@@ -1,8 +1,13 @@
 #!/usr/bin/env python
 """bench.py -- GCN10 Curve Number hot path on B200: CN Gpixel/s (9 LUT variants).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes, after the K timed kernel-resident steps, what the last of them computed: the nine
+drained Curve Number planes of rank 0, as float32 DIR/cn_drained.npy [9, n] at n seeded pixel positions
+(DIR/cn_drained_index.npy, float64 flat indices y * W + x; every pixel when the tile has at most 2**20).  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 
 One "step" = one pass of the hot path over one synthetic 3x3 degree block: a 36000 x 36000 uint8
 WorldCover-like tile plus its 1440 x 1440 HSG window, all nine lookup variants (p/f/g x ARC
@@ -54,7 +59,7 @@ LON0, LAT0 = -114.0, 42.0
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the kernel-resident leg (the headline value)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--profile", default="worldcover", choices=["worldcover", "random", "coastal"])
@@ -66,7 +71,33 @@ def parse_args():
     ap.add_argument("--ship", type=int, default=None, choices=[0, 1], help="override the library's strip hand-over path")
     ap.add_argument("--queue-blocks", type=int, default=64, help="blocks of the e2e.queue64 leg (0 = skip)")
     ap.add_argument("--program-blocks", type=int, default=4, help="blocks of the e2e.program leg per GPU (0 = skip)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a seeded sample of the last timed step's output planes to DIR (see the module docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm keeps no outputs)")
+    return args
+
+
+DUMP_SAMPLE = 1 << 20           # pixels per plane in --dump-outputs: 9 x 4 MB of float32 + 8 MB of indices
+DUMP_SEED = 20240601
+
+
+def dump_outputs(directory, d_out, w, h):
+    """The drained planes of the last timed step at DUMP_SAMPLE seeded pixel positions (all pixels of a small tile)."""
+    import numpy as np
+    import torch
+    n = w * h
+    if n <= DUMP_SAMPLE:
+        idx = np.arange(n, dtype=np.int64)
+    else:
+        idx = np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, DUMP_SAMPLE, dtype=np.int64))
+    vals = d_out.view(NVAR, n)[:, torch.from_numpy(idx).to(d_out.device)]
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "cn_drained.npy"), vals.to(torch.float32).cpu().numpy())
+    np.save(os.path.join(directory, "cn_drained_index.npy"), idx.astype(np.float64))
 
 
 def workload_config(args, extra=None):
@@ -336,6 +367,9 @@ def run_ours(args):
     mean_step_ms = sum(step_ms) / len(step_ms)
     px = float(w) * h
     value = world * px * args.steps / (total_ms * 1e-3) / 1e9
+    # before the legs below write into d_out
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out, w, h)
 
     # ---- the drop-in pass: both drainage conditions, all 18 rasters of a block in one launch (19 B/px)
     all18 = None
@@ -934,6 +968,7 @@ print_json = None
 
 
 def main():
+    sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
     args = parse_args()
     # stdout must carry exactly one JSON line: libraries (NCCL prints its version banner to stdout on the
     # first collective) are diverted to stderr for the whole run and the line is written to the real stdout

@@ -134,6 +134,23 @@ class Port:
             raise MemoryError("cn_oracle_block_rows")
         return out
 
+    def run_block(self, esa_raster, esa_t, hsg_raster, hsg_t, bbox, lookup_dir, *, block_id=1):
+        """What ``Ref.run_block`` returns for the rasters process_block() saves (nplanes, w, h, gt, paths,
+        planes), restated: both windows cut from ``bbox``, a block whose window is invalid in either raster is
+        skipped (nplanes == 0, cn.c:188-192), else the 18 planes in the save order (cn.c:236,258-259,308)."""
+        esa_raster = np.ascontiguousarray(esa_raster, dtype=np.uint8)
+        hsg_raster = np.ascontiguousarray(hsg_raster, dtype=np.uint8)
+        we = self.window(esa_raster.shape[1], esa_raster.shape[0], esa_t, bbox)
+        wh = self.window(hsg_raster.shape[1], hsg_raster.shape[0], hsg_t, bbox)
+        if we is None or wh is None:
+            return dict(nplanes=0, w=0, h=0, gt=(0.0,) * 6, paths=[], planes=None)
+        xo, yo, xc, yc, gt = we
+        hxo, hyo, hxc, hyc, sgt = wh
+        planes = self.block_rows(esa_raster[yo:yo + yc, xo:xo + xc], gt, hsg_raster[hyo:hyo + hyc, hxo:hxo + hxc], sgt,
+                                 self.load_tables(lookup_dir))
+        paths = [f"cn_rasters_{c}/cn_{h}_{a}_{block_id}.tif" for c in CONDS for h in HCS for a in ARCS]
+        return dict(nplanes=NPLANES, w=xc, h=yc, gt=gt, paths=paths, planes=planes)
+
 
 class Ref:
     """The reference's own object code (oracle/_ref/libgcn10_ref.so)."""

@@ -1,5 +1,6 @@
 import os
 import sys
+import warnings
 
 import pytest
 
@@ -33,6 +34,19 @@ def ref():
     if not O.Ref.available():
         pytest.skip("oracle/_ref/libgcn10_ref.so not present")
     return O.Ref()
+
+
+@pytest.fixture(scope="session")
+def reference(port):
+    """What process_block() saves (``run_block``) and its window arithmetic (``window``): the reference's own object
+    code where oracle/_ref is built, else the plain-C restatement, which the golden fixtures in tests/golden/ (outputs
+    of that object code) pin to it.  The substitution is reported as a warning in the test summary."""
+    from oracle import oracle as O
+    if O.Ref.available():
+        return O.Ref()
+    warnings.warn("oracle/_ref/libgcn10_ref.so not present: expected rasters and windows come from the plain-C "
+                  "restatement (oracle/cn_oracle.c), pinned to the reference by tests/golden/")
+    return port
 
 
 @pytest.fixture(scope="session")

@@ -59,3 +59,25 @@ def test_program_leg_always_reaches_both_barriers(monkeypatch):
     if os.path.exists(hostlib.EXE_PATH):
         assert "skipped" in res
     assert len(calls) == 2
+
+
+def test_dump_outputs_is_a_fixed_sample_of_the_planes(tmp_path):
+    """--dump-outputs: float32 values at float64 flat indices, the same positions on every run, under 64 MB in all;
+    every pixel of a tile small enough."""
+    import torch
+    small = torch.from_numpy(np.stack([synth.esa_tile(40, 30, k) for k in range(bench.NVAR)]))
+    bench.dump_outputs(str(tmp_path / "small"), small, 40, 30)
+    vals = np.load(tmp_path / "small" / "cn_drained.npy")
+    idx = np.load(tmp_path / "small" / "cn_drained_index.npy")
+    assert vals.dtype == np.float32 and idx.dtype == np.float64
+    assert np.array_equal(idx, np.arange(40 * 30)) and np.array_equal(vals, small.reshape(bench.NVAR, -1).numpy())
+    w = h = 1500
+    big = torch.from_numpy(np.stack([synth.esa_tile(w, h, k, "random") for k in range(bench.NVAR)]))
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), big, w, h)
+    idx = np.load(tmp_path / "a" / "cn_drained_index.npy")
+    vals = np.load(tmp_path / "a" / "cn_drained.npy")
+    assert np.array_equal(idx, np.load(tmp_path / "b" / "cn_drained_index.npy"))
+    assert idx.size <= bench.DUMP_SAMPLE and (np.diff(idx) > 0).all() and vals.shape == (bench.NVAR, idx.size)
+    assert np.array_equal(vals, big.reshape(bench.NVAR, -1).numpy()[:, idx.astype(np.int64)])
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 << 20

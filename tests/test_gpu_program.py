@@ -1,6 +1,7 @@
 """End to end on a GPU: the gcn10 executable (C host program + libgcn10cuda) against the reference's
 own process_block() on the same rasters -- decoded planes must be identical, file names, log lines
-and the no-overwrite underscore rule must match the reference's observable behaviour."""
+and the no-overwrite underscore rule must match the reference's observable behaviour.  Where the reference's object
+code (oracle/_ref) is not built, the expected rasters come from the plain-C restatement the golden fixtures pin to it."""
 import os
 import re
 import subprocess
@@ -56,7 +57,7 @@ def _run(world, *extra, host_deflate=False, host_inflate=False):
 
 @pytest.mark.parametrize("host_deflate,host_inflate", [(False, False), (False, True), (True, True)],
                          ids=["gpu_inflate_gpu_deflate", "host_inflate_gpu_deflate", "host_inflate_host_deflate"])
-def test_program_matches_reference_process_block(world, ref, host_deflate, host_inflate):
+def test_program_matches_reference_process_block(world, reference, host_deflate, host_inflate):
     from PIL import Image
     import shutil
     shutil.rmtree(world["root"] / "logs", ignore_errors=True)      # log files are opened for append (log.c:79)
@@ -66,7 +67,7 @@ def test_program_matches_reference_process_block(world, ref, host_deflate, host_
     assert ("land cover inflated on the gpu" in log_all) == (not host_deflate and not host_inflate)
     root = world["root"]
     for bid, x0, y0, x1, y1 in world["blocks"][:2]:
-        want = ref.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
+        want = reference.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
                              str(root / "lookups"), block_id=bid)
         assert want["nplanes"] == 18
         for k, rel in enumerate(want["paths"]):                 # the reference's own file names, save order
@@ -140,7 +141,7 @@ def test_block_rows_bands_equal_whole_block(gpu_ctx, port, tables):
         assert np.array_equal(got, want[:, y0:y0 + n]), (y0, n)
 
 
-def test_program_reads_a_vrt_mosaic(world, ref, tmp_path):
+def test_program_reads_a_vrt_mosaic(world, reference, tmp_path):
     """esa_data_path = *.vrt, as in the reference's shipped config (landcover/esa_worldcover_2021.vrt, opened at
     raster.c:119): the land cover is a 2 x 2 mosaic of GeoTIFFs whose borders (x = 1290, y = 1210) cross both block
     windows, so every block is assembled from four sources -- on the GPU from their compressed tiles, and on the
@@ -174,7 +175,7 @@ def test_program_reads_a_vrt_mosaic(world, ref, tmp_path):
         log = (vroot / "logs" / "rank_0.log").read_text()
         assert ("mosaic parts inflated on the gpu" in log) == (host_inflate == "0")
         for bid, x0, y0, x1, y1 in world["blocks"][:2]:
-            want = ref.run_block(esa, esa_t, world["hsg"], world["hsg_t"], (x0, y0, x1, y1), str(root / "lookups"),
+            want = reference.run_block(esa, esa_t, world["hsg"], world["hsg_t"], (x0, y0, x1, y1), str(root / "lookups"),
                                  block_id=bid)
             for k, rel in enumerate(want["paths"]):
                 t = hostlib.Tiff(str(out / rel))
@@ -191,7 +192,7 @@ def test_program_reads_a_vrt_mosaic(world, ref, tmp_path):
     assert not list(out.glob("cn_rasters_*/cn_*_12*"))
 
 
-def test_program_with_the_gdal_backend(world, ref, tmp_path):
+def test_program_with_the_gdal_backend(world, reference, tmp_path):
     """The optional GDAL input backend (host_raster_gdal.c, make GDAL=1) inside the whole program: gcn10 is rebuilt
     here with -DGCN10_WITH_GDAL against the oracle's RAM stand-in for GDAL, the land cover is served by that GDAL under
     a /vsicurl/ name no file has (the soil raster stays a GeoTIFF on disk, read by the built-in reader), and the 18
@@ -243,7 +244,7 @@ def test_program_with_the_gdal_backend(world, ref, tmp_path):
     assert f"{name} opened with gdal" in log and "hsg.tif opened with gdal" not in log
     assert "inflated on the gpu" not in log
     for bid, x0, y0, x1, y1 in world["blocks"][:2]:
-        want = ref.run_block(esa, esa_t, world["hsg"], world["hsg_t"], (x0, y0, x1, y1), str(root / "lookups"),
+        want = reference.run_block(esa, esa_t, world["hsg"], world["hsg_t"], (x0, y0, x1, y1), str(root / "lookups"),
                              block_id=bid)
         for k, rel in enumerate(want["paths"]):
             t = hostlib.Tiff(str(out / rel))

@@ -47,7 +47,7 @@ def test_window_arithmetic_matches_golden():
             assert got == (e["xoff"], e["yoff"], e["xsize"], e["ysize"], tuple(e["gt"])), c
 
 
-def test_window_matches_reference_live(ref):
+def test_window_matches_reference_live(reference):
     rng = np.random.default_rng(7)
     for _ in range(300):
         rw, rh = int(rng.integers(1, 5000)), int(rng.integers(1, 5000))
@@ -56,7 +56,7 @@ def test_window_matches_reference_live(ref):
         x0, x1 = sorted(rng.uniform(-0.2 * rw, 1.2 * rw, 2))
         y0, y1 = sorted(rng.uniform(-0.2 * rh, 1.2 * rh, 2))
         bbox = (t[0] + x0 * px, t[3] - y1 * px, t[0] + x1 * px, t[3] - y0 * px)
-        assert hostlib.raster_window(rw, rh, t, bbox) == ref.window(rw, rh, t, bbox)
+        assert hostlib.raster_window(rw, rh, t, bbox) == reference.window(rw, rh, t, bbox)
 
 
 def test_config_parser(tmp_path):

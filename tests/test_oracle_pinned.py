@@ -34,13 +34,19 @@ def _window_inputs(port, c):
 
 
 @pytest.mark.parametrize("name", sorted(BLOCKS))
-def test_restatement_matches_golden_blocks(name, port, tables):
+def test_restatement_matches_golden_blocks(name, port, tables, lookup_dir):
     c = BLOCKS[name]
     esa, gt, hsg, sgt = _window_inputs(port, c)
     assert np.array_equal(np.array(gt), c["gt"]), "clipped geotransform differs from the reference's"
     got = port.block_rows(esa, gt, hsg, sgt, tables)
     assert got.shape == c["planes"].shape
     assert np.array_equal(got, c["planes"])
+    # Port.run_block, the stand-in for process_block() where oracle/_ref is not built: the same block from the whole
+    # rasters, and a bbox west of the land cover skipped
+    r = port.run_block(c["esa"], c["esa_t"], c["hsg"], c["hsg_t"], c["bbox"], lookup_dir)
+    assert (r["nplanes"], r["gt"]) == (18, gt) and np.array_equal(r["planes"], c["planes"])
+    t0, t3 = float(c["esa_t"][0]), float(c["esa_t"][3])
+    assert port.run_block(c["esa"], c["esa_t"], c["hsg"], c["hsg_t"], (t0 - 2, t3 - 1, t0 - 1, t3), lookup_dir)["nplanes"] == 0
 
 
 @pytest.mark.parametrize("name", sorted(BLOCKS))
