@@ -41,7 +41,30 @@ class TileStrip(C.Structure):
     """gcn10_tile_strip of include/gcn10_cuda.h."""
     _fields_ = [("tile_row0", C.c_int), ("n_tile_rows", C.c_int), ("tiles_x", C.c_int), ("n_planes", C.c_int),
                 ("plane_ids", C.POINTER(C.c_int)), ("offsets", C.POINTER(C.c_uint64)),
-                ("sizes", C.POINTER(C.c_uint32)), ("blob", C.POINTER(C.c_uint8)), ("blob_bytes", C.c_size_t)]
+                ("sizes", C.POINTER(C.c_uint32)), ("blob", C.POINTER(C.c_uint8)), ("blob_bytes", C.c_size_t),
+                ("level", C.c_int), ("level_w", C.c_int), ("level_h", C.c_int)]
+
+
+def _tile_collector(tiles, overviews, total, on_strip=None):
+    """A sink that files every tile of a strip: level 0 into tiles = {plane: {(tile_row, tile_x): bytes}}, overview
+    level k into overviews = {k: {plane: {...}}}; with ``on_strip(strip_struct)`` the tiles are not copied."""
+
+    def _sink(_user, sp):
+        st = sp.contents
+        total[0] += st.blob_bytes
+        if on_strip is not None:
+            return int(on_strip(st) or 0)
+        blob = C.string_at(st.blob, st.blob_bytes)
+        dest = tiles if st.level == 0 else overviews.setdefault(st.level, {})
+        for k in range(st.n_planes):
+            d = dest.setdefault(st.plane_ids[k], {})
+            for tr in range(st.n_tile_rows):
+                for tx in range(st.tiles_x):
+                    i = (k * st.n_tile_rows + tr) * st.tiles_x + tx
+                    d[(st.tile_row0 + tr, tx)] = blob[st.offsets[i]: st.offsets[i] + st.sizes[i]]
+        return 0
+
+    return _sink
 
 
 TILE_SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(TileStrip))
@@ -315,34 +338,33 @@ class Context:
         return out
 
     def block_deflate(self, esa, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
-        """Compressed-tile call.  Returns dict(tiles={plane: {(tile_row, tile_x): bytes}}, bytes=total)
-        unless ``on_strip(strip_struct)`` is given, in which case tiles are not copied."""
+        """Compressed-tile call.  Returns dict(tiles={plane: {(tile_row, tile_x): bytes}},
+        overviews={level: {plane: {(tile_row, tile_x): bytes}}} (option "overviews"), bytes=total); with
+        ``on_strip(strip_struct)`` the tiles are not copied."""
         esa, esa_pitch = _rows(esa)
         hsg, hsg_pitch = _rows(hsg)
         h, w = esa.shape
         hsy, hsx = hsg.shape
-        tiles = {}
-        total = [0]
-
-        def _sink(_user, sp):
-            st = sp.contents
-            total[0] += st.blob_bytes
-            if on_strip is not None:
-                return int(on_strip(st) or 0)
-            blob = C.string_at(st.blob, st.blob_bytes)
-            for k in range(st.n_planes):
-                d = tiles.setdefault(st.plane_ids[k], {})
-                for tr in range(st.n_tile_rows):
-                    for tx in range(st.tiles_x):
-                        i = (k * st.n_tile_rows + tr) * st.tiles_x + tx
-                        d[(st.tile_row0 + tr, tx)] = blob[st.offsets[i]: st.offsets[i] + st.sizes[i]]
-            return 0
-
-        cb = TILE_SINK(_sink)
+        tiles, overviews, total = {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
         self._check(self.lib.gcn10_cuda_block_deflate(
             self.h, esa.ctypes.data, w, h, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
             _d6(soil_gt), plane_mask, cb, None))
-        return dict(tiles=tiles, bytes=total[0])
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
+
+    def block_deflate_rows(self, esa_rows, h, row0, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
+        """Band form of block_deflate: esa_rows holds rows [row0, row0+len) of a block that is h rows tall; the
+        result holds this band's tiles (and, for the band that ends the block, its overview levels)."""
+        esa_rows, esa_pitch = _rows(esa_rows)
+        hsg, hsg_pitch = _rows(hsg)
+        nrows, w = esa_rows.shape
+        hsy, hsx = hsg.shape
+        tiles, overviews, total = {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
+        self._check(self.lib.gcn10_cuda_block_deflate_rows(
+            self.h, esa_rows.ctypes.data, w, h, row0, nrows, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
+            _d6(soil_gt), plane_mask, cb, None))
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
 
     def inflate_tiles(self, src: "TileSource", w, h, out=None, want_status=False):
         """GPU inflate of a tile source into a host raster uint8 [h, w]."""
@@ -362,29 +384,13 @@ class Context:
         block_deflate)."""
         hsg, hsg_pitch = _rows(hsg)
         hsy, hsx = hsg.shape
-        tiles = {}
-        total = [0]
-
-        def _sink(_user, sp):
-            st = sp.contents
-            total[0] += st.blob_bytes
-            if on_strip is not None:
-                return int(on_strip(st) or 0)
-            blob = C.string_at(st.blob, st.blob_bytes)
-            for k in range(st.n_planes):
-                d = tiles.setdefault(st.plane_ids[k], {})
-                for tr in range(st.n_tile_rows):
-                    for tx in range(st.tiles_x):
-                        i = (k * st.n_tile_rows + tr) * st.tiles_x + tx
-                        d[(st.tile_row0 + tr, tx)] = blob[st.offsets[i]: st.offsets[i] + st.sizes[i]]
-            return 0
-
-        cb = TILE_SINK(_sink)
+        tiles, overviews, total = {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
         st = src.struct()
         self._check(self.lib.gcn10_cuda_block_tiles_deflate(
             self.h, C.byref(st), w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
             cb, None))
-        return dict(tiles=tiles, bytes=total[0])
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
 
     def inflate_parts(self, parts, fill, w, h, want_status=False):
         """GPU inflate of a mosaic ([(TileSource, dst_x, dst_y, w, h), ...]) into a host raster uint8 [h, w]."""
@@ -399,31 +405,17 @@ class Context:
         self._check(rc)
         return out
 
-    def block_parts_deflate(self, parts, fill, w, h, gt, hsg, soil_gt, plane_mask=MASK_ALL):
+    def block_parts_deflate(self, parts, fill, w, h, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
         """Mosaic form of block_tiles_deflate; same result layout."""
         hsg, hsg_pitch = _rows(hsg)
         hsy, hsx = hsg.shape
-        tiles = {}
-        total = [0]
-
-        def _sink(_user, sp):
-            st = sp.contents
-            total[0] += st.blob_bytes
-            blob = C.string_at(st.blob, st.blob_bytes)
-            for k in range(st.n_planes):
-                d = tiles.setdefault(st.plane_ids[k], {})
-                for tr in range(st.n_tile_rows):
-                    for tx in range(st.tiles_x):
-                        i = (k * st.n_tile_rows + tr) * st.tiles_x + tx
-                        d[(st.tile_row0 + tr, tx)] = blob[st.offsets[i]: st.offsets[i] + st.sizes[i]]
-            return 0
-
-        cb = TILE_SINK(_sink)
+        tiles, overviews, total = {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
         arr = parts_array(parts)
         self._check(self.lib.gcn10_cuda_block_parts_deflate(
             self.h, arr, len(parts), fill, w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
             cb, None))
-        return dict(tiles=tiles, bytes=total[0])
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
 
     def tiles_prefetch(self, src: "TileSource", w, h):
         """Start upload + GPU inflate of a block's tiles; the next block_tiles_deflate / inflate_tiles call with the

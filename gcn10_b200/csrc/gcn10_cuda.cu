@@ -11,6 +11,7 @@
 #include "deflate_tiles.cuh"
 #include "inflate_tiles.cuh"
 #include "cn_deflate_fused.cuh"
+#include "overviews.cuh"
 #include "tile_code.h"
 
 #include <algorithm>
@@ -70,7 +71,9 @@ struct StripSlot {
     DevBuf blob2, order;        // option "ordered": the strip re-laid in table order, and the scan's offsets
     HostBuf h_blob, h_table;    // page-locked mirrors
     cudaEvent_t enc_done = nullptr;
+    cudaEvent_t ov = nullptr;   // option "overviews": behind the strip's overview_decimate_kernel
     int y0 = 0, rows = 0;
+    int level = 0, y_base = 0, tiles_x = 0, level_w = 0, level_h = 0;     // what the strip reports to the sink
     bool busy = false;
 };
 
@@ -134,6 +137,13 @@ struct gcn10_ctx {
     float last_inflate_ms = 0.f;
     float last_kernel_ms = 0.f;
     uint64_t launches = 0;
+    // option "overviews": the land cover and index maps of every overview level of the block in hand, filled strip by
+    // strip (and band by band: ov_next is the block row the next band must start at, -1 = no block open)
+    int overviews = 0;
+    DevBuf ov_buf;
+    OverviewLevel ov_lv[GCN10_MAX_OVERVIEWS] = {};
+    int ov_h[GCN10_MAX_OVERVIEWS] = {};
+    int ov_w = 0, ov_hb = 0, ov_next = -1;
     // asynchronous raw-plane blocks (gcn10_cuda_block_async): frame guard, per-stream end-of-block marks, timer events
     cudaEvent_t frame_ready = nullptr;
     cudaEvent_t tail[kMaxStreams] = {};
@@ -484,7 +494,7 @@ int launch_index_maps(gcn10_ctx *c, int w, int h, const double gt[6], int hsx, i
 int launch_rows(gcn10_ctx *c, const LaunchPlan &lp, int lut_slot, const uint8_t *d_esa, size_t esa_pitch, int w,
                 int rows, int y_base, const uint8_t *d_hsg, size_t hsg_pitch, int hsx, int hsy,
                 const CUtensorMap &map, int tma_ok, uint8_t *const d_out[GCN10_NPLANES], size_t out_pitch,
-                cudaStream_t st)
+                cudaStream_t st, const int32_t *col_idx = nullptr, const int32_t *row_idx = nullptr)
 {
     BlockParams p;
     memset(&p, 0, sizeof(p));
@@ -493,8 +503,8 @@ int launch_rows(gcn10_ctx *c, const LaunchPlan &lp, int lut_slot, const uint8_t 
     p.w = w;
     p.h = rows;
     p.y_base = y_base;
-    p.col_idx = (const int32_t *)c->col_idx.p;
-    p.row_idx = (const int32_t *)c->row_idx.p;
+    p.col_idx = col_idx ? col_idx : (const int32_t *)c->col_idx.p;      // (an overview level's maps, or the block's)
+    p.row_idx = row_idx ? row_idx : (const int32_t *)c->row_idx.p;
     p.hsg = d_hsg;
     p.hsg_pitch = hsg_pitch;
     p.hsx = hsx;
@@ -726,6 +736,7 @@ int gcn10_cuda_create(int device, gcn10_ctx **out)
         CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].k2, cudaEventDisableTiming));
         CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].done, cudaEventDisableTiming));
         CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].enc_done, cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].ov, cudaEventDisableTiming));
     }
     CUDA_TRY(cudaFuncSetAttribute((const void *)deflate_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   kEncSmem));
@@ -775,6 +786,7 @@ void gcn10_cuda_destroy(gcn10_ctx *c)
     release(c->row_idx);
     release(c->hsg);
     release(c->fused_tab);
+    release(c->ov_buf);
     for (int i = 0; i < 2; i++) {
         release(c->tslot[i].in_blob);
         release(c->tslot[i].in_table);
@@ -801,6 +813,7 @@ void gcn10_cuda_destroy(gcn10_ctx *c)
         release_host(c->slots[i].h_blob);
         release_host(c->slots[i].h_table);
         if (c->slots[i].enc_done) cudaEventDestroy(c->slots[i].enc_done);
+        if (c->slots[i].ov) cudaEventDestroy(c->slots[i].ov);
         if (c->slots[i].k0) cudaEventDestroy(c->slots[i].k0);
         if (c->slots[i].k1) cudaEventDestroy(c->slots[i].k1);
         if (c->slots[i].k2) cudaEventDestroy(c->slots[i].k2);
@@ -838,6 +851,10 @@ int gcn10_cuda_set_option(gcn10_ctx *c, const char *key, long value)
     else if (!strcmp(key, "fused") && (value == 0 || value == 1)) c->fused = (int)value;
     else if (!strcmp(key, "ship") && (value == 0 || value == 1)) c->ship = (int)value;
     else if (!strcmp(key, "ordered") && (value == 0 || value == 1)) c->ordered = (int)value;
+    else if (!strcmp(key, "overviews") && value >= 0 && value <= GCN10_MAX_OVERVIEWS) {
+        c->overviews = (int)value;
+        c->ov_next = -1;
+    }
     else if (!strcmp(key, "inflate_probe") && value >= 0 && value <= 2) c->inflate_probe = (int)value;
     else if (!strcmp(key, "tuned_code") && (value == 0 || value == 1)) {
         c->tuned_code = (int)value;
@@ -1193,7 +1210,43 @@ static int deflate_rows_impl(gcn10_ctx *c,
         return fail(GCN10_ENOLUT, "gcn10_cuda_set_luts() has not been called");
     if (c->pending_events)
         return fail(GCN10_EINVAL, "asynchronous blocks are pending on this context: gcn10_cuda_wait() for them first");
+    // option "overviews": every band feeds the block's levels, so the bands of a block must come in order and without
+    // gaps; the band that ends the block emits the levels
+    const int nlev = c->overviews ? gcn10_overview_levels(w, h, c->overviews) : 0;
+    if (nlev && row0 != 0 && (row0 != c->ov_next || w != c->ov_w || h != c->ov_hb)) {
+        rc = fail(GCN10_EINVAL, "overviews: band [%d, +%d) of a %d x %d block does not continue the block's previous band "
+                                "(next row %d); a block starts with row 0", row0, nrows, w, h, c->ov_next);
+        c->ov_next = -1;
+        return rc;
+    }
+    c->ov_next = -1;            // (until this call has succeeded)
+    const bool emit_levels = nlev && row0 + nrows == h;
     CUDA_TRY(cudaSetDevice(c->device));
+    if (nlev && row0 == 0) {
+        size_t off[GCN10_MAX_OVERVIEWS][3], total = 0;
+        for (int k = 1; k <= nlev; k++) {
+            OverviewLevel &L = c->ov_lv[k - 1];
+            L.k = k;
+            L.w = gcn10_overview_dim(w, k);
+            c->ov_h[k - 1] = gcn10_overview_dim(h, k);
+            L.pitch = round_up((size_t)L.w, 256);
+            off[k - 1][0] = total;
+            total += L.pitch * (size_t)c->ov_h[k - 1];
+            off[k - 1][1] = total;
+            total += round_up(sizeof(int32_t) * round_up((size_t)L.w, kVecPx), 256);
+            off[k - 1][2] = total;
+            total += round_up(sizeof(int32_t) * (size_t)c->ov_h[k - 1], 256);
+        }
+        if ((rc = ensure(c->ov_buf, total)))
+            return rc;
+        for (int k = 0; k < nlev; k++) {
+            c->ov_lv[k].esa = (uint8_t *)c->ov_buf.p + off[k][0];
+            c->ov_lv[k].col_idx = (int32_t *)((uint8_t *)c->ov_buf.p + off[k][1]);
+            c->ov_lv[k].row_idx = (int32_t *)((uint8_t *)c->ov_buf.p + off[k][2]);
+        }
+        c->ov_w = w;
+        c->ov_hb = h;
+    }
 
     LaunchPlan plans[2];
     const int nplans = plan_launches(plane_mask, plans);
@@ -1225,7 +1278,28 @@ static int deflate_rows_impl(gcn10_ctx *c,
     const int ns = c->nstreams;
     const int strip = std::max(kTile, std::min(c->strip_rows, (int)round_up((size_t)nrows, kTile)) / kTile * kTile);
     const int tiles_x = (w + kTile - 1) / kTile;
-    const int strip_tile_rows = strip / kTile;
+    // the strips of this call: the band's full-resolution rows; then, when the band ends the block, every overview
+    // level, level 1 first, in strips of at most `lstrip` level rows (they use the same slots, at most tiles_x wide)
+    struct StripJob {
+        int level, y0, rows, w, h, y_base;      // y0: row in the caller's band (level 0) or in the level
+        const uint8_t *d_esa;                   // nullptr: staged from the caller's host raster
+        size_t pitch;
+        const int32_t *col_idx, *row_idx;       // nullptr: the block's
+    };
+    std::vector<StripJob> jobs;
+    for (int y0 = 0; y0 < nrows; y0 += strip)
+        jobs.push_back({ 0, y0, std::min(strip, nrows - y0), w, h, row0 + y0,
+                         d_esa ? d_esa + (size_t)y0 * d_esa_pitch : nullptr, d_esa_pitch, nullptr, nullptr });
+    const int lstrip = emit_levels ? std::max(kTile, std::min(c->strip_rows, (int)round_up((size_t)c->ov_h[0], kTile)) / kTile * kTile)
+                                   : 0;
+    for (int k = 0; k < (emit_levels ? nlev : 0); k++) {
+        const OverviewLevel &L = c->ov_lv[k];
+        for (int y0 = 0; y0 < c->ov_h[k]; y0 += lstrip)
+            jobs.push_back({ k + 1, y0, std::min(lstrip, c->ov_h[k] - y0), L.w, c->ov_h[k], y0,
+                             L.esa + (size_t)y0 * L.pitch, L.pitch, L.col_idx, L.row_idx });
+    }
+    const int strip_cap = std::max(strip, lstrip);
+    const int strip_tile_rows = strip_cap / kTile;
     const size_t ntile_slot = (size_t)nplanes * strip_tile_rows * tiles_x;
     const size_t blob_cap = ntile_slot * (size_t)round_up(kStoredBytes, 16);
     const size_t table_bytes = 16 + ntile_slot * (sizeof(unsigned long long) + sizeof(uint32_t));
@@ -1235,7 +1309,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
     for (int i = 0; i < ns; i++) {
         StripSlot &sl = c->slots[i];
         if ((esa && (rc = ensure(sl.esa, dpitch * (size_t)strip))) ||
-            (!fused && (rc = ensure(sl.out, dpitch * (size_t)strip * nplanes))) ||
+            (!fused && (rc = ensure(sl.out, dpitch * (size_t)strip_cap * nplanes))) ||
             (rc = ensure(sl.blob, blob_cap)) || (rc = ensure(sl.table, table_bytes)) ||
             (c->ordered && ((rc = ensure(sl.blob2, blob2_cap)) || (rc = ensure(sl.order, ntile_slot * sizeof(unsigned long long))))) ||
             (rc = ensure_host(sl.h_table, table_bytes)))
@@ -1250,7 +1324,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
             CUDA_TRY(cudaStreamWaitEvent(c->streams[i], esa_ready, 0));
     }
 
-    const int nstrips = (nrows + strip - 1) / strip;
+    const int nstrips = (int)jobs.size();
     float kernel_ms = 0.f;
 
     // behind the encoder on the strip's stream: either the ship kernel (exact bytes + tables straight into the
@@ -1258,7 +1332,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
     auto hand_over = [&](StripSlot &sl, cudaStream_t st) -> int {
         CUDA_TRY(cudaEventRecord(sl.k1, st));
         if (c->ordered) {
-            const int n = nplanes * ((sl.rows + kTile - 1) / kTile) * tiles_x;
+            const int n = nplanes * ((sl.rows + kTile - 1) / kTile) * sl.tiles_x;
             unsigned long long *d_offsets = (unsigned long long *)((uint8_t *)sl.table.p + 16);
             const uint32_t *d_sizes = (const uint32_t *)((uint8_t *)sl.table.p + 16 + ntile_slot * sizeof(unsigned long long));
             order_scan_kernel<<<1, 1024, 0, st>>>(d_sizes, n, (unsigned long long *)sl.order.p,
@@ -1294,19 +1368,69 @@ static int deflate_rows_impl(gcn10_ctx *c,
     auto issue = [&](int s) -> int {
         StripSlot &sl = c->slots[s % ns];
         cudaStream_t st = c->streams[s % ns];
-        const int y0 = s * strip, rows = std::min(strip, nrows - y0);      // y0 counts rows of the caller's band
+        const StripJob &jb = jobs[s];
+        const int y0 = jb.y0, rows = jb.rows;
         const int tile_rows = (rows + kTile - 1) / kTile;
+        const int sw = jb.w, stx = (jb.w + kTile - 1) / kTile;
         sl.y0 = y0;
         sl.rows = rows;
-        const uint8_t *strip_esa = d_esa ? d_esa + (size_t)y0 * d_esa_pitch : (const uint8_t *)sl.esa.p;
-        const size_t strip_esa_pitch = d_esa ? d_esa_pitch : dpitch;
-        if (!d_esa)
+        sl.level = jb.level;
+        sl.y_base = jb.y_base;
+        sl.tiles_x = stx;
+        sl.level_w = jb.w;
+        sl.level_h = jb.h;
+        const uint8_t *strip_esa = jb.d_esa ? jb.d_esa : (const uint8_t *)sl.esa.p;
+        const size_t strip_esa_pitch = jb.d_esa ? jb.pitch : dpitch;
+        if (!jb.d_esa)
             CUDA_TRY(cudaMemcpy2DAsync(sl.esa.p, dpitch, esa + (size_t)y0 * esa_pitch, esa_pitch, (size_t)w, (size_t)rows,
                                        cudaMemcpyHostToDevice, st));
+        if (nlev && jb.level == 0) {
+            // the overview levels' share of this strip, while its land cover is on the device
+            OverviewParams op;
+            memset(&op, 0, sizeof(op));
+            op.src = strip_esa;
+            op.src_pitch = strip_esa_pitch;
+            op.src_y0 = jb.y_base;
+            op.w = w;
+            op.h = h;
+            op.col_idx = (const int32_t *)c->col_idx.p;
+            op.row_idx = (const int32_t *)c->row_idx.p;
+            op.with_cols = jb.y_base == 0;
+            op.nlev = nlev;
+            // level row i samples block row R(i), which is non-decreasing in i: the first level row at or below block row y
+            auto first_row = [&](int y, int k) -> int {
+                const int hk = c->ov_h[k - 1];
+                if (y >= h)
+                    return hk;
+                const long long f = 1LL << k, a = (long long)y - f / 2;
+                return a <= 0 ? 0 : (int)std::min<long long>(hk, (a + f - 1) / f);
+            };
+            long long most = 0;
+            for (int k = 1; k <= nlev; k++) {
+                op.lv[k - 1] = c->ov_lv[k - 1];
+                op.lv[k - 1].i_lo = first_row(jb.y_base, k);
+                op.lv[k - 1].i_hi = first_row(jb.y_base + rows, k);
+                most = std::max(most, (long long)(op.lv[k - 1].i_hi - op.lv[k - 1].i_lo) * ((op.lv[k - 1].w + 3) / 4));
+            }
+            most = std::max<long long>(most, op.with_cols ? round_up((size_t)op.lv[0].w, kVecPx) : 1);
+            const int blocks = (int)std::max<long long>(1, std::min<long long>((most + 255) / 256, (long long)c->sm_count * 8));
+            overview_decimate_kernel<<<dim3(blocks, nlev), 256, 0, st>>>(op);
+            c->launches++;
+            CUDA_TRY(cudaGetLastError());
+            CUDA_TRY(cudaEventRecord(sl.ov, st));
+        }
+        else if (jb.level) {
+            // the level's land cover is complete once every full-resolution strip of the block has been sampled: the
+            // last decimation on each stream (earlier bands finished theirs before their call returned)
+            for (int i = 0; i < ns; i++)
+                CUDA_TRY(cudaStreamWaitEvent(st, c->slots[i].ov, 0));
+        }
         // The encoder kernels run in strip order, at most two at a time (the second fills the first one's last wave):
         // launched side by side on all streams they would all finish together, and the copy of strip 0 -- the head of
         // the chain of copies that ends the block -- would wait for the others.
-        if (s >= 2)
+        // Overview strips are not chained: their grids are small (level k has 1/4^k of the tiles), one alone leaves
+        // most SMs idle, and they end the block, so no later copy waits on them.
+        if (s >= 2 && jb.level == 0)
             CUDA_TRY(cudaStreamWaitEvent(st, c->slots[(s - 2) % ns].k1, 0));
         CUDA_TRY(cudaEventRecord(sl.k0, st));
         if (fused) {
@@ -1314,11 +1438,11 @@ static int deflate_rows_impl(gcn10_ctx *c,
             memset(&fp, 0, sizeof(fp));
             fp.esa = strip_esa;
             fp.esa_pitch = strip_esa_pitch;
-            fp.w = w;
+            fp.w = sw;
             fp.rows = rows;
-            fp.y_base = row0 + y0;
-            fp.col_idx = (const int32_t *)c->col_idx.p;
-            fp.row_idx = (const int32_t *)c->row_idx.p;
+            fp.y_base = jb.y_base;
+            fp.col_idx = jb.col_idx ? jb.col_idx : (const int32_t *)c->col_idx.p;
+            fp.row_idx = jb.row_idx ? jb.row_idx : (const int32_t *)c->row_idx.p;
             fp.hsg = (const uint8_t *)c->hsg.p;
             fp.hsg_pitch = hsg_dpitch;
             fp.idmap = (const uint8_t *)c->fused_tab.p;
@@ -1327,7 +1451,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
             memcpy(fp.cls, c->fused_cls, sizeof(fp.cls));
             fp.code = c->fused_code;
             fp.nsel = nplanes;
-            fp.tiles_x = tiles_x;
+            fp.tiles_x = stx;
             fp.tile_rows = tile_rows;
             fp.blob = (uint8_t *)sl.blob.p;
             fp.cursor = (unsigned long long *)sl.table.p;
@@ -1335,19 +1459,19 @@ static int deflate_rows_impl(gcn10_ctx *c,
             fp.sizes = (uint32_t *)((uint8_t *)sl.table.p + 16 + ntile_slot * sizeof(unsigned long long));
             CUDA_TRY(cudaMemsetAsync(sl.table.p, 0, 16, st));
             if (nplanes <= 9)
-                cn_deflate_fused_kernel<9><<<dim3(tiles_x, tile_rows), kTile, fused_smem_bytes<9>(), st>>>(fp);
+                cn_deflate_fused_kernel<9><<<dim3(stx, tile_rows), kTile, fused_smem_bytes<9>(), st>>>(fp);
             else
-                cn_deflate_fused_kernel<18><<<dim3(tiles_x, tile_rows), kTile, fused_smem_bytes<18>(), st>>>(fp);
+                cn_deflate_fused_kernel<18><<<dim3(stx, tile_rows), kTile, fused_smem_bytes<18>(), st>>>(fp);
             c->launches++;
             CUDA_TRY(cudaGetLastError());
             return hand_over(sl, st);
         }
         uint8_t *d_out[GCN10_NPLANES] = { nullptr };
         for (int k = 0; k < nplanes; k++)
-            d_out[plane_ids[k]] = (uint8_t *)sl.out.p + (size_t)k * dpitch * (size_t)strip;
+            d_out[plane_ids[k]] = (uint8_t *)sl.out.p + (size_t)k * dpitch * (size_t)strip_cap;
         for (int i = 0; i < nplans; i++) {
-            int r2 = launch_rows(c, plans[i], i, strip_esa, strip_esa_pitch, w, rows, row0 + y0, (const uint8_t *)c->hsg.p,
-                                 hsg_dpitch, hsx, hsy, map, tma_ok, d_out, dpitch, st);
+            int r2 = launch_rows(c, plans[i], i, strip_esa, strip_esa_pitch, sw, rows, jb.y_base, (const uint8_t *)c->hsg.p,
+                                 hsg_dpitch, hsx, hsy, map, tma_ok, d_out, dpitch, st, jb.col_idx, jb.row_idx);
             if (r2)
                 return r2;
         }
@@ -1356,16 +1480,16 @@ static int deflate_rows_impl(gcn10_ctx *c,
         for (int k = 0; k < nplanes; k++)
             ep.plane[k] = d_out[plane_ids[k]];
         ep.pitch = dpitch;
-        ep.w = w;
+        ep.w = sw;
         ep.rows = rows;
-        ep.tiles_x = tiles_x;
+        ep.tiles_x = stx;
         ep.tile_rows = tile_rows;
         ep.blob = (uint8_t *)sl.blob.p;
         ep.cursor = (unsigned long long *)sl.table.p;
         ep.offsets = (unsigned long long *)((uint8_t *)sl.table.p + 16);
         ep.sizes = (uint32_t *)((uint8_t *)sl.table.p + 16 + ntile_slot * sizeof(unsigned long long));
         CUDA_TRY(cudaMemsetAsync(sl.table.p, 0, 16, st));
-        deflate_tiles_kernel<<<dim3(tiles_x, tile_rows, nplanes), kTile, kEncSmem, st>>>(ep);
+        deflate_tiles_kernel<<<dim3(stx, tile_rows, nplanes), kTile, kEncSmem, st>>>(ep);
         c->launches++;
         CUDA_TRY(cudaGetLastError());
         return hand_over(sl, st);
@@ -1382,7 +1506,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
         return code;
     };
 
-    // the last strip is on its way: a prefetched block's inflate kernel may have the SMs behind it.  (Letting it go
+    // the last strip (of any level) is on its way: a prefetched block's inflate kernel may have the SMs behind it.  (Letting it go
     // earlier -- once every strip slot is in use -- was measured: its CTAs keep the SMs until they retire, the encoder
     // kernels of the remaining strips wait for milliseconds and the chain of copies runs dry; 10.6 ms against 7.5.)
     auto release = [&](int s) -> int {
@@ -1427,15 +1551,18 @@ static int deflate_rows_impl(gcn10_ctx *c,
         if (s == 0 && before_first_sink && (rc = before_first_sink()))
             return bail(rc);
         gcn10_tile_strip ts;
-        ts.tile_row0 = (row0 + sl.y0) / kTile;
+        ts.tile_row0 = sl.y_base / kTile;
         ts.n_tile_rows = (sl.rows + kTile - 1) / kTile;
-        ts.tiles_x = tiles_x;
+        ts.tiles_x = sl.tiles_x;
         ts.n_planes = nplanes;
         ts.plane_ids = plane_ids;
         ts.offsets = (const uint64_t *)((const uint8_t *)sl.h_table.p + 16);
         ts.sizes = (const uint32_t *)((const uint8_t *)sl.h_table.p + 16 + ntile_slot * sizeof(unsigned long long));
         ts.blob = (const uint8_t *)sl.h_blob.p;
         ts.blob_bytes = used;
+        ts.level = sl.level;
+        ts.level_w = sl.level_w;
+        ts.level_h = sl.level_h;
         // NB: the tables are laid out [plane][strip_tile_rows (capacity)][tiles_x] only when the strip is
         // full; the kernel indexes with the strip's own tile_rows, which is what n_tile_rows reports
         const int sink_rc = sink(user, &ts);
@@ -1446,6 +1573,8 @@ static int deflate_rows_impl(gcn10_ctx *c,
             return bail(rc);
     }
     c->last_kernel_ms = kernel_ms;
+    if (nlev && !emit_levels)
+        c->ov_next = row0 + nrows;
     return GCN10_OK;
 }
 

@@ -8,6 +8,7 @@
  * Extra flags: --gpus N (default: all), --io-threads N (per worker), --outdir DIR (default: CWD).
  */
 #include "gcn10_host.h"
+#include "../../include/gcn10_cuda.h"
 
 #include <stdio.h>
 #include <stdlib.h>
@@ -34,6 +35,8 @@ static void usage(FILE *fp)
             "  --io-threads <n>	decode/encode threads per worker (default: cores / workers)\n"
             "  --workers-per-gpu <n>	blocks in flight per GPU, each with its own context (default: 1)\n"
             "  --outdir <dir>	where cn_rasters_<condition>/ are created (default: .)\n"
+            "  --overviews		also write reduced-resolution overview levels into every output\n"
+            "			(nearest neighbour, halving until a level fits one 256 x 256 tile)\n"
             "  --help, -h		show this help and exit\n"
             "  --version, -v	print version and exit\n"
             "\n"
@@ -74,6 +77,8 @@ int main(int argc, char **argv)
             opt.workers_per_gpu = atoi(argv[++i]);
         else if (!strcmp(argv[i], "--outdir") && i + 1 < argc)
             opt.out_root = argv[++i];
+        else if (!strcmp(argv[i], "--overviews"))
+            opt.overviews = GCN10_MAX_OVERVIEWS;
     }
     if (!conf) {
         fprintf(stderr, "[rank 0] missing -c/--config <file>; see 'gcn10 -h' for usage.\n");    /* main.c:103-107 */

@@ -186,6 +186,11 @@ static int open_writers(worker *wk)
             gh_tiffw_set_geokeys(wk->writers[k], &gk);
         pthread_mutex_unlock(&wk->rmu);
         opened++;
+        if (gh_tiffw_set_overviews(wk->writers[k], wk->opt->overviews)) {
+            snprintf(err, sizeof err, "write error 3 on %s (overviews)", wk->paths[k]);
+            gh_log_message(wk->log, "ERROR", err, 1);
+            break;
+        }
     }
     if (opened < NPLANES) {
         for (int k = 0; k < opened; k++) {
@@ -281,7 +286,7 @@ typedef struct {
     const gcn10_tile_strip *st;
 } sink_job;
 
-/* one plane of a strip: append its tile rows to that plane's GeoTIFF */
+/* one plane of a strip: append its tile rows to that plane's GeoTIFF (to the strip's level of it) */
 static void sink_plane(void *arg, int k)
 {
     sink_job *j = arg;
@@ -289,7 +294,8 @@ static void sink_plane(void *arg, int k)
     gh_tiffw *tw = j->wk->writers[st->plane_ids[k]];
     /* the context runs with "ordered" strips: a plane's share of the strip is one contiguous piece of the blob */
     size_t base = (size_t)k * st->n_tile_rows * (size_t)st->tiles_x;
-    if (gh_tiffw_put_tile_rows(tw, st->tile_row0, st->n_tile_rows, st->blob, st->offsets + base, st->sizes + base))
+    if (gh_tiffw_put_level_tile_rows(tw, st->level, st->tile_row0, st->n_tile_rows, st->blob, st->offsets + base,
+                                     st->sizes + base))
         atomic_store(&j->wk->encode_failed, 1);
 }
 
@@ -715,7 +721,8 @@ static void *worker_main(void *arg)
     /* ordered strips: a plane's share of a strip is one write; ship kernel: from four GPUs on one host fabric its posted
      * writes beat the copy engine's size read-back + copy (measured on 8 x B200: +4..7 %), below that the copy engine wins */
     if (gcn10_cuda_create(wk->device, &wk->ctx) || gcn10_cuda_set_luts(wk->ctx, wk->tables) ||
-        gcn10_cuda_set_option(wk->ctx, "ordered", 1) || gcn10_cuda_set_option(wk->ctx, "ship", wk->n_gpus >= 4)) {
+        gcn10_cuda_set_option(wk->ctx, "ordered", 1) || gcn10_cuda_set_option(wk->ctx, "ship", wk->n_gpus >= 4) ||
+        gcn10_cuda_set_option(wk->ctx, "overviews", wk->opt->overviews)) {
         snprintf(msg, sizeof msg, "cannot initialise GPU %d: %s", wk->device, gcn10_cuda_last_error());
         fatal(wk, msg);
     }

@@ -742,6 +742,15 @@ int gh_tiff_window_tiles_read(gh_tiff *t, const gh_tile_plan *plan, uint8_t *blo
 
 enum { TILE = 256 };
 
+/* the tile grid of one level of the file: level 0 = the full-resolution raster, k >= 1 = overview level k */
+typedef struct {
+    int w, h;
+    int tiles_x, tiles_y;
+    uint32_t *offsets, *counts;
+    int next_tile_row;
+    uint8_t *band;              /* gh_tiffw_write_rows, levels >= 1: the level's tile row being sampled, TILE x w */
+} tw_grid;
+
 struct gh_tiffw {
     FILE *fp;
     char *path, *tmp;           /* written as <path>.part, renamed on a successful close, removed otherwise */
@@ -751,18 +760,17 @@ struct gh_tiffw {
     size_t n_geo_doubles;
     char *geo_ascii;
     size_t n_geo_ascii;
-    int w, h;
-    int tiles_x, tiles_y;
     double gt[6];
-    uint32_t *offsets, *counts;
     uint64_t pos;
-    int next_tile_row;
-    int level;
+    int nlev;                   /* overview levels (gh_tiffw_set_overviews) */
+    tw_grid g[1 + GCN10_MAX_OVERVIEWS];
+    int level;                  /* zlib level */
     int failed;
 };
 
 typedef struct {
     gh_tiffw *tw;
+    const tw_grid *g;
     const uint8_t *data;        /* first row of this band */
     size_t pitch;
     int rows;                   /* rows available in the band */
@@ -775,10 +783,10 @@ static void compress_tile(void *arg, int index)
 {
     write_job *j = arg;
     gh_tiffw *tw = j->tw;
-    int tx = index % tw->tiles_x, tr = index / tw->tiles_x;
+    int tx = index % j->g->tiles_x, tr = index / j->g->tiles_x;
     unsigned char tile[TILE * TILE];
     int x0 = tx * TILE, y0 = tr * TILE;
-    int cols = tw->w - x0 < TILE ? tw->w - x0 : TILE;
+    int cols = j->g->w - x0 < TILE ? j->g->w - x0 : TILE;
     int rows = j->rows - y0 < TILE ? j->rows - y0 : TILE;
     if (cols < TILE || rows < TILE)
         memset(tile, 0, sizeof tile);       /* edge tiles are padded with zeros */
@@ -794,6 +802,27 @@ static void compress_tile(void *arg, int index)
     }
     j->comp[index] = out;
     j->comp_len[index] = cap;
+}
+
+static int grid_init(tw_grid *g, int w, int h)
+{
+    g->w = w;
+    g->h = h;
+    g->tiles_x = (w + TILE - 1) / TILE;
+    g->tiles_y = (h + TILE - 1) / TILE;
+    size_t nt = (size_t)g->tiles_x * (size_t)g->tiles_y;
+    g->offsets = calloc(nt, sizeof(uint32_t));
+    g->counts = calloc(nt, sizeof(uint32_t));
+    return g->offsets && g->counts ? 0 : -1;
+}
+
+static void free_grids(gh_tiffw *tw)
+{
+    for (int k = 0; k <= tw->nlev; k++) {
+        free(tw->g[k].offsets);
+        free(tw->g[k].counts);
+        free(tw->g[k].band);
+    }
 }
 
 int gh_tiffw_open(const char *path, int w, int h, const double gt[6], gh_tiffw **out, char *err, size_t errlen)
@@ -822,17 +851,10 @@ int gh_tiffw_open(const char *path, int w, int h, const double gt[6], gh_tiffw *
         return -1;
     }
     setvbuf(tw->fp, NULL, _IOFBF, 1 << 20);     /* tiles arrive as ~1.5 KB pieces: one write(2) per MB, not per tile */
-    tw->w = w;
-    tw->h = h;
-    tw->tiles_x = (w + TILE - 1) / TILE;
-    tw->tiles_y = (h + TILE - 1) / TILE;
     tw->level = 6;              /* GDAL's default ZLEVEL */
     memcpy(tw->gt, gt, sizeof tw->gt);
-    size_t nt = (size_t)tw->tiles_x * (size_t)tw->tiles_y;
-    tw->offsets = calloc(nt, sizeof(uint32_t));
-    tw->counts = calloc(nt, sizeof(uint32_t));
     unsigned char hdr[8] = { 'I', 'I', 42, 0, 0, 0, 0, 0 };      /* IFD offset patched on close */
-    if (!tw->offsets || !tw->counts || fwrite(hdr, 1, 8, tw->fp) != 8) {
+    if (grid_init(&tw->g[0], w, h) || fwrite(hdr, 1, 8, tw->fp) != 8) {
         set_err(err, errlen, "write error 3 on %s", path);
         gh_tiffw_abort(tw);
         return -1;
@@ -877,14 +899,29 @@ int gh_tiffw_set_geokeys(gh_tiffw *tw, const gh_geokeys *gk)
     return 0;
 }
 
-int gh_tiffw_write_rows(gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0, int nrows, int threads)
+int gh_tiffw_set_overviews(gh_tiffw *tw, int n)
 {
-    if (tw->failed || y0 != tw->next_tile_row * TILE || y0 + nrows > tw->h ||
-        (nrows % TILE != 0 && y0 + nrows != tw->h))
+    if (!tw || tw->failed || n < 0 || n > GCN10_MAX_OVERVIEWS || tw->nlev || tw->pos != 8 || tw->g[0].next_tile_row)
         return -1;
-    int tile_rows = (nrows + TILE - 1) / TILE;
-    int n = tile_rows * tw->tiles_x;
-    write_job j = { tw, data, pitch, nrows, tw->next_tile_row, NULL, NULL };
+    const int nlev = gcn10_overview_levels(tw->g[0].w, tw->g[0].h, n);
+    for (int k = 1; k <= nlev; k++) {
+        tw->nlev = k;
+        if (grid_init(&tw->g[k], gcn10_overview_dim(tw->g[0].w, k), gcn10_overview_dim(tw->g[0].h, k))) {
+            tw->failed = 1;
+            return -1;
+        }
+    }
+    return 0;
+}
+
+int gh_tiffw_levels(const gh_tiffw *tw) { return tw ? tw->nlev : -1; }
+
+/* Compresses the tile rows [0, rows) held in data (pitch bytes apart) as the next tile rows of grid g. */
+static int append_tile_rows(gh_tiffw *tw, tw_grid *g, const uint8_t *data, size_t pitch, int rows, int threads)
+{
+    int tile_rows = (rows + TILE - 1) / TILE;
+    int n = tile_rows * g->tiles_x;
+    write_job j = { tw, g, data, pitch, rows, g->next_tile_row, NULL, NULL };
     j.comp = calloc((size_t)n, sizeof(unsigned char *));
     j.comp_len = calloc((size_t)n, sizeof(uLongf));
     if (!j.comp || !j.comp_len) {
@@ -895,47 +932,97 @@ int gh_tiffw_write_rows(gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0,
     }
     parallel_for(n, threads, compress_tile, &j);
     for (int i = 0; i < n; i++) {
-        size_t ti = (size_t)(tw->next_tile_row + i / tw->tiles_x) * (size_t)tw->tiles_x + (size_t)(i % tw->tiles_x);
+        size_t ti = (size_t)(g->next_tile_row + i / g->tiles_x) * (size_t)g->tiles_x + (size_t)(i % g->tiles_x);
         if (!tw->failed && j.comp[i]) {
             if (tw->pos + j.comp_len[i] > 0xFFFFFFF0ull || fwrite(j.comp[i], 1, j.comp_len[i], tw->fp) != j.comp_len[i])
                 tw->failed = 1;
-            tw->offsets[ti] = (uint32_t)tw->pos;
-            tw->counts[ti] = (uint32_t)j.comp_len[i];
+            g->offsets[ti] = (uint32_t)tw->pos;
+            g->counts[ti] = (uint32_t)j.comp_len[i];
             tw->pos += j.comp_len[i];
         }
         free(j.comp[i]);
     }
     free(j.comp);
     free(j.comp_len);
-    tw->next_tile_row += tile_rows;
+    g->next_tile_row += tile_rows;
     return tw->failed ? -1 : 0;
+}
+
+int gh_tiffw_write_rows(gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0, int nrows, int threads)
+{
+    tw_grid *g0 = &tw->g[0];
+    if (tw->failed || y0 != g0->next_tile_row * TILE || y0 + nrows > g0->h ||
+        (nrows % TILE != 0 && y0 + nrows != g0->h))
+        return -1;
+    if (append_tile_rows(tw, g0, data, pitch, nrows, threads))
+        return -1;
+    /* the overview levels, sampled from this band by the rule of gcn10_overview_src: each level keeps one tile row
+     * and appends it compressed when it is full, so the levels cost a few MB, not a third of the raster */
+    for (int k = 1; k <= tw->nlev; k++) {
+        tw_grid *g = &tw->g[k];
+        if (!g->band && !(g->band = malloc((size_t)TILE * (size_t)g->w))) {
+            tw->failed = 1;
+            return -1;
+        }
+        for (int i = g->next_tile_row * TILE; i < g->h; i++) {
+            const int src = gcn10_overview_src(i, k, g0->h);
+            if (src < y0)
+                continue;       /* (a band boundary inside a tile row: rows before it were sampled already) */
+            if (src >= y0 + nrows)
+                break;
+            const uint8_t *row = data + (size_t)(src - y0) * pitch;
+            uint8_t *dst = g->band + (size_t)(i % TILE) * (size_t)g->w;
+            for (int x = 0; x < g->w; x++)
+                dst[x] = row[gcn10_overview_src(x, k, g0->w)];
+            if (i % TILE == TILE - 1 || i == g->h - 1) {
+                if (append_tile_rows(tw, g, g->band, (size_t)g->w, i % TILE + 1, threads))
+                    return -1;
+            }
+        }
+    }
+    return 0;
+}
+
+static int put_grid_tile_row(gh_tiffw *tw, tw_grid *g, int tile_row, const uint8_t *blob, const uint64_t *offsets,
+                             const uint32_t *sizes)
+{
+    if (tw->failed || tile_row != g->next_tile_row || tile_row >= g->tiles_y)
+        return -1;
+    for (int tx = 0; tx < g->tiles_x; tx++) {
+        size_t ti = (size_t)tile_row * (size_t)g->tiles_x + (size_t)tx;
+        if (tw->pos + sizes[tx] > 0xFFFFFFF0ull || fwrite(blob + offsets[tx], 1, sizes[tx], tw->fp) != sizes[tx]) {
+            tw->failed = 1;
+            return -1;
+        }
+        g->offsets[ti] = (uint32_t)tw->pos;
+        g->counts[ti] = sizes[tx];
+        tw->pos += sizes[tx];
+    }
+    g->next_tile_row++;
+    return 0;
 }
 
 int gh_tiffw_put_tile_row(gh_tiffw *tw, int tile_row, const uint8_t *blob, const uint64_t *offsets,
                           const uint32_t *sizes)
 {
-    if (tw->failed || tile_row != tw->next_tile_row || tile_row >= tw->tiles_y)
-        return -1;
-    for (int tx = 0; tx < tw->tiles_x; tx++) {
-        size_t ti = (size_t)tile_row * (size_t)tw->tiles_x + (size_t)tx;
-        if (tw->pos + sizes[tx] > 0xFFFFFFF0ull || fwrite(blob + offsets[tx], 1, sizes[tx], tw->fp) != sizes[tx]) {
-            tw->failed = 1;
-            return -1;
-        }
-        tw->offsets[ti] = (uint32_t)tw->pos;
-        tw->counts[ti] = sizes[tx];
-        tw->pos += sizes[tx];
-    }
-    tw->next_tile_row++;
-    return 0;
+    return put_grid_tile_row(tw, &tw->g[0], tile_row, blob, offsets, sizes);
 }
 
 int gh_tiffw_put_tile_rows(gh_tiffw *tw, int tile_row0, int nrows, const uint8_t *blob, const uint64_t *offsets,
                            const uint32_t *sizes)
 {
-    if (tw->failed || tile_row0 != tw->next_tile_row || nrows < 1 || tile_row0 + nrows > tw->tiles_y)
+    return gh_tiffw_put_level_tile_rows(tw, 0, tile_row0, nrows, blob, offsets, sizes);
+}
+
+int gh_tiffw_put_level_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nrows, const uint8_t *blob,
+                                 const uint64_t *offsets, const uint32_t *sizes)
+{
+    if (!tw || level < 0 || level > tw->nlev)
         return -1;
-    const size_t n = (size_t)nrows * (size_t)tw->tiles_x;
+    tw_grid *g = &tw->g[level];
+    if (tw->failed || tile_row0 != g->next_tile_row || nrows < 1 || tile_row0 + nrows > g->tiles_y)
+        return -1;
+    const size_t n = (size_t)nrows * (size_t)g->tiles_x;
     /* laid out in table order with small gaps (the library's "ordered" strips)?  Then the whole share is one write;
      * the gaps (< 16 bytes per tile, alignment padding) go into the file as unused bytes, which TIFF allows */
     int ordered = 1;
@@ -943,7 +1030,7 @@ int gh_tiffw_put_tile_rows(gh_tiffw *tw, int tile_row0, int nrows, const uint8_t
         ordered = offsets[i + 1] >= offsets[i] + sizes[i] && offsets[i + 1] - (offsets[i] + sizes[i]) < 64;
     if (!ordered) {
         for (int r = 0; r < nrows; r++)
-            if (gh_tiffw_put_tile_row(tw, tile_row0 + r, blob, offsets + (size_t)r * tw->tiles_x, sizes + (size_t)r * tw->tiles_x))
+            if (put_grid_tile_row(tw, g, tile_row0 + r, blob, offsets + (size_t)r * g->tiles_x, sizes + (size_t)r * g->tiles_x))
                 return -1;
         return 0;
     }
@@ -953,12 +1040,12 @@ int gh_tiffw_put_tile_rows(gh_tiffw *tw, int tile_row0, int nrows, const uint8_t
         return -1;
     }
     for (size_t i = 0; i < n; i++) {
-        const size_t ti = (size_t)tile_row0 * (size_t)tw->tiles_x + i;
-        tw->offsets[ti] = (uint32_t)(tw->pos + (offsets[i] - first));
-        tw->counts[ti] = sizes[i];
+        const size_t ti = (size_t)tile_row0 * (size_t)g->tiles_x + i;
+        g->offsets[ti] = (uint32_t)(tw->pos + (offsets[i] - first));
+        g->counts[ti] = sizes[i];
     }
     tw->pos += bytes;
-    tw->next_tile_row += nrows;
+    g->next_tile_row += nrows;
     return 0;
 }
 
@@ -980,8 +1067,12 @@ int gh_tiffw_close(gh_tiffw *tw)
     if (!tw)
         return -1;
     int rc = -1;
-    size_t nt = (size_t)tw->tiles_x * (size_t)tw->tiles_y;
-    if (!tw->failed && tw->next_tile_row == tw->tiles_y) {
+    const tw_grid *g0 = &tw->g[0];
+    size_t nt = (size_t)g0->tiles_x * (size_t)g0->tiles_y;
+    int complete = !tw->failed;
+    for (int k = 0; k <= tw->nlev; k++)
+        complete = complete && tw->g[k].next_tile_row == tw->g[k].tiles_y;
+    if (complete) {
         /* trailing data area: tile offsets, tile byte counts, pixel scale, tiepoint, geo keys, ascii */
         static const uint16_t geokeys[] = {
             1, 1, 0, 4,
@@ -1002,11 +1093,19 @@ int gh_tiffw_close(gh_tiffw *tw)
         uint64_t off_ascii = off_dbl + 8 * ndbl;
         uint64_t off_ifd = (off_ascii + nascii + 1) & ~(uint64_t)1;
         const int nent = 14 + 1 + (ndbl ? 1 : 0) + (nascii ? 1 : 0);
-        size_t tail = (size_t)(off_ifd - tw->pos) + 2 + (size_t)nent * 12 + 4;
+        /* behind IFD0, per overview level: its tile offsets, byte counts and IFD (reduced-resolution image, no geo tags:
+         * readers derive the level's georeferencing from the size ratio) */
+        enum { LEVEL_ENTRIES = 13 };
+        uint64_t off_lv[1 + GCN10_MAX_OVERVIEWS], end = off_ifd + 2 + (uint64_t)nent * 12 + 4;
+        for (int k = 1; k <= tw->nlev; k++) {
+            off_lv[k] = end;            /* offsets | counts | IFD */
+            end += 8 * (uint64_t)tw->g[k].tiles_x * (uint64_t)tw->g[k].tiles_y + 2 + LEVEL_ENTRIES * 12 + 4;
+        }
+        size_t tail = (size_t)(end - tw->pos);
         unsigned char *buf = calloc(1, tail), *p = buf;
-        if (buf && off_ifd + 256 < 0xFFFFFFF0ull) {
-            for (size_t i = 0; i < nt; i++) put32(&p, tw->offsets[i]);
-            for (size_t i = 0; i < nt; i++) put32(&p, tw->counts[i]);
+        if (buf && end + 256 < 0xFFFFFFF0ull) {
+            for (size_t i = 0; i < nt; i++) put32(&p, g0->offsets[i]);
+            for (size_t i = 0; i < nt; i++) put32(&p, g0->counts[i]);
             put_f64(&p, tw->gt[1]); put_f64(&p, -tw->gt[5]); put_f64(&p, 0.0);
             put_f64(&p, 0.0); put_f64(&p, 0.0); put_f64(&p, 0.0);
             put_f64(&p, tw->gt[0]); put_f64(&p, tw->gt[3]); put_f64(&p, 0.0);
@@ -1016,8 +1115,8 @@ int gh_tiffw_close(gh_tiffw *tw)
                 memcpy(p, ascii, nascii);
             p = buf + (off_ifd - tw->pos);
             put16(&p, (uint16_t)nent);
-            put_entry(&p, 256, 4, 1, (uint32_t)tw->w);
-            put_entry(&p, 257, 4, 1, (uint32_t)tw->h);
+            put_entry(&p, 256, 4, 1, (uint32_t)g0->w);
+            put_entry(&p, 257, 4, 1, (uint32_t)g0->h);
             put_entry(&p, 258, 3, 1, 8);
             put_entry(&p, 259, 3, 1, 8);                /* Adobe DEFLATE, what GDAL writes */
             put_entry(&p, 262, 3, 1, 1);                /* BlackIsZero */
@@ -1025,8 +1124,8 @@ int gh_tiffw_close(gh_tiffw *tw)
             put_entry(&p, 284, 3, 1, 1);
             put_entry(&p, 322, 3, 1, TILE);
             put_entry(&p, 323, 3, 1, TILE);
-            put_entry(&p, 324, 4, (uint32_t)nt, nt == 1 ? tw->offsets[0] : (uint32_t)off_offsets);
-            put_entry(&p, 325, 4, (uint32_t)nt, nt == 1 ? tw->counts[0] : (uint32_t)off_counts);
+            put_entry(&p, 324, 4, (uint32_t)nt, nt == 1 ? g0->offsets[0] : (uint32_t)off_offsets);
+            put_entry(&p, 325, 4, (uint32_t)nt, nt == 1 ? g0->counts[0] : (uint32_t)off_counts);
             put_entry(&p, 339, 3, 1, 1);                /* SampleFormat = unsigned */
             put_entry(&p, 33550, 12, 3, (uint32_t)off_scale);
             put_entry(&p, 33922, 12, 6, (uint32_t)off_tie);
@@ -1035,7 +1134,30 @@ int gh_tiffw_close(gh_tiffw *tw)
                 put_entry(&p, 34736, 12, (uint32_t)ndbl, (uint32_t)off_dbl);
             if (nascii)
                 put_entry(&p, 34737, 2, (uint32_t)nascii, (uint32_t)off_ascii);
-            put32(&p, 0);
+            put32(&p, tw->nlev ? (uint32_t)(off_lv[1] + 8 * (uint64_t)tw->g[1].tiles_x * (uint64_t)tw->g[1].tiles_y) : 0);
+            for (int k = 1; k <= tw->nlev; k++) {
+                const tw_grid *g = &tw->g[k];
+                const size_t n = (size_t)g->tiles_x * (size_t)g->tiles_y;
+                p = buf + (off_lv[k] - tw->pos);
+                for (size_t i = 0; i < n; i++) put32(&p, g->offsets[i]);
+                for (size_t i = 0; i < n; i++) put32(&p, g->counts[i]);
+                put16(&p, LEVEL_ENTRIES);
+                put_entry(&p, 254, 4, 1, 1);            /* NewSubfileType = reduced-resolution version */
+                put_entry(&p, 256, 4, 1, (uint32_t)g->w);
+                put_entry(&p, 257, 4, 1, (uint32_t)g->h);
+                put_entry(&p, 258, 3, 1, 8);
+                put_entry(&p, 259, 3, 1, 8);
+                put_entry(&p, 262, 3, 1, 1);
+                put_entry(&p, 277, 3, 1, 1);
+                put_entry(&p, 284, 3, 1, 1);
+                put_entry(&p, 322, 3, 1, TILE);
+                put_entry(&p, 323, 3, 1, TILE);
+                put_entry(&p, 324, 4, (uint32_t)n, n == 1 ? g->offsets[0] : (uint32_t)off_lv[k]);
+                put_entry(&p, 325, 4, (uint32_t)n, n == 1 ? g->counts[0] : (uint32_t)(off_lv[k] + 4 * n));
+                put_entry(&p, 339, 3, 1, 1);
+                put32(&p, k < tw->nlev ? (uint32_t)(off_lv[k + 1] + 8 * (uint64_t)tw->g[k + 1].tiles_x * (uint64_t)tw->g[k + 1].tiles_y)
+                                       : 0);
+            }
             if (fwrite(buf, 1, tail, tw->fp) == tail && fseek(tw->fp, 4, SEEK_SET) == 0) {
                 unsigned char o[4], *q = o;
                 put32(&q, (uint32_t)off_ifd);
@@ -1056,8 +1178,7 @@ int gh_tiffw_close(gh_tiffw *tw)
     free(tw->geo_ascii);
     free(tw->path);
     free(tw->tmp);
-    free(tw->offsets);
-    free(tw->counts);
+    free_grids(tw);
     free(tw);
     return rc;
 }
@@ -1075,8 +1196,7 @@ void gh_tiffw_abort(gh_tiffw *tw)
     free(tw->geo_ascii);
     free(tw->path);
     free(tw->tmp);
-    free(tw->offsets);
-    free(tw->counts);
+    free_grids(tw);
     free(tw);
 }
 

@@ -5,6 +5,8 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include "../../include/gcn10_cuda.h"      /* the overview rules: gcn10_overview_dim / _src / _levels */
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -17,8 +19,15 @@ int gh_tiffw_open(const char *path, int w, int h, const double gt[6], gh_tiffw *
  * PixelIsArea because the tiepoint written is a pixel corner).  Call before gh_tiffw_close. */
 #include "gcn10_host.h"
 int gh_tiffw_set_geokeys(gh_tiffw *tw, const gh_geokeys *gk);
+/* Overview levels: the file gets gcn10_overview_levels(w, h, n) reduced-resolution images behind the full-resolution
+ * one (one IFD each, NewSubfileType 1, chained from IFD0; n = 0: none).  Call after open, before the first data.
+ * gh_tiffw_levels returns how many levels the file will have.  gh_tiffw_close fails (and removes the file) unless
+ * every tile of every level has been written. */
+int gh_tiffw_set_overviews(gh_tiffw *tw, int n);
+int gh_tiffw_levels(const gh_tiffw *tw);
 /* Appends rows [y0, y0+nrows): y0 must continue where the previous call stopped and be a multiple
- * of 256; nrows must be a multiple of 256 except for the last band of the raster. */
+ * of 256; nrows must be a multiple of 256 except for the last band of the raster.  With overviews, the levels are
+ * sampled from the same rows (gcn10_overview_src) and compressed here too, a level's tile row as soon as it is full. */
 int gh_tiffw_write_rows(gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0, int nrows, int threads);
 /* Appends tiles that are already compressed (complete zlib streams of 256 x 256 bytes, e.g. from
  * gcn10_cuda_block_deflate): tile row `tile_row` must be the next one not yet written; sizes / offsets
@@ -29,6 +38,10 @@ int gh_tiffw_put_tile_row(gh_tiffw *tw, int tile_row, const uint8_t *blob, const
  * order with at most alignment gaps between them (gcn10_cuda_set_option "ordered") they are written with one write. */
 int gh_tiffw_put_tile_rows(gh_tiffw *tw, int tile_row0, int nrows, const uint8_t *blob, const uint64_t *offsets,
                            const uint32_t *sizes);
+/* The same for the tile grid of overview level `level` (0 = the full-resolution image, as gh_tiffw_put_tile_rows):
+ * its tile rows too must come in order. */
+int gh_tiffw_put_level_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nrows, const uint8_t *blob,
+                                 const uint64_t *offsets, const uint32_t *sizes);
 /* Runs fn(arg, 0..n-1) on up to `threads` threads (the calling thread included). */
 void gh_parallel_for(int n, int threads, void (*fn)(void *arg, int index), void *arg);
 /* Writes the tile tables, georeferencing and IFD; 0 ok. */

@@ -73,6 +73,10 @@ def load(path: str | None = None) -> C.CDLL:
     L.gh_tiffw_put_tile_row.argtypes = [_vp, C.c_int, _vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]
     L.gh_tiffw_put_tile_rows.argtypes = [_vp, C.c_int, C.c_int, _vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]
     L.gh_tiffw_write_rows.argtypes = [_vp, _vp, C.c_size_t, C.c_int, C.c_int, C.c_int]
+    L.gh_tiffw_set_overviews.argtypes = [_vp, C.c_int]
+    L.gh_tiffw_levels.argtypes = [_vp]
+    L.gh_tiffw_put_level_tile_rows.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, C.POINTER(C.c_uint64),
+                                               C.POINTER(C.c_uint32)]
     L.gh_tiffw_close.argtypes = [_vp]
     L.gh_tiffw_abort.argtypes = [_vp]
     L.gh_tiffw_abort.restype = None
@@ -314,9 +318,10 @@ class Raster:
 
 
 class TiffWriter:
-    """Incremental tiled-DEFLATE GeoTIFF writer (gh_tiffw_*): raw row bands or pre-compressed tile rows."""
+    """Incremental tiled-DEFLATE GeoTIFF writer (gh_tiffw_*): raw row bands or pre-compressed tile rows.
+    ``overviews=n`` adds up to n overview levels (gh_tiffw_set_overviews); ``levels`` is how many the file gets."""
 
-    def __init__(self, path: str, w: int, h: int, gt):
+    def __init__(self, path: str, w: int, h: int, gt, overviews: int = 0):
         self.L = load()
         h_ = _vp()
         e = _err()
@@ -325,10 +330,16 @@ class TiffWriter:
             raise HostError(rc, e.value.decode(errors="replace"))
         self.h = h_
         self.tiles_x = (w + 255) // 256
+        if overviews and self.L.gh_tiffw_set_overviews(h_, overviews):
+            self.L.gh_tiffw_abort(h_)
+            self.h = None
+            raise HostError(-1, f"gh_tiffw_set_overviews({overviews}) failed")
+        self.levels = self.L.gh_tiffw_levels(h_)
 
-    def put_tile_row(self, tile_row: int, streams):
-        """streams: tiles_x zlib streams (bytes) of one tile row."""
-        assert len(streams) == self.tiles_x
+    def put_tile_row(self, tile_row: int, streams, level: int = 0):
+        """streams: the zlib streams (bytes) of one tile row of ``level`` (0 = full resolution)."""
+        if level == 0:
+            assert len(streams) == self.tiles_x
         blob = b"".join(streams)
         offs = (C.c_uint64 * len(streams))()
         sizes = (C.c_uint32 * len(streams))()
@@ -336,8 +347,10 @@ class TiffWriter:
         for i, z in enumerate(streams):
             offs[i], sizes[i] = pos, len(z)
             pos += len(z)
-        buf = C.create_string_buffer(blob, len(blob))
-        return self.L.gh_tiffw_put_tile_row(self.h, tile_row, buf, offs, sizes)
+        buf = C.create_string_buffer(blob, max(len(blob), 1))
+        if level == 0:
+            return self.L.gh_tiffw_put_tile_row(self.h, tile_row, buf, offs, sizes)
+        return self.L.gh_tiffw_put_level_tile_rows(self.h, level, tile_row, 1, buf, offs, sizes)
 
     def write_rows(self, data: np.ndarray, y0: int, threads: int = 2):
         data = np.ascontiguousarray(data, dtype=np.uint8)

@@ -151,7 +151,15 @@ int gcn10_cuda_block_rows(gcn10_ctx *ctx,
  * edge are zero padded to 256 x 256.  The block is processed in strips of whole tile rows; `sink` is
  * called once per strip, in order, from the calling thread.  The memory behind strip->blob / offsets /
  * sizes is page-locked, owned by the library and valid only during the call: copy or write it out.
- * A non-zero return from `sink` aborts the block (returned as GCN10_EINVAL). */
+ * A non-zero return from `sink` aborts the block (returned as GCN10_EINVAL).
+ *
+ * Overviews (option "overviews" = n > 0): after the block's last full-resolution strip the same sink receives the
+ * block's overview levels 1 .. gcn10_overview_levels(w, h, n), level 1 first, each in tile-row order, in strips of at
+ * most "strip_rows" rows of that level (strip->level, level_w, level_h say which level and its size).  Level k of every
+ * plane is the plane sampled by gcn10_overview_src, so each of its pixels is a full-resolution output pixel.  This
+ * holds for gcn10_cuda_block_deflate, _block_deflate_rows, _block_tiles_deflate and _block_parts_deflate; the raw-plane
+ * calls (gcn10_cuda_block*, _block_device) ignore the option.  The levels cost device memory of about a third of the
+ * block (about 0.44 GB for 36001 x 36001), kept on the context. */
 typedef struct {
     int tile_row0;              /* first tile row (of the block) in this strip                    */
     int n_tile_rows;            /* tile rows in this strip                                        */
@@ -162,7 +170,45 @@ typedef struct {
     const uint32_t *sizes;      /* [n_planes][n_tile_rows][tiles_x] bytes of its zlib stream      */
     const uint8_t *blob;        /* the compressed tiles of the strip                              */
     size_t blob_bytes;
+    /* overview levels (option "overviews"): 0 = a full-resolution strip; k >= 1 = a strip of overview level k,
+     * whose level_w x level_h raster has its own tile grid (tile_row0 and tiles_x then refer to that grid).
+     * level_w x level_h is the raster the strip's tile grid covers: the block itself at level 0. */
+    int level;
+    int level_w, level_h;
 } gcn10_tile_strip;
+
+/* Overview levels: nearest-neighbour reductions by 2^k of a block, sampled from full resolution.
+ * Every layer (library, GeoTIFF writer, tests) uses these three rules.
+ *
+ *   gcn10_overview_dim(n, k)        pixels of level k along an n-pixel axis: ceil(n / 2^k) (GDAL's overview size)
+ *   gcn10_overview_src(i, k, n)     the full-resolution pixel that level pixel i samples: the one holding the centre
+ *                                   of the level cell, min(i * 2^k + 2^(k-1), n - 1); every level samples level 0
+ *   gcn10_overview_levels(w, h, m)  levels k = 1, 2, ... are made while level k - 1 is wider or taller than one
+ *                                   256-pixel tile, at most m (gdaladdo's automatic rule): 8 for 36000 x 36000 and
+ *                                   36001 x 36001, none for a block that fits in one tile */
+#ifdef __CUDACC__
+#define GCN10_HOST_DEVICE __host__ __device__        /* the library's kernels sample by the same rule */
+#else
+#define GCN10_HOST_DEVICE
+#endif
+
+static inline GCN10_HOST_DEVICE int gcn10_overview_dim(int n, int k) { return (int)(((long long)n + (1LL << k) - 1) >> k); }
+
+static inline GCN10_HOST_DEVICE int gcn10_overview_src(int i, int k, int n)
+{
+    const long long s = ((long long)i << k) + ((1LL << k) >> 1);
+    return s < n - 1 ? (int)s : n - 1;
+}
+
+static inline int gcn10_overview_levels(int w, int h, int max_levels)
+{
+    int k = 0;
+    while (k < max_levels && (gcn10_overview_dim(w, k) > 256 || gcn10_overview_dim(h, k) > 256))
+        k++;
+    return k;
+}
+
+#define GCN10_MAX_OVERVIEWS 16
 
 typedef int (*gcn10_tile_sink)(void *user, const gcn10_tile_strip *strip);
 
@@ -172,7 +218,11 @@ int gcn10_cuda_block_deflate(gcn10_ctx *ctx,
                              unsigned plane_mask, gcn10_tile_sink sink, void *user);
 
 /* Band form of gcn10_cuda_block_deflate (see gcn10_cuda_block_rows): esa points at block row `row0`,
- * which must be a multiple of 256; nrows must be a multiple of 256 unless the band ends the block. */
+ * which must be a multiple of 256; nrows must be a multiple of 256 unless the band ends the block.
+ * With option "overviews" the bands of a block feed its levels, which stay on the context between calls: a band with
+ * row0 == 0 starts a block, every later band must start where the previous one ended (same w and h; anything else is
+ * refused with GCN10_EINVAL), and the band that ends the block (row0 + nrows == h) delivers the levels after its own
+ * strips. */
 int gcn10_cuda_block_deflate_rows(gcn10_ctx *ctx,
                                   const uint8_t *esa, int w, int h, int row0, int nrows, size_t esa_pitch,
                                   const double gt[6],
@@ -286,7 +336,7 @@ int gcn10_cuda_index_maps(gcn10_ctx *ctx, int w, int h, const double gt[6],
 int gcn10_cuda_synchronize(gcn10_ctx *ctx);
 
 /* Device time of the fused kernels of the most recent gcn10_cuda_block() call (sum over its
- * strips), measured with CUDA events on the launching streams. */
+ * strips, overview strips included), measured with CUDA events on the launching streams. */
 int gcn10_cuda_last_kernel_ms(gcn10_ctx *ctx, float *ms);
 
 /* Number of kernels this context has launched since it was created. */
@@ -300,7 +350,8 @@ int gcn10_cuda_launch_count(gcn10_ctx *ctx, uint64_t *launches);
  * 16-byte boundaries, offsets ascending -- so that a consumer can write a plane's share of a strip with one write),
  * "tuned_code" (0 = tile streams use RFC 1951's fixed Huffman code instead
  * of the tuned one), "defer_inflate" (0 = the inflate kernel of a prefetched block starts at once instead of behind
- * the last strip of the block in hand), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
+ * the last strip of the block in hand), "overviews" (0..16, default 0: the compressed-tile calls also deliver up to that
+ * many overview levels of the block, see gcn10_cuda_block_deflate), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
  * kernel's writer off; results are then invalid). */
 int gcn10_cuda_set_option(gcn10_ctx *ctx, const char *key, long value);
 
