@@ -31,6 +31,7 @@ EXPORTS = (
     "gcn10_cuda_inflate_tiles", "gcn10_cuda_block_tiles_deflate", "gcn10_cuda_last_inflate_ms",
     "gcn10_cuda_tiles_prefetch", "gcn10_cuda_block_async", "gcn10_cuda_wait", "gcn10_cuda_event_query",
     "gcn10_cuda_pcie_probe", "gcn10_cuda_parts_prefetch", "gcn10_cuda_inflate_parts", "gcn10_cuda_block_parts_deflate",
+    "gcn10_cuda_last_histograms",
 )
 
 _vp = C.c_void_p
@@ -177,6 +178,7 @@ def load(path: str = LIB_PATH) -> C.CDLL:
     lib.gcn10_cuda_synchronize.argtypes = [_vp]
     lib.gcn10_cuda_last_kernel_ms.argtypes = [_vp, C.POINTER(C.c_float)]
     lib.gcn10_cuda_launch_count.argtypes = [_vp, C.POINTER(C.c_uint64)]
+    lib.gcn10_cuda_last_histograms.argtypes = [_vp, _vp]
     lib.gcn10_cuda_set_option.argtypes = [_vp, C.c_char_p, C.c_long]
     lib.gcn10_cuda_host_alloc.argtypes = [C.c_size_t]
     lib.gcn10_cuda_host_alloc.restype = _vp
@@ -239,6 +241,7 @@ class Context:
         self._check(self.lib.gcn10_cuda_create(device, C.byref(h)))
         self.h = h
         self.device = device
+        self._stats = False
 
     def _check(self, rc):
         if rc != 0:
@@ -262,6 +265,23 @@ class Context:
 
     def set_option(self, key: str, value: int):
         self._check(self.lib.gcn10_cuda_set_option(self.h, key.encode(), int(value)))
+        if key == "stats":
+            self._stats = bool(value)
+
+    def last_histograms(self) -> np.ndarray:
+        """uint64 [18, 256]: per plane, the pixels of each value in the last block a compressed-tile call completed
+        with option "stats" on (gcn10_cuda_last_histograms)."""
+        out = np.zeros((NPLANES, 256), dtype=np.uint64)
+        self._check(self.lib.gcn10_cuda_last_histograms(self.h, out.ctypes.data))
+        return out
+
+    def _histograms(self):
+        """The result dicts' ``histograms``: None while option "stats" is off, or no block has completed (a band
+        that does not end its block)."""
+        if not self._stats:
+            return None
+        out = np.zeros((NPLANES, 256), dtype=np.uint64)
+        return out if self.lib.gcn10_cuda_last_histograms(self.h, out.ctypes.data) == 0 else None
 
     def index_maps(self, w, h, gt, hsx, hsy, soil_gt):
         ci = np.empty(w, dtype=np.int32)
@@ -339,8 +359,9 @@ class Context:
 
     def block_deflate(self, esa, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
         """Compressed-tile call.  Returns dict(tiles={plane: {(tile_row, tile_x): bytes}},
-        overviews={level: {plane: {(tile_row, tile_x): bytes}}} (option "overviews"), bytes=total); with
-        ``on_strip(strip_struct)`` the tiles are not copied."""
+        overviews={level: {plane: {(tile_row, tile_x): bytes}}} (option "overviews"), bytes=total,
+        histograms=uint64 [18, 256] (option "stats", else None)); with ``on_strip(strip_struct)`` the tiles are not
+        copied."""
         esa, esa_pitch = _rows(esa)
         hsg, hsg_pitch = _rows(hsg)
         h, w = esa.shape
@@ -350,7 +371,7 @@ class Context:
         self._check(self.lib.gcn10_cuda_block_deflate(
             self.h, esa.ctypes.data, w, h, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
             _d6(soil_gt), plane_mask, cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
 
     def block_deflate_rows(self, esa_rows, h, row0, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
         """Band form of block_deflate: esa_rows holds rows [row0, row0+len) of a block that is h rows tall; the
@@ -364,7 +385,7 @@ class Context:
         self._check(self.lib.gcn10_cuda_block_deflate_rows(
             self.h, esa_rows.ctypes.data, w, h, row0, nrows, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
             _d6(soil_gt), plane_mask, cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
 
     def inflate_tiles(self, src: "TileSource", w, h, out=None, want_status=False):
         """GPU inflate of a tile source into a host raster uint8 [h, w]."""
@@ -390,7 +411,7 @@ class Context:
         self._check(self.lib.gcn10_cuda_block_tiles_deflate(
             self.h, C.byref(st), w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
             cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
 
     def inflate_parts(self, parts, fill, w, h, want_status=False):
         """GPU inflate of a mosaic ([(TileSource, dst_x, dst_y, w, h), ...]) into a host raster uint8 [h, w]."""
@@ -415,7 +436,7 @@ class Context:
         self._check(self.lib.gcn10_cuda_block_parts_deflate(
             self.h, arr, len(parts), fill, w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
             cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0])
+        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
 
     def tiles_prefetch(self, src: "TileSource", w, h):
         """Start upload + GPU inflate of a block's tiles; the next block_tiles_deflate / inflate_tiles call with the

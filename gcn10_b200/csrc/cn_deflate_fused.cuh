@@ -98,6 +98,7 @@ struct FusedParams {
     unsigned long long *cursor;
     unsigned long long *offsets;    // [nsel][tile_rows][tiles_x]
     uint32_t *sizes;
+    unsigned long long *id_hist;    // [256] option "stats": raster pixels per record id, summed over the tiles (null = off)
 };
 
 // soil class of a raw HYSOGs byte: 0 = code 0, 1..4 = A..D, 5..8 = A/D..D/D (11..14), 9 = anything else
@@ -707,6 +708,10 @@ cn_deflate_fused_kernel(const __grid_constant__ FusedParams p)
             s_perm[at + q] = (uint16_t)(tid | (q << 8));
     }
     __syncthreads();
+    // option "stats": s_cnt is final and stays intact until step 6 reuses it for s_desc.  Id kFusedPad is the padding
+    // beyond the raster, never a raster pixel.
+    if (p.id_hist && tid != kFusedPad && s_cnt[tid])
+        atomicAdd(p.id_hist + tid, (unsigned long long)s_cnt[tid]);
 
     // ---- 3. pass 1: thread t parses items perm[t] and perm[t + 256]; (common bits, 9-bit-literal counts) -> item slot
     const uint32_t n_items = s_nitems;

@@ -12,6 +12,7 @@
 #include "inflate_tiles.cuh"
 #include "cn_deflate_fused.cuh"
 #include "overviews.cuh"
+#include "stats.cuh"
 #include "tile_code.h"
 
 #include <algorithm>
@@ -137,13 +138,23 @@ struct gcn10_ctx {
     float last_inflate_ms = 0.f;
     float last_kernel_ms = 0.f;
     uint64_t launches = 0;
-    // option "overviews": the land cover and index maps of every overview level of the block in hand, filled strip by
-    // strip (and band by band: ov_next is the block row the next band must start at, -1 = no block open)
+    // options "overviews" and "stats" gather the block in hand strip by strip, and band by band: blk_next is the block
+    // row the next band must start at (-1 = no block open), blk_w x blk_h and blk_mask what the block's first band had
+    int blk_w = 0, blk_h = 0, blk_next = -1;
+    unsigned blk_mask = 0;
+    // option "overviews": the land cover and index maps of every overview level of the block in hand
     int overviews = 0;
     DevBuf ov_buf;
     OverviewLevel ov_lv[GCN10_MAX_OVERVIEWS] = {};
     int ov_h[GCN10_MAX_OVERVIEWS] = {};
-    int ov_w = 0, ov_hb = 0, ov_next = -1;
+    // option "stats": the block's pixel counts on the device, [256] per record id (fused path) | [18][256] per plane and
+    // value (two-kernel path); the last completed block's histograms on the host (gcn10_cuda_last_histograms)
+    int stats = 0;
+    DevBuf stats_buf;
+    bool blk_fused = false;             // a strip of the block in hand counted record ids
+    bool stats_ready = false;
+    uint64_t stats_hist[GCN10_NPLANES][256] = {};
+    uint8_t fused_rec[kFusedIds][GCN10_NPLANES] = {};  // value record of every id of the fused tables (fused_mask)
     // asynchronous raw-plane blocks (gcn10_cuda_block_async): frame guard, per-stream end-of-block marks, timer events
     cudaEvent_t frame_ready = nullptr;
     cudaEvent_t tail[kMaxStreams] = {};
@@ -622,9 +633,10 @@ int build_fused_tables(gcn10_ctx *c, unsigned plane_mask, cudaStream_t st)
         c->fused_cls[j] = (uint8_t)q;
     }
     if (c->fused_ok) {
+        memset(c->fused_rec, 0, sizeof(c->fused_rec));
         for (size_t id = 0; id < records.size(); id++) {
             for (int j = 0; j < nsel; j++)
-                val[id * valb + j] = records[id][j];
+                val[id * valb + j] = c->fused_rec[id][j] = records[id][j];
             for (size_t q = 0; q < patterns.size() && !tuned; q++)      // (all literals equally long in the tuned code)
                 if (patterns[q][id])
                     lit9[id] |= 1ull << (21 * q);
@@ -787,6 +799,7 @@ void gcn10_cuda_destroy(gcn10_ctx *c)
     release(c->hsg);
     release(c->fused_tab);
     release(c->ov_buf);
+    release(c->stats_buf);
     for (int i = 0; i < 2; i++) {
         release(c->tslot[i].in_blob);
         release(c->tslot[i].in_table);
@@ -853,7 +866,12 @@ int gcn10_cuda_set_option(gcn10_ctx *c, const char *key, long value)
     else if (!strcmp(key, "ordered") && (value == 0 || value == 1)) c->ordered = (int)value;
     else if (!strcmp(key, "overviews") && value >= 0 && value <= GCN10_MAX_OVERVIEWS) {
         c->overviews = (int)value;
-        c->ov_next = -1;
+        c->blk_next = -1;
+    }
+    else if (!strcmp(key, "stats") && (value == 0 || value == 1)) {
+        c->stats = (int)value;
+        c->blk_next = -1;
+        c->stats_ready = false;
     }
     else if (!strcmp(key, "inflate_probe") && value >= 0 && value <= 2) c->inflate_probe = (int)value;
     else if (!strcmp(key, "tuned_code") && (value == 0 || value == 1)) {
@@ -889,6 +907,16 @@ int gcn10_cuda_launch_count(gcn10_ctx *c, uint64_t *launches)
     if (!c || !launches)
         return fail(GCN10_EINVAL, "NULL argument");
     *launches = c->launches;
+    return GCN10_OK;
+}
+
+int gcn10_cuda_last_histograms(gcn10_ctx *c, uint64_t hist[GCN10_NPLANES][256])
+{
+    if (!c || !hist)
+        return fail(GCN10_EINVAL, "NULL argument");
+    if (!c->stats_ready)
+        return fail(GCN10_EINVAL, "no block has completed with option \"stats\" on since it was set");
+    memcpy(hist, c->stats_hist, sizeof(c->stats_hist));
     return GCN10_OK;
 }
 
@@ -1187,6 +1215,33 @@ int gcn10_cuda_block_deflate(gcn10_ctx *c,
 // device-resident plane (d_esa, valid once `esa_ready` has fired: the compressed-input path).
 static int launch_inflate(gcn10_ctx *c, TileSlot &sl, cudaEvent_t after);
 
+// Option "stats", after the block's last strip has been handed over (so every kernel that counted has finished): the
+// device counts come back once, and the per-id counts of the fused path become plane histograms through the value
+// records of the block's plane mask -- a pixel's value in every plane is a function of its record id.
+static int finish_histograms(gcn10_ctx *c, cudaStream_t st)
+{
+    std::vector<unsigned long long> h((size_t)kFusedIds + (size_t)GCN10_NPLANES * 256);
+    CUDA_TRY(cudaMemcpyAsync(h.data(), c->stats_buf.p, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    for (int p = 0; p < GCN10_NPLANES; p++)
+        for (int v = 0; v < 256; v++)
+            c->stats_hist[p][v] = h[(size_t)kFusedIds + (size_t)p * 256 + v];
+    if (c->blk_fused) {
+        int rc = build_fused_tables(c, c->blk_mask, st);        // (the tables of the block's mask: cached, no work)
+        if (rc)
+            return rc;
+        int plane_ids[GCN10_NPLANES], nsel = 0;
+        for (int p = 0; p < GCN10_NPLANES; p++)
+            if (c->blk_mask & (1u << p))
+                plane_ids[nsel++] = p;
+        for (int id = 0; id < kFusedPad; id++)
+            for (int j = 0; j < nsel && h[id]; j++)
+                c->stats_hist[plane_ids[j]][c->fused_rec[id][j]] += h[id];
+    }
+    c->stats_ready = true;
+    return GCN10_OK;
+}
+
 static int deflate_rows_impl(gcn10_ctx *c,
                              const uint8_t *esa, size_t esa_pitch, const uint8_t *d_esa, size_t d_esa_pitch,
                              cudaEvent_t esa_ready, int w, int h, int row0, int nrows,
@@ -1210,18 +1265,28 @@ static int deflate_rows_impl(gcn10_ctx *c,
         return fail(GCN10_ENOLUT, "gcn10_cuda_set_luts() has not been called");
     if (c->pending_events)
         return fail(GCN10_EINVAL, "asynchronous blocks are pending on this context: gcn10_cuda_wait() for them first");
-    // option "overviews": every band feeds the block's levels, so the bands of a block must come in order and without
-    // gaps; the band that ends the block emits the levels
+    // options "overviews" and "stats": every band feeds the block's levels and histograms, so the bands of a block must
+    // come in order and without gaps (with "stats" also with the same planes); the band that ends the block emits the
+    // levels and completes the histograms
     const int nlev = c->overviews ? gcn10_overview_levels(w, h, c->overviews) : 0;
-    if (nlev && row0 != 0 && (row0 != c->ov_next || w != c->ov_w || h != c->ov_hb)) {
-        rc = fail(GCN10_EINVAL, "overviews: band [%d, +%d) of a %d x %d block does not continue the block's previous band "
-                                "(next row %d); a block starts with row 0", row0, nrows, w, h, c->ov_next);
-        c->ov_next = -1;
+    const bool gather = nlev || c->stats;
+    if (gather && row0 != 0 &&
+        (row0 != c->blk_next || w != c->blk_w || h != c->blk_h || (c->stats && plane_mask != c->blk_mask))) {
+        rc = fail(GCN10_EINVAL, "%s: band [%d, +%d) of a %d x %d block does not continue the block's previous band "
+                                "(next row %d); a block starts with row 0", nlev ? "overviews" : "stats", row0, nrows, w,
+                  h, c->blk_next);
+        c->blk_next = -1;
         return rc;
     }
-    c->ov_next = -1;            // (until this call has succeeded)
-    const bool emit_levels = nlev && row0 + nrows == h;
+    c->blk_next = -1;           // (until this call has succeeded)
+    const bool ends_block = row0 + nrows == h;
+    const bool emit_levels = nlev && ends_block;
     CUDA_TRY(cudaSetDevice(c->device));
+    if (gather && row0 == 0) {
+        c->blk_w = w;
+        c->blk_h = h;
+        c->blk_mask = plane_mask;
+    }
     if (nlev && row0 == 0) {
         size_t off[GCN10_MAX_OVERVIEWS][3], total = 0;
         for (int k = 1; k <= nlev; k++) {
@@ -1244,8 +1309,6 @@ static int deflate_rows_impl(gcn10_ctx *c,
             c->ov_lv[k].col_idx = (int32_t *)((uint8_t *)c->ov_buf.p + off[k][1]);
             c->ov_lv[k].row_idx = (int32_t *)((uint8_t *)c->ov_buf.p + off[k][2]);
         }
-        c->ov_w = w;
-        c->ov_hb = h;
     }
 
     LaunchPlan plans[2];
@@ -1256,6 +1319,17 @@ static int deflate_rows_impl(gcn10_ctx *c,
             plane_ids[nplanes++] = k;
 
     cudaStream_t s0 = c->streams[0];
+    constexpr size_t kStatsWords = (size_t)kFusedIds + (size_t)GCN10_NPLANES * 256;
+    if (c->stats && row0 == 0) {
+        // (done before the strips start: s0 is synchronised below)
+        if ((rc = ensure(c->stats_buf, kStatsWords * sizeof(unsigned long long))))
+            return rc;
+        CUDA_TRY(cudaMemsetAsync(c->stats_buf.p, 0, kStatsWords * sizeof(unsigned long long), s0));
+        c->blk_fused = false;
+        c->stats_ready = false;
+    }
+    unsigned long long *id_hist = c->stats ? (unsigned long long *)c->stats_buf.p : nullptr;
+    unsigned long long *plane_hist = c->stats ? id_hist + kFusedIds : nullptr;
     for (int i = 0; i < nplans; i++)
         if ((rc = upload_lut(c, plans[i].variant_mask, i, s0)))
             return rc;
@@ -1272,6 +1346,8 @@ static int deflate_rows_impl(gcn10_ctx *c,
     CUDA_TRY(cudaStreamSynchronize(s0));
 
     const bool fused = c->fused && !build_fused_tables(c, plane_mask & GCN10_MASK_ALL, s0) && c->fused_ok;
+    if (c->stats && fused)
+        c->blk_fused = true;
 
     // strips of whole tile rows
     const size_t dpitch = round_up((size_t)w, 256);
@@ -1457,6 +1533,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
             fp.cursor = (unsigned long long *)sl.table.p;
             fp.offsets = (unsigned long long *)((uint8_t *)sl.table.p + 16);
             fp.sizes = (uint32_t *)((uint8_t *)sl.table.p + 16 + ntile_slot * sizeof(unsigned long long));
+            fp.id_hist = jb.level == 0 ? id_hist : nullptr;     // (the levels' pixels are level-0 pixels again)
             CUDA_TRY(cudaMemsetAsync(sl.table.p, 0, 16, st));
             if (nplanes <= 9)
                 cn_deflate_fused_kernel<9><<<dim3(stx, tile_rows), kTile, fused_smem_bytes<9>(), st>>>(fp);
@@ -1474,6 +1551,23 @@ static int deflate_rows_impl(gcn10_ctx *c,
                                  hsg_dpitch, hsx, hsy, map, tma_ok, d_out, dpitch, st, jb.col_idx, jb.row_idx);
             if (r2)
                 return r2;
+        }
+        if (plane_hist && jb.level == 0) {
+            PlaneHistParams hp;
+            memset(&hp, 0, sizeof(hp));
+            hp.planes = (const uint8_t *)sl.out.p;
+            hp.plane_stride = dpitch * (size_t)strip_cap;
+            hp.pitch = dpitch;
+            hp.w = sw;
+            hp.rows = rows;
+            memcpy(hp.plane_ids, plane_ids, sizeof(int) * (size_t)nplanes);
+            hp.hist = plane_hist;
+            // (at least one CTA per 2^31 pixels of a plane, for the kernel's 32-bit counts)
+            const long long ctas_wanted = std::max<long long>(4 * c->sm_count / nplanes, ((long long)rows * sw >> 31) + 1);
+            const int ctas = (int)std::max<long long>(1, std::min<long long>(rows, ctas_wanted));
+            plane_histogram_kernel<<<dim3(ctas, nplanes), 256, 0, st>>>(hp);
+            c->launches++;
+            CUDA_TRY(cudaGetLastError());
         }
         TileEncParams ep;
         memset(&ep, 0, sizeof(ep));
@@ -1573,8 +1667,10 @@ static int deflate_rows_impl(gcn10_ctx *c,
             return bail(rc);
     }
     c->last_kernel_ms = kernel_ms;
-    if (nlev && !emit_levels)
-        c->ov_next = row0 + nrows;
+    if (c->stats && ends_block && (rc = finish_histograms(c, s0)))
+        return rc;
+    if (gather && !ends_block)
+        c->blk_next = row0 + nrows;
     return GCN10_OK;
 }
 

@@ -176,6 +176,7 @@ typedef struct {
     int workers_per_gpu;        /* blocks in flight per GPU (each with its own context); <= 0 means 1 */
     const char *out_root;       /* directory that receives cn_rasters_<cond>/ (reference: CWD)     */
     int overviews;              /* --overviews: at most this many overview levels per output (0 = none) */
+    int stats;                  /* --stats: NoData tag and band statistics in every output                   */
 } gh_run_options;
 
 /* Runs a list of blocks on the GPUs of this box: one worker thread (+ one gcn10_ctx) per GPU, block

@@ -37,6 +37,8 @@ static void usage(FILE *fp)
             "  --outdir <dir>	where cn_rasters_<condition>/ are created (default: .)\n"
             "  --overviews		also write reduced-resolution overview levels into every output\n"
             "			(nearest neighbour, halving until a level fits one 256 x 256 tile)\n"
+            "  --stats		tag every output with NoData 255 and its band statistics (minimum, maximum,\n"
+            "			mean, standard deviation, valid percent), counted on the GPU\n"
             "  --help, -h		show this help and exit\n"
             "  --version, -v	print version and exit\n"
             "\n"
@@ -79,6 +81,8 @@ int main(int argc, char **argv)
             opt.out_root = argv[++i];
         else if (!strcmp(argv[i], "--overviews"))
             opt.overviews = GCN10_MAX_OVERVIEWS;
+        else if (!strcmp(argv[i], "--stats"))
+            opt.stats = 1;
     }
     if (!conf) {
         fprintf(stderr, "[rank 0] missing -c/--config <file>; see 'gcn10 -h' for usage.\n");    /* main.c:103-107 */

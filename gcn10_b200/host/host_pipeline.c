@@ -186,8 +186,8 @@ static int open_writers(worker *wk)
             gh_tiffw_set_geokeys(wk->writers[k], &gk);
         pthread_mutex_unlock(&wk->rmu);
         opened++;
-        if (gh_tiffw_set_overviews(wk->writers[k], wk->opt->overviews)) {
-            snprintf(err, sizeof err, "write error 3 on %s (overviews)", wk->paths[k]);
+        if (gh_tiffw_set_overviews(wk->writers[k], wk->opt->overviews) || gh_tiffw_set_stats(wk->writers[k], wk->opt->stats)) {
+            snprintf(err, sizeof err, "write error 3 on %s (overviews / stats)", wk->paths[k]);
             gh_log_message(wk->log, "ERROR", err, 1);
             break;
         }
@@ -315,6 +315,22 @@ static int tile_sink(void *user, const gcn10_tile_strip *st)
     return atomic_load(&wk->encode_failed) ? 1 : 0;
 }
 
+/* option "stats" on the GPU-deflate paths: the histograms the GPU counted while it encoded the block go to the writers,
+ * which turn them into the files' statistics on close (after the block's last band, or its one call).  Runs on the
+ * thread that called the library, which is also the one whose tile sink opened the writers.  (The host-deflate path
+ * needs none: gh_tiffw_write_rows counts the rows it compresses.) */
+static void put_gpu_histograms(worker *wk)
+{
+    if (!wk->opt->stats || !wk->writers_open || atomic_load(&wk->encode_failed))
+        return;
+    uint64_t hist[NPLANES][256];
+    int rc = gcn10_cuda_last_histograms(wk->ctx, hist);
+    for (int k = 0; k < NPLANES && !rc; k++)
+        rc = gh_tiffw_put_histogram(wk->writers[k], hist[k]);
+    if (rc)
+        atomic_store(&wk->encode_failed, 1);
+}
+
 /* returns 0 ok, 1 = land-cover read failed (recoverable tier) */
 static int bands_gpu_deflate(worker *wk, int block_id, const gh_window *we, const uint8_t *hsg, const gh_window *wh,
                              size_t pitch, double *t_read, double *t_gpu)
@@ -358,6 +374,8 @@ static int bands_gpu_deflate(worker *wk, int block_id, const gh_window *we, cons
             break;
     }
     gcn10_cuda_set_option(wk->ctx, "strip_rows", 2048);
+    if (!failed)
+        put_gpu_histograms(wk);
     pthread_mutex_lock(&wk->mu);
     wk->encoder_quit = 1;
     pthread_cond_broadcast(&wk->cv);
@@ -387,6 +405,8 @@ static int block_gpu_tiles(worker *wk, const block_input *in, double *t_gpu)
         snprintf(msg, sizeof msg, "cuda failure on block %d: %s", in->block_id, gcn10_cuda_last_error());
         fatal(wk, msg);
     }
+    if (!rc)
+        put_gpu_histograms(wk);
     return 0;
 }
 
@@ -722,7 +742,7 @@ static void *worker_main(void *arg)
      * writes beat the copy engine's size read-back + copy (measured on 8 x B200: +4..7 %), below that the copy engine wins */
     if (gcn10_cuda_create(wk->device, &wk->ctx) || gcn10_cuda_set_luts(wk->ctx, wk->tables) ||
         gcn10_cuda_set_option(wk->ctx, "ordered", 1) || gcn10_cuda_set_option(wk->ctx, "ship", wk->n_gpus >= 4) ||
-        gcn10_cuda_set_option(wk->ctx, "overviews", wk->opt->overviews)) {
+        gcn10_cuda_set_option(wk->ctx, "overviews", wk->opt->overviews) || gcn10_cuda_set_option(wk->ctx, "stats", wk->opt->stats)) {
         snprintf(msg, sizeof msg, "cannot initialise GPU %d: %s", wk->device, gcn10_cuda_last_error());
         fatal(wk, msg);
     }

@@ -9,14 +9,15 @@
  * compression none (1), LZW (5), DEFLATE (8 / 32946), predictor 1 or 2.
  * Writer: what GDAL's GTiff driver produces for COMPRESS=DEFLATE, TILED=YES with defaults
  * (raster.c:206-207): 256 x 256 tiles, zlib level 6, no predictor, PixelIsArea, EPSG:4326 keys,
- * no NoData tag.  Tiles are compressed in parallel (pthreads) and appended band by band, so a
- * 36000 x 36000 plane never has to be resident in full.
+ * no NoData tag (gh_tiffw_set_stats adds one, and the band statistics GDAL would compute).  Tiles are compressed in
+ * parallel (pthreads) and appended band by band, so a 36000 x 36000 plane never has to be resident in full.
  */
 #define _GNU_SOURCE
 #include "gcn10_host.h"
 #include "host_tiff.h"
 
 #include <errno.h>
+#include <math.h>
 #include <pthread.h>
 #include <stdarg.h>
 #include <stdio.h>
@@ -764,6 +765,8 @@ struct gh_tiffw {
     uint64_t pos;
     int nlev;                   /* overview levels (gh_tiffw_set_overviews) */
     tw_grid g[1 + GCN10_MAX_OVERVIEWS];
+    int stats;                  /* gh_tiffw_set_stats: NoData tag + GDAL_METADATA statistics from hist */
+    uint64_t hist[256];         /* full-resolution pixels per value */
     int level;                  /* zlib level */
     int failed;
 };
@@ -777,6 +780,7 @@ typedef struct {
     int tile_row0;
     unsigned char **comp;
     uLongf *comp_len;
+    uint32_t (*hist)[256];      /* per tile: its pixels per value (NULL: not counted) */
 } write_job;
 
 static void compress_tile(void *arg, int index)
@@ -792,6 +796,13 @@ static void compress_tile(void *arg, int index)
         memset(tile, 0, sizeof tile);       /* edge tiles are padded with zeros */
     for (int r = 0; r < rows; r++)
         memcpy(tile + r * TILE, j->data + (size_t)(y0 + r) * j->pitch + x0, (size_t)cols);
+    if (j->hist) {
+        uint32_t *hc = j->hist[index];
+        memset(hc, 0, sizeof j->hist[index]);
+        for (int r = 0; r < rows; r++)
+            for (int x = 0; x < cols; x++)
+                hc[tile[r * TILE + x]]++;
+    }
     uLongf cap = compressBound(sizeof tile);
     unsigned char *out = malloc(cap);
     if (!out || compress2(out, &cap, tile, sizeof tile, tw->level) != Z_OK) {
@@ -916,21 +927,87 @@ int gh_tiffw_set_overviews(gh_tiffw *tw, int n)
 
 int gh_tiffw_levels(const gh_tiffw *tw) { return tw ? tw->nlev : -1; }
 
-/* Compresses the tile rows [0, rows) held in data (pitch bytes apart) as the next tile rows of grid g. */
-static int append_tile_rows(gh_tiffw *tw, tw_grid *g, const uint8_t *data, size_t pitch, int rows, int threads)
+int gh_tiffw_set_stats(gh_tiffw *tw, int on)
+{
+    if (!tw || tw->failed || (on != 0 && on != 1) || tw->pos != 8 || tw->g[0].next_tile_row)
+        return -1;
+    tw->stats = on;
+    return 0;
+}
+
+int gh_tiffw_put_histogram(gh_tiffw *tw, const uint64_t hist[256])
+{
+    if (!tw || !hist || !tw->stats)
+        return -1;
+    for (int v = 0; v < 256; v++)
+        tw->hist[v] += hist[v];
+    return 0;
+}
+
+/* The band statistics GDAL computes for a file whose NoData value is 255, as GDAL stores them in GDAL_METADATA: only
+ * pixels other than 255 count, the standard deviation is the population one, VALID_PERCENT = 100 * valid / pixels.  A
+ * plane without a valid pixel gets VALID_PERCENT 0 and nothing else.  The sums are exact integers: N * sum(v^2) needs
+ * more than 64 bits at 36001 x 36001.  Returns the length of the NUL-terminated text, or -1 if cap is too small. */
+static int stats_metadata(const uint64_t hist[256], uint64_t pixels, char *out, size_t cap)
+{
+    uint64_t valid = 0, sum = 0;
+    unsigned __int128 sum2 = 0;
+    int lo = -1, hi = -1;
+    for (int v = 0; v < GCN10_NODATA; v++) {
+        if (!hist[v])
+            continue;
+        if (lo < 0)
+            lo = v;
+        hi = v;
+        valid += hist[v];
+        sum += hist[v] * (uint64_t)v;
+        sum2 += (unsigned __int128)hist[v] * (unsigned)(v * v);
+    }
+    const double pct = pixels ? 100.0 * (double)valid / (double)pixels : 0.0;
+    int n;
+    if (!valid) {
+        n = snprintf(out, cap, "<GDALMetadata>\n  <Item name=\"STATISTICS_VALID_PERCENT\" sample=\"0\">%.17g</Item>\n"
+                               "</GDALMetadata>\n", pct);
+    }
+    else {
+        const unsigned __int128 var_n2 = (unsigned __int128)valid * sum2 - (unsigned __int128)sum * sum;   /* N^2 var */
+        const double mean = (double)sum / (double)valid, sd = sqrt((double)var_n2) / (double)valid;
+        n = snprintf(out, cap,
+                     "<GDALMetadata>\n"
+                     "  <Item name=\"STATISTICS_MAXIMUM\" sample=\"0\">%.17g</Item>\n"
+                     "  <Item name=\"STATISTICS_MEAN\" sample=\"0\">%.17g</Item>\n"
+                     "  <Item name=\"STATISTICS_MINIMUM\" sample=\"0\">%.17g</Item>\n"
+                     "  <Item name=\"STATISTICS_STDDEV\" sample=\"0\">%.17g</Item>\n"
+                     "  <Item name=\"STATISTICS_VALID_PERCENT\" sample=\"0\">%.17g</Item>\n"
+                     "</GDALMetadata>\n",
+                     (double)hi, mean, (double)lo, sd, pct);
+    }
+    return n < 0 || (size_t)n >= cap ? -1 : n;
+}
+
+/* Compresses the tile rows [0, rows) held in data (pitch bytes apart) as the next tile rows of grid g; with `count`
+ * their pixels are added to the file's histogram. */
+static int append_tile_rows(gh_tiffw *tw, tw_grid *g, const uint8_t *data, size_t pitch, int rows, int threads, int count)
 {
     int tile_rows = (rows + TILE - 1) / TILE;
     int n = tile_rows * g->tiles_x;
-    write_job j = { tw, g, data, pitch, rows, g->next_tile_row, NULL, NULL };
+    write_job j = { tw, g, data, pitch, rows, g->next_tile_row, NULL, NULL, NULL };
     j.comp = calloc((size_t)n, sizeof(unsigned char *));
     j.comp_len = calloc((size_t)n, sizeof(uLongf));
-    if (!j.comp || !j.comp_len) {
+    if (count)
+        j.hist = malloc((size_t)n * sizeof *j.hist);
+    if (!j.comp || !j.comp_len || (count && !j.hist)) {
         free(j.comp);
         free(j.comp_len);
+        free(j.hist);
         tw->failed = 1;
         return -1;
     }
     parallel_for(n, threads, compress_tile, &j);
+    for (int i = 0; count && i < n; i++)
+        for (int v = 0; v < 256; v++)
+            tw->hist[v] += j.hist[i][v];
+    free(j.hist);
     for (int i = 0; i < n; i++) {
         size_t ti = (size_t)(g->next_tile_row + i / g->tiles_x) * (size_t)g->tiles_x + (size_t)(i % g->tiles_x);
         if (!tw->failed && j.comp[i]) {
@@ -954,7 +1031,7 @@ int gh_tiffw_write_rows(gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0,
     if (tw->failed || y0 != g0->next_tile_row * TILE || y0 + nrows > g0->h ||
         (nrows % TILE != 0 && y0 + nrows != g0->h))
         return -1;
-    if (append_tile_rows(tw, g0, data, pitch, nrows, threads))
+    if (append_tile_rows(tw, g0, data, pitch, nrows, threads, tw->stats))
         return -1;
     /* the overview levels, sampled from this band by the rule of gcn10_overview_src: each level keeps one tile row
      * and appends it compressed when it is full, so the levels cost a few MB, not a third of the raster */
@@ -975,7 +1052,7 @@ int gh_tiffw_write_rows(gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0,
             for (int x = 0; x < g->w; x++)
                 dst[x] = row[gcn10_overview_src(x, k, g0->w)];
             if (i % TILE == TILE - 1 || i == g->h - 1) {
-                if (append_tile_rows(tw, g, g->band, (size_t)g->w, i % TILE + 1, threads))
+                if (append_tile_rows(tw, g, g->band, (size_t)g->w, i % TILE + 1, threads, 0))
                     return -1;
             }
         }
@@ -1072,6 +1149,19 @@ int gh_tiffw_close(gh_tiffw *tw)
     int complete = !tw->failed;
     for (int k = 0; k <= tw->nlev; k++)
         complete = complete && tw->g[k].next_tile_row == tw->g[k].tiles_y;
+    /* statistics: GDAL_METADATA (42112) in IFD0 and GDAL_NODATA (42113) "255" in every IFD; a histogram that does not
+     * count every pixel exactly once (never handed over, or not this raster's) would publish wrong numbers */
+    char meta[1024];
+    size_t nmeta = 0;
+    if (complete && tw->stats) {
+        uint64_t total = 0;
+        for (int v = 0; v < 256; v++)
+            total += tw->hist[v];
+        const int n = total == (uint64_t)g0->w * (uint64_t)g0->h ? stats_metadata(tw->hist, total, meta, sizeof meta) : -1;
+        complete = n > 0;
+        nmeta = n > 0 ? (size_t)n + 1 : 0;
+    }
+    const uint32_t nodata_ascii = '2' | '5' << 8 | '5' << 16;     /* "255\0", held in the entry itself */
     if (complete) {
         /* trailing data area: tile offsets, tile byte counts, pixel scale, tiepoint, geo keys, ascii */
         static const uint16_t geokeys[] = {
@@ -1090,16 +1180,16 @@ int gh_tiffw_close(gh_tiffw *tw)
         if (tw->pos & 1) { fputc(0, tw->fp); tw->pos++; }
         uint64_t off_offsets = tw->pos, off_counts = off_offsets + 4 * nt, off_scale = off_counts + 4 * nt;
         uint64_t off_tie = off_scale + 24, off_keys = off_tie + 48, off_dbl = off_keys + 2 * nkeys;
-        uint64_t off_ascii = off_dbl + 8 * ndbl;
-        uint64_t off_ifd = (off_ascii + nascii + 1) & ~(uint64_t)1;
-        const int nent = 14 + 1 + (ndbl ? 1 : 0) + (nascii ? 1 : 0);
+        uint64_t off_ascii = off_dbl + 8 * ndbl, off_meta = (off_ascii + nascii + 1) & ~(uint64_t)1;     /* word aligned */
+        uint64_t off_ifd = (off_meta + nmeta + 1) & ~(uint64_t)1;
+        const int nent = 14 + 1 + (ndbl ? 1 : 0) + (nascii ? 1 : 0) + (tw->stats ? 2 : 0);
         /* behind IFD0, per overview level: its tile offsets, byte counts and IFD (reduced-resolution image, no geo tags:
          * readers derive the level's georeferencing from the size ratio) */
-        enum { LEVEL_ENTRIES = 13 };
+        const int level_entries = 13 + (tw->stats ? 1 : 0);
         uint64_t off_lv[1 + GCN10_MAX_OVERVIEWS], end = off_ifd + 2 + (uint64_t)nent * 12 + 4;
         for (int k = 1; k <= tw->nlev; k++) {
             off_lv[k] = end;            /* offsets | counts | IFD */
-            end += 8 * (uint64_t)tw->g[k].tiles_x * (uint64_t)tw->g[k].tiles_y + 2 + LEVEL_ENTRIES * 12 + 4;
+            end += 8 * (uint64_t)tw->g[k].tiles_x * (uint64_t)tw->g[k].tiles_y + 2 + (uint64_t)level_entries * 12 + 4;
         }
         size_t tail = (size_t)(end - tw->pos);
         unsigned char *buf = calloc(1, tail), *p = buf;
@@ -1113,6 +1203,8 @@ int gh_tiffw_close(gh_tiffw *tw)
             for (size_t i = 0; i < ndbl; i++) put_f64(&p, tw->geo_doubles[i]);
             if (nascii)
                 memcpy(p, ascii, nascii);
+            if (nmeta)
+                memcpy(buf + (off_meta - tw->pos), meta, nmeta);
             p = buf + (off_ifd - tw->pos);
             put16(&p, (uint16_t)nent);
             put_entry(&p, 256, 4, 1, (uint32_t)g0->w);
@@ -1134,6 +1226,10 @@ int gh_tiffw_close(gh_tiffw *tw)
                 put_entry(&p, 34736, 12, (uint32_t)ndbl, (uint32_t)off_dbl);
             if (nascii)
                 put_entry(&p, 34737, 2, (uint32_t)nascii, (uint32_t)off_ascii);
+            if (tw->stats) {
+                put_entry(&p, 42112, 2, (uint32_t)nmeta, (uint32_t)off_meta);
+                put_entry(&p, 42113, 2, 4, nodata_ascii);
+            }
             put32(&p, tw->nlev ? (uint32_t)(off_lv[1] + 8 * (uint64_t)tw->g[1].tiles_x * (uint64_t)tw->g[1].tiles_y) : 0);
             for (int k = 1; k <= tw->nlev; k++) {
                 const tw_grid *g = &tw->g[k];
@@ -1141,7 +1237,7 @@ int gh_tiffw_close(gh_tiffw *tw)
                 p = buf + (off_lv[k] - tw->pos);
                 for (size_t i = 0; i < n; i++) put32(&p, g->offsets[i]);
                 for (size_t i = 0; i < n; i++) put32(&p, g->counts[i]);
-                put16(&p, LEVEL_ENTRIES);
+                put16(&p, (uint16_t)level_entries);
                 put_entry(&p, 254, 4, 1, 1);            /* NewSubfileType = reduced-resolution version */
                 put_entry(&p, 256, 4, 1, (uint32_t)g->w);
                 put_entry(&p, 257, 4, 1, (uint32_t)g->h);
@@ -1155,6 +1251,8 @@ int gh_tiffw_close(gh_tiffw *tw)
                 put_entry(&p, 324, 4, (uint32_t)n, n == 1 ? g->offsets[0] : (uint32_t)off_lv[k]);
                 put_entry(&p, 325, 4, (uint32_t)n, n == 1 ? g->counts[0] : (uint32_t)(off_lv[k] + 4 * n));
                 put_entry(&p, 339, 3, 1, 1);
+                if (tw->stats)
+                    put_entry(&p, 42113, 2, 4, nodata_ascii);
                 put32(&p, k < tw->nlev ? (uint32_t)(off_lv[k + 1] + 8 * (uint64_t)tw->g[k + 1].tiles_x * (uint64_t)tw->g[k + 1].tiles_y)
                                        : 0);
             }

@@ -25,6 +25,13 @@ int gh_tiffw_set_geokeys(gh_tiffw *tw, const gh_geokeys *gk);
  * every tile of every level has been written. */
 int gh_tiffw_set_overviews(gh_tiffw *tw, int n);
 int gh_tiffw_levels(const gh_tiffw *tw);
+/* Statistics (on = 1): the file gets GDAL_NODATA "255" (tag 42113) in every IFD and, in IFD0, GDAL_METADATA (42112)
+ * with the band statistics GDAL computes for that NoData value (STATISTICS_MINIMUM / MAXIMUM / MEAN / STDDEV /
+ * VALID_PERCENT of sample 0), taken from the full-resolution histogram: gh_tiffw_write_rows counts the rows it
+ * compresses, and tiles appended already compressed need gh_tiffw_put_histogram (which adds to the counts).  Call after
+ * open, before the first data.  gh_tiffw_close fails (and removes the file) unless the histogram counts w * h pixels. */
+int gh_tiffw_set_stats(gh_tiffw *tw, int on);
+int gh_tiffw_put_histogram(gh_tiffw *tw, const uint64_t hist[256]);
 /* Appends rows [y0, y0+nrows): y0 must continue where the previous call stopped and be a multiple
  * of 256; nrows must be a multiple of 256 except for the last band of the raster.  With overviews, the levels are
  * sampled from the same rows (gcn10_overview_src) and compressed here too, a level's tile row as soon as it is full. */

@@ -75,6 +75,8 @@ def load(path: str | None = None) -> C.CDLL:
     L.gh_tiffw_write_rows.argtypes = [_vp, _vp, C.c_size_t, C.c_int, C.c_int, C.c_int]
     L.gh_tiffw_set_overviews.argtypes = [_vp, C.c_int]
     L.gh_tiffw_levels.argtypes = [_vp]
+    L.gh_tiffw_set_stats.argtypes = [_vp, C.c_int]
+    L.gh_tiffw_put_histogram.argtypes = [_vp, C.POINTER(C.c_uint64)]
     L.gh_tiffw_put_level_tile_rows.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, C.POINTER(C.c_uint64),
                                                C.POINTER(C.c_uint32)]
     L.gh_tiffw_close.argtypes = [_vp]
@@ -319,9 +321,11 @@ class Raster:
 
 class TiffWriter:
     """Incremental tiled-DEFLATE GeoTIFF writer (gh_tiffw_*): raw row bands or pre-compressed tile rows.
-    ``overviews=n`` adds up to n overview levels (gh_tiffw_set_overviews); ``levels`` is how many the file gets."""
+    ``overviews=n`` adds up to n overview levels (gh_tiffw_set_overviews); ``levels`` is how many the file gets.
+    ``stats=True`` adds the NoData tag and the band statistics (gh_tiffw_set_stats): write_rows counts the pixels itself,
+    tiles put already compressed need ``put_histogram``."""
 
-    def __init__(self, path: str, w: int, h: int, gt, overviews: int = 0):
+    def __init__(self, path: str, w: int, h: int, gt, overviews: int = 0, stats: bool = False):
         self.L = load()
         h_ = _vp()
         e = _err()
@@ -334,7 +338,17 @@ class TiffWriter:
             self.L.gh_tiffw_abort(h_)
             self.h = None
             raise HostError(-1, f"gh_tiffw_set_overviews({overviews}) failed")
+        if stats and self.L.gh_tiffw_set_stats(h_, 1):
+            self.L.gh_tiffw_abort(h_)
+            self.h = None
+            raise HostError(-1, "gh_tiffw_set_stats(1) failed")
         self.levels = self.L.gh_tiffw_levels(h_)
+
+    def put_histogram(self, hist):
+        """hist: 256 pixel counts of the full-resolution raster (added to what the writer has counted)."""
+        a = np.ascontiguousarray(hist, dtype=np.uint64)
+        assert a.shape == (256,), a.shape
+        return self.L.gh_tiffw_put_histogram(self.h, a.ctypes.data_as(C.POINTER(C.c_uint64)))
 
     def put_tile_row(self, tile_row: int, streams, level: int = 0):
         """streams: the zlib streams (bytes) of one tile row of ``level`` (0 = full resolution)."""

@@ -219,10 +219,10 @@ int gcn10_cuda_block_deflate(gcn10_ctx *ctx,
 
 /* Band form of gcn10_cuda_block_deflate (see gcn10_cuda_block_rows): esa points at block row `row0`,
  * which must be a multiple of 256; nrows must be a multiple of 256 unless the band ends the block.
- * With option "overviews" the bands of a block feed its levels, which stay on the context between calls: a band with
- * row0 == 0 starts a block, every later band must start where the previous one ended (same w and h; anything else is
- * refused with GCN10_EINVAL), and the band that ends the block (row0 + nrows == h) delivers the levels after its own
- * strips. */
+ * With option "overviews" or "stats" the bands of a block feed its levels and histograms, which stay on the context
+ * between calls: a band with row0 == 0 starts a block, every later band must start where the previous one ended (same
+ * w and h, and with "stats" the same plane mask; anything else is refused with GCN10_EINVAL), and the band that ends
+ * the block (row0 + nrows == h) delivers the levels after its own strips and completes the histograms. */
 int gcn10_cuda_block_deflate_rows(gcn10_ctx *ctx,
                                   const uint8_t *esa, int w, int h, int row0, int nrows, size_t esa_pitch,
                                   const double gt[6],
@@ -342,6 +342,15 @@ int gcn10_cuda_last_kernel_ms(gcn10_ctx *ctx, float *ms);
 /* Number of kernels this context has launched since it was created. */
 int gcn10_cuda_launch_count(gcn10_ctx *ctx, uint64_t *launches);
 
+/* Per-plane histograms of the full-resolution pixels of the last block that a compressed-tile call completed with
+ * option "stats" on: hist[p][v] = pixels of plane p with value v (255 = nodata).  Rows of planes outside the mask are
+ * zero; every selected row sums to w * h.  GCN10_EINVAL if no such block has completed since the option was set
+ * (a band call completes its block with the band that ends it; a call that starts a block clears the last one).
+ * The GPU counts them while it encodes (gcn10_cuda_block_deflate, _block_deflate_rows, _block_tiles_deflate and
+ * _block_parts_deflate; the raw-plane calls ignore the option, their callers hold the planes): overview levels are
+ * not counted, and the tiles are the same bytes as without the option. */
+int gcn10_cuda_last_histograms(gcn10_ctx *ctx, uint64_t hist[GCN10_NPLANES][256]);
+
 /* Tunables: "strip_rows" (rows per pipelined strip in the host-buffer calls), "streams" (1..8), "rows_per_cta"
  * (0 = automatic), "tma" (0 = always use the gather fallback for HSG staging), "fused" (0 = compressed-tile
  * calls run the Curve Number kernel and the per-plane tile encoder instead of the fused kernel), "ship" (1 = a strip's
@@ -351,7 +360,8 @@ int gcn10_cuda_launch_count(gcn10_ctx *ctx, uint64_t *launches);
  * "tuned_code" (0 = tile streams use RFC 1951's fixed Huffman code instead
  * of the tuned one), "defer_inflate" (0 = the inflate kernel of a prefetched block starts at once instead of behind
  * the last strip of the block in hand), "overviews" (0..16, default 0: the compressed-tile calls also deliver up to that
- * many overview levels of the block, see gcn10_cuda_block_deflate), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
+ * many overview levels of the block, see gcn10_cuda_block_deflate), "stats" (0 / 1, default 0: the compressed-tile calls
+ * also count every selected plane's histogram, see gcn10_cuda_last_histograms), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
  * kernel's writer off; results are then invalid). */
 int gcn10_cuda_set_option(gcn10_ctx *ctx, const char *key, long value);
 

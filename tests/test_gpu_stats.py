@@ -1,0 +1,326 @@
+"""GPU tests of option "stats": the compressed-tile calls count the histogram of every selected plane while they encode
+(gcn10_cuda_last_histograms).  Every histogram must equal np.bincount of the oracle's planes, and the tiles must be
+byte-identical to the same call without the option.  The program's --stats outputs must carry the tags of
+tests/stats_rule.py applied to their decoded planes."""
+import os
+import shutil
+import subprocess
+
+import numpy as np
+import pytest
+
+from gcn10_b200 import capi, hostlib, synth
+from tests import overview_rule as R
+from tests import stats_rule as S
+from tests.cases import SMALL_CASES, make_block
+from tests.test_gpu_overviews import _parts, world  # noqa: F401  (world: the program's input fixture)
+
+pytestmark = pytest.mark.gpu
+
+MASKS = [capi.MASK_ALL, capi.MASK_DRAINED, 1 << 13]
+# (mask, fused, ordered, ship): all 24 combinations, dealt out over the cases x calls below
+CONFIGS = [(m, f, o, s) for m in MASKS for f in (1, 0) for o in (0, 1) for s in (0, 1)]
+CALLS = ["deflate", "rows", "tiles", "parts"]
+
+
+@pytest.fixture(scope="module")
+def ctx(tables):
+    with capi.Context(0) as c:
+        c.set_luts(tables)
+        yield c
+
+
+def _set(ctx, stats=0, overviews=0, fused=1, ordered=0, ship=0, strip_rows=2048):
+    for k, v in dict(stats=stats, overviews=overviews, fused=fused, ordered=ordered, ship=ship,
+                     strip_rows=strip_rows).items():
+        ctx.set_option(k, v)
+
+
+def _want(planes, mask):
+    """[18, 256] bincount of the selected planes of an oracle block, zero rows elsewhere."""
+    out = np.zeros((18, 256), np.uint64)
+    for p in range(18):
+        if mask >> p & 1:
+            out[p] = np.bincount(planes[p].ravel(), minlength=256)
+    return out
+
+
+def _run(ctx, call, b, mask, band=768):
+    esa = b["esa"]
+    h, w = esa.shape
+    if call == "deflate":
+        return ctx.block_deflate(esa, b["gt"], b["hsg"], b["soil_gt"], mask)
+    if call == "rows":
+        res = dict(tiles={}, histograms=None)
+        for y0 in range(0, h, band):
+            r = ctx.block_deflate_rows(esa[y0:y0 + band], h, y0, b["gt"], b["hsg"], b["soil_gt"], mask)
+            for k, d in r["tiles"].items():
+                res["tiles"].setdefault(k, {}).update(d)
+            assert r["histograms"] is None or y0 + band >= h, "histograms before the band that ends the block"
+            res["histograms"] = r["histograms"]
+        return res
+    if call == "tiles":
+        src = capi.TileSource.from_raster(esa, 256, 256)
+        return ctx.block_tiles_deflate(src, w, h, b["gt"], b["hsg"], b["soil_gt"], mask)
+    return ctx.block_parts_deflate(_parts(esa), 0, w, h, b["gt"], b["hsg"], b["soil_gt"], mask)
+
+
+@pytest.mark.parametrize("call", CALLS)
+@pytest.mark.parametrize("name,kw", SMALL_CASES, ids=[c[0] for c in SMALL_CASES])
+def test_histograms_equal_oracle(name, kw, call, ctx, port, tables):
+    i = [c[0] for c in SMALL_CASES].index(name) * len(CALLS) + CALLS.index(call)
+    mask, fused, ordered, ship = CONFIGS[i % len(CONFIGS)]
+    b = make_block(**kw)
+    want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
+    _set(ctx, 0, 0, fused, ordered, ship)
+    base = _run(ctx, call, b, mask)
+    assert base["histograms"] is None
+    _set(ctx, 1, 0, fused, ordered, ship)
+    try:
+        res = _run(ctx, call, b, mask)
+        assert np.array_equal(ctx.last_histograms(), res["histograms"])
+    finally:
+        _set(ctx)
+    assert res["tiles"] == base["tiles"]            # the same bytes as without the option
+    assert np.array_equal(res["histograms"], _want(want, mask))
+
+
+@pytest.mark.parametrize("fused", [1, 0], ids=["fused_on", "fused_off"])
+def test_random_tables_two_kernel_path(fused, ctx, port, tables):
+    """Random tables give more than 255 distinct value records: the two-kernel path runs with option fused on too."""
+    rng = np.random.default_rng(1)
+    t = rng.integers(0, 256, size=tables.shape).astype(np.int32)
+    b = make_block(w=1040, h=700, profile="random", seed=9)
+    b["esa"] = rng.integers(0, 256, size=b["esa"].shape, dtype=np.uint8)
+    b["hsg"] = rng.integers(0, 15, size=b["hsg"].shape, dtype=np.uint8)
+    want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], t)
+    try:
+        ctx.set_luts(t)
+        for mask in (capi.MASK_ALL, capi.MASK_UNDRAINED):
+            _set(ctx, 1, fused=fused, strip_rows=256)
+            n0 = ctx.launch_count()
+            res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
+            n_on = ctx.launch_count() - n0
+            _set(ctx, 0, fused=fused, strip_rows=256)
+            n0 = ctx.launch_count()
+            ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
+            assert n_on - (ctx.launch_count() - n0) == 3        # one histogram kernel per strip (3 of 256 rows)
+            assert np.array_equal(res["histograms"], _want(want, mask)), mask
+    finally:
+        _set(ctx)
+        ctx.set_luts(tables)
+
+
+def test_with_overviews_level_zero_only(ctx, port, tables):
+    b = make_block(w=2100, h=1900, seed=41)
+    want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
+    for fused in (1, 0):
+        _set(ctx, 1, 16, fused)
+        try:
+            res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])
+        finally:
+            _set(ctx)
+        assert sorted(res["overviews"]) == list(range(1, R.levels(2100, 1900) + 1))
+        assert np.array_equal(res["histograms"], _want(want, capi.MASK_ALL)), fused
+        assert all(int(res["histograms"][p].sum()) == 2100 * 1900 for p in range(18))
+
+
+def test_bands_order_and_restart(ctx, port, tables):
+    b = make_block(w=700, h=1100, seed=23)
+    esa, h = b["esa"], 1100
+    want = port.block_rows(esa, b["gt"], b["hsg"], b["soil_gt"], tables)
+    _set(ctx, 1)
+    try:
+        with pytest.raises(capi.Gcn10Error) as e:       # no block open
+            ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])
+        assert e.value.code == -1
+        with pytest.raises(capi.Gcn10Error):            # nothing completed since the option was set
+            ctx.last_histograms()
+        ctx.block_deflate_rows(esa[:256], h, 0, b["gt"], b["hsg"], b["soil_gt"])
+        with pytest.raises(capi.Gcn10Error):            # a gap
+            ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])
+        ctx.block_deflate_rows(esa[:256], h, 0, b["gt"], b["hsg"], b["soil_gt"])
+        with pytest.raises(capi.Gcn10Error):            # another plane mask inside the block
+            ctx.block_deflate_rows(esa[256:512], h, 256, b["gt"], b["hsg"], b["soil_gt"], capi.MASK_DRAINED)
+        # a block that starts over at row 0 counts from zero: the rows of the abandoned bands are not in it
+        ctx.block_deflate_rows(esa[:512], h, 0, b["gt"], b["hsg"], b["soil_gt"])
+        r1 = ctx.block_deflate_rows(esa[:512], h, 0, b["gt"], b["hsg"], b["soil_gt"])
+        assert r1["histograms"] is None
+        r2 = ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])
+        assert np.array_equal(r2["histograms"], _want(want, capi.MASK_ALL))
+        # the whole block again in one call: the same counts, not twice them
+        r3 = ctx.block_deflate(esa, b["gt"], b["hsg"], b["soil_gt"])
+        assert np.array_equal(r3["histograms"], r2["histograms"])
+    finally:
+        _set(ctx)
+    ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])     # free again without the option
+
+
+def test_launch_counts(ctx, tables):
+    b = make_block(w=1300, h=1100, seed=22)
+    args = (b["esa"], b["gt"], b["hsg"], b["soil_gt"])
+    with capi.Context(0) as fresh:
+        fresh.set_luts(tables)
+        n0 = fresh.launch_count()
+        fresh.block_deflate(*args)
+        base = fresh.launch_count() - n0
+
+    def count(stats, fused):
+        _set(ctx, stats, fused=fused, strip_rows=512)
+        n0 = ctx.launch_count()
+        ctx.block_deflate(*args)
+        return ctx.launch_count() - n0
+
+    try:
+        _set(ctx, 1)
+        _set(ctx, 0)                                    # set, then back off: exactly the launches of a fresh context
+        n0 = ctx.launch_count()
+        ctx.block_deflate(*args)
+        assert ctx.launch_count() - n0 == base
+        assert count(1, 1) == count(0, 1)               # fused: no launch of its own
+        assert count(1, 0) == count(0, 0) + 3           # two-kernel path: one per strip (1100 rows in 512-row strips)
+    finally:
+        _set(ctx)
+
+
+def test_prefetch_and_ship_paths(ctx, port, tables):
+    blocks = [make_block(w=2100, h=1900, seed=24 + i) for i in range(3)]
+    srcs = [capi.TileSource.from_raster(b["esa"], 256, 256) for b in blocks]
+    for ordered, ship in ((0, 0), (1, 1)):
+        _set(ctx, 1, ordered=ordered, ship=ship)
+        try:
+            ctx.tiles_prefetch(srcs[0], 2100, 1900)
+            results = []
+            for i, b in enumerate(blocks):
+                if i + 1 < len(blocks):
+                    ctx.tiles_prefetch(srcs[i + 1], 2100, 1900)
+                results.append(ctx.block_tiles_deflate(srcs[i], 2100, 1900, b["gt"], b["hsg"], b["soil_gt"]))
+        finally:
+            _set(ctx)
+        for b, res in zip(blocks, results):
+            want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
+            assert np.array_equal(res["histograms"], _want(want, capi.MASK_ALL))
+
+
+def _oracle_histograms(port, tables, esa, gt, hsg, sgt, n):
+    """The oracle's planes of an n x n block in 256-row bands, counted (with torch on the GPU: numpy's bincount would
+    take minutes for 23 G pixels)."""
+    import torch
+    hist = torch.zeros((18, 256), dtype=torch.int64, device="cuda")
+    for y in range(0, n, 256):
+        y1 = min(n, y + 256)
+        planes = torch.from_numpy(port.block_rows(esa[y:y1], gt, hsg, sgt, tables, y0=y, y1=y1, h=n)).cuda()
+        for p in range(18):
+            hist[p] += torch.bincount(planes[p].flatten(), minlength=256)
+    return hist.cpu().numpy().astype(np.uint64)
+
+
+@pytest.mark.parametrize("shape", ["worldcover_36000", "vrt_36001_four_parts"])
+def test_full_size_block(shape, ctx, port, tables):
+    if shape == "worldcover_36000":
+        n, px, lon0, lat0 = 36000, 1.0 / 12000.0, -114.0, 42.0
+    else:
+        n, px, lon0, lat0 = 36001, 8.3333333333330430e-05, 33.0, -3.0
+    gt, sgt, hsx, hsy = synth.block_geometry(lon0, lat0, n, n, px, 1.0 / 480.0, (0.0011, 0.0004), 2)
+    esa = synth.esa_tile(n, n, 77, patch=64)
+    hsg = synth.hsg_tile(hsx, hsy, 78, patch=3)
+    _set(ctx, 1)
+    try:
+        if shape == "worldcover_36000":
+            res = ctx.block_tiles_deflate(capi.TileSource.from_raster(esa, 1024, 1024), n, n, gt, hsg, sgt,
+                                          on_strip=lambda st: 0)
+        else:                                           # the real VRT's four files around a block corner
+            c = 35000
+            parts = [(capi.TileSource.from_raster(np.ascontiguousarray(esa[y:y + hh, x:x + ww]), 1024, 1024), x, y,
+                      ww, hh) for (y, hh) in ((0, c), (c, n - c)) for (x, ww) in ((0, c), (c, n - c))]
+            res = ctx.block_parts_deflate(parts, 0, n, n, gt, hsg, sgt, on_strip=lambda st: 0)
+    finally:
+        _set(ctx)
+    got = res["histograms"]
+    assert all(int(got[p].sum()) == n * n for p in range(18))
+    assert np.array_equal(got, _oracle_histograms(port, tables, esa, gt, hsg, sgt, n))
+
+
+# ---- the program, file to file ---------------------------------------------------------------------------------
+
+def _program(world, config, outdir, stats, host_deflate=False, host_inflate=False):
+    env = dict(os.environ, GCN10_HOST_DEFLATE="1" if host_deflate else "0",
+               GCN10_HOST_INFLATE="1" if host_inflate else "0")
+    root = world["root"]
+    shutil.rmtree(outdir, ignore_errors=True)
+    os.makedirs(outdir)
+    r = subprocess.run([hostlib.EXE_PATH, "-c", str(root / config), "-l", str(root / "blocks.txt"), "--gpus", "1",
+                        "--io-threads", "4", "-o", "--outdir", str(outdir)] + (["--stats"] if stats else []),
+                       cwd=str(root), capture_output=True, text=True, timeout=300, env=env)
+    assert r.returncode == 0, r.stderr
+
+
+def _tags(path):
+    from PIL import Image
+    with Image.open(path) as im:
+        return np.array(im), im.tag_v2.get(42113), im.tag_v2.get(42112)
+
+
+@pytest.mark.parametrize("config", ["config.txt", "config_vrt.txt"], ids=["geotiff", "vrt_mosaic"])
+def test_program_stats(world, reference, config, tmp_path):
+    root = world["root"]
+    modes = dict(gpu=(False, False), host_inflate=(False, True), host_deflate=(True, True))
+    for mode, (hd, hi) in modes.items():
+        _program(world, config, tmp_path / mode, True, hd, hi)
+    _program(world, config, tmp_path / "plain", False)
+    for bid, x0, y0, x1, y1 in world["blocks"]:
+        want = reference.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
+                                   str(root / "lookups"), block_id=bid)
+        for k, rel in enumerate(want["paths"]):
+            tags = {m: _tags(str(tmp_path / m / rel)) for m in modes}
+            img, nodata, meta = tags["gpu"]
+            assert np.array_equal(img, want["planes"][k]), rel
+            assert nodata == "255", rel
+            assert S.close(S.parse(meta), S.of_plane(img)), rel
+            for m in modes:                             # the three paths write the same tags
+                assert tags[m][1:] == tags["gpu"][1:], (rel, m)
+                assert np.array_equal(tags[m][0], img), (rel, m)
+            img, nodata, meta = _tags(str(tmp_path / "plain" / rel))
+            assert nodata is None and meta is None, rel
+            assert np.array_equal(img, want["planes"][k]), rel
+
+
+@pytest.fixture(scope="module")
+def tall_world(tmp_path_factory):
+    """A block of 4500 rows: three 2048-row bands on the host-decode and host-deflate paths of the program."""
+    from tests import fixtures, lookups
+    root = tmp_path_factory.mktemp("gcn10_stats_tall")
+    px, hpx = 1.0 / 12000.0, 1.0 / 480.0
+    esa_t = (-114.0, px, 0.0, 42.0, 0.0, -px)
+    esa = synth.esa_tile(1200, 4800, 61, patch=96)
+    esa[::37, ::11] = 255                               # some nodata land cover too
+    hsg_t = (-114.0 - 1.3 * hpx, hpx, 0.0, 42.0 + 2.6 * hpx, 0.0, -hpx)
+    hsg = synth.hsg_tile(60, 200, 62, "coastal", patch=3)
+    hostlib.tiff_write(str(root / "esa.tif"), esa, esa_t)
+    hostlib.tiff_write(str(root / "hsg.tif"), hsg, hsg_t)
+    blocks = [(31, -114.0 + 100 * px, 42.0 - 4600 * px, -114.0 + 1000 * px, 42.0 - 100 * px)]
+    fixtures.write_block_shapefile(str(root / "blocks.shp"), blocks)
+    lookups.write_default_lookups(str(root / "lookups"))
+    (root / "blocks.txt").write_text("31\n")
+    fixtures.write_config(str(root / "config.txt"), str(root / "esa.tif"), str(root / "hsg.tif"), str(root / "blocks.shp"),
+                          str(root / "lookups"), str(root / "logs"))
+    return dict(root=root, esa=esa, esa_t=esa_t, hsg=hsg, hsg_t=hsg_t, blocks=blocks)
+
+
+def test_program_stats_multi_band_block(tall_world, reference, tmp_path):
+    """A block taller than two 2048-row bands: the host-decode path hands the GPU's histograms over after its last band,
+    the host-deflate path counts in the writer; every path writes the tags of the decoded planes."""
+    root = tall_world["root"]
+    modes = dict(gpu=(False, False), host_inflate=(False, True), host_deflate=(True, True))
+    for mode, (hd, hi) in modes.items():
+        _program(tall_world, "config.txt", tmp_path / mode, True, hd, hi)
+    bid, x0, y0, x1, y1 = tall_world["blocks"][0]
+    want = reference.run_block(tall_world["esa"], tall_world["esa_t"], tall_world["hsg"], tall_world["hsg_t"],
+                               (x0, y0, x1, y1), str(root / "lookups"), block_id=bid)
+    assert want["h"] > 2 * 2048
+    for k, rel in enumerate(want["paths"]):
+        for m in modes:
+            img, nodata, meta = _tags(str(tmp_path / m / rel))
+            assert np.array_equal(img, want["planes"][k]), (rel, m)
+            assert nodata == "255", (rel, m)
+            assert S.close(S.parse(meta), S.of_plane(img)), (rel, m)
