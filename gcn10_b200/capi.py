@@ -43,12 +43,13 @@ class TileStrip(C.Structure):
     _fields_ = [("tile_row0", C.c_int), ("n_tile_rows", C.c_int), ("tiles_x", C.c_int), ("n_planes", C.c_int),
                 ("plane_ids", C.POINTER(C.c_int)), ("offsets", C.POINTER(C.c_uint64)),
                 ("sizes", C.POINTER(C.c_uint32)), ("blob", C.POINTER(C.c_uint8)), ("blob_bytes", C.c_size_t),
-                ("level", C.c_int), ("level_w", C.c_int), ("level_h", C.c_int)]
+                ("level", C.c_int), ("level_w", C.c_int), ("level_h", C.c_int), ("aggregate", C.c_int)]
 
 
-def _tile_collector(tiles, overviews, total, on_strip=None):
+def _tile_collector(tiles, overviews, total, on_strip=None, aggregate=None):
     """A sink that files every tile of a strip: level 0 into tiles = {plane: {(tile_row, tile_x): bytes}}, overview
-    level k into overviews = {k: {plane: {...}}}; with ``on_strip(strip_struct)`` the tiles are not copied."""
+    level k into overviews = {k: {plane: {...}}}, the mean rasters (option "aggregate") into aggregate = {plane: {...}};
+    with ``on_strip(strip_struct)`` the tiles are not copied."""
 
     def _sink(_user, sp):
         st = sp.contents
@@ -56,7 +57,7 @@ def _tile_collector(tiles, overviews, total, on_strip=None):
         if on_strip is not None:
             return int(on_strip(st) or 0)
         blob = C.string_at(st.blob, st.blob_bytes)
-        dest = tiles if st.level == 0 else overviews.setdefault(st.level, {})
+        dest = aggregate if st.aggregate else tiles if st.level == 0 else overviews.setdefault(st.level, {})
         for k in range(st.n_planes):
             d = dest.setdefault(st.plane_ids[k], {})
             for tr in range(st.n_tile_rows):
@@ -360,32 +361,33 @@ class Context:
     def block_deflate(self, esa, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
         """Compressed-tile call.  Returns dict(tiles={plane: {(tile_row, tile_x): bytes}},
         overviews={level: {plane: {(tile_row, tile_x): bytes}}} (option "overviews"), bytes=total,
-        histograms=uint64 [18, 256] (option "stats", else None)); with ``on_strip(strip_struct)`` the tiles are not
+        histograms=uint64 [18, 256] (option "stats", else None), aggregate={plane: {(tile_row, tile_x): bytes}} (the f x f mean
+        rasters of option "aggregate", else empty)); with ``on_strip(strip_struct)`` the tiles are not
         copied."""
         esa, esa_pitch = _rows(esa)
         hsg, hsg_pitch = _rows(hsg)
         h, w = esa.shape
         hsy, hsx = hsg.shape
-        tiles, overviews, total = {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
+        tiles, overviews, aggregate, total = {}, {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
         self._check(self.lib.gcn10_cuda_block_deflate(
             self.h, esa.ctypes.data, w, h, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
             _d6(soil_gt), plane_mask, cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
+        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
 
     def block_deflate_rows(self, esa_rows, h, row0, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
         """Band form of block_deflate: esa_rows holds rows [row0, row0+len) of a block that is h rows tall; the
-        result holds this band's tiles (and, for the band that ends the block, its overview levels)."""
+        result holds this band's tiles (and, for the band that ends the block, its overview levels and mean rasters)."""
         esa_rows, esa_pitch = _rows(esa_rows)
         hsg, hsg_pitch = _rows(hsg)
         nrows, w = esa_rows.shape
         hsy, hsx = hsg.shape
-        tiles, overviews, total = {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
+        tiles, overviews, aggregate, total = {}, {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
         self._check(self.lib.gcn10_cuda_block_deflate_rows(
             self.h, esa_rows.ctypes.data, w, h, row0, nrows, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
             _d6(soil_gt), plane_mask, cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
+        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
 
     def inflate_tiles(self, src: "TileSource", w, h, out=None, want_status=False):
         """GPU inflate of a tile source into a host raster uint8 [h, w]."""
@@ -405,13 +407,13 @@ class Context:
         block_deflate)."""
         hsg, hsg_pitch = _rows(hsg)
         hsy, hsx = hsg.shape
-        tiles, overviews, total = {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
+        tiles, overviews, aggregate, total = {}, {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
         st = src.struct()
         self._check(self.lib.gcn10_cuda_block_tiles_deflate(
             self.h, C.byref(st), w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
             cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
+        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
 
     def inflate_parts(self, parts, fill, w, h, want_status=False):
         """GPU inflate of a mosaic ([(TileSource, dst_x, dst_y, w, h), ...]) into a host raster uint8 [h, w]."""
@@ -430,13 +432,13 @@ class Context:
         """Mosaic form of block_tiles_deflate; same result layout."""
         hsg, hsg_pitch = _rows(hsg)
         hsy, hsx = hsg.shape
-        tiles, overviews, total = {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip))
+        tiles, overviews, aggregate, total = {}, {}, {}, [0]
+        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
         arr = parts_array(parts)
         self._check(self.lib.gcn10_cuda_block_parts_deflate(
             self.h, arr, len(parts), fill, w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
             cb, None))
-        return dict(tiles=tiles, overviews=overviews, bytes=total[0], histograms=self._histograms())
+        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
 
     def tiles_prefetch(self, src: "TileSource", w, h):
         """Start upload + GPU inflate of a block's tiles; the next block_tiles_deflate / inflate_tiles call with the

@@ -11,6 +11,7 @@
 #include "deflate_tiles.cuh"
 #include "inflate_tiles.cuh"
 #include "cn_deflate_fused.cuh"
+#include "aggregate.cuh"
 #include "overviews.cuh"
 #include "stats.cuh"
 #include "tile_code.h"
@@ -73,8 +74,10 @@ struct StripSlot {
     HostBuf h_blob, h_table;    // page-locked mirrors
     cudaEvent_t enc_done = nullptr;
     cudaEvent_t ov = nullptr;   // option "overviews": behind the strip's overview_decimate_kernel
+    cudaEvent_t ag = nullptr;   // option "aggregate": behind the strip's aggregate_accumulate_kernel
     int y0 = 0, rows = 0;
     int level = 0, y_base = 0, tiles_x = 0, level_w = 0, level_h = 0;     // what the strip reports to the sink
+    int agg = 0;                // ... and the factor of a mean-raster strip (0 = a Curve Number strip)
     bool busy = false;
 };
 
@@ -155,6 +158,12 @@ struct gcn10_ctx {
     bool stats_ready = false;
     uint64_t stats_hist[GCN10_NPLANES][256] = {};
     uint8_t fused_rec[kFusedIds][GCN10_NPLANES] = {};  // value record of every id of the fused tables (fused_mask)
+    // option "aggregate": the block's per-cell (sum, count) accumulators [selected planes][ch][cw], all zero between
+    // blocks (agg_clean), and the mean rasters the finish kernel makes of them [selected planes][ch][pitch]
+    int aggregate = 0;
+    DevBuf agg_acc, agg_out;
+    bool agg_clean = false;
+    cudaEvent_t agg_ready = nullptr;    // behind aggregate_finish_kernel
     // asynchronous raw-plane blocks (gcn10_cuda_block_async): frame guard, per-stream end-of-block marks, timer events
     cudaEvent_t frame_ready = nullptr;
     cudaEvent_t tail[kMaxStreams] = {};
@@ -749,6 +758,7 @@ int gcn10_cuda_create(int device, gcn10_ctx **out)
         CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].done, cudaEventDisableTiming));
         CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].enc_done, cudaEventDisableTiming));
         CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].ov, cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&c->slots[i].ag, cudaEventDisableTiming));
     }
     CUDA_TRY(cudaFuncSetAttribute((const void *)deflate_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   kEncSmem));
@@ -766,6 +776,7 @@ int gcn10_cuda_create(int device, gcn10_ctx **out)
                                   cudaSharedmemCarveoutMaxShared));
     CUDA_TRY(cudaStreamCreateWithPriority(&c->pre_stream, cudaStreamNonBlocking, prio_lo));
     CUDA_TRY(cudaEventCreateWithFlags(&c->frame_ready, cudaEventDisableTiming));
+    CUDA_TRY(cudaEventCreateWithFlags(&c->agg_ready, cudaEventDisableTiming));
     for (int i = 0; i < kMaxStreams; i++)
         CUDA_TRY(cudaEventCreateWithFlags(&c->tail[i], cudaEventDisableTiming));
     for (int i = 0; i < 2; i++) {
@@ -800,6 +811,9 @@ void gcn10_cuda_destroy(gcn10_ctx *c)
     release(c->fused_tab);
     release(c->ov_buf);
     release(c->stats_buf);
+    release(c->agg_acc);
+    release(c->agg_out);
+    if (c->agg_ready) cudaEventDestroy(c->agg_ready);
     for (int i = 0; i < 2; i++) {
         release(c->tslot[i].in_blob);
         release(c->tslot[i].in_table);
@@ -827,6 +841,7 @@ void gcn10_cuda_destroy(gcn10_ctx *c)
         release_host(c->slots[i].h_table);
         if (c->slots[i].enc_done) cudaEventDestroy(c->slots[i].enc_done);
         if (c->slots[i].ov) cudaEventDestroy(c->slots[i].ov);
+        if (c->slots[i].ag) cudaEventDestroy(c->slots[i].ag);
         if (c->slots[i].k0) cudaEventDestroy(c->slots[i].k0);
         if (c->slots[i].k1) cudaEventDestroy(c->slots[i].k1);
         if (c->slots[i].k2) cudaEventDestroy(c->slots[i].k2);
@@ -872,6 +887,10 @@ int gcn10_cuda_set_option(gcn10_ctx *c, const char *key, long value)
         c->stats = (int)value;
         c->blk_next = -1;
         c->stats_ready = false;
+    }
+    else if (!strcmp(key, "aggregate") && (value == 0 || (value >= 2 && value <= GCN10_MAX_AGGREGATE))) {
+        c->aggregate = (int)value;
+        c->blk_next = -1;
     }
     else if (!strcmp(key, "inflate_probe") && value >= 0 && value <= 2) c->inflate_probe = (int)value;
     else if (!strcmp(key, "tuned_code") && (value == 0 || value == 1)) {
@@ -1265,22 +1284,24 @@ static int deflate_rows_impl(gcn10_ctx *c,
         return fail(GCN10_ENOLUT, "gcn10_cuda_set_luts() has not been called");
     if (c->pending_events)
         return fail(GCN10_EINVAL, "asynchronous blocks are pending on this context: gcn10_cuda_wait() for them first");
-    // options "overviews" and "stats": every band feeds the block's levels and histograms, so the bands of a block must
-    // come in order and without gaps (with "stats" also with the same planes); the band that ends the block emits the
-    // levels and completes the histograms
+    // options "overviews", "stats" and "aggregate": every band feeds the block's levels, histograms and mean rasters, so
+    // the bands of a block must come in order and without gaps (with "stats" or "aggregate" also with the same planes);
+    // the band that ends the block emits the levels and the mean rasters and completes the histograms
     const int nlev = c->overviews ? gcn10_overview_levels(w, h, c->overviews) : 0;
-    const bool gather = nlev || c->stats;
+    const int agg = c->aggregate;
+    const bool gather = nlev || c->stats || agg;
     if (gather && row0 != 0 &&
-        (row0 != c->blk_next || w != c->blk_w || h != c->blk_h || (c->stats && plane_mask != c->blk_mask))) {
+        (row0 != c->blk_next || w != c->blk_w || h != c->blk_h || ((c->stats || agg) && plane_mask != c->blk_mask))) {
         rc = fail(GCN10_EINVAL, "%s: band [%d, +%d) of a %d x %d block does not continue the block's previous band "
-                                "(next row %d); a block starts with row 0", nlev ? "overviews" : "stats", row0, nrows, w,
-                  h, c->blk_next);
+                                "(next row %d); a block starts with row 0",
+                  nlev ? "overviews" : c->stats ? "stats" : "aggregate", row0, nrows, w, h, c->blk_next);
         c->blk_next = -1;
         return rc;
     }
     c->blk_next = -1;           // (until this call has succeeded)
     const bool ends_block = row0 + nrows == h;
     const bool emit_levels = nlev && ends_block;
+    const bool emit_agg = agg && ends_block;
     CUDA_TRY(cudaSetDevice(c->device));
     if (gather && row0 == 0) {
         c->blk_w = w;
@@ -1328,6 +1349,19 @@ static int deflate_rows_impl(gcn10_ctx *c,
         c->blk_fused = false;
         c->stats_ready = false;
     }
+    // option "aggregate": a block starts with zero accumulators (the finish kernel leaves them so; a new buffer or an
+    // abandoned block is cleared here)
+    const int acw = agg ? gcn10_aggregate_dim(w, agg) : 0, ach = agg ? gcn10_aggregate_dim(h, agg) : 0;
+    const size_t apitch = round_up((size_t)acw, 256);
+    if (agg && row0 == 0) {
+        const size_t cap_was = c->agg_acc.cap;
+        if ((rc = ensure(c->agg_acc, sizeof(uint2) * (size_t)nplanes * ach * acw)) ||
+            (rc = ensure(c->agg_out, apitch * (size_t)ach * nplanes)))
+            return rc;
+        if (c->agg_acc.cap != cap_was || !c->agg_clean)
+            CUDA_TRY(cudaMemsetAsync(c->agg_acc.p, 0, c->agg_acc.cap, s0));
+        c->agg_clean = false;
+    }
     unsigned long long *id_hist = c->stats ? (unsigned long long *)c->stats_buf.p : nullptr;
     unsigned long long *plane_hist = c->stats ? id_hist + kFusedIds : nullptr;
     for (int i = 0; i < nplans; i++)
@@ -1361,6 +1395,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
         const uint8_t *d_esa;                   // nullptr: staged from the caller's host raster
         size_t pitch;
         const int32_t *col_idx, *row_idx;       // nullptr: the block's
+        int agg;                                // a strip of the mean rasters (d_esa: their first row)
     };
     std::vector<StripJob> jobs;
     for (int y0 = 0; y0 < nrows; y0 += strip)
@@ -1374,7 +1409,13 @@ static int deflate_rows_impl(gcn10_ctx *c,
             jobs.push_back({ k + 1, y0, std::min(lstrip, c->ov_h[k] - y0), L.w, c->ov_h[k], y0,
                              L.esa + (size_t)y0 * L.pitch, L.pitch, L.col_idx, L.row_idx });
     }
-    const int strip_cap = std::max(strip, lstrip);
+    // then, when the band ends the block, the mean rasters in strips of at most `astrip` cell rows
+    const int astrip = emit_agg ? std::max(kTile, std::min(c->strip_rows, (int)round_up((size_t)ach, kTile)) / kTile * kTile) : 0;
+    const int first_agg = (int)jobs.size();
+    for (int y0 = 0; emit_agg && y0 < ach; y0 += astrip)
+        jobs.push_back({ 0, y0, std::min(astrip, ach - y0), acw, ach, y0, (const uint8_t *)c->agg_out.p + (size_t)y0 * apitch,
+                         apitch, nullptr, nullptr, agg });
+    const int strip_cap = std::max(std::max(strip, lstrip), astrip);
     const int strip_tile_rows = strip_cap / kTile;
     const size_t ntile_slot = (size_t)nplanes * strip_tile_rows * tiles_x;
     const size_t blob_cap = ntile_slot * (size_t)round_up(kStoredBytes, 16);
@@ -1402,6 +1443,40 @@ static int deflate_rows_impl(gcn10_ctx *c,
 
     const int nstrips = (int)jobs.size();
     float kernel_ms = 0.f;
+
+    // option "aggregate": what every accumulate launch shares -- a thread's segment of at most 32 pixel columns, a cell
+    // row's rows walked in equal chunks of at most 32 per CTA, and each launch plan's records and outputs
+    AggParams ap;
+    memset(&ap, 0, sizeof(ap));
+    if (agg) {
+        ap.w = w;
+        ap.f = agg;
+        ap.cw = acw;
+        ap.ch = ach;
+        ap.spc = (agg + 31) / 32;
+        ap.seg = (agg + ap.spc - 1) / ap.spc;
+        ap.nchunk = (agg + 31) / 32;
+        ap.chunk_rows = (agg + ap.nchunk - 1) / ap.nchunk;
+        ap.col_idx = (const int32_t *)c->col_idx.p;
+        ap.row_idx = (const int32_t *)c->row_idx.p;
+        ap.hsg = (const uint8_t *)c->hsg.p;
+        ap.hsg_pitch = hsg_dpitch;
+        ap.swz_shift = c->swz_shift;
+        ap.nplans = nplans;
+        for (int i = 0; i < nplans; i++) {
+            AggPlan &P = ap.plan[i];
+            P.lut = (const uint8_t *)c->lut.p + (size_t)i * kLutBytes;
+            P.rec_bytes = plans[i].np <= kNarrowPlanes ? 4 : 16;
+            P.np = plans[i].np;
+            P.groups = plans[i].groups;
+            P.drained[0] = plans[i].drained[0];
+            P.drained[1] = plans[i].drained[1];
+            for (int k = 0; k < plans[i].np * plans[i].groups; k++)
+                P.acc[k] = (int)(std::find(plane_ids, plane_ids + nplanes, plans[i].plane_ids[k]) - plane_ids);
+        }
+        ap.nsel = nplanes;
+        ap.acc = (uint2 *)c->agg_acc.p;
+    }
 
     // behind the encoder on the strip's stream: either the ship kernel (exact bytes + tables straight into the
     // page-locked arena, nothing for the host to do but wait), or the table read-back of the two-phase path
@@ -1455,12 +1530,13 @@ static int deflate_rows_impl(gcn10_ctx *c,
         sl.tiles_x = stx;
         sl.level_w = jb.w;
         sl.level_h = jb.h;
+        sl.agg = jb.agg;
         const uint8_t *strip_esa = jb.d_esa ? jb.d_esa : (const uint8_t *)sl.esa.p;
         const size_t strip_esa_pitch = jb.d_esa ? jb.pitch : dpitch;
         if (!jb.d_esa)
             CUDA_TRY(cudaMemcpy2DAsync(sl.esa.p, dpitch, esa + (size_t)y0 * esa_pitch, esa_pitch, (size_t)w, (size_t)rows,
                                        cudaMemcpyHostToDevice, st));
-        if (nlev && jb.level == 0) {
+        if (nlev && jb.level == 0 && !jb.agg) {
             // the overview levels' share of this strip, while its land cover is on the device
             OverviewParams op;
             memset(&op, 0, sizeof(op));
@@ -1501,15 +1577,55 @@ static int deflate_rows_impl(gcn10_ctx *c,
             for (int i = 0; i < ns; i++)
                 CUDA_TRY(cudaStreamWaitEvent(st, c->slots[i].ov, 0));
         }
+        if (agg && jb.level == 0 && !jb.agg) {
+            // the mean rasters' share of this strip, while its land cover is on the device
+            AggParams a = ap;
+            a.esa = strip_esa;
+            a.esa_pitch = strip_esa_pitch;
+            a.y0 = jb.y_base;
+            a.rows = rows;
+            a.ncr = (jb.y_base + rows - 1) / agg - jb.y_base / agg + 1;
+            const int cells = kAggThreads / a.spc;
+            const dim3 grid((acw + cells - 1) / cells, (unsigned)std::min(a.ncr * a.nchunk, 65535));
+            aggregate_accumulate_kernel<<<grid, kAggThreads, 0, st>>>(a);
+            c->launches++;
+            CUDA_TRY(cudaGetLastError());
+            CUDA_TRY(cudaEventRecord(sl.ag, st));
+        }
+        if (jb.agg) {
+            // the accumulators are complete once every full-resolution strip of the block has been added (earlier bands
+            // finished theirs before their call returned): the first mean strip turns them into the mean rasters, the
+            // others wait for that
+            if (s == first_agg) {
+                for (int i = 0; i < ns; i++)
+                    CUDA_TRY(cudaStreamWaitEvent(st, c->slots[i].ag, 0));
+                AggFinishParams fp;
+                fp.acc = (uint2 *)c->agg_acc.p;
+                fp.out = (uint8_t *)c->agg_out.p;
+                fp.pitch = apitch;
+                fp.plane_stride = apitch * (size_t)ach;
+                fp.cw = acw;
+                fp.ch = ach;
+                fp.nsel = nplanes;
+                const long long n = (long long)acw * ach * nplanes;
+                aggregate_finish_kernel<<<(int)std::min<long long>((n + 255) / 256, (long long)c->sm_count * 8), 256, 0, st>>>(fp);
+                c->launches++;
+                CUDA_TRY(cudaGetLastError());
+                CUDA_TRY(cudaEventRecord(c->agg_ready, st));
+            }
+            else {
+                CUDA_TRY(cudaStreamWaitEvent(st, c->agg_ready, 0));
+            }
+        }
         // The encoder kernels run in strip order, at most two at a time (the second fills the first one's last wave):
         // launched side by side on all streams they would all finish together, and the copy of strip 0 -- the head of
         // the chain of copies that ends the block -- would wait for the others.
         // Overview strips are not chained: their grids are small (level k has 1/4^k of the tiles), one alone leaves
         // most SMs idle, and they end the block, so no later copy waits on them.
-        if (s >= 2 && jb.level == 0)
+        if (s >= 2 && jb.level == 0 && !jb.agg)
             CUDA_TRY(cudaStreamWaitEvent(st, c->slots[(s - 2) % ns].k1, 0));
         CUDA_TRY(cudaEventRecord(sl.k0, st));
-        if (fused) {
+        if (fused && !jb.agg) {
             FusedParams fp;
             memset(&fp, 0, sizeof(fp));
             fp.esa = strip_esa;
@@ -1545,14 +1661,15 @@ static int deflate_rows_impl(gcn10_ctx *c,
         }
         uint8_t *d_out[GCN10_NPLANES] = { nullptr };
         for (int k = 0; k < nplanes; k++)
-            d_out[plane_ids[k]] = (uint8_t *)sl.out.p + (size_t)k * dpitch * (size_t)strip_cap;
-        for (int i = 0; i < nplans; i++) {
+            d_out[plane_ids[k]] = jb.agg ? (uint8_t *)jb.d_esa + (size_t)k * apitch * (size_t)ach     // the mean rasters
+                                         : (uint8_t *)sl.out.p + (size_t)k * dpitch * (size_t)strip_cap;
+        for (int i = 0; i < nplans && !jb.agg; i++) {
             int r2 = launch_rows(c, plans[i], i, strip_esa, strip_esa_pitch, sw, rows, jb.y_base, (const uint8_t *)c->hsg.p,
                                  hsg_dpitch, hsx, hsy, map, tma_ok, d_out, dpitch, st, jb.col_idx, jb.row_idx);
             if (r2)
                 return r2;
         }
-        if (plane_hist && jb.level == 0) {
+        if (plane_hist && jb.level == 0 && !jb.agg) {
             PlaneHistParams hp;
             memset(&hp, 0, sizeof(hp));
             hp.planes = (const uint8_t *)sl.out.p;
@@ -1573,7 +1690,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
         memset(&ep, 0, sizeof(ep));
         for (int k = 0; k < nplanes; k++)
             ep.plane[k] = d_out[plane_ids[k]];
-        ep.pitch = dpitch;
+        ep.pitch = jb.agg ? apitch : dpitch;
         ep.w = sw;
         ep.rows = rows;
         ep.tiles_x = stx;
@@ -1657,6 +1774,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
         ts.level = sl.level;
         ts.level_w = sl.level_w;
         ts.level_h = sl.level_h;
+        ts.aggregate = sl.agg;
         // NB: the tables are laid out [plane][strip_tile_rows (capacity)][tiles_x] only when the strip is
         // full; the kernel indexes with the strip's own tile_rows, which is what n_tile_rows reports
         const int sink_rc = sink(user, &ts);
@@ -1667,6 +1785,8 @@ static int deflate_rows_impl(gcn10_ctx *c,
             return bail(rc);
     }
     c->last_kernel_ms = kernel_ms;
+    if (emit_agg)
+        c->agg_clean = true;
     if (c->stats && ends_block && (rc = finish_histograms(c, s0)))
         return rc;
     if (gather && !ends_block)

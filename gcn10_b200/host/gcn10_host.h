@@ -177,6 +177,7 @@ typedef struct {
     const char *out_root;       /* directory that receives cn_rasters_<cond>/ (reference: CWD)     */
     int overviews;              /* --overviews: at most this many overview levels per output (0 = none) */
     int stats;                  /* --stats: NoData tag and band statistics in every output                   */
+    int aggregate;              /* --aggregate f: also the f x f mean rasters, in cn_rasters_<cond>_agg<f>/ (0 = none) */
 } gh_run_options;
 
 /* Runs a list of blocks on the GPUs of this box: one worker thread (+ one gcn10_ctx) per GPU, block

@@ -39,6 +39,9 @@ static void usage(FILE *fp)
             "			(nearest neighbour, halving until a level fits one 256 x 256 tile)\n"
             "  --stats		tag every output with NoData 255 and its band statistics (minimum, maximum,\n"
             "			mean, standard deviation, valid percent), counted on the GPU\n"
+            "  --aggregate <f>	also write the f x f mean of every output (the composite Curve Number of\n"
+            "			cells of f x f pixels, nodata 255 left out; f = 2..1024, 25 = the 250 m soil\n"
+            "			grid) to cn_rasters_<condition>_agg<f>/, computed on the GPU\n"
             "  --help, -h		show this help and exit\n"
             "  --version, -v	print version and exit\n"
             "\n"
@@ -83,6 +86,15 @@ int main(int argc, char **argv)
             opt.overviews = GCN10_MAX_OVERVIEWS;
         else if (!strcmp(argv[i], "--stats"))
             opt.stats = 1;
+        else if (!strcmp(argv[i], "--aggregate") && i + 1 < argc) {
+            char *end = NULL;
+            const long f = strtol(argv[++i], &end, 10);
+            if (!end || *end || f < 2 || f > GCN10_MAX_AGGREGATE) {
+                fprintf(stderr, "[rank 0] --aggregate takes a factor from 2 to %d, not '%s'\n", GCN10_MAX_AGGREGATE, argv[i]);
+                return 1;
+            }
+            opt.aggregate = (int)f;
+        }
     }
     if (!conf) {
         fprintf(stderr, "[rank 0] missing -c/--config <file>; see 'gcn10 -h' for usage.\n");    /* main.c:103-107 */

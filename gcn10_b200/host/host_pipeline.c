@@ -104,6 +104,11 @@ typedef struct worker {
     gh_tiffw *writers[NPLANES];
     int writers_open;
     char paths[NPLANES][PATH_MAX];
+    /* --aggregate: the mean rasters' files, opened and closed with the 18 outputs, and (host-deflate path) the host
+     * aggregation of each plane */
+    gh_tiffw *agg_writers[NPLANES];
+    gh_aggregate *aggs[NPLANES];
+    char agg_paths[NPLANES][PATH_MAX];
     int out_w, out_h;
     double out_gt[6];
     int cur_block;
@@ -148,20 +153,67 @@ static int ensure_bands(worker *wk, size_t pitch, int need_planes)
     return 0;
 }
 
-/* cn.c:293-360: "<outdir>/cn_<hc>_<arc>_<id>.tif", or "..._<id>_.tif" when the file exists and
- * overwrite is off */
-static void output_path(const worker *wk, int cond, int hi, int ai, int block_id, char *path, size_t n)
+/* cn.c:293-360: "<outdir>/cn_rasters_<cond>/cn_<hc>_<arc>_<id>.tif", or "..._<id>_.tif" when the file exists and
+ * overwrite is off; the f x f mean rasters (agg = f) go to "cn_rasters_<cond>_agg<f>/" by the same rule */
+static void output_path(const worker *wk, int cond, int hi, int ai, int block_id, int agg, char *path, size_t n)
 {
     const char *root = (wk->opt->out_root && *wk->opt->out_root) ? wk->opt->out_root : ".";
-    snprintf(path, n, "%s/cn_rasters_%s/cn_%s_%s_%d.tif", root, k_conds[cond], k_hcs[hi], k_arcs[ai], block_id);
+    char sfx[32] = "";
+    if (agg)
+        snprintf(sfx, sizeof sfx, "_agg%d", agg);
+    snprintf(path, n, "%s/cn_rasters_%s%s/cn_%s_%s_%d.tif", root, k_conds[cond], sfx, k_hcs[hi], k_arcs[ai], block_id);
     if (!wk->opt->overwrite) {
         FILE *f = fopen(path, "r");
         if (f) {
             fclose(f);
-            snprintf(path, n, "%s/cn_rasters_%s/cn_%s_%s_%d_.tif", root, k_conds[cond], k_hcs[hi], k_arcs[ai],
+            snprintf(path, n, "%s/cn_rasters_%s%s/cn_%s_%s_%d_.tif", root, k_conds[cond], sfx, k_hcs[hi], k_arcs[ai],
                      block_id);
         }
     }
+}
+
+/* --aggregate: drop the mean rasters' files of a block that failed (or that never got its outputs) */
+static void abort_agg_writers(worker *wk)
+{
+    for (int k = 0; k < NPLANES; k++) {
+        if (wk->agg_writers[k])
+            gh_tiffw_abort(wk->agg_writers[k]);
+        wk->agg_writers[k] = NULL;
+        gh_aggregate_free(wk->aggs[k]);
+        wk->aggs[k] = NULL;
+    }
+}
+
+/* --aggregate: the 18 mean rasters of the block, w / f x h / f with the scaled geotransform, the land cover's GeoKeys and
+ * NoData 255 (a mean grid without it would get 255 averaged in by the next resampling).  0 ok. */
+static int open_agg_writers(worker *wk)
+{
+    const int f = wk->opt->aggregate;
+    char err[GH_ERRLEN] = "";
+    double gt[6];
+    gcn10_aggregate_gt(wk->out_gt, f, gt);
+    for (int k = 0; k < NPLANES; k++) {
+        if (gh_tiffw_open(wk->agg_paths[k], gcn10_aggregate_dim(wk->out_w, f), gcn10_aggregate_dim(wk->out_h, f), gt,
+                          &wk->agg_writers[k], err, sizeof err)) {
+            gh_log_message(wk->log, "ERROR", err, 1);
+            wk->agg_writers[k] = NULL;
+            abort_agg_writers(wk);
+            return -1;
+        }
+        gh_geokeys gk;
+        pthread_mutex_lock(&wk->rmu);
+        if (wk->esa_r && gh_raster_geokeys(wk->esa_r, &gk) == 0)
+            gh_tiffw_set_geokeys(wk->agg_writers[k], &gk);
+        pthread_mutex_unlock(&wk->rmu);
+        wk->aggs[k] = gh_aggregate_new(wk->out_w, wk->out_h, f);
+        if (gh_tiffw_set_nodata(wk->agg_writers[k], 1) || !wk->aggs[k]) {
+            snprintf(err, sizeof err, "write error 3 on %s (aggregate)", wk->agg_paths[k]);
+            gh_log_message(wk->log, "ERROR", err, 1);
+            abort_agg_writers(wk);
+            return -1;
+        }
+    }
+    return 0;
 }
 
 
@@ -192,7 +244,8 @@ static int open_writers(worker *wk)
             break;
         }
     }
-    if (opened < NPLANES) {
+    const int agg_failed = opened == NPLANES && wk->opt->aggregate && open_agg_writers(wk);
+    if (opened < NPLANES || agg_failed) {
         for (int k = 0; k < opened; k++) {
             gh_tiffw_abort(wk->writers[k]);
             wk->writers[k] = NULL;
@@ -221,7 +274,9 @@ static void *encoder_main(void *arg)
         if (open_writers(wk))
             atomic_store(&wk->encode_failed, 1);
         for (int k = 0; k < NPLANES && !atomic_load(&wk->encode_failed); k++)
-            if (gh_tiffw_write_rows(wk->writers[k], bb->planes[k], wk->pitch, bb->y0, bb->rows, wk->io_threads))
+            if (gh_tiffw_write_rows(wk->writers[k], bb->planes[k], wk->pitch, bb->y0, bb->rows, wk->io_threads) ||
+                (wk->opt->aggregate && gh_aggregate_write_rows(wk->aggs[k], wk->agg_writers[k], bb->planes[k], wk->pitch,
+                                                               bb->y0, bb->rows, wk->io_threads)))
                 atomic_store(&wk->encode_failed, 1);
         pthread_mutex_lock(&wk->mu);
         bb->state = 0;
@@ -286,12 +341,13 @@ typedef struct {
     const gcn10_tile_strip *st;
 } sink_job;
 
-/* one plane of a strip: append its tile rows to that plane's GeoTIFF (to the strip's level of it) */
+/* one plane of a strip: append its tile rows to that plane's GeoTIFF (to the strip's level of it), or to its mean
+ * raster's */
 static void sink_plane(void *arg, int k)
 {
     sink_job *j = arg;
     const gcn10_tile_strip *st = j->st;
-    gh_tiffw *tw = j->wk->writers[st->plane_ids[k]];
+    gh_tiffw *tw = st->aggregate ? j->wk->agg_writers[st->plane_ids[k]] : j->wk->writers[st->plane_ids[k]];
     /* the context runs with "ordered" strips: a plane's share of the strip is one contiguous piece of the blob */
     size_t base = (size_t)k * st->n_tile_rows * (size_t)st->tiles_x;
     if (gh_tiffw_put_level_tile_rows(tw, st->level, st->tile_row0, st->n_tile_rows, st->blob, st->offsets + base,
@@ -671,15 +727,24 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
         fatal(wk, msg);
     }
     for (int c = 0; c < 2; c++) {
-        char outdir[PATH_MAX];
-        snprintf(outdir, sizeof outdir, "%s/cn_rasters_%s", root, k_conds[c]);
-        if (mkdir(outdir, 0755) != 0 && errno != EEXIST) {
-            snprintf(msg, sizeof msg, "failed to create output directory %s", outdir);   /* cn.c:250 */
-            fatal(wk, msg);
+        for (int a = 0; a < (wk->opt->aggregate ? 2 : 1); a++) {
+            char outdir[PATH_MAX];
+            if (a)
+                snprintf(outdir, sizeof outdir, "%s/cn_rasters_%s_agg%d", root, k_conds[c], wk->opt->aggregate);
+            else
+                snprintf(outdir, sizeof outdir, "%s/cn_rasters_%s", root, k_conds[c]);
+            if (mkdir(outdir, 0755) != 0 && errno != EEXIST) {
+                snprintf(msg, sizeof msg, "failed to create output directory %s", outdir);   /* cn.c:250 */
+                fatal(wk, msg);
+            }
         }
     }
-    for (int k = 0; k < NPLANES; k++)
-        output_path(wk, k / 9, (k % 9) / 3, k % 3, block_id, wk->paths[k], sizeof wk->paths[k]);
+    for (int k = 0; k < NPLANES; k++) {
+        output_path(wk, k / 9, (k % 9) / 3, k % 3, block_id, 0, wk->paths[k], sizeof wk->paths[k]);
+        if (wk->opt->aggregate)
+            output_path(wk, k / 9, (k % 9) / 3, k % 3, block_id, wk->opt->aggregate, wk->agg_paths[k],
+                        sizeof wk->agg_paths[k]);
+    }
     wk->writers_open = 0;
     wk->out_w = w;
     wk->out_h = h;
@@ -697,6 +762,7 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
             for (int k = 0; k < NPLANES; k++)
                 gh_tiffw_abort(wk->writers[k]);
         wk->writers_open = 0;
+        abort_agg_writers(wk);
         if (failed) {
             snprintf(msg, sizeof msg, "esa load failed for block %d", block_id);    /* cn.c:189 */
             gh_log_message(wk->log, "ERROR", msg, 1);
@@ -718,6 +784,21 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
         snprintf(msg, sizeof msg, "progress: completed block %d / total %d", block_id, total_blocks);
         gh_log_message(wk->log0, "INFO", msg, 0);                                   /* log.c:199-207 */
     }
+    /* the mean rasters: complete only if the block is (a failed block leaves none of them behind) */
+    for (int k = 0; k < NPLANES && wk->opt->aggregate; k++) {
+        if (ok && !atomic_load(&wk->encode_failed)) {
+            if (gh_tiffw_close(wk->agg_writers[k])) {
+                snprintf(msg, sizeof msg, "write error 3 on %s", wk->agg_paths[k]);
+                gh_log_message(wk->log, "ERROR", msg, 1);
+                ok = 0;
+            }
+        }
+        else {
+            gh_tiffw_abort(wk->agg_writers[k]);
+        }
+        wk->agg_writers[k] = NULL;
+    }
+    abort_agg_writers(wk);                      /* (frees the host aggregation; no writer is left to abort) */
     wk->writers_open = 0;
     double dt = now_s() - t_start;
     snprintf(msg, sizeof msg,
@@ -742,7 +823,8 @@ static void *worker_main(void *arg)
      * writes beat the copy engine's size read-back + copy (measured on 8 x B200: +4..7 %), below that the copy engine wins */
     if (gcn10_cuda_create(wk->device, &wk->ctx) || gcn10_cuda_set_luts(wk->ctx, wk->tables) ||
         gcn10_cuda_set_option(wk->ctx, "ordered", 1) || gcn10_cuda_set_option(wk->ctx, "ship", wk->n_gpus >= 4) ||
-        gcn10_cuda_set_option(wk->ctx, "overviews", wk->opt->overviews) || gcn10_cuda_set_option(wk->ctx, "stats", wk->opt->stats)) {
+        gcn10_cuda_set_option(wk->ctx, "overviews", wk->opt->overviews) || gcn10_cuda_set_option(wk->ctx, "stats", wk->opt->stats) ||
+        gcn10_cuda_set_option(wk->ctx, "aggregate", wk->opt->aggregate)) {
         snprintf(msg, sizeof msg, "cannot initialise GPU %d: %s", wk->device, gcn10_cuda_last_error());
         fatal(wk, msg);
     }

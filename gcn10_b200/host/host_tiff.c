@@ -767,6 +767,7 @@ struct gh_tiffw {
     tw_grid g[1 + GCN10_MAX_OVERVIEWS];
     int stats;                  /* gh_tiffw_set_stats: NoData tag + GDAL_METADATA statistics from hist */
     uint64_t hist[256];         /* full-resolution pixels per value */
+    int nodata;                 /* gh_tiffw_set_nodata: NoData tag without statistics */
     int level;                  /* zlib level */
     int failed;
 };
@@ -932,6 +933,14 @@ int gh_tiffw_set_stats(gh_tiffw *tw, int on)
     if (!tw || tw->failed || (on != 0 && on != 1) || tw->pos != 8 || tw->g[0].next_tile_row)
         return -1;
     tw->stats = on;
+    return 0;
+}
+
+int gh_tiffw_set_nodata(gh_tiffw *tw, int on)
+{
+    if (!tw || tw->failed || (on != 0 && on != 1))
+        return -1;
+    tw->nodata = on;
     return 0;
 }
 
@@ -1162,6 +1171,7 @@ int gh_tiffw_close(gh_tiffw *tw)
         nmeta = n > 0 ? (size_t)n + 1 : 0;
     }
     const uint32_t nodata_ascii = '2' | '5' << 8 | '5' << 16;     /* "255\0", held in the entry itself */
+    const int tag_nodata = tw->stats || tw->nodata;                 /* GDAL_NODATA in every IFD */
     if (complete) {
         /* trailing data area: tile offsets, tile byte counts, pixel scale, tiepoint, geo keys, ascii */
         static const uint16_t geokeys[] = {
@@ -1182,10 +1192,10 @@ int gh_tiffw_close(gh_tiffw *tw)
         uint64_t off_tie = off_scale + 24, off_keys = off_tie + 48, off_dbl = off_keys + 2 * nkeys;
         uint64_t off_ascii = off_dbl + 8 * ndbl, off_meta = (off_ascii + nascii + 1) & ~(uint64_t)1;     /* word aligned */
         uint64_t off_ifd = (off_meta + nmeta + 1) & ~(uint64_t)1;
-        const int nent = 14 + 1 + (ndbl ? 1 : 0) + (nascii ? 1 : 0) + (tw->stats ? 2 : 0);
+        const int nent = 14 + 1 + (ndbl ? 1 : 0) + (nascii ? 1 : 0) + (tw->stats ? 1 : 0) + tag_nodata;
         /* behind IFD0, per overview level: its tile offsets, byte counts and IFD (reduced-resolution image, no geo tags:
          * readers derive the level's georeferencing from the size ratio) */
-        const int level_entries = 13 + (tw->stats ? 1 : 0);
+        const int level_entries = 13 + tag_nodata;
         uint64_t off_lv[1 + GCN10_MAX_OVERVIEWS], end = off_ifd + 2 + (uint64_t)nent * 12 + 4;
         for (int k = 1; k <= tw->nlev; k++) {
             off_lv[k] = end;            /* offsets | counts | IFD */
@@ -1226,10 +1236,10 @@ int gh_tiffw_close(gh_tiffw *tw)
                 put_entry(&p, 34736, 12, (uint32_t)ndbl, (uint32_t)off_dbl);
             if (nascii)
                 put_entry(&p, 34737, 2, (uint32_t)nascii, (uint32_t)off_ascii);
-            if (tw->stats) {
+            if (tw->stats)
                 put_entry(&p, 42112, 2, (uint32_t)nmeta, (uint32_t)off_meta);
+            if (tag_nodata)
                 put_entry(&p, 42113, 2, 4, nodata_ascii);
-            }
             put32(&p, tw->nlev ? (uint32_t)(off_lv[1] + 8 * (uint64_t)tw->g[1].tiles_x * (uint64_t)tw->g[1].tiles_y) : 0);
             for (int k = 1; k <= tw->nlev; k++) {
                 const tw_grid *g = &tw->g[k];
@@ -1251,7 +1261,7 @@ int gh_tiffw_close(gh_tiffw *tw)
                 put_entry(&p, 324, 4, (uint32_t)n, n == 1 ? g->offsets[0] : (uint32_t)off_lv[k]);
                 put_entry(&p, 325, 4, (uint32_t)n, n == 1 ? g->counts[0] : (uint32_t)(off_lv[k] + 4 * n));
                 put_entry(&p, 339, 3, 1, 1);
-                if (tw->stats)
+                if (tag_nodata)
                     put_entry(&p, 42113, 2, 4, nodata_ascii);
                 put32(&p, k < tw->nlev ? (uint32_t)(off_lv[k + 1] + 8 * (uint64_t)tw->g[k + 1].tiles_x * (uint64_t)tw->g[k + 1].tiles_y)
                                        : 0);
@@ -1316,6 +1326,113 @@ int gh_tiff_write(const char *path, const uint8_t *data, int w, int h, size_t pi
     if (gh_tiffw_close(tw)) {
         set_err(err, errlen, "write error 3 on %s", path);
         return -1;
+    }
+    return 0;
+}
+
+/* ---- mean rasters on the host (gh_aggregate_*) ---- */
+
+struct gh_aggregate {
+    int w, h, f, cw, ch;
+    uint32_t *sum, *cnt;        /* the cell row in progress */
+    int next_y, next_cell;      /* the next plane row and cell row */
+    uint8_t *buf;               /* completed cell rows not yet written: rows buf_row0 .. + buf_rows */
+    int buf_rows, buf_cap, buf_row0;
+};
+
+gh_aggregate *gh_aggregate_new(int w, int h, int f)
+{
+    if (w <= 0 || h <= 0 || f < 2 || f > GCN10_MAX_AGGREGATE)
+        return NULL;
+    gh_aggregate *a = calloc(1, sizeof *a);
+    if (!a)
+        return NULL;
+    a->w = w;
+    a->h = h;
+    a->f = f;
+    a->cw = gcn10_aggregate_dim(w, f);
+    a->ch = gcn10_aggregate_dim(h, f);
+    a->sum = calloc((size_t)a->cw, sizeof *a->sum);
+    a->cnt = calloc((size_t)a->cw, sizeof *a->cnt);
+    if (!a->sum || !a->cnt) {
+        gh_aggregate_free(a);
+        return NULL;
+    }
+    return a;
+}
+
+void gh_aggregate_free(gh_aggregate *a)
+{
+    if (!a)
+        return;
+    free(a->sum);
+    free(a->cnt);
+    free(a->buf);
+    free(a);
+}
+
+int gh_aggregate_rows(gh_aggregate *a, const uint8_t *data, size_t pitch, int y0, int nrows, uint8_t *out, size_t out_pitch,
+                      int *row0)
+{
+    if (!a || !data || !out || nrows < 0 || y0 != a->next_y || nrows > a->h - y0 || out_pitch < (size_t)a->cw)
+        return -1;
+    if (row0)
+        *row0 = a->next_cell;
+    int n = 0;
+    for (int y = y0; y < y0 + nrows; y++) {
+        const uint8_t *row = data + (size_t)(y - y0) * pitch;
+        for (int cx = 0, x = 0; cx < a->cw; cx++) {
+            const int xe = x + a->f < a->w ? x + a->f : a->w;
+            uint32_t s = 0, c = 0;
+            for (; x < xe; x++)
+                if (row[x] != GCN10_NODATA) {
+                    s += row[x];
+                    c++;
+                }
+            a->sum[cx] += s;
+            a->cnt[cx] += c;
+        }
+        if ((y + 1) % a->f == 0 || y + 1 == a->h) {
+            uint8_t *o = out + (size_t)n * out_pitch;
+            for (int cx = 0; cx < a->cw; cx++)
+                o[cx] = gcn10_aggregate_value(a->sum[cx], a->cnt[cx]);
+            memset(a->sum, 0, (size_t)a->cw * sizeof *a->sum);
+            memset(a->cnt, 0, (size_t)a->cw * sizeof *a->cnt);
+            n++;
+        }
+    }
+    a->next_y = y0 + nrows;
+    a->next_cell += n;
+    return n;
+}
+
+int gh_aggregate_write_rows(gh_aggregate *a, gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0, int nrows, int threads)
+{
+    if (!a || !tw)
+        return -1;
+    const int most = nrows / a->f + 2;                  /* cell rows this band can complete (the last one short) */
+    if (a->buf_rows + most > a->buf_cap) {
+        const int cap = a->buf_rows + most + TILE;
+        uint8_t *b = realloc(a->buf, (size_t)cap * (size_t)a->cw);
+        if (!b)
+            return -1;
+        a->buf = b;
+        a->buf_cap = cap;
+    }
+    if (a->buf_rows == 0)
+        a->buf_row0 = a->next_cell;
+    const int n = gh_aggregate_rows(a, data, pitch, y0, nrows, a->buf + (size_t)a->buf_rows * a->cw, (size_t)a->cw, NULL);
+    if (n < 0)
+        return -1;
+    a->buf_rows += n;
+    const int done = a->buf_row0 + a->buf_rows == a->ch;
+    const int put = done ? a->buf_rows : a->buf_rows / TILE * TILE;
+    if (put > 0) {
+        if (gh_tiffw_write_rows(tw, a->buf, (size_t)a->cw, a->buf_row0, put, threads))
+            return -1;
+        memmove(a->buf, a->buf + (size_t)put * a->cw, (size_t)(a->buf_rows - put) * a->cw);
+        a->buf_rows -= put;
+        a->buf_row0 += put;
     }
     return 0;
 }

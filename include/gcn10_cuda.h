@@ -159,7 +159,15 @@ int gcn10_cuda_block_rows(gcn10_ctx *ctx,
  * plane is the plane sampled by gcn10_overview_src, so each of its pixels is a full-resolution output pixel.  This
  * holds for gcn10_cuda_block_deflate, _block_deflate_rows, _block_tiles_deflate and _block_parts_deflate; the raw-plane
  * calls (gcn10_cuda_block*, _block_device) ignore the option.  The levels cost device memory of about a third of the
- * block (about 0.44 GB for 36001 x 36001), kept on the context. */
+ * block (about 0.44 GB for 36001 x 36001), kept on the context.
+ *
+ * Mean rasters (option "aggregate" = f >= 2): after the full-resolution strips and the overview levels the same sink
+ * receives, for every selected plane, the block's f x f mean raster (gcn10_aggregate_dim / _value below) as 256 x 256
+ * DEFLATE tiles, in tile-row order, in strips of at most "strip_rows" rows (strip->aggregate = f, level = 0, level_w x
+ * level_h = the mean raster's size).  The same four calls deliver it; the raw-plane calls ignore the option.  The
+ * full-resolution strips and overview levels are the same bytes as without the option, and "stats" does not count the
+ * mean strips.  The accumulators cost 8 bytes per cell and selected plane on the context (computed: about 0.3 GB for
+ * 18 planes of 36001 x 36001 at f = 25). */
 typedef struct {
     int tile_row0;              /* first tile row (of the block) in this strip                    */
     int n_tile_rows;            /* tile rows in this strip                                        */
@@ -175,6 +183,10 @@ typedef struct {
      * level_w x level_h is the raster the strip's tile grid covers: the block itself at level 0. */
     int level;
     int level_w, level_h;
+    /* mean rasters (option "aggregate"): 0 = a Curve Number strip (full resolution or overview); f = a strip of the
+     * block's f x f mean raster, whose level_w x level_h = gcn10_aggregate_dim(w, f) x gcn10_aggregate_dim(h, f)
+     * cells have their own tile grid (level is then 0) */
+    int aggregate;
 } gcn10_tile_strip;
 
 /* Overview levels: nearest-neighbour reductions by 2^k of a block, sampled from full resolution.
@@ -210,6 +222,44 @@ static inline int gcn10_overview_levels(int w, int h, int max_levels)
 
 #define GCN10_MAX_OVERVIEWS 16
 
+/* Mean rasters (option "aggregate" = f): the f x f mean of every selected plane, the composite Curve Number of a
+ * coarse cell (TR-55; GDAL's "-r average").  Every layer (library, GeoTIFF writer, host program, tests) uses these
+ * rules.
+ *
+ *   gcn10_aggregate_dim(n, f)          cells along an n-pixel axis: ceil(n / f).  Cells are aligned to the block's
+ *                                      pixel (0, 0); an edge cell covers the pixels it has (GDAL's edge overview cell)
+ *   gcn10_aggregate_value(sum, count)  a cell's value from the sum and the number of its pixels that are not 255:
+ *                                      the mean rounded half up, (2 sum + count) / (2 count) in integers, and 255
+ *                                      only when every pixel of the cell is 255 (GDAL's "average" rule).  Valid values
+ *                                      are <= 254, so the mean never collides with nodata.
+ *   gcn10_aggregate_gt(gt, f, out)     the mean raster's geotransform: { gt0, gt1 f, gt2 f, gt3, gt4 f, gt5 f }
+ *
+ * f <= GCN10_MAX_AGGREGATE keeps a cell's sum (<= 1024^2 * 254) and count inside uint32.
+ *
+ * Edge wart: a window of the shipped VRT is 36001 x 36001 pixels (ceil of 36000.00000000125), so at f = 25 its last
+ * cell row and column are one pixel wide.  That pixel is the first pixel of the neighbouring block's window (both
+ * windows' pixel offsets are floor of the block's origin in VRT pixels, and the origins are 36000 pixels apart), so
+ * the neighbour's first cell covers the footprint in full; the one-pixel cell is the same duplicated pixel that the
+ * full-resolution outputs already carry. */
+#define GCN10_MAX_AGGREGATE 1024
+
+static inline GCN10_HOST_DEVICE int gcn10_aggregate_dim(int n, int f) { return (int)(((long long)n + f - 1) / f); }
+
+static inline GCN10_HOST_DEVICE uint8_t gcn10_aggregate_value(uint32_t sum, uint32_t count)
+{
+    return count ? (uint8_t)((2ull * sum + count) / (2ull * count)) : (uint8_t)GCN10_NODATA;
+}
+
+static inline void gcn10_aggregate_gt(const double gt[6], int f, double out[6])
+{
+    out[0] = gt[0];
+    out[1] = gt[1] * f;
+    out[2] = gt[2] * f;
+    out[3] = gt[3];
+    out[4] = gt[4] * f;
+    out[5] = gt[5] * f;
+}
+
 typedef int (*gcn10_tile_sink)(void *user, const gcn10_tile_strip *strip);
 
 int gcn10_cuda_block_deflate(gcn10_ctx *ctx,
@@ -219,10 +269,11 @@ int gcn10_cuda_block_deflate(gcn10_ctx *ctx,
 
 /* Band form of gcn10_cuda_block_deflate (see gcn10_cuda_block_rows): esa points at block row `row0`,
  * which must be a multiple of 256; nrows must be a multiple of 256 unless the band ends the block.
- * With option "overviews" or "stats" the bands of a block feed its levels and histograms, which stay on the context
- * between calls: a band with row0 == 0 starts a block, every later band must start where the previous one ended (same
- * w and h, and with "stats" the same plane mask; anything else is refused with GCN10_EINVAL), and the band that ends
- * the block (row0 + nrows == h) delivers the levels after its own strips and completes the histograms. */
+ * With option "overviews", "stats" or "aggregate" the bands of a block feed its levels, histograms and mean rasters,
+ * which stay on the context between calls: a band with row0 == 0 starts a block, every later band must start where the
+ * previous one ended (same w and h, and with "stats" or "aggregate" the same plane mask; anything else is refused with
+ * GCN10_EINVAL), and the band that ends the block (row0 + nrows == h) delivers the levels and the mean rasters after
+ * its own strips and completes the histograms. */
 int gcn10_cuda_block_deflate_rows(gcn10_ctx *ctx,
                                   const uint8_t *esa, int w, int h, int row0, int nrows, size_t esa_pitch,
                                   const double gt[6],
@@ -361,7 +412,9 @@ int gcn10_cuda_last_histograms(gcn10_ctx *ctx, uint64_t hist[GCN10_NPLANES][256]
  * of the tuned one), "defer_inflate" (0 = the inflate kernel of a prefetched block starts at once instead of behind
  * the last strip of the block in hand), "overviews" (0..16, default 0: the compressed-tile calls also deliver up to that
  * many overview levels of the block, see gcn10_cuda_block_deflate), "stats" (0 / 1, default 0: the compressed-tile calls
- * also count every selected plane's histogram, see gcn10_cuda_last_histograms), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
+ * also count every selected plane's histogram, see gcn10_cuda_last_histograms), "aggregate" (0 or 2 ..
+ * GCN10_MAX_AGGREGATE, default 0: the compressed-tile calls also deliver every selected plane's f x f mean raster, see
+ * gcn10_cuda_block_deflate), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
  * kernel's writer off; results are then invalid). */
 int gcn10_cuda_set_option(gcn10_ctx *ctx, const char *key, long value);
 
