@@ -4,6 +4,7 @@ import numpy as np
 import pytest
 
 from gcn10_b200 import capi
+from tests import stream_ref as S
 from tests.cases import make_block, PX, PX_VRT
 
 pytestmark = pytest.mark.gpu
@@ -36,7 +37,7 @@ def test_random_block(seed, gpu_ctx, port, tables):
 def test_random_block_through_the_compressed_tile_chain(seed, gpu_ctx, port, tables):
     """The same property through gcn10_cuda_block_tiles_deflate: random input tile sizes and zlib levels, the
     window at a random position inside the tile grid, random plane masks; every output tile is inflated with
-    zlib and compared with the oracle's plane."""
+    zlib and compared with the oracle's plane, and equals the reference encoder's stream byte for byte."""
     import zlib
     rng = np.random.default_rng(5000 + seed)
     w = int(rng.choice([1, 16, 255, 256, 257, 700, 1023, 1025, int(rng.integers(1, 2600))]))
@@ -67,3 +68,4 @@ def test_random_block_through_the_compressed_tile_chain(seed, gpu_ctx, port, tab
             full[r * T:(r + 1) * T, c * T:(c + 1) * T] = np.frombuffer(zlib.decompress(z), dtype=np.uint8).reshape(T, T)
         assert np.array_equal(full[:h, :w], want[k]), (kw, (tw, th, x_off, y_off), hex(mask), k)
         assert not full[h:, :].any() and not full[:, w:].any()
+    S.check_tiles(res["tiles"], {k: want[k] for k in res["tiles"]}, S.regime(tables, mask), f"seed {seed}")
