@@ -43,7 +43,8 @@ class TileStrip(C.Structure):
     _fields_ = [("tile_row0", C.c_int), ("n_tile_rows", C.c_int), ("tiles_x", C.c_int), ("n_planes", C.c_int),
                 ("plane_ids", C.POINTER(C.c_int)), ("offsets", C.POINTER(C.c_uint64)),
                 ("sizes", C.POINTER(C.c_uint32)), ("blob", C.POINTER(C.c_uint8)), ("blob_bytes", C.c_size_t),
-                ("level", C.c_int), ("level_w", C.c_int), ("level_h", C.c_int), ("aggregate", C.c_int)]
+                ("level", C.c_int), ("level_w", C.c_int), ("level_h", C.c_int), ("aggregate", C.c_int),
+                ("framed", C.c_int)]
 
 
 def _tile_collector(tiles, overviews, total, on_strip=None, aggregate=None):

@@ -115,6 +115,8 @@ struct gcn10_ctx {
     int inflate_probe = 0;      // measurement aid for tools/inflate_bench.py (see InflateParams::probe)
     int fused = 1;              // compressed-tile calls use cn_deflate_fused_kernel (0 = CN kernel + tile encoder)
     int ordered = 0;            // 1 = strips are re-laid in table order before they leave the device
+    int cog = 0;                // 1 = Cloud Optimized GeoTIFF order: overview levels first, smallest first; with
+                                // "ordered" every tile also gets its block leader and trailer on the device
     int ship = 0;               // 1 = strips leave through ship_strip_kernel; 0 = size read-back, then a D2H copy of that size
                                 // (measured on B200: 11.8 vs 12.2 ms per block -- the copy engine does not compete for SMs)
     DevBuf fused_tab;           // idmap [256][16] | val [256][32] | lit9 [256][6] u64
@@ -325,11 +327,25 @@ constexpr int kShipCtas = 2 * 148;
 // 16-byte boundary -- before it leaves the device, so that the consumer can write a plane's share of the strip (or a
 // whole tile row of it) to its GeoTIFF with ONE write instead of one per tile.  Two small kernels behind the
 // encoder: an exclusive scan of the rounded sizes (one CTA) and a warp-per-tile copy.  The total is unchanged.
+//
+// FRAMED (options "cog" and "ordered"): every stream also gets the block leader and trailer of a Cloud Optimized
+// GeoTIFF -- its byte count as a uint32 LE in the 4 bytes before it, its last 4 bytes repeated after it.  A tile's slot
+// is round16(size + 8): [stream | trailer | zero padding | the NEXT tile's leader], and the first tile's leader sits
+// in the strip's first 16 bytes, so every stream still starts on a 16-byte boundary and the uint4 copy stays.  The
+// total changes: the scan writes it to the word `cursor` points at (the table's second 8 bytes), 0 when the re-laid
+// strip does not fit the second arena.
+template <bool FRAMED>
+__device__ __forceinline__ unsigned long long laid_bytes(uint32_t size)
+{
+    return ((unsigned long long)size + (FRAMED ? 8ull : 0ull) + 15ull) & ~15ull;
+}
+
+template <bool FRAMED>
 __global__ void __launch_bounds__(1024)
 order_scan_kernel(const uint32_t *__restrict__ sizes, int n, unsigned long long *__restrict__ new_off,
-                  const unsigned long long *__restrict__ cursor, unsigned long long cap2)
+                  unsigned long long *__restrict__ cursor, unsigned long long cap2)
 {
-    if (*cursor > cap2)
+    if (!FRAMED && *cursor > cap2)
         return;                 // the strip does not fit the second arena: it leaves unordered
     __shared__ unsigned long long s_part[32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -337,7 +353,7 @@ order_scan_kernel(const uint32_t *__restrict__ sizes, int n, unsigned long long 
     const int i0 = tid * per, i1 = min(n, i0 + per);
     unsigned long long sum = 0;
     for (int i = i0; i < i1; i++)
-        sum += ((unsigned long long)sizes[i] + 15ull) & ~15ull;
+        sum += laid_bytes<FRAMED>(sizes[i]);
     unsigned long long inc = sum;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -359,28 +375,55 @@ order_scan_kernel(const uint32_t *__restrict__ sizes, int n, unsigned long long 
         s_part[lane] = w - v;
     }
     __syncthreads();
-    unsigned long long at = s_part[warp] + inc - sum;
+    unsigned long long at = s_part[warp] + inc - sum + (FRAMED ? 16ull : 0ull);
     for (int i = i0; i < i1; i++) {
         new_off[i] = at;
-        at += ((unsigned long long)sizes[i] + 15ull) & ~15ull;
+        at += laid_bytes<FRAMED>(sizes[i]);
     }
+    if (FRAMED && tid == 1023)
+        *cursor = at <= cap2 ? at : 0ull;
 }
 
+template <bool FRAMED>
 __global__ void __launch_bounds__(256)
 order_copy_kernel(const uint8_t *__restrict__ blob, unsigned long long *__restrict__ offsets, const uint32_t *__restrict__ sizes,
                   const unsigned long long *__restrict__ new_off, uint8_t *__restrict__ blob2, int n,
                   const unsigned long long *__restrict__ cursor, unsigned long long cap2)
 {
-    if (*cursor > cap2)
+    if (FRAMED ? *cursor == 0ull : *cursor > cap2)
         return;
     const int lane = threadIdx.x & 31;
     const int warps = (gridDim.x * blockDim.x) >> 5;
     for (int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += warps) {
         const uint4 *src = reinterpret_cast<const uint4 *>(blob + offsets[i]);
         uint4 *dst = reinterpret_cast<uint4 *>(blob2 + new_off[i]);
-        const uint32_t n16 = (sizes[i] + 15u) >> 4;
+        const uint32_t size = sizes[i];
+        const uint32_t n16 = FRAMED ? size >> 4 : (size + 15u) >> 4;
         for (uint32_t k = lane; k < n16; k += 32u)
             dst[k] = src[k];
+        if (FRAMED) {
+            // the slot's last one or two words: the stream's tail, the trailer, zeros, the next tile's leader
+            const uint8_t *sb = blob + offsets[i];
+            const uint32_t end = (uint32_t)laid_bytes<true>(size);
+            const uint32_t lead = i + 1 < n ? sizes[i + 1] : 0u;
+            for (uint32_t k = n16 + lane; k < end >> 4; k += 32u) {
+                uint32_t v[4];
+#pragma unroll
+                for (int q = 0; q < 4; q++) {
+                    v[q] = 0u;
+#pragma unroll
+                    for (int b = 0; b < 4; b++) {
+                        const uint32_t p = k * 16u + (uint32_t)(q * 4 + b);
+                        const uint32_t byte = p < size + 4u ? (uint32_t)sb[p < size ? p : p - 4u]
+                                              : p >= end - 4u ? (lead >> (8u * (p - (end - 4u)))) & 255u : 0u;
+                        v[q] |= byte << (8 * b);
+                    }
+                }
+                dst[k] = make_uint4(v[0], v[1], v[2], v[3]);
+            }
+            if (i == 0 && lane == 0)
+                reinterpret_cast<uint4 *>(blob2)[0] = make_uint4(0u, 0u, 0u, size);     // the first tile's leader
+        }
         __syncwarp();
         if (lane == 0)
             offsets[i] = new_off[i];
@@ -879,6 +922,7 @@ int gcn10_cuda_set_option(gcn10_ctx *c, const char *key, long value)
     else if (!strcmp(key, "fused") && (value == 0 || value == 1)) c->fused = (int)value;
     else if (!strcmp(key, "ship") && (value == 0 || value == 1)) c->ship = (int)value;
     else if (!strcmp(key, "ordered") && (value == 0 || value == 1)) c->ordered = (int)value;
+    else if (!strcmp(key, "cog") && (value == 0 || value == 1)) c->cog = (int)value;
     else if (!strcmp(key, "overviews") && value >= 0 && value <= GCN10_MAX_OVERVIEWS) {
         c->overviews = (int)value;
         c->blk_next = -1;
@@ -1220,13 +1264,46 @@ int gcn10_cuda_block_rows(gcn10_ctx *c,
     return gcn10_cuda_wait(ev);
 }
 
+static int deflate_rows_impl(gcn10_ctx *c,
+                             const uint8_t *esa, size_t esa_pitch, const uint8_t *d_esa, size_t d_esa_pitch,
+                             cudaEvent_t esa_ready, int w, int h, int row0, int nrows,
+                             const double gt[6],
+                             const uint8_t *hsg, int hsx, int hsy, size_t hsg_pitch, const double soil_gt[6],
+                             unsigned plane_mask, gcn10_tile_sink sink, void *user,
+                             const std::function<int()> &before_first_sink = nullptr);
+static int free_slot(gcn10_ctx *c, TileSlot **out);
+
 int gcn10_cuda_block_deflate(gcn10_ctx *c,
                              const uint8_t *esa, int w, int h, size_t esa_pitch, const double gt[6],
                              const uint8_t *hsg, int hsx, int hsy, size_t hsg_pitch, const double soil_gt[6],
                              unsigned plane_mask, gcn10_tile_sink sink, void *user)
 {
-    return gcn10_cuda_block_deflate_rows(c, esa, w, h, 0, h, esa_pitch, gt, hsg, hsx, hsy, hsg_pitch, soil_gt,
-                                         plane_mask, sink, user);
+    if (!c || !c->cog)
+        return gcn10_cuda_block_deflate_rows(c, esa, w, h, 0, h, esa_pitch, gt, hsg, hsx, hsy, hsg_pitch, soil_gt,
+                                             plane_mask, sink, user);
+    // option "cog": the levels are made before the first strip, so the whole raster goes to the device first, into the
+    // land-cover plane of a tile slot that holds no prefetched block; from there the block runs as the tiles path does
+    int rc = check_geometry(esa, w, h, esa_pitch, gt, hsg, hsx, hsy, hsg_pitch, soil_gt, plane_mask, (const void *)sink,
+                            (size_t)w);
+    if (rc)
+        return rc;
+    if (!c->have_lut)
+        return fail(GCN10_ENOLUT, "gcn10_cuda_set_luts() has not been called");
+    if (c->pending_events)
+        return fail(GCN10_EINVAL, "asynchronous blocks are pending on this context: gcn10_cuda_wait() for them first");
+    CUDA_TRY(cudaSetDevice(c->device));
+    TileSlot *sl = nullptr;
+    if ((rc = free_slot(c, &sl)))
+        return rc;
+    const size_t dpitch = round_up((size_t)w, 256);
+    if ((rc = ensure(sl->esa_full, dpitch * (size_t)h)))
+        return rc;
+    // (on the upload stream: a dropped prefetch of this slot may still have work on the plane queued there)
+    CUDA_TRY(cudaMemcpy2DAsync(sl->esa_full.p, dpitch, esa, esa_pitch, (size_t)w, (size_t)h, cudaMemcpyHostToDevice,
+                               c->pre_stream));
+    CUDA_TRY(cudaEventRecord(sl->done, c->pre_stream));
+    return deflate_rows_impl(c, nullptr, 0, (const uint8_t *)sl->esa_full.p, dpitch, sl->done, w, h, 0, h, gt, hsg, hsx,
+                             hsy, hsg_pitch, soil_gt, plane_mask, sink, user);
 }
 
 // Strips of whole tile rows: [H2D of the land-cover rows ->] Curve Number kernel -> tile DEFLATE -> D2H of
@@ -1267,7 +1344,7 @@ static int deflate_rows_impl(gcn10_ctx *c,
                              const double gt[6],
                              const uint8_t *hsg, int hsx, int hsy, size_t hsg_pitch, const double soil_gt[6],
                              unsigned plane_mask, gcn10_tile_sink sink, void *user,
-                             const std::function<int()> &before_first_sink = nullptr)
+                             const std::function<int()> &before_first_sink)
 {
     if (!c)
         return fail(GCN10_EINVAL, "NULL context");
@@ -1284,6 +1361,11 @@ static int deflate_rows_impl(gcn10_ctx *c,
         return fail(GCN10_ENOLUT, "gcn10_cuda_set_luts() has not been called");
     if (c->pending_events)
         return fail(GCN10_EINVAL, "asynchronous blocks are pending on this context: gcn10_cuda_wait() for them first");
+    // option "cog": the levels come first, so the whole block's land cover must be on the device before the first strip
+    // (the callers upload or inflate it there)
+    const bool cog = c->cog;
+    if (cog && (!d_esa || row0 != 0 || nrows != h))
+        return fail(GCN10_EINVAL, "option cog: the block must be resident on the device and handed over in one call");
     // options "overviews", "stats" and "aggregate": every band feeds the block's levels, histograms and mean rasters, so
     // the bands of a block must come in order and without gaps (with "stats" or "aggregate" also with the same planes);
     // the band that ends the block emits the levels and the mean rasters and completes the histograms
@@ -1389,7 +1471,8 @@ static int deflate_rows_impl(gcn10_ctx *c,
     const int strip = std::max(kTile, std::min(c->strip_rows, (int)round_up((size_t)nrows, kTile)) / kTile * kTile);
     const int tiles_x = (w + kTile - 1) / kTile;
     // the strips of this call: the band's full-resolution rows; then, when the band ends the block, every overview
-    // level, level 1 first, in strips of at most `lstrip` level rows (they use the same slots, at most tiles_x wide)
+    // level, level 1 first, in strips of at most `lstrip` level rows (they use the same slots, at most tiles_x wide).
+    // With option "cog" the levels come first instead, the smallest first (nlev .. 1), then the full resolution.
     struct StripJob {
         int level, y0, rows, w, h, y_base;      // y0: row in the caller's band (level 0) or in the level
         const uint8_t *d_esa;                   // nullptr: staged from the caller's host raster
@@ -1398,17 +1481,22 @@ static int deflate_rows_impl(gcn10_ctx *c,
         int agg;                                // a strip of the mean rasters (d_esa: their first row)
     };
     std::vector<StripJob> jobs;
-    for (int y0 = 0; y0 < nrows; y0 += strip)
-        jobs.push_back({ 0, y0, std::min(strip, nrows - y0), w, h, row0 + y0,
-                         d_esa ? d_esa + (size_t)y0 * d_esa_pitch : nullptr, d_esa_pitch, nullptr, nullptr });
     const int lstrip = emit_levels ? std::max(kTile, std::min(c->strip_rows, (int)round_up((size_t)c->ov_h[0], kTile)) / kTile * kTile)
                                    : 0;
-    for (int k = 0; k < (emit_levels ? nlev : 0); k++) {
+    auto push_level = [&](int k) {
         const OverviewLevel &L = c->ov_lv[k];
         for (int y0 = 0; y0 < c->ov_h[k]; y0 += lstrip)
             jobs.push_back({ k + 1, y0, std::min(lstrip, c->ov_h[k] - y0), L.w, c->ov_h[k], y0,
                              L.esa + (size_t)y0 * L.pitch, L.pitch, L.col_idx, L.row_idx });
-    }
+    };
+    for (int k = (cog && emit_levels ? nlev : 0) - 1; k >= 0; k--)
+        push_level(k);
+    const int first_full = (int)jobs.size();
+    for (int y0 = 0; y0 < nrows; y0 += strip)
+        jobs.push_back({ 0, y0, std::min(strip, nrows - y0), w, h, row0 + y0,
+                         d_esa ? d_esa + (size_t)y0 * d_esa_pitch : nullptr, d_esa_pitch, nullptr, nullptr });
+    for (int k = 0; k < (!cog && emit_levels ? nlev : 0); k++)
+        push_level(k);
     // then, when the band ends the block, the mean rasters in strips of at most `astrip` cell rows
     const int astrip = emit_agg ? std::max(kTile, std::min(c->strip_rows, (int)round_up((size_t)ach, kTile)) / kTile * kTile) : 0;
     const int first_agg = (int)jobs.size();
@@ -1480,17 +1568,33 @@ static int deflate_rows_impl(gcn10_ctx *c,
 
     // behind the encoder on the strip's stream: either the ship kernel (exact bytes + tables straight into the
     // page-locked arena, nothing for the host to do but wait), or the table read-back of the two-phase path
+    // option "cog" with "ordered": the re-laid strip carries every tile's leader and trailer, and its size is the table's
+    // second word (framed_bytes; 0 = it did not fit the second arena and leaves unordered and unframed)
+    const bool framed = cog && c->ordered;
     auto hand_over = [&](StripSlot &sl, cudaStream_t st) -> int {
         CUDA_TRY(cudaEventRecord(sl.k1, st));
+        unsigned long long *framed_bytes = (unsigned long long *)sl.table.p + 1;
         if (c->ordered) {
             const int n = nplanes * ((sl.rows + kTile - 1) / kTile) * sl.tiles_x;
             unsigned long long *d_offsets = (unsigned long long *)((uint8_t *)sl.table.p + 16);
             const uint32_t *d_sizes = (const uint32_t *)((uint8_t *)sl.table.p + 16 + ntile_slot * sizeof(unsigned long long));
-            order_scan_kernel<<<1, 1024, 0, st>>>(d_sizes, n, (unsigned long long *)sl.order.p,
-                                                  (const unsigned long long *)sl.table.p, (unsigned long long)blob2_cap);
-            order_copy_kernel<<<2 * c->sm_count, 256, 0, st>>>((const uint8_t *)sl.blob.p, d_offsets, d_sizes,
-                                                              (const unsigned long long *)sl.order.p, (uint8_t *)sl.blob2.p, n,
-                                                              (const unsigned long long *)sl.table.p, (unsigned long long)blob2_cap);
+            if (framed) {
+                order_scan_kernel<true><<<1, 1024, 0, st>>>(d_sizes, n, (unsigned long long *)sl.order.p, framed_bytes,
+                                                            (unsigned long long)blob2_cap);
+                order_copy_kernel<true><<<2 * c->sm_count, 256, 0, st>>>((const uint8_t *)sl.blob.p, d_offsets, d_sizes,
+                                                                         (const unsigned long long *)sl.order.p,
+                                                                         (uint8_t *)sl.blob2.p, n, framed_bytes,
+                                                                         (unsigned long long)blob2_cap);
+            }
+            else {
+                order_scan_kernel<false><<<1, 1024, 0, st>>>(d_sizes, n, (unsigned long long *)sl.order.p,
+                                                             (unsigned long long *)sl.table.p, (unsigned long long)blob2_cap);
+                order_copy_kernel<false><<<2 * c->sm_count, 256, 0, st>>>((const uint8_t *)sl.blob.p, d_offsets, d_sizes,
+                                                                          (const unsigned long long *)sl.order.p,
+                                                                          (uint8_t *)sl.blob2.p, n,
+                                                                          (const unsigned long long *)sl.table.p,
+                                                                          (unsigned long long)blob2_cap);
+            }
             c->launches += 2;
             CUDA_TRY(cudaGetLastError());
         }
@@ -1499,7 +1603,8 @@ static int deflate_rows_impl(gcn10_ctx *c,
         if (c->ship) {
             cudaStream_t ss = c->ship_streams[&sl - c->slots];
             CUDA_TRY(cudaStreamWaitEvent(ss, sl.k2, 0));
-            ship_strip_kernel<<<kShipCtas, kShipThreads, 0, ss>>>((const uint4 *)out_blob, (const unsigned long long *)sl.table.p,
+            ship_strip_kernel<<<kShipCtas, kShipThreads, 0, ss>>>((const uint4 *)out_blob,
+                                                                  framed ? framed_bytes : (const unsigned long long *)sl.table.p,
                                                                   (const uint32_t *)sl.table.p, (uint32_t)(table_bytes / 4),
                                                                   (uint4 *)sl.h_blob.p,
                                                                   (unsigned long long)(sl.h_blob.cap & ~(size_t)15),
@@ -1513,6 +1618,42 @@ static int deflate_rows_impl(gcn10_ctx *c,
             CUDA_TRY(cudaEventRecord(sl.enc_done, st));
         }
         sl.busy = true;
+        return GCN10_OK;
+    };
+
+    // the overview levels' share of block rows [y_base, y_base + rows) of the land cover at src: one launch
+    auto decimate = [&](const uint8_t *src, size_t src_pitch, int y_base, int rows, cudaStream_t st) -> int {
+        OverviewParams op;
+        memset(&op, 0, sizeof(op));
+        op.src = src;
+        op.src_pitch = src_pitch;
+        op.src_y0 = y_base;
+        op.w = w;
+        op.h = h;
+        op.col_idx = (const int32_t *)c->col_idx.p;
+        op.row_idx = (const int32_t *)c->row_idx.p;
+        op.with_cols = y_base == 0;
+        op.nlev = nlev;
+        // level row i samples block row R(i), which is non-decreasing in i: the first level row at or below block row y
+        auto first_row = [&](int y, int k) -> int {
+            const int hk = c->ov_h[k - 1];
+            if (y >= h)
+                return hk;
+            const long long f = 1LL << k, a = (long long)y - f / 2;
+            return a <= 0 ? 0 : (int)std::min<long long>(hk, (a + f - 1) / f);
+        };
+        long long most = 0;
+        for (int k = 1; k <= nlev; k++) {
+            op.lv[k - 1] = c->ov_lv[k - 1];
+            op.lv[k - 1].i_lo = first_row(y_base, k);
+            op.lv[k - 1].i_hi = first_row(y_base + rows, k);
+            most = std::max(most, (long long)(op.lv[k - 1].i_hi - op.lv[k - 1].i_lo) * ((op.lv[k - 1].w + 3) / 4));
+        }
+        most = std::max<long long>(most, op.with_cols ? round_up((size_t)op.lv[0].w, kVecPx) : 1);
+        const int blocks = (int)std::max<long long>(1, std::min<long long>((most + 255) / 256, (long long)c->sm_count * 8));
+        overview_decimate_kernel<<<dim3(blocks, nlev), 256, 0, st>>>(op);
+        c->launches++;
+        CUDA_TRY(cudaGetLastError());
         return GCN10_OK;
     };
 
@@ -1536,39 +1677,11 @@ static int deflate_rows_impl(gcn10_ctx *c,
         if (!jb.d_esa)
             CUDA_TRY(cudaMemcpy2DAsync(sl.esa.p, dpitch, esa + (size_t)y0 * esa_pitch, esa_pitch, (size_t)w, (size_t)rows,
                                        cudaMemcpyHostToDevice, st));
-        if (nlev && jb.level == 0 && !jb.agg) {
+        if (nlev && jb.level == 0 && !jb.agg && !cog) {
             // the overview levels' share of this strip, while its land cover is on the device
-            OverviewParams op;
-            memset(&op, 0, sizeof(op));
-            op.src = strip_esa;
-            op.src_pitch = strip_esa_pitch;
-            op.src_y0 = jb.y_base;
-            op.w = w;
-            op.h = h;
-            op.col_idx = (const int32_t *)c->col_idx.p;
-            op.row_idx = (const int32_t *)c->row_idx.p;
-            op.with_cols = jb.y_base == 0;
-            op.nlev = nlev;
-            // level row i samples block row R(i), which is non-decreasing in i: the first level row at or below block row y
-            auto first_row = [&](int y, int k) -> int {
-                const int hk = c->ov_h[k - 1];
-                if (y >= h)
-                    return hk;
-                const long long f = 1LL << k, a = (long long)y - f / 2;
-                return a <= 0 ? 0 : (int)std::min<long long>(hk, (a + f - 1) / f);
-            };
-            long long most = 0;
-            for (int k = 1; k <= nlev; k++) {
-                op.lv[k - 1] = c->ov_lv[k - 1];
-                op.lv[k - 1].i_lo = first_row(jb.y_base, k);
-                op.lv[k - 1].i_hi = first_row(jb.y_base + rows, k);
-                most = std::max(most, (long long)(op.lv[k - 1].i_hi - op.lv[k - 1].i_lo) * ((op.lv[k - 1].w + 3) / 4));
-            }
-            most = std::max<long long>(most, op.with_cols ? round_up((size_t)op.lv[0].w, kVecPx) : 1);
-            const int blocks = (int)std::max<long long>(1, std::min<long long>((most + 255) / 256, (long long)c->sm_count * 8));
-            overview_decimate_kernel<<<dim3(blocks, nlev), 256, 0, st>>>(op);
-            c->launches++;
-            CUDA_TRY(cudaGetLastError());
+            const int r2 = decimate(strip_esa, strip_esa_pitch, jb.y_base, rows, st);
+            if (r2)
+                return r2;
             CUDA_TRY(cudaEventRecord(sl.ov, st));
         }
         else if (jb.level) {
@@ -1621,8 +1734,9 @@ static int deflate_rows_impl(gcn10_ctx *c,
         // launched side by side on all streams they would all finish together, and the copy of strip 0 -- the head of
         // the chain of copies that ends the block -- would wait for the others.
         // Overview strips are not chained: their grids are small (level k has 1/4^k of the tiles), one alone leaves
-        // most SMs idle, and they end the block, so no later copy waits on them.
-        if (s >= 2 && jb.level == 0 && !jb.agg)
+        // most SMs idle, and they end the block, so no later copy waits on them (with option "cog" they start it, and
+        // the chain begins with the first full-resolution strip).
+        if (s - 2 >= first_full && jb.level == 0 && !jb.agg)
             CUDA_TRY(cudaStreamWaitEvent(st, c->slots[(s - 2) % ns].k1, 0));
         CUDA_TRY(cudaEventRecord(sl.k0, st));
         if (fused && !jb.agg) {
@@ -1731,6 +1845,14 @@ static int deflate_rows_impl(gcn10_ctx *c,
             }
         return GCN10_OK;
     };
+    if (cog && emit_levels) {
+        // the whole plane is resident: one decimation over rows [0, h), behind the land cover (esa_ready) on stream 0,
+        // before the first level strip; the level strips wait for every slot's mark
+        if ((rc = decimate(d_esa, d_esa_pitch, 0, h, c->streams[0])))
+            return bail(rc);
+        for (int i = 0; i < ns; i++)
+            CUDA_TRY(cudaEventRecord(c->slots[i].ov, c->streams[0]));
+    }
     for (int s = 0; s < std::min(ns, nstrips); s++)
         if ((rc = issue(s)) || (rc = release(s)))
             return bail(rc);
@@ -1746,12 +1868,15 @@ static int deflate_rows_impl(gcn10_ctx *c,
         const size_t used = (size_t) * (const unsigned long long *)sl.h_table.p;
         if (used > blob_cap)
             return bail(fail(GCN10_ECUDA, "tile encoder overran its arena (%zu > %zu)", used, blob_cap));
-        if (!c->ship || used > (sl.h_blob.cap & ~(size_t)15) || (c->ordered && used > blob2_cap)) {
-            // two-phase path, or a strip that outgrew the host arena: (grow it and) copy exactly `used` bytes
-            if ((rc = ensure_host(sl.h_blob, used ? used + used / 4 : 16)))
+        // where the strip leaves from: the re-laid copy when it fit the second arena, with framed_bytes bytes when framed
+        const size_t laid = framed ? (size_t)((const unsigned long long *)sl.h_table.p)[1] : 0;
+        const bool relaid = c->ordered && (framed ? laid != 0 : used <= blob2_cap);
+        const size_t bytes = relaid && framed ? laid : used;
+        if (!c->ship || bytes > (sl.h_blob.cap & ~(size_t)15) || (c->ordered && !relaid)) {
+            // two-phase path, or a strip that outgrew the host arena: (grow it and) copy exactly `bytes` bytes
+            if ((rc = ensure_host(sl.h_blob, bytes ? bytes + bytes / 4 : 16)))
                 return bail(rc);
-            ce = cudaMemcpyAsync(sl.h_blob.p, (c->ordered && used <= blob2_cap) ? sl.blob2.p : sl.blob.p, used,
-                                 cudaMemcpyDeviceToHost, st);
+            ce = cudaMemcpyAsync(sl.h_blob.p, relaid ? sl.blob2.p : sl.blob.p, bytes, cudaMemcpyDeviceToHost, st);
             if (ce == cudaSuccess)
                 ce = cudaStreamSynchronize(st);
             if (ce != cudaSuccess)
@@ -1770,11 +1895,12 @@ static int deflate_rows_impl(gcn10_ctx *c,
         ts.offsets = (const uint64_t *)((const uint8_t *)sl.h_table.p + 16);
         ts.sizes = (const uint32_t *)((const uint8_t *)sl.h_table.p + 16 + ntile_slot * sizeof(unsigned long long));
         ts.blob = (const uint8_t *)sl.h_blob.p;
-        ts.blob_bytes = used;
+        ts.blob_bytes = bytes;
         ts.level = sl.level;
         ts.level_w = sl.level_w;
         ts.level_h = sl.level_h;
         ts.aggregate = sl.agg;
+        ts.framed = framed && relaid;
         // NB: the tables are laid out [plane][strip_tile_rows (capacity)][tiles_x] only when the strip is
         // full; the kernel indexes with the strip's own tile_rows, which is what n_tile_rows reports
         const int sink_rc = sink(user, &ts);
@@ -1802,6 +1928,8 @@ int gcn10_cuda_block_deflate_rows(gcn10_ctx *c,
 {
     if (!esa)
         return fail(GCN10_EINVAL, "NULL argument");
+    if (c && c->cog)
+        return fail(GCN10_EINVAL, "option cog: a band does not hold the whole block; use gcn10_cuda_block_deflate");
     return deflate_rows_impl(c, esa, esa_pitch, nullptr, 0, nullptr, w, h, row0, nrows, gt, hsg, hsx, hsy, hsg_pitch,
                              soil_gt, plane_mask, sink, user);
 }
@@ -2016,6 +2144,22 @@ static int finish_slot(gcn10_ctx *c, TileSlot &sl, int *tile_status)
     return GCN10_OK;
 }
 
+// a slot without pending work (or, both pending, the older one, whose prefetch is dropped)
+static int free_slot(gcn10_ctx *c, TileSlot **out)
+{
+    TileSlot *sl = !c->tslot[0].pending ? &c->tslot[0] : !c->tslot[1].pending ? &c->tslot[1]
+                   : c->tslot[0].seq < c->tslot[1].seq ? &c->tslot[0] : &c->tslot[1];
+    if (sl->pending) {
+        if (sl->deferred)
+            sl->deferred = false;                       // never launched: its uploads drain in stream order
+        else
+            CUDA_TRY(cudaEventSynchronize(sl->done));
+        sl->pending = false;
+    }
+    *out = sl;
+    return GCN10_OK;
+}
+
 // the slot a call works with: the oldest prefetched one that matches, else a free one (inflated now)
 static int acquire_slot(gcn10_ctx *c, const gcn10_tile_part *parts, int nparts, int fill, int w, int h, TileSlot **out)
 {
@@ -2035,18 +2179,9 @@ static int acquire_slot(gcn10_ctx *c, const gcn10_tile_part *parts, int nparts, 
             hit = &sl;
     }
     if (!hit) {
-        // not prefetched: take the slot without pending work (or, both pending, drop the older prefetch)
-        TileSlot *sl = !c->tslot[0].pending ? &c->tslot[0] : !c->tslot[1].pending ? &c->tslot[1]
-                       : c->tslot[0].seq < c->tslot[1].seq ? &c->tslot[0] : &c->tslot[1];
-        if (sl->pending) {
-            if (sl->deferred)
-                sl->deferred = false;                       // never launched: its uploads drain in stream order
-            else
-                CUDA_TRY(cudaEventSynchronize(sl->done));
-            sl->pending = false;
-        }
-        int rc = inflate_to_device(c, *sl, parts, nparts, fill, w, h);
-        if (rc)
+        TileSlot *sl = nullptr;
+        int rc = free_slot(c, &sl);
+        if (rc || (rc = inflate_to_device(c, *sl, parts, nparts, fill, w, h)))
             return rc;
         hit = sl;
     }

@@ -156,6 +156,10 @@ void gh_raster_close(gh_raster *r);
  * COMPRESS=DEFLATE (zlib level 6, no predictor), geotransform + EPSG:4326 keys, no NoData tag. */
 int gh_tiff_write(const char *path, const uint8_t *data, int w, int h, size_t pitch, const double gt[6],
                   int threads, char *err, size_t errlen);
+/* The same raster as a Cloud Optimized GeoTIFF (gh_tiffw_set_cog) with up to `overviews` overview levels
+ * (gcn10_overview_levels), sampled on the host and written smallest first, then the full resolution. */
+int gh_tiff_write_cog(const char *path, const uint8_t *data, int w, int h, size_t pitch, const double gt[6], int overviews,
+                      int threads, char *err, size_t errlen);
 
 /* ---- logging (log.c) ----------------------------------------------------------------------- */
 
@@ -178,6 +182,7 @@ typedef struct {
     int overviews;              /* --overviews: at most this many overview levels per output (0 = none) */
     int stats;                  /* --stats: NoData tag and band statistics in every output                   */
     int aggregate;              /* --aggregate f: also the f x f mean rasters, in cn_rasters_<cond>_agg<f>/ (0 = none) */
+    int cog;                    /* --cog: every output (and mean raster) as a Cloud Optimized GeoTIFF               */
 } gh_run_options;
 
 /* Runs a list of blocks on the GPUs of this box: one worker thread (+ one gcn10_ctx) per GPU, block

@@ -42,6 +42,9 @@ static void usage(FILE *fp)
             "  --aggregate <f>	also write the f x f mean of every output (the composite Curve Number of\n"
             "			cells of f x f pixels, nodata 255 left out; f = 2..1024, 25 = the 250 m soil\n"
             "			grid) to cn_rasters_<condition>_agg<f>/, computed on the GPU\n"
+            "  --cog		write every output as a Cloud Optimized GeoTIFF: header first, overview\n"
+            "			levels before the full resolution (turns --overviews on), tiles framed as\n"
+            "			GDAL's COG driver frames them; with --aggregate the mean rasters too\n"
             "  --help, -h		show this help and exit\n"
             "  --version, -v	print version and exit\n"
             "\n"
@@ -86,6 +89,8 @@ int main(int argc, char **argv)
             opt.overviews = GCN10_MAX_OVERVIEWS;
         else if (!strcmp(argv[i], "--stats"))
             opt.stats = 1;
+        else if (!strcmp(argv[i], "--cog"))
+            opt.cog = 1;
         else if (!strcmp(argv[i], "--aggregate") && i + 1 < argc) {
             char *end = NULL;
             const long f = strtol(argv[++i], &end, 10);
@@ -99,6 +104,18 @@ int main(int argc, char **argv)
     if (!conf) {
         fprintf(stderr, "[rank 0] missing -c/--config <file>; see 'gcn10 -h' for usage.\n");    /* main.c:103-107 */
         return 1;
+    }
+    if (opt.cog) {
+        /* a COG's levels come before its full resolution: the GPU makes them from the whole block first.  The
+         * host-deflate path encodes band by band on the host and cannot. */
+        const char *hd = getenv("GCN10_HOST_DEFLATE");
+        if (hd && *hd && *hd != '0') {
+            fprintf(stderr, "[rank 0] --cog cannot be combined with GCN10_HOST_DEFLATE=1: that diagnostic path encodes "
+                            "the outputs band by band on the host, and a COG's overview levels must precede its full "
+                            "resolution\n");
+            return 1;
+        }
+        opt.overviews = GCN10_MAX_OVERVIEWS;
     }
     char err[GH_ERRLEN] = "";
     if (gh_config_parse(conf, &opt.cfg, err, sizeof err)) {

@@ -98,6 +98,8 @@ typedef struct worker {
     size_t pitch_cap;
     int have_planes;
     band_buf bands[2];
+    uint8_t *whole;                 /* --cog, land cover decoded on the host: the whole window, pinned */
+    size_t whole_cap;
     /* encoder hand-off */
     pthread_mutex_t mu;
     pthread_cond_t cv;
@@ -206,7 +208,8 @@ static int open_agg_writers(worker *wk)
             gh_tiffw_set_geokeys(wk->agg_writers[k], &gk);
         pthread_mutex_unlock(&wk->rmu);
         wk->aggs[k] = gh_aggregate_new(wk->out_w, wk->out_h, f);
-        if (gh_tiffw_set_nodata(wk->agg_writers[k], 1) || !wk->aggs[k]) {
+        if (gh_tiffw_set_nodata(wk->agg_writers[k], 1) || (wk->opt->cog && gh_tiffw_set_cog(wk->agg_writers[k], 1)) ||
+            !wk->aggs[k]) {
             snprintf(err, sizeof err, "write error 3 on %s (aggregate)", wk->agg_paths[k]);
             gh_log_message(wk->log, "ERROR", err, 1);
             abort_agg_writers(wk);
@@ -238,8 +241,9 @@ static int open_writers(worker *wk)
             gh_tiffw_set_geokeys(wk->writers[k], &gk);
         pthread_mutex_unlock(&wk->rmu);
         opened++;
-        if (gh_tiffw_set_overviews(wk->writers[k], wk->opt->overviews) || gh_tiffw_set_stats(wk->writers[k], wk->opt->stats)) {
-            snprintf(err, sizeof err, "write error 3 on %s (overviews / stats)", wk->paths[k]);
+        if (gh_tiffw_set_overviews(wk->writers[k], wk->opt->overviews) || gh_tiffw_set_stats(wk->writers[k], wk->opt->stats) ||
+            (wk->opt->cog && gh_tiffw_set_cog(wk->writers[k], 1))) {
+            snprintf(err, sizeof err, "write error 3 on %s (overviews / stats / cog)", wk->paths[k]);
             gh_log_message(wk->log, "ERROR", err, 1);
             break;
         }
@@ -348,10 +352,11 @@ static void sink_plane(void *arg, int k)
     sink_job *j = arg;
     const gcn10_tile_strip *st = j->st;
     gh_tiffw *tw = st->aggregate ? j->wk->agg_writers[st->plane_ids[k]] : j->wk->writers[st->plane_ids[k]];
-    /* the context runs with "ordered" strips: a plane's share of the strip is one contiguous piece of the blob */
+    /* the context runs with "ordered" strips: a plane's share of the strip is one contiguous piece of the blob (with
+     * --cog framed on the device already, unless the strip left unordered) */
     size_t base = (size_t)k * st->n_tile_rows * (size_t)st->tiles_x;
-    if (gh_tiffw_put_level_tile_rows(tw, st->level, st->tile_row0, st->n_tile_rows, st->blob, st->offsets + base,
-                                     st->sizes + base))
+    if ((st->framed ? gh_tiffw_put_framed_tile_rows : gh_tiffw_put_level_tile_rows)(tw, st->level, st->tile_row0, st->n_tile_rows,
+                                                                                   st->blob, st->offsets + base, st->sizes + base))
         atomic_store(&j->wk->encode_failed, 1);
 }
 
@@ -461,6 +466,43 @@ static int block_gpu_tiles(worker *wk, const block_input *in, double *t_gpu)
         snprintf(msg, sizeof msg, "cuda failure on block %d: %s", in->block_id, gcn10_cuda_last_error());
         fatal(wk, msg);
     }
+    if (!rc)
+        put_gpu_histograms(wk);
+    return 0;
+}
+
+/* ---- --cog with land cover decoded on the host: a COG's levels come first, so the GPU needs the whole block before
+ * its first strip -- the window is read into one page-locked buffer (about 1.3 GB for 36001 x 36001) and handed to
+ * gcn10_cuda_block_deflate in one call.  Returns 0 ok, 1 = land-cover read failed (recoverable tier) */
+static int block_gpu_whole(worker *wk, int block_id, const gh_window *we, const uint8_t *hsg, const gh_window *wh,
+                           size_t pitch, double *t_read, double *t_gpu)
+{
+    char msg[1024], err[GH_ERRLEN] = "";
+    const int w = we->xcount, h = we->ycount;
+    if (wk->whole_cap < pitch * (size_t)h) {
+        gcn10_cuda_host_free(wk->whole);
+        wk->whole_cap = pitch * (size_t)h;
+        wk->whole = gcn10_cuda_host_alloc(wk->whole_cap);
+        if (!wk->whole) {
+            wk->whole_cap = 0;
+            snprintf(msg, sizeof msg, "pinned allocation failed for block %d: %s", block_id, gcn10_cuda_last_error());
+            fatal(wk, msg);
+        }
+    }
+    double t0 = now_s();
+    if (read_band(wk, we, 0, h, wk->whole, pitch, err, sizeof err)) {
+        gh_log_message(wk->log, "ERROR", err, 1);                                   /* raster.c:182-186 */
+        return 1;
+    }
+    double t1 = now_s();
+    int rc = gcn10_cuda_block_deflate(wk->ctx, wk->whole, w, h, pitch, we->gt, hsg, wh->xcount, wh->ycount,
+                                      (size_t)wh->xcount, wh->gt, GCN10_MASK_ALL, tile_sink, wk);
+    if (rc && !atomic_load(&wk->encode_failed)) {
+        snprintf(msg, sizeof msg, "cuda failure on block %d: %s", block_id, gcn10_cuda_last_error());
+        fatal(wk, msg);                             /* CUDA errors are the fatal tier; there is no CPU path */
+    }
+    *t_read += t1 - t0;
+    *t_gpu += now_s() - t1;
     if (!rc)
         put_gpu_histograms(wk);
     return 0;
@@ -714,7 +756,7 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
     const size_t pitch = ((size_t)w + 255) / 256 * 256;
     const char *hd = getenv("GCN10_HOST_DEFLATE");
     const int host_deflate = hd && *hd && *hd != '0';
-    if (!in->gpu_inflate && ensure_bands(wk, pitch, host_deflate)) {
+    if (!in->gpu_inflate && !wk->opt->cog && ensure_bands(wk, pitch, host_deflate)) {
         snprintf(msg, sizeof msg, "pinned allocation failed for block %d: %s", block_id, gcn10_cuda_last_error());
         fatal(wk, msg);
     }
@@ -755,6 +797,7 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
     double t_read = in->t_read, t_gpu = 0;
     int failed = in->gpu_inflate ? block_gpu_tiles(wk, in, &t_gpu)
                  : host_deflate ? bands_host_deflate(wk, block_id, we, in->hsg, wh, pitch, &t_read, &t_gpu)
+                 : wk->opt->cog ? block_gpu_whole(wk, block_id, we, in->hsg, wh, pitch, &t_read, &t_gpu)
                                 : bands_gpu_deflate(wk, block_id, we, in->hsg, wh, pitch, &t_read, &t_gpu);
 
     if (failed || !wk->writers_open) {
@@ -824,7 +867,7 @@ static void *worker_main(void *arg)
     if (gcn10_cuda_create(wk->device, &wk->ctx) || gcn10_cuda_set_luts(wk->ctx, wk->tables) ||
         gcn10_cuda_set_option(wk->ctx, "ordered", 1) || gcn10_cuda_set_option(wk->ctx, "ship", wk->n_gpus >= 4) ||
         gcn10_cuda_set_option(wk->ctx, "overviews", wk->opt->overviews) || gcn10_cuda_set_option(wk->ctx, "stats", wk->opt->stats) ||
-        gcn10_cuda_set_option(wk->ctx, "aggregate", wk->opt->aggregate)) {
+        gcn10_cuda_set_option(wk->ctx, "aggregate", wk->opt->aggregate) || gcn10_cuda_set_option(wk->ctx, "cog", wk->opt->cog)) {
         snprintf(msg, sizeof msg, "cannot initialise GPU %d: %s", wk->device, gcn10_cuda_last_error());
         fatal(wk, msg);
     }
@@ -866,6 +909,7 @@ static void *worker_main(void *arg)
         for (int k = 0; k < NPLANES; k++)
             gcn10_cuda_host_free(wk->bands[b].planes[k]);
     }
+    gcn10_cuda_host_free(wk->whole);
     for (int i = 0; i < LOAD_SLOTS; i++) {
         gcn10_cuda_host_free(wk->in[i].blob);
         free(wk->in[i].tile_off);

@@ -743,6 +743,10 @@ int gh_tiff_window_tiles_read(gh_tiff *t, const gh_tile_plan *plan, uint8_t *blo
 
 enum { TILE = 256 };
 
+static void put16(unsigned char **p, uint16_t v) { (*p)[0] = (unsigned char)v; (*p)[1] = (unsigned char)(v >> 8); *p += 2; }
+static void put32(unsigned char **p, uint32_t v) { for (int i = 0; i < 4; i++) (*p)[i] = (unsigned char)(v >> (8 * i)); *p += 4; }
+static void put_f64(unsigned char **p, double d) { uint64_t v; memcpy(&v, &d, 8); for (int i = 0; i < 8; i++) (*p)[i] = (unsigned char)(v >> (8 * i)); *p += 8; }
+
 /* the tile grid of one level of the file: level 0 = the full-resolution raster, k >= 1 = overview level k */
 typedef struct {
     int w, h;
@@ -768,6 +772,9 @@ struct gh_tiffw {
     int stats;                  /* gh_tiffw_set_stats: NoData tag + GDAL_METADATA statistics from hist */
     uint64_t hist[256];         /* full-resolution pixels per value */
     int nodata;                 /* gh_tiffw_set_nodata: NoData tag without statistics */
+    int cog;                    /* gh_tiffw_set_cog: Cloud Optimized GeoTIFF layout */
+    int cog_level;              /* ... the level whose tiles come next (nlev .. 0) */
+    uint64_t cog_data;          /* ... the first byte after the header region */
     int level;                  /* zlib level */
     int failed;
 };
@@ -814,6 +821,27 @@ static void compress_tile(void *arg, int index)
     }
     j->comp[index] = out;
     j->comp_len[index] = cap;
+}
+
+/* Appends one compressed tile as tile ti of grid g.  In a COG it is framed: its byte count as a uint32 LE before it,
+ * its last 4 bytes repeated after it (GDAL's BLOCK_LEADER=SIZE_AS_UINT4, BLOCK_TRAILER=LAST_4_BYTES_REPEATED); the
+ * tile's offset and byte count are those of the stream itself. */
+static int put_tile(gh_tiffw *tw, tw_grid *g, size_t ti, const uint8_t *z, uint32_t n)
+{
+    const uint32_t frame = tw->cog ? 8 : 0;
+    if (tw->pos + n + frame > 0xFFFFFFF0ull || (tw->cog && n < 4)) {
+        tw->failed = 1;
+        return -1;
+    }
+    unsigned char lead[4], *q = lead;
+    put32(&q, n);
+    if ((tw->cog && fwrite(lead, 1, 4, tw->fp) != 4) || fwrite(z, 1, n, tw->fp) != n ||
+        (tw->cog && fwrite(z + n - 4, 1, 4, tw->fp) != 4))
+        tw->failed = 1;
+    g->offsets[ti] = (uint32_t)(tw->pos + frame / 2);
+    g->counts[ti] = n;
+    tw->pos += n + frame;
+    return tw->failed ? -1 : 0;
 }
 
 static int grid_init(tw_grid *g, int w, int h)
@@ -878,7 +906,7 @@ int gh_tiffw_open(const char *path, int w, int h, const double gt[6], gh_tiffw *
 
 int gh_tiffw_set_geokeys(gh_tiffw *tw, const gh_geokeys *gk)
 {
-    if (!tw || !gk || !gk->keys || gk->n_keys < 4)
+    if (!tw || !gk || !gk->keys || gk->n_keys < 4 || tw->cog)
         return -1;
     free(tw->geo_keys);
     free(tw->geo_doubles);
@@ -938,7 +966,7 @@ int gh_tiffw_set_stats(gh_tiffw *tw, int on)
 
 int gh_tiffw_set_nodata(gh_tiffw *tw, int on)
 {
-    if (!tw || tw->failed || (on != 0 && on != 1))
+    if (!tw || tw->failed || (on != 0 && on != 1) || tw->cog)
         return -1;
     tw->nodata = on;
     return 0;
@@ -957,6 +985,17 @@ int gh_tiffw_put_histogram(gh_tiffw *tw, const uint64_t hist[256])
  * pixels other than 255 count, the standard deviation is the population one, VALID_PERCENT = 100 * valid / pixels.  A
  * plane without a valid pixel gets VALID_PERCENT 0 and nothing else.  The sums are exact integers: N * sum(v^2) needs
  * more than 64 bits at 36001 x 36001.  Returns the length of the NUL-terminated text, or -1 if cap is too small. */
+static const char k_stats_none[] =
+    "<GDALMetadata>\n  <Item name=\"STATISTICS_VALID_PERCENT\" sample=\"0\">%.17g</Item>\n</GDALMetadata>\n";
+static const char k_stats_all[] =
+    "<GDALMetadata>\n"
+    "  <Item name=\"STATISTICS_MAXIMUM\" sample=\"0\">%.17g</Item>\n"
+    "  <Item name=\"STATISTICS_MEAN\" sample=\"0\">%.17g</Item>\n"
+    "  <Item name=\"STATISTICS_MINIMUM\" sample=\"0\">%.17g</Item>\n"
+    "  <Item name=\"STATISTICS_STDDEV\" sample=\"0\">%.17g</Item>\n"
+    "  <Item name=\"STATISTICS_VALID_PERCENT\" sample=\"0\">%.17g</Item>\n"
+    "</GDALMetadata>\n";
+
 static int stats_metadata(const uint64_t hist[256], uint64_t pixels, char *out, size_t cap)
 {
     uint64_t valid = 0, sum = 0;
@@ -975,23 +1014,23 @@ static int stats_metadata(const uint64_t hist[256], uint64_t pixels, char *out, 
     const double pct = pixels ? 100.0 * (double)valid / (double)pixels : 0.0;
     int n;
     if (!valid) {
-        n = snprintf(out, cap, "<GDALMetadata>\n  <Item name=\"STATISTICS_VALID_PERCENT\" sample=\"0\">%.17g</Item>\n"
-                               "</GDALMetadata>\n", pct);
+        n = snprintf(out, cap, k_stats_none, pct);
     }
     else {
         const unsigned __int128 var_n2 = (unsigned __int128)valid * sum2 - (unsigned __int128)sum * sum;   /* N^2 var */
         const double mean = (double)sum / (double)valid, sd = sqrt((double)var_n2) / (double)valid;
-        n = snprintf(out, cap,
-                     "<GDALMetadata>\n"
-                     "  <Item name=\"STATISTICS_MAXIMUM\" sample=\"0\">%.17g</Item>\n"
-                     "  <Item name=\"STATISTICS_MEAN\" sample=\"0\">%.17g</Item>\n"
-                     "  <Item name=\"STATISTICS_MINIMUM\" sample=\"0\">%.17g</Item>\n"
-                     "  <Item name=\"STATISTICS_STDDEV\" sample=\"0\">%.17g</Item>\n"
-                     "  <Item name=\"STATISTICS_VALID_PERCENT\" sample=\"0\">%.17g</Item>\n"
-                     "</GDALMetadata>\n",
-                     (double)hi, mean, (double)lo, sd, pct);
+        n = snprintf(out, cap, k_stats_all, (double)hi, mean, (double)lo, sd, pct);
     }
     return n < 0 || (size_t)n >= cap ? -1 : n;
+}
+
+/* The most bytes stats_metadata can produce, its NUL included: every number at the longest %.17g prints (24
+ * characters: sign, 17 digits, point, a three-digit exponent).  A COG reserves this much before the data, because the
+ * statistics are only known at close. */
+static size_t stats_metadata_cap(void)
+{
+    const double x = -1.2345678901234567e-300;
+    return (size_t)snprintf(NULL, 0, k_stats_all, x, x, x, x, x) + 1;
 }
 
 /* Compresses the tile rows [0, rows) held in data (pitch bytes apart) as the next tile rows of grid g; with `count`
@@ -1019,13 +1058,8 @@ static int append_tile_rows(gh_tiffw *tw, tw_grid *g, const uint8_t *data, size_
     free(j.hist);
     for (int i = 0; i < n; i++) {
         size_t ti = (size_t)(g->next_tile_row + i / g->tiles_x) * (size_t)g->tiles_x + (size_t)(i % g->tiles_x);
-        if (!tw->failed && j.comp[i]) {
-            if (tw->pos + j.comp_len[i] > 0xFFFFFFF0ull || fwrite(j.comp[i], 1, j.comp_len[i], tw->fp) != j.comp_len[i])
-                tw->failed = 1;
-            g->offsets[ti] = (uint32_t)tw->pos;
-            g->counts[ti] = (uint32_t)j.comp_len[i];
-            tw->pos += j.comp_len[i];
-        }
+        if (!tw->failed && j.comp[i])
+            put_tile(tw, g, ti, j.comp[i], (uint32_t)j.comp_len[i]);
         free(j.comp[i]);
     }
     free(j.comp);
@@ -1037,7 +1071,7 @@ static int append_tile_rows(gh_tiffw *tw, tw_grid *g, const uint8_t *data, size_
 int gh_tiffw_write_rows(gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0, int nrows, int threads)
 {
     tw_grid *g0 = &tw->g[0];
-    if (tw->failed || y0 != g0->next_tile_row * TILE || y0 + nrows > g0->h ||
+    if (tw->failed || tw->cog || y0 != g0->next_tile_row * TILE || y0 + nrows > g0->h ||
         (nrows % TILE != 0 && y0 + nrows != g0->h))
         return -1;
     if (append_tile_rows(tw, g0, data, pitch, nrows, threads, tw->stats))
@@ -1074,23 +1108,31 @@ static int put_grid_tile_row(gh_tiffw *tw, tw_grid *g, int tile_row, const uint8
 {
     if (tw->failed || tile_row != g->next_tile_row || tile_row >= g->tiles_y)
         return -1;
-    for (int tx = 0; tx < g->tiles_x; tx++) {
-        size_t ti = (size_t)tile_row * (size_t)g->tiles_x + (size_t)tx;
-        if (tw->pos + sizes[tx] > 0xFFFFFFF0ull || fwrite(blob + offsets[tx], 1, sizes[tx], tw->fp) != sizes[tx]) {
-            tw->failed = 1;
+    for (int tx = 0; tx < g->tiles_x; tx++)
+        if (put_tile(tw, g, (size_t)tile_row * (size_t)g->tiles_x + (size_t)tx, blob + offsets[tx], sizes[tx]))
             return -1;
-        }
-        g->offsets[ti] = (uint32_t)tw->pos;
-        g->counts[ti] = sizes[tx];
-        tw->pos += sizes[tx];
-    }
     g->next_tile_row++;
+    return 0;
+}
+
+/* COG: the levels come smallest first (nlev .. 1), then the full resolution; anything else fails the file */
+static int cog_accepts(gh_tiffw *tw, int level)
+{
+    if (!tw->cog)
+        return 1;
+    while (tw->cog_level > 0 && tw->g[tw->cog_level].next_tile_row == tw->g[tw->cog_level].tiles_y)
+        tw->cog_level--;
+    if (level == tw->cog_level)
+        return 1;
+    tw->failed = 1;
     return 0;
 }
 
 int gh_tiffw_put_tile_row(gh_tiffw *tw, int tile_row, const uint8_t *blob, const uint64_t *offsets,
                           const uint32_t *sizes)
 {
+    if (!cog_accepts(tw, 0))
+        return -1;
     return put_grid_tile_row(tw, &tw->g[0], tile_row, blob, offsets, sizes);
 }
 
@@ -1106,12 +1148,13 @@ int gh_tiffw_put_level_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nro
     if (!tw || level < 0 || level > tw->nlev)
         return -1;
     tw_grid *g = &tw->g[level];
-    if (tw->failed || tile_row0 != g->next_tile_row || nrows < 1 || tile_row0 + nrows > g->tiles_y)
+    if (tw->failed || tile_row0 != g->next_tile_row || nrows < 1 || tile_row0 + nrows > g->tiles_y || !cog_accepts(tw, level))
         return -1;
     const size_t n = (size_t)nrows * (size_t)g->tiles_x;
     /* laid out in table order with small gaps (the library's "ordered" strips)?  Then the whole share is one write;
-     * the gaps (< 16 bytes per tile, alignment padding) go into the file as unused bytes, which TIFF allows */
-    int ordered = 1;
+     * the gaps (< 16 bytes per tile, alignment padding) go into the file as unused bytes, which TIFF allows.  (A COG's
+     * tiles need their framing between them: the writer adds it tile by tile.) */
+    int ordered = !tw->cog;
     for (size_t i = 0; i + 1 < n && ordered; i++)
         ordered = offsets[i + 1] >= offsets[i] + sizes[i] && offsets[i + 1] - (offsets[i] + sizes[i]) < 64;
     if (!ordered) {
@@ -1135,9 +1178,41 @@ int gh_tiffw_put_level_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nro
     return 0;
 }
 
-static void put16(unsigned char **p, uint16_t v) { (*p)[0] = (unsigned char)v; (*p)[1] = (unsigned char)(v >> 8); *p += 2; }
-static void put32(unsigned char **p, uint32_t v) { for (int i = 0; i < 4; i++) (*p)[i] = (unsigned char)(v >> (8 * i)); *p += 4; }
-static void put_f64(unsigned char **p, double d) { uint64_t v; memcpy(&v, &d, 8); for (int i = 0; i < 8; i++) (*p)[i] = (unsigned char)(v >> (8 * i)); *p += 8; }
+int gh_tiffw_put_framed_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nrows, const uint8_t *blob,
+                                  const uint64_t *offsets, const uint32_t *sizes)
+{
+    if (!tw || !tw->cog || level < 0 || level > tw->nlev)
+        return -1;
+    tw_grid *g = &tw->g[level];
+    if (tw->failed || tile_row0 != g->next_tile_row || nrows < 1 || tile_row0 + nrows > g->tiles_y || !cog_accepts(tw, level))
+        return -1;
+    const size_t n = (size_t)nrows * (size_t)g->tiles_x;
+    /* every tile framed in place, in table order, with at most alignment padding between one trailer and the next
+     * leader: then the share from the first leader to the last trailer is one write */
+    for (size_t i = 0; i < n; i++) {
+        const uint8_t *z = blob + offsets[i];
+        if (offsets[i] < 4 || sizes[i] < 4 ||
+            ((uint32_t)z[-4] | (uint32_t)z[-3] << 8 | (uint32_t)z[-2] << 16 | (uint32_t)z[-1] << 24) != sizes[i] ||
+            memcmp(z + sizes[i], z + sizes[i] - 4, 4) != 0 ||
+            (i + 1 < n && (offsets[i + 1] < offsets[i] + sizes[i] + 8 || offsets[i + 1] - (offsets[i] + sizes[i]) >= 64))) {
+            tw->failed = 1;
+            return -1;
+        }
+    }
+    const uint64_t first = offsets[0] - 4, bytes = offsets[n - 1] + sizes[n - 1] + 4 - first;
+    if (tw->pos + bytes > 0xFFFFFFF0ull || fwrite(blob + first, 1, (size_t)bytes, tw->fp) != (size_t)bytes) {
+        tw->failed = 1;
+        return -1;
+    }
+    for (size_t i = 0; i < n; i++) {
+        const size_t ti = (size_t)tile_row0 * (size_t)g->tiles_x + i;
+        g->offsets[ti] = (uint32_t)(tw->pos + (offsets[i] - first));
+        g->counts[ti] = sizes[i];
+    }
+    tw->pos += bytes;
+    g->next_tile_row += nrows;
+    return 0;
+}
 
 static void put_entry(unsigned char **p, uint16_t tag, uint16_t type, uint32_t count, uint32_t value)
 {
@@ -1146,6 +1221,132 @@ static void put_entry(unsigned char **p, uint16_t tag, uint16_t type, uint32_t c
     put32(p, count);
     if (type == 3 && count == 1) { put16(p, (uint16_t)value); put16(p, 0); }
     else put32(p, value);
+}
+
+/* What IFD0 and the level IFDs hold besides the tile tables: the georeferencing (the land cover's GeoKeys, or
+ * EPSG:4326) and the NoData / statistics tags */
+typedef struct {
+    const uint16_t *keys;
+    size_t nkeys;
+    const char *ascii;
+    size_t nascii, ndbl;
+    int tag_nodata;             /* GDAL_NODATA in every IFD */
+    int nent, level_entries;    /* entries of IFD0 and of a level's IFD */
+} tw_tags;
+
+static void tags_of(const gh_tiffw *tw, tw_tags *t)
+{
+    static const uint16_t geokeys[] = {
+        1, 1, 0, 4,
+        1024, 0, 1, 2,          /* GTModelTypeGeoKey      = ModelTypeGeographic */
+        1025, 0, 1, 1,          /* GTRasterTypeGeoKey     = RasterPixelIsArea   */
+        2048, 0, 1, 4326,       /* GeographicTypeGeoKey   = WGS 84              */
+        2054, 0, 1, 9102,       /* GeogAngularUnitsGeoKey = degree              */
+    };
+    static const char ascii_default[] = "WGS 84|";
+    t->keys = tw->geo_keys ? tw->geo_keys : geokeys;
+    t->nkeys = tw->geo_keys ? tw->n_geo_keys : sizeof geokeys / 2;
+    t->ascii = tw->geo_keys ? tw->geo_ascii : ascii_default;
+    t->nascii = tw->geo_keys ? tw->n_geo_ascii : sizeof ascii_default;
+    t->ndbl = tw->geo_keys ? tw->n_geo_doubles : 0;
+    t->tag_nodata = tw->stats || tw->nodata;
+    t->nent = 14 + 1 + (t->ndbl ? 1 : 0) + (t->nascii ? 1 : 0) + (tw->stats ? 1 : 0) + t->tag_nodata;
+    t->level_entries = 13 + t->tag_nodata;
+}
+
+/* File offsets of everything the IFDs hold or point to.  end = the first byte after all of it. */
+typedef struct {
+    uint64_t offsets, counts, scale, tie, keys, dbl, ascii, meta, ifd0;
+    uint64_t lv_tables[1 + GCN10_MAX_OVERVIEWS];        /* a level's tile offsets, then its byte counts */
+    uint64_t lv_ifd[1 + GCN10_MAX_OVERVIEWS];
+    uint64_t end;
+} tw_layout;
+
+/* IFD0's arrays and IFD0 at the current (even) end of the data, then per overview level its tables and IFD */
+static void trailing_layout(const gh_tiffw *tw, const tw_tags *t, size_t nmeta, tw_layout *L)
+{
+    const uint64_t nt = (uint64_t)tw->g[0].tiles_x * (uint64_t)tw->g[0].tiles_y;
+    L->offsets = tw->pos;
+    L->counts = L->offsets + 4 * nt;
+    L->scale = L->counts + 4 * nt;
+    L->tie = L->scale + 24;
+    L->keys = L->tie + 48;
+    L->dbl = L->keys + 2 * t->nkeys;
+    L->ascii = L->dbl + 8 * t->ndbl;
+    L->meta = (L->ascii + t->nascii + 1) & ~(uint64_t)1;     /* word aligned */
+    L->ifd0 = (L->meta + nmeta + 1) & ~(uint64_t)1;
+    L->end = L->ifd0 + 2 + (uint64_t)t->nent * 12 + 4;
+    /* behind IFD0, per overview level: its tile offsets, byte counts and IFD (reduced-resolution image, no geo tags:
+     * readers derive the level's georeferencing from the size ratio) */
+    for (int k = 1; k <= tw->nlev; k++) {
+        L->lv_tables[k] = L->end;
+        L->lv_ifd[k] = L->end + 8 * (uint64_t)tw->g[k].tiles_x * (uint64_t)tw->g[k].tiles_y;
+        L->end = L->lv_ifd[k] + 2 + (uint64_t)t->level_entries * 12 + 4;
+    }
+}
+
+/* GDAL's ghost area of a COG (its COG driver writes it; its validator reads it): the layout promises a reader that the
+ * IFDs come before the data, tiles in row-major order, each framed by its size and its last 4 bytes */
+static const char k_cog_ghost[] = "LAYOUT=IFDS_BEFORE_DATA\n"
+                                  "BLOCK_ORDER=ROW_MAJOR\n"
+                                  "BLOCK_LEADER=SIZE_AS_UINT4\n"
+                                  "BLOCK_TRAILER=LAST_4_BYTES_REPEATED\n"
+                                  "KNOWN_INCOMPATIBLE_EDITION=NO\n ";
+
+/* A COG's header region: the TIFF header and the ghost area, IFD0 at the next even offset, the level IFDs from the
+ * largest level to the smallest, then every array they point to -- the GDAL_METADATA slot sized for the longest
+ * statistics text -- and the data after it.  Known as soon as the tile grids, the georeferencing and the tags are. */
+static void cog_layout(const gh_tiffw *tw, const tw_tags *t, tw_layout *L)
+{
+    const uint64_t ghost = 8 + strlen("GDAL_STRUCTURAL_METADATA_SIZE=000000 bytes\n") + (sizeof k_cog_ghost - 1);
+    L->ifd0 = (ghost + 1) & ~(uint64_t)1;
+    uint64_t at = L->ifd0 + 2 + (uint64_t)t->nent * 12 + 4;
+    for (int k = 1; k <= tw->nlev; k++) {
+        L->lv_ifd[k] = at;
+        at += 2 + (uint64_t)t->level_entries * 12 + 4;
+    }
+    const uint64_t nt = (uint64_t)tw->g[0].tiles_x * (uint64_t)tw->g[0].tiles_y;
+    L->offsets = at;
+    L->counts = L->offsets + 4 * nt;
+    at = L->counts + 4 * nt;
+    for (int k = 1; k <= tw->nlev; k++) {
+        L->lv_tables[k] = at;
+        at += 8 * (uint64_t)tw->g[k].tiles_x * (uint64_t)tw->g[k].tiles_y;
+    }
+    L->scale = at;
+    L->tie = L->scale + 24;
+    L->keys = L->tie + 48;
+    L->dbl = L->keys + 2 * t->nkeys;
+    L->ascii = L->dbl + 8 * t->ndbl;
+    L->meta = (L->ascii + t->nascii + 1) & ~(uint64_t)1;
+    L->end = (L->meta + (tw->stats ? stats_metadata_cap() : 0) + 1) & ~(uint64_t)1;
+}
+
+int gh_tiffw_set_cog(gh_tiffw *tw, int on)
+{
+    if (!tw || tw->failed || (on != 0 && on != 1) || tw->cog || tw->pos != 8)
+        return -1;
+    for (int k = 0; k <= tw->nlev; k++)
+        if (tw->g[k].next_tile_row)
+            return -1;
+    if (!on)
+        return 0;
+    tw_tags t;
+    tw_layout L;
+    tw->cog = 1;
+    tags_of(tw, &t);
+    cog_layout(tw, &t, &L);
+    /* the header region is filled in on close; the tiles follow it */
+    unsigned char *zero = calloc(1, (size_t)(L.end - 8));
+    if (!zero || fwrite(zero, 1, (size_t)(L.end - 8), tw->fp) != (size_t)(L.end - 8) || L.end + 256 >= 0xFFFFFFF0ull) {
+        free(zero);
+        tw->failed = 1;
+        return -1;
+    }
+    free(zero);
+    tw->pos = tw->cog_data = L.end;
+    tw->cog_level = tw->nlev;
+    return 0;
 }
 
 int gh_tiffw_close(gh_tiffw *tw)
@@ -1171,52 +1372,40 @@ int gh_tiffw_close(gh_tiffw *tw)
         nmeta = n > 0 ? (size_t)n + 1 : 0;
     }
     const uint32_t nodata_ascii = '2' | '5' << 8 | '5' << 16;     /* "255\0", held in the entry itself */
-    const int tag_nodata = tw->stats || tw->nodata;                 /* GDAL_NODATA in every IFD */
     if (complete) {
-        /* trailing data area: tile offsets, tile byte counts, pixel scale, tiepoint, geo keys, ascii */
-        static const uint16_t geokeys[] = {
-            1, 1, 0, 4,
-            1024, 0, 1, 2,          /* GTModelTypeGeoKey      = ModelTypeGeographic */
-            1025, 0, 1, 1,          /* GTRasterTypeGeoKey     = RasterPixelIsArea   */
-            2048, 0, 1, 4326,       /* GeographicTypeGeoKey   = WGS 84              */
-            2054, 0, 1, 9102,       /* GeogAngularUnitsGeoKey = degree              */
-        };
-        static const char ascii_default[] = "WGS 84|";
-        const uint16_t *keys = tw->geo_keys ? tw->geo_keys : geokeys;
-        const size_t nkeys = tw->geo_keys ? tw->n_geo_keys : sizeof geokeys / 2;
-        const char *ascii = tw->geo_keys ? tw->geo_ascii : ascii_default;
-        const size_t nascii = tw->geo_keys ? tw->n_geo_ascii : sizeof ascii_default;
-        const size_t ndbl = tw->geo_keys ? tw->n_geo_doubles : 0;
-        if (tw->pos & 1) { fputc(0, tw->fp); tw->pos++; }
-        uint64_t off_offsets = tw->pos, off_counts = off_offsets + 4 * nt, off_scale = off_counts + 4 * nt;
-        uint64_t off_tie = off_scale + 24, off_keys = off_tie + 48, off_dbl = off_keys + 2 * nkeys;
-        uint64_t off_ascii = off_dbl + 8 * ndbl, off_meta = (off_ascii + nascii + 1) & ~(uint64_t)1;     /* word aligned */
-        uint64_t off_ifd = (off_meta + nmeta + 1) & ~(uint64_t)1;
-        const int nent = 14 + 1 + (ndbl ? 1 : 0) + (nascii ? 1 : 0) + (tw->stats ? 1 : 0) + tag_nodata;
-        /* behind IFD0, per overview level: its tile offsets, byte counts and IFD (reduced-resolution image, no geo tags:
-         * readers derive the level's georeferencing from the size ratio) */
-        const int level_entries = 13 + tag_nodata;
-        uint64_t off_lv[1 + GCN10_MAX_OVERVIEWS], end = off_ifd + 2 + (uint64_t)nent * 12 + 4;
-        for (int k = 1; k <= tw->nlev; k++) {
-            off_lv[k] = end;            /* offsets | counts | IFD */
-            end += 8 * (uint64_t)tw->g[k].tiles_x * (uint64_t)tw->g[k].tiles_y + 2 + (uint64_t)level_entries * 12 + 4;
+        tw_tags t;
+        tw_layout L;
+        tags_of(tw, &t);
+        uint64_t at;            /* buf holds the file's bytes [at, L.end) */
+        if (tw->cog) {
+            if (nmeta > stats_metadata_cap())
+                complete = 0;
+            cog_layout(tw, &t, &L);
+            at = 0;
         }
-        size_t tail = (size_t)(end - tw->pos);
-        unsigned char *buf = calloc(1, tail), *p = buf;
-        if (buf && end + 256 < 0xFFFFFFF0ull) {
+        else {
+            if (tw->pos & 1) { fputc(0, tw->fp); tw->pos++; }
+            trailing_layout(tw, &t, nmeta, &L);
+            at = tw->pos;
+        }
+        size_t tail = (size_t)(L.end - at);
+        unsigned char *buf = complete ? calloc(1, tail) : NULL, *p = buf;
+        if (buf && L.end + 256 < 0xFFFFFFF0ull) {
+            p = buf + (L.offsets - at);
             for (size_t i = 0; i < nt; i++) put32(&p, g0->offsets[i]);
             for (size_t i = 0; i < nt; i++) put32(&p, g0->counts[i]);
+            p = buf + (L.scale - at);
             put_f64(&p, tw->gt[1]); put_f64(&p, -tw->gt[5]); put_f64(&p, 0.0);
             put_f64(&p, 0.0); put_f64(&p, 0.0); put_f64(&p, 0.0);
             put_f64(&p, tw->gt[0]); put_f64(&p, tw->gt[3]); put_f64(&p, 0.0);
-            for (size_t i = 0; i < nkeys; i++) put16(&p, keys[i]);
-            for (size_t i = 0; i < ndbl; i++) put_f64(&p, tw->geo_doubles[i]);
-            if (nascii)
-                memcpy(p, ascii, nascii);
+            for (size_t i = 0; i < t.nkeys; i++) put16(&p, t.keys[i]);
+            for (size_t i = 0; i < t.ndbl; i++) put_f64(&p, tw->geo_doubles[i]);
+            if (t.nascii)
+                memcpy(p, t.ascii, t.nascii);
             if (nmeta)
-                memcpy(buf + (off_meta - tw->pos), meta, nmeta);
-            p = buf + (off_ifd - tw->pos);
-            put16(&p, (uint16_t)nent);
+                memcpy(buf + (L.meta - at), meta, nmeta);
+            p = buf + (L.ifd0 - at);
+            put16(&p, (uint16_t)t.nent);
             put_entry(&p, 256, 4, 1, (uint32_t)g0->w);
             put_entry(&p, 257, 4, 1, (uint32_t)g0->h);
             put_entry(&p, 258, 3, 1, 8);
@@ -1226,28 +1415,29 @@ int gh_tiffw_close(gh_tiffw *tw)
             put_entry(&p, 284, 3, 1, 1);
             put_entry(&p, 322, 3, 1, TILE);
             put_entry(&p, 323, 3, 1, TILE);
-            put_entry(&p, 324, 4, (uint32_t)nt, nt == 1 ? g0->offsets[0] : (uint32_t)off_offsets);
-            put_entry(&p, 325, 4, (uint32_t)nt, nt == 1 ? g0->counts[0] : (uint32_t)off_counts);
+            put_entry(&p, 324, 4, (uint32_t)nt, nt == 1 ? g0->offsets[0] : (uint32_t)L.offsets);
+            put_entry(&p, 325, 4, (uint32_t)nt, nt == 1 ? g0->counts[0] : (uint32_t)L.counts);
             put_entry(&p, 339, 3, 1, 1);                /* SampleFormat = unsigned */
-            put_entry(&p, 33550, 12, 3, (uint32_t)off_scale);
-            put_entry(&p, 33922, 12, 6, (uint32_t)off_tie);
-            put_entry(&p, 34735, 3, (uint32_t)nkeys, (uint32_t)off_keys);
-            if (ndbl)
-                put_entry(&p, 34736, 12, (uint32_t)ndbl, (uint32_t)off_dbl);
-            if (nascii)
-                put_entry(&p, 34737, 2, (uint32_t)nascii, (uint32_t)off_ascii);
+            put_entry(&p, 33550, 12, 3, (uint32_t)L.scale);
+            put_entry(&p, 33922, 12, 6, (uint32_t)L.tie);
+            put_entry(&p, 34735, 3, (uint32_t)t.nkeys, (uint32_t)L.keys);
+            if (t.ndbl)
+                put_entry(&p, 34736, 12, (uint32_t)t.ndbl, (uint32_t)L.dbl);
+            if (t.nascii)
+                put_entry(&p, 34737, 2, (uint32_t)t.nascii, (uint32_t)L.ascii);
             if (tw->stats)
-                put_entry(&p, 42112, 2, (uint32_t)nmeta, (uint32_t)off_meta);
-            if (tag_nodata)
+                put_entry(&p, 42112, 2, (uint32_t)nmeta, (uint32_t)L.meta);
+            if (t.tag_nodata)
                 put_entry(&p, 42113, 2, 4, nodata_ascii);
-            put32(&p, tw->nlev ? (uint32_t)(off_lv[1] + 8 * (uint64_t)tw->g[1].tiles_x * (uint64_t)tw->g[1].tiles_y) : 0);
+            put32(&p, tw->nlev ? (uint32_t)L.lv_ifd[1] : 0);
             for (int k = 1; k <= tw->nlev; k++) {
                 const tw_grid *g = &tw->g[k];
                 const size_t n = (size_t)g->tiles_x * (size_t)g->tiles_y;
-                p = buf + (off_lv[k] - tw->pos);
+                p = buf + (L.lv_tables[k] - at);
                 for (size_t i = 0; i < n; i++) put32(&p, g->offsets[i]);
                 for (size_t i = 0; i < n; i++) put32(&p, g->counts[i]);
-                put16(&p, (uint16_t)level_entries);
+                p = buf + (L.lv_ifd[k] - at);
+                put16(&p, (uint16_t)t.level_entries);
                 put_entry(&p, 254, 4, 1, 1);            /* NewSubfileType = reduced-resolution version */
                 put_entry(&p, 256, 4, 1, (uint32_t)g->w);
                 put_entry(&p, 257, 4, 1, (uint32_t)g->h);
@@ -1258,17 +1448,27 @@ int gh_tiffw_close(gh_tiffw *tw)
                 put_entry(&p, 284, 3, 1, 1);
                 put_entry(&p, 322, 3, 1, TILE);
                 put_entry(&p, 323, 3, 1, TILE);
-                put_entry(&p, 324, 4, (uint32_t)n, n == 1 ? g->offsets[0] : (uint32_t)off_lv[k]);
-                put_entry(&p, 325, 4, (uint32_t)n, n == 1 ? g->counts[0] : (uint32_t)(off_lv[k] + 4 * n));
+                put_entry(&p, 324, 4, (uint32_t)n, n == 1 ? g->offsets[0] : (uint32_t)L.lv_tables[k]);
+                put_entry(&p, 325, 4, (uint32_t)n, n == 1 ? g->counts[0] : (uint32_t)(L.lv_tables[k] + 4 * n));
                 put_entry(&p, 339, 3, 1, 1);
-                if (tag_nodata)
+                if (t.tag_nodata)
                     put_entry(&p, 42113, 2, 4, nodata_ascii);
-                put32(&p, k < tw->nlev ? (uint32_t)(off_lv[k + 1] + 8 * (uint64_t)tw->g[k + 1].tiles_x * (uint64_t)tw->g[k + 1].tiles_y)
-                                       : 0);
+                put32(&p, k < tw->nlev ? (uint32_t)L.lv_ifd[k + 1] : 0);
             }
-            if (fwrite(buf, 1, tail, tw->fp) == tail && fseek(tw->fp, 4, SEEK_SET) == 0) {
+            if (tw->cog) {
+                /* the header region: TIFF header, GDAL's ghost area, then everything above, in place before the data */
+                p = buf;
+                put16(&p, 'I' | 'I' << 8);
+                put16(&p, 42);
+                put32(&p, (uint32_t)L.ifd0);
+                snprintf((char *)buf + 8, L.ifd0 - 8, "GDAL_STRUCTURAL_METADATA_SIZE=%06d bytes\n%s",
+                         (int)(sizeof k_cog_ghost - 1), k_cog_ghost);
+                if (L.end == tw->cog_data && fseek(tw->fp, 0, SEEK_SET) == 0 && fwrite(buf, 1, tail, tw->fp) == tail)
+                    rc = 0;
+            }
+            else if (fwrite(buf, 1, tail, tw->fp) == tail && fseek(tw->fp, 4, SEEK_SET) == 0) {
                 unsigned char o[4], *q = o;
-                put32(&q, (uint32_t)off_ifd);
+                put32(&q, (uint32_t)L.ifd0);
                 if (fwrite(o, 1, 4, tw->fp) == 4)
                     rc = 0;
             }
@@ -1322,6 +1522,45 @@ int gh_tiff_write(const char *path, const uint8_t *data, int w, int h, size_t pi
             gh_tiffw_abort(tw);
             return -1;
         }
+    }
+    if (gh_tiffw_close(tw)) {
+        set_err(err, errlen, "write error 3 on %s", path);
+        return -1;
+    }
+    return 0;
+}
+
+int gh_tiff_write_cog(const char *path, const uint8_t *data, int w, int h, size_t pitch, const double gt[6], int overviews,
+                      int threads, char *err, size_t errlen)
+{
+    gh_tiffw *tw;
+    if (gh_tiffw_open(path, w, h, gt, &tw, err, errlen))
+        return -1;
+    int rc = gh_tiffw_set_overviews(tw, overviews) || gh_tiffw_set_cog(tw, 1);
+    /* the levels first, the smallest first, each sampled whole (a level is at most a quarter of the raster); then the
+     * full resolution, in bands of 16 tile rows */
+    for (int k = tw->nlev; k >= 0 && !rc; k--) {
+        tw_grid *g = &tw->g[k];
+        uint8_t *lv = k ? malloc((size_t)g->w * (size_t)g->h) : NULL;
+        if (k && !lv) {
+            rc = -1;
+            break;
+        }
+        for (int i = 0; k && i < g->h; i++) {
+            const uint8_t *row = data + (size_t)gcn10_overview_src(i, k, h) * pitch;
+            for (int x = 0; x < g->w; x++)
+                lv[(size_t)i * g->w + x] = row[gcn10_overview_src(x, k, w)];
+        }
+        const uint8_t *src = k ? lv : data;
+        const size_t sp = k ? (size_t)g->w : pitch;
+        for (int y0 = 0; y0 < g->h && !rc; y0 += 16 * TILE)
+            rc = append_tile_rows(tw, g, src + (size_t)y0 * sp, sp, g->h - y0 < 16 * TILE ? g->h - y0 : 16 * TILE, threads, 0);
+        free(lv);
+    }
+    if (rc) {
+        set_err(err, errlen, "write error 3 on %s", path);
+        gh_tiffw_abort(tw);
+        return -1;
     }
     if (gh_tiffw_close(tw)) {
         set_err(err, errlen, "write error 3 on %s", path);

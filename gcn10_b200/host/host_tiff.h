@@ -35,6 +35,18 @@ int gh_tiffw_put_histogram(gh_tiffw *tw, const uint64_t hist[256]);
 /* NoData alone (on = 1): GDAL_NODATA "255" in every IFD and no GDAL_METADATA (what the mean rasters of option
  * "aggregate" carry).  gh_tiffw_set_stats writes the tag as well, with its statistics. */
 int gh_tiffw_set_nodata(gh_tiffw *tw, int on);
+/* Cloud Optimized GeoTIFF layout (on = 1), the order GDAL's COG driver writes and its validator checks: GDAL's ghost
+ * area at offset 8 (LAYOUT=IFDS_BEFORE_DATA, BLOCK_ORDER=ROW_MAJOR, BLOCK_LEADER=SIZE_AS_UINT4,
+ * BLOCK_TRAILER=LAST_4_BYTES_REPEATED), IFD0 and the level IFDs (largest to smallest) and every table and tag value they
+ * point to before the first tile; then the tiles of the smallest level first and the full resolution last, each tile
+ * framed by its byte count (uint32 LE) before it and its last 4 bytes after it.  Call after gh_tiffw_set_overviews,
+ * _set_stats, _set_nodata and _set_geokeys (which refuse afterwards) and before the first tile: the header region is
+ * reserved here, with a GDAL_METADATA slot for the longest statistics text, and filled in by gh_tiffw_close.  The tiles
+ * must then come level by level in that order (levels nlev .. 1, then 0), each level in tile-row order: anything else
+ * fails the file, which close removes.  gh_tiffw_write_rows refuses a COG (its levels would trail the full resolution);
+ * gh_tiffw_put_tile_row(s) / _put_level_tile_rows frame the tiles they are given, gh_tiffw_put_framed_tile_rows takes
+ * tiles framed already. */
+int gh_tiffw_set_cog(gh_tiffw *tw, int on);
 /* Appends rows [y0, y0+nrows): y0 must continue where the previous call stopped and be a multiple
  * of 256; nrows must be a multiple of 256 except for the last band of the raster.  With overviews, the levels are
  * sampled from the same rows (gcn10_overview_src) and compressed here too, a level's tile row as soon as it is full. */
@@ -52,6 +64,12 @@ int gh_tiffw_put_tile_rows(gh_tiffw *tw, int tile_row0, int nrows, const uint8_t
  * its tile rows too must come in order. */
 int gh_tiffw_put_level_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nrows, const uint8_t *blob,
                                  const uint64_t *offsets, const uint32_t *sizes);
+/* COG only: tile rows whose tiles already carry their leader and trailer in blob (gcn10_tile_strip.framed: the 4 bytes
+ * before blob + offsets[i] hold sizes[i], the 4 after the stream repeat its last 4), in table order with at most
+ * alignment padding between them: the share from the first leader to the last trailer is written with one write.  A
+ * tile whose framing is wrong fails the file. */
+int gh_tiffw_put_framed_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nrows, const uint8_t *blob,
+                                  const uint64_t *offsets, const uint32_t *sizes);
 /* Mean rasters on the host (option "aggregate" where the raw planes come back): the rule of gcn10_aggregate_dim /
  * _value (include/gcn10_cuda.h) applied band by band.  A gh_aggregate belongs to one plane of a w x h block and keeps the
  * partial cell row between bands.

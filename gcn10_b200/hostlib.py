@@ -69,6 +69,8 @@ def load(path: str | None = None) -> C.CDLL:
     L.gh_tiff_window_tiles_plan.argtypes = [_vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp]
     L.gh_tiff_window_tiles_read.argtypes = [_vp, _vp, _vp, _vp, _vp, C.c_int, C.c_char_p, C.c_size_t]
     L.gh_tiff_write.argtypes = [C.c_char_p, _vp, C.c_int, C.c_int, C.c_size_t, _dp, C.c_int, C.c_char_p, C.c_size_t]
+    L.gh_tiff_write_cog.argtypes = [C.c_char_p, _vp, C.c_int, C.c_int, C.c_size_t, _dp, C.c_int, C.c_int, C.c_char_p,
+                                    C.c_size_t]
     L.gh_tiffw_open.argtypes = [C.c_char_p, C.c_int, C.c_int, _dp, C.POINTER(_vp), C.c_char_p, C.c_size_t]
     L.gh_tiffw_put_tile_row.argtypes = [_vp, C.c_int, _vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]
     L.gh_tiffw_put_tile_rows.argtypes = [_vp, C.c_int, C.c_int, _vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]
@@ -78,6 +80,9 @@ def load(path: str | None = None) -> C.CDLL:
     L.gh_tiffw_set_stats.argtypes = [_vp, C.c_int]
     L.gh_tiffw_put_histogram.argtypes = [_vp, C.POINTER(C.c_uint64)]
     L.gh_tiffw_set_nodata.argtypes = [_vp, C.c_int]
+    L.gh_tiffw_set_cog.argtypes = [_vp, C.c_int]
+    L.gh_tiffw_put_framed_tile_rows.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, C.POINTER(C.c_uint64),
+                                                C.POINTER(C.c_uint32)]
     L.gh_aggregate_new.argtypes = [C.c_int, C.c_int, C.c_int]
     L.gh_aggregate_new.restype = _vp
     L.gh_aggregate_rows.argtypes = [_vp, _vp, C.c_size_t, C.c_int, C.c_int, _vp, C.c_size_t, _ip]
@@ -198,6 +203,25 @@ def tiff_write(path: str, data: np.ndarray, gt, threads: int = 4):
     rc = L.gh_tiff_write(os.fsencode(path), data.ctypes.data, w, h, w, (C.c_double * 6)(*gt), threads, e, ERRLEN)
     if rc:
         raise HostError(rc, e.value.decode(errors="replace"))
+
+
+def tiff_write_cog(path: str, data: np.ndarray, gt, overviews: int = 16, threads: int = 4):
+    """The whole raster as a Cloud Optimized GeoTIFF with up to ``overviews`` levels sampled on the host
+    (gh_tiff_write_cog): the CPU reference of the COG layout."""
+    L = load()
+    data = np.ascontiguousarray(data, dtype=np.uint8)
+    h, w = data.shape
+    e = _err()
+    rc = L.gh_tiff_write_cog(os.fsencode(path), data.ctypes.data, w, h, w, (C.c_double * 6)(*gt), overviews, threads, e,
+                             ERRLEN)
+    if rc:
+        raise HostError(rc, e.value.decode(errors="replace"))
+
+
+class GeoKeys(C.Structure):
+    """gh_geokeys of gcn10_host.h."""
+    _fields_ = [("keys", C.POINTER(C.c_uint16)), ("n_keys", C.c_size_t), ("doubles", _dp), ("n_doubles", C.c_size_t),
+                ("ascii", C.c_char_p), ("n_ascii", C.c_size_t)]
 
 
 class Tiff:
@@ -335,7 +359,7 @@ class TiffWriter:
     geotransform scaled by f, NoData 255, and ``write_plane_rows`` feeds it the plane's rows (gh_aggregate_write_rows)."""
 
     def __init__(self, path: str, w: int, h: int, gt, overviews: int = 0, stats: bool = False, nodata: bool = False,
-                 aggregate: int = 0):
+                 aggregate: int = 0, geokeys=None, cog: bool = False):
         self.agg = Aggregate(w, h, aggregate) if aggregate else None
         if aggregate:
             f = aggregate
@@ -361,6 +385,22 @@ class TiffWriter:
             self.L.gh_tiffw_abort(h_)
             self.h = None
             raise HostError(-1, "gh_tiffw_set_nodata(1) failed")
+        if geokeys is not None:
+            keys, doubles, ascii = geokeys
+            k = (C.c_uint16 * len(keys))(*keys)
+            d = (C.c_double * max(len(doubles), 1))(*doubles)
+            a = ascii.encode() if ascii else None
+            gk = GeoKeys(k, len(keys), d if doubles else None, len(doubles), a, len(a) if a else 0)
+            fn = self.L["gh_tiffw_set_geokeys"]     # (a function object of its own: tests bind the symbol their way)
+            fn.argtypes = [_vp, C.POINTER(GeoKeys)]
+            if fn(h_, C.byref(gk)):
+                self.L.gh_tiffw_abort(h_)
+                self.h = None
+                raise HostError(-1, "gh_tiffw_set_geokeys failed")
+        if cog and self.L.gh_tiffw_set_cog(h_, 1):
+            self.L.gh_tiffw_abort(h_)
+            self.h = None
+            raise HostError(-1, "gh_tiffw_set_cog(1) failed")
         self.levels = self.L.gh_tiffw_levels(h_)
 
     def put_histogram(self, hist):
@@ -384,6 +424,17 @@ class TiffWriter:
         if level == 0:
             return self.L.gh_tiffw_put_tile_row(self.h, tile_row, buf, offs, sizes)
         return self.L.gh_tiffw_put_level_tile_rows(self.h, level, tile_row, 1, buf, offs, sizes)
+
+    def put_tile_rows(self, level: int, tile_row0: int, nrows: int, blob, offsets, sizes, framed: bool = False):
+        """``nrows`` tile rows of ``level`` at once, [nrows][tiles_x] tiles: tile i is blob[offsets[i] : offsets[i] +
+        sizes[i]] (gh_tiffw_put_level_tile_rows; ``framed``: the tiles carry their COG leader and trailer in blob,
+        gh_tiffw_put_framed_tile_rows)."""
+        n = len(sizes)
+        buf = C.create_string_buffer(bytes(blob), max(len(blob), 1))
+        offs = (C.c_uint64 * n)(*[int(v) for v in offsets])
+        sz = (C.c_uint32 * n)(*[int(v) for v in sizes])
+        f = self.L.gh_tiffw_put_framed_tile_rows if framed else self.L.gh_tiffw_put_level_tile_rows
+        return f(self.h, level, tile_row0, nrows, buf, offs, sz)
 
     def write_rows(self, data: np.ndarray, y0: int, threads: int = 2):
         data = np.ascontiguousarray(data, dtype=np.uint8)

@@ -167,7 +167,19 @@ int gcn10_cuda_block_rows(gcn10_ctx *ctx,
  * level_h = the mean raster's size).  The same four calls deliver it; the raw-plane calls ignore the option.  The
  * full-resolution strips and overview levels are the same bytes as without the option, and "stats" does not count the
  * mean strips.  The accumulators cost 8 bytes per cell and selected plane on the context (computed: about 0.3 GB for
- * 18 planes of 36001 x 36001 at f = 25). */
+ * 18 planes of 36001 x 36001 at f = 25).
+ *
+ * Cloud Optimized GeoTIFF order (option "cog" = 1): a COG holds the smallest overview level's tiles first and the full
+ * resolution last, so gcn10_cuda_block_deflate, _block_tiles_deflate and _block_parts_deflate then deliver the strips
+ * in that order: the overview levels nlev .. 1 (the smallest first, each in tile-row order), then the full-resolution
+ * strips, then the mean rasters.  The levels are made in one pass over the block's land cover before the first strip,
+ * so the whole block must be on the device: the tiles and parts calls inflate it there anyway, and
+ * gcn10_cuda_block_deflate uploads the caller's raster whole (w x h bytes of device memory, in a tile slot that holds
+ * no prefetched block) instead of strip by strip.  _block_deflate_rows refuses the option (GCN10_EINVAL): a band does
+ * not hold the whole block.  With "ordered" on as well, every tile of a re-laid strip also gets the block leader and
+ * trailer of the COG layout on the device (strip->framed, 8 more bytes per tile), so a consumer still writes a plane's
+ * share of a strip with one write.  The tile streams, the histograms of "stats" and the mean rasters are the same
+ * bytes as without the option; only their order and framing change.  The raw-plane calls ignore the option. */
 typedef struct {
     int tile_row0;              /* first tile row (of the block) in this strip                    */
     int n_tile_rows;            /* tile rows in this strip                                        */
@@ -187,6 +199,11 @@ typedef struct {
      * block's f x f mean raster, whose level_w x level_h = gcn10_aggregate_dim(w, f) x gcn10_aggregate_dim(h, f)
      * cells have their own tile grid (level is then 0) */
     int aggregate;
+    /* option "cog" with "ordered": 1 = every tile in blob carries the block leader and trailer of a Cloud Optimized
+     * GeoTIFF -- the 4 bytes before blob + offsets[i] hold sizes[i] as a uint32 LE, the 4 bytes after the stream repeat
+     * its last 4 bytes (offsets and sizes still address the stream itself).  0 without the option, and for a strip
+     * that did not fit the re-laying arena and left unordered. */
+    int framed;
 } gcn10_tile_strip;
 
 /* Overview levels: nearest-neighbour reductions by 2^k of a block, sampled from full resolution.
@@ -414,7 +431,9 @@ int gcn10_cuda_last_histograms(gcn10_ctx *ctx, uint64_t hist[GCN10_NPLANES][256]
  * many overview levels of the block, see gcn10_cuda_block_deflate), "stats" (0 / 1, default 0: the compressed-tile calls
  * also count every selected plane's histogram, see gcn10_cuda_last_histograms), "aggregate" (0 or 2 ..
  * GCN10_MAX_AGGREGATE, default 0: the compressed-tile calls also deliver every selected plane's f x f mean raster, see
- * gcn10_cuda_block_deflate), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
+ * gcn10_cuda_block_deflate), "cog" (0 / 1, default 0: the whole-block compressed-tile calls deliver the overview levels
+ * first, smallest first, and with "ordered" frame every tile for a Cloud Optimized GeoTIFF, see gcn10_cuda_block_deflate;
+ * _block_deflate_rows refuses it), "inflate_probe" (measurement aid of tools/inflate_bench.py: 1 / 2 switch parts of the inflate
  * kernel's writer off; results are then invalid). */
 int gcn10_cuda_set_option(gcn10_ctx *ctx, const char *key, long value);
 
