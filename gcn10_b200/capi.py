@@ -77,31 +77,52 @@ class TileSourceStruct(C.Structure):
     """gcn10_tile_source of include/gcn10_cuda.h."""
     _fields_ = [("tile_w", C.c_int), ("tile_h", C.c_int), ("tiles_x", C.c_int), ("tiles_y", C.c_int),
                 ("x_off", C.c_int), ("y_off", C.c_int), ("blob", C.c_void_p), ("blob_bytes", C.c_size_t),
-                ("offsets", C.c_void_p), ("sizes", C.c_void_p)]
+                ("offsets", C.c_void_p), ("sizes", C.c_void_p), ("compression", C.c_int)]
+
+
+COMPRESSION = {"deflate": 8, "lzw": 5}          # TIFF Compression tag values of the codecs the GPU decodes
 
 
 class TileSource:
-    """Compressed tiles of a raster window as a tiled DEFLATE GeoTIFF holds them (one zlib stream per tile).
+    """Compressed tiles of a raster window as a tiled GeoTIFF holds them: one zlib stream per tile (``compression``
+    0, 8 or 32946) or one LZW stream per tile (5).
 
     ``blob`` uint8 [n], ``offsets`` uint64 [tiles_y*tiles_x], ``sizes`` uint32 [tiles_y*tiles_x] (0 = sparse
-    tile).  ``from_raster`` builds one from a decoded raster with zlib on the host: a test / benchmark
-    convenience standing in for "read the tile bytes from the file"."""
+    tile).  ``from_raster`` builds one from a decoded raster on the host (zlib, or libtiff's LZW encoder): a test /
+    benchmark convenience standing in for "read the tile bytes from the file"."""
 
-    def __init__(self, tile_w, tile_h, tiles_x, tiles_y, x_off, y_off, blob, offsets, sizes):
+    def __init__(self, tile_w, tile_h, tiles_x, tiles_y, x_off, y_off, blob, offsets, sizes, compression=0):
         self.tile_w, self.tile_h, self.tiles_x, self.tiles_y = tile_w, tile_h, tiles_x, tiles_y
         self.x_off, self.y_off = x_off, y_off
         self.blob = blob
         self.offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
         self.sizes = np.ascontiguousarray(sizes, dtype=np.uint32)
+        self.compression = compression
 
     @classmethod
     def from_raster(cls, raster, tile_w=1024, tile_h=1024, level=6, x_off=0, y_off=0, sparse=(), gap=0,
-                    pad_value=0, blob_alloc=None):
+                    pad_value=0, blob_alloc=None, codec="deflate"):
         """Tile ``raster`` (the window occupies raster[y_off:, x_off:] of the grid's pixel space only in the
-        sense that the CALLER passes x_off / y_off to say where its window starts)."""
+        sense that the CALLER passes x_off / y_off to say where its window starts).  ``codec`` "deflate" (zlib at
+        ``level``; level < 0 stores the raw bytes) or "lzw" (libtiff's encoder, gcn10_b200.tiff_lzw)."""
         import zlib
+        if codec not in COMPRESSION:
+            raise ValueError(f"codec {codec!r}: expected one of {sorted(COMPRESSION)}")
         h, w = raster.shape
         tiles_x, tiles_y = (w + tile_w - 1) // tile_w, (h + tile_h - 1) // tile_h
+        cells = [(ty, tx) for ty in range(tiles_y) for tx in range(tiles_x) if (ty, tx) not in sparse]
+
+        def grid():
+            for ty, tx in cells:
+                t = np.full((tile_h, tile_w), pad_value, dtype=np.uint8)
+                part = raster[ty * tile_h:(ty + 1) * tile_h, tx * tile_w:(tx + 1) * tile_w]
+                t[:part.shape[0], :part.shape[1]] = part
+                yield t
+        if codec == "lzw":
+            from . import tiff_lzw
+            coded = iter(tiff_lzw.encode(grid(), tile_w, tile_h, len(cells)))
+        else:
+            coded = (zlib.compress(t.tobytes(), level) if level >= 0 else t.tobytes() for t in grid())
         streams, offsets, sizes = [], [], []
         pos = 0
         for ty in range(tiles_y):
@@ -110,10 +131,7 @@ class TileSource:
                     offsets.append(0)
                     sizes.append(0)
                     continue
-                t = np.full((tile_h, tile_w), pad_value, dtype=np.uint8)
-                part = raster[ty * tile_h:(ty + 1) * tile_h, tx * tile_w:(tx + 1) * tile_w]
-                t[:part.shape[0], :part.shape[1]] = part
-                z = zlib.compress(t.tobytes(), level) if level >= 0 else t.tobytes()
+                z = next(coded)
                 pos += gap
                 streams.append(b"\x00" * gap + z)
                 offsets.append(pos)
@@ -126,12 +144,12 @@ class TileSource:
             blob = blob[:len(data)]
         else:
             blob = np.frombuffer(data, dtype=np.uint8).copy()
-        return cls(tile_w, tile_h, tiles_x, tiles_y, x_off, y_off, blob, offsets, sizes)
+        return cls(tile_w, tile_h, tiles_x, tiles_y, x_off, y_off, blob, offsets, sizes, COMPRESSION[codec])
 
     def struct(self):
         return TileSourceStruct(self.tile_w, self.tile_h, self.tiles_x, self.tiles_y, self.x_off, self.y_off,
                                 self.blob.ctypes.data, self.blob.size, self.offsets.ctypes.data,
-                                self.sizes.ctypes.data)
+                                self.sizes.ctypes.data, self.compression)
 
 
 class TilePartStruct(C.Structure):

@@ -10,6 +10,7 @@
 #include "cn_kernels.cuh"
 #include "deflate_tiles.cuh"
 #include "inflate_tiles.cuh"
+#include "lzw_tiles.cuh"
 #include "cn_deflate_fused.cuh"
 #include "aggregate.cuh"
 #include "overviews.cuh"
@@ -97,6 +98,7 @@ struct TileSlot {
     bool pending = false;       // inflate issued, result not consumed yet
     bool deferred = false;      // ... uploads issued, the kernel waits for the strips of the block in hand (launch_inflate)
     InflateParams ip;           // the deferred launch
+    size_t n_lzw = 0;           // LZW tiles: the last n_lzw entries of the launch order, decoded by lzw_tiles_kernel
     uint64_t seq = 0;           // issue order of pending slots
     const void *key_blob = nullptr, *key_off = nullptr;
     size_t key_bytes = 0, ntiles = 0, dpitch = 0;
@@ -815,6 +817,9 @@ int gcn10_cuda_create(int device, gcn10_ctx **out)
                                   cudaSharedmemCarveoutMaxShared));
     CUDA_TRY(cudaFuncSetAttribute((const void *)inflate_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   kInflateSmem));
+    CUDA_TRY(cudaFuncSetAttribute((const void *)lzw_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kLzwSmem));
+    CUDA_TRY(cudaFuncSetAttribute((const void *)lzw_tiles_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                  cudaSharedmemCarveoutMaxShared));
     CUDA_TRY(cudaFuncSetAttribute((const void *)inflate_tiles_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                   cudaSharedmemCarveoutMaxShared));
     CUDA_TRY(cudaStreamCreateWithPriority(&c->pre_stream, cudaStreamNonBlocking, prio_lo));
@@ -1950,9 +1955,19 @@ static int launch_inflate(gcn10_ctx *c, TileSlot &sl, cudaEvent_t after)
     if (after)
         CUDA_TRY(cudaStreamWaitEvent(st, after, 0));
     CUDA_TRY(cudaEventRecord(sl.inf0, st));
-    inflate_tiles_kernel<<<(unsigned)sl.ntiles, kInflateThreads, kInflateSmem, st>>>(sl.ip);
-    c->launches++;
-    CUDA_TRY(cudaGetLastError());
+    // a window whose tiles are all of one codec is one launch; a mosaic that mixes codecs takes one per codec
+    if (sl.ntiles > sl.n_lzw) {
+        inflate_tiles_kernel<<<(unsigned)(sl.ntiles - sl.n_lzw), kInflateThreads, kInflateSmem, st>>>(sl.ip);
+        c->launches++;
+        CUDA_TRY(cudaGetLastError());
+    }
+    if (sl.n_lzw) {
+        InflateParams lp = sl.ip;
+        lp.order += sl.ntiles - sl.n_lzw;
+        lzw_tiles_kernel<<<(unsigned)sl.n_lzw, kLzwThreads, kLzwSmem, st>>>(lp);
+        c->launches++;
+        CUDA_TRY(cudaGetLastError());
+    }
     CUDA_TRY(cudaEventRecord(sl.inf1, st));
     CUDA_TRY(cudaMemcpyAsync(sl.h_status.p, sl.ip.status, sl.ntiles * sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaEventRecord(sl.done, st));
@@ -1978,6 +1993,9 @@ static int inflate_to_device(gcn10_ctx *c, TileSlot &sl, const gcn10_tile_part *
             return fail(GCN10_EINVAL, "NULL argument");
         if (pt.w <= 0 || pt.h <= 0 || src->tile_w <= 0 || src->tile_h <= 0 || src->tiles_x <= 0 || src->tiles_y <= 0)
             return fail(GCN10_EINVAL, "non-positive size");
+        if (src->compression != 0 && src->compression != 8 && src->compression != 32946 && src->compression != 5)
+            return fail(GCN10_EINVAL, "part %d: TIFF compression %d is not supported (0, 8 and 32946 = zlib, 5 = LZW)", k,
+                        src->compression);
         if ((long long)src->tile_w * src->tile_h > (1ll << 28))
             return fail(GCN10_EINVAL, "tile of %d x %d pixels is too large", src->tile_w, src->tile_h);
         if (pt.dst_x < 0 || pt.dst_y < 0 || (long long)pt.dst_x + pt.w > w || (long long)pt.dst_y + pt.h > h)
@@ -2020,6 +2038,7 @@ static int inflate_to_device(gcn10_ctx *c, TileSlot &sl, const gcn10_tile_part *
     unsigned long long *h_off = (unsigned long long *)((int *)sl.h_status.p + 2 * ntiles);
     uint32_t *h_size = (uint32_t *)(h_off + ntiles);
     int *h_scratch = (int *)(h_size + ntiles);
+    std::vector<uint8_t> is_lzw(ntiles);
     // tiles that are not stored whole in the plane (clipped by their part's rectangle) keep a scratch copy: the
     // inflater reads history older than its 8 KB ring back from where the bytes were flushed to
     size_t nscratch = 0, scratch_stride = 0;
@@ -2043,6 +2062,7 @@ static int inflate_to_device(gcn10_ctx *c, TileSlot &sl, const gcn10_tile_part *
         for (size_t i = 0; i < n; i++) {
             h_off[t0 + i] = (unsigned long long)b0 + src->offsets[i];
             h_size[t0 + i] = src->sizes[i];
+            is_lzw[t0 + i] = src->compression == 5;
         }
         if (same < 0) {
             if (src->blob_bytes)
@@ -2071,10 +2091,16 @@ static int inflate_to_device(gcn10_ctx *c, TileSlot &sl, const gcn10_tile_part *
         t0 += n;
     }
     // longest streams first: a tile's decode time grows with its compressed size, and a block has only a
-    // few tiles per resident CTA slot, so the order sets the tail
-    for (size_t i = 0; i < ntiles; i++)
+    // few tiles per resident CTA slot, so the order sets the tail.  LZW tiles go behind the zlib ones (their kernel
+    // takes the tail of the order).
+    size_t n_lzw = 0;
+    for (size_t i = 0; i < ntiles; i++) {
         h_order[i] = (int)i;
-    std::stable_sort(h_order, h_order + ntiles, [&](int a, int b) { return h_size[a] > h_size[b]; });
+        n_lzw += is_lzw[i];
+    }
+    std::stable_sort(h_order, h_order + ntiles, [&](int a, int b) {
+        return is_lzw[a] != is_lzw[b] ? is_lzw[a] < is_lzw[b] : h_size[a] > h_size[b];
+    });
     CUDA_TRY(cudaMemcpyAsync(d_order, h_order, ntiles * 4, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(d_off, h_off, ntiles * 8, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemcpyAsync(d_size, h_size, ntiles * 4, cudaMemcpyHostToDevice, st));
@@ -2094,6 +2120,7 @@ static int inflate_to_device(gcn10_ctx *c, TileSlot &sl, const gcn10_tile_part *
     ip.nparts = nparts;
     sl.ip = ip;
     sl.ntiles = ntiles;
+    sl.n_lzw = n_lzw;
     sl.deferred = true;
     if (!defer && (rc = launch_inflate(c, sl, nullptr)))
         return rc;

@@ -104,8 +104,8 @@ int gh_tiff_geokeys(const gh_tiff *t, gh_geokeys *out);
 int gh_tiff_read_window(gh_tiff *t, int xoff, int yoff, int xcount, int ycount, uint8_t *dst, size_t pitch,
                         int threads, char *err, size_t errlen);
 /* The compressed tiles of a pixel window, as they lie in the file, for gcn10_cuda_block_tiles_deflate (GPU-side
- * inflate).  gh_tiff_window_tiles_plan returns 0 and fills the plan when the dataset can be handed over that
- * way (tiled, DEFLATE, no predictor), 1 when it cannot (the caller then decodes on the host with
+ * decode).  gh_tiff_window_tiles_plan returns 0 and fills the plan when the dataset can be handed over that
+ * way (tiled, DEFLATE or LZW, no predictor), 1 when it cannot (the caller then decodes on the host with
  * gh_tiff_read_window).  gh_tiff_window_tiles_read copies the tiles' bytes into blob (plan->blob_bytes, tiles
  * adjacent in the file are read with one pread) and fills offsets / sizes [tiles_y * tiles_x] (size 0 = sparse). */
 typedef struct {
@@ -114,6 +114,7 @@ typedef struct {
     int tiles_x, tiles_y;       /* tile grid covering the window */
     int x_in, y_in;             /* window pixel (0,0) inside that grid */
     size_t blob_bytes;
+    int compression;            /* the file's TIFF Compression tag (8 / 32946 DEFLATE, 5 LZW): gcn10_tile_source.compression */
 } gh_tile_plan;
 int gh_tiff_window_tiles_plan(const gh_tiff *t, int xoff, int yoff, int xcount, int ycount, gh_tile_plan *plan);
 int gh_tiff_window_tiles_read(gh_tiff *t, const gh_tile_plan *plan, uint8_t *blob, uint64_t *offsets, uint32_t *sizes,
@@ -140,7 +141,8 @@ int gh_raster_geokeys(const gh_raster *r, gh_geokeys *out);
 int gh_raster_read_window(gh_raster *r, int xoff, int yoff, int xcount, int ycount, uint8_t *dst, size_t pitch,
                           int threads, char *err, size_t errlen);
 /* The window as compressed tiles, source by source, for gcn10_cuda_block_parts_deflate.  Returns 0 and fills
- * parts[0..*nparts) when every source that touches the window is a tiled DEFLATE GeoTIFF without predictor; 1 when
+ * parts[0..*nparts) when every source that touches the window is a tiled DEFLATE or LZW GeoTIFF without predictor
+ * (the codec may differ from source to source); 1 when
  * the window has to be decoded on the host instead (other formats, overlapping sources, more than max_parts
  * sources); -1 when a source cannot be opened (err set: the read fails like GDAL's would). */
 typedef struct {

@@ -640,8 +640,8 @@ static void load_block(worker *wk, block_input *in, int block_id)
         goto out;
     }
 
-    /* a tiled DEFLATE land-cover file (what GDAL writes for COMPRESS=DEFLATE TILED=YES, and what the ESA WorldCover
-     * files are) is handed to the GPU compressed; anything else is decoded later, band by band */
+    /* a tiled DEFLATE or LZW land-cover file without predictor (what GDAL writes for COMPRESS=DEFLATE / LZW TILED=YES;
+     * the ESA WorldCover files are DEFLATE) is handed to the GPU compressed; anything else is decoded later, band by band */
     const char *hd = getenv("GCN10_HOST_DEFLATE"), *hi = getenv("GCN10_HOST_INFLATE");
     const int host_side = (hd && *hd && *hd != '0') || (hi && *hi && *hi != '0');
     gh_raster_part rp[MAX_PARTS];
@@ -697,6 +697,7 @@ static void load_block(worker *wk, block_input *in, int block_id)
             cp->tiles.blob_bytes = rp[k].plan.blob_bytes;
             cp->tiles.offsets = in->tile_off + t_at;
             cp->tiles.sizes = in->tile_size + t_at;
+            cp->tiles.compression = rp[k].plan.compression;
             cp->dst_x = rp[k].dst_x;
             cp->dst_y = rp[k].dst_y;
             cp->w = rp[k].w;
@@ -844,11 +845,17 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
     abort_agg_writers(wk);                      /* (frees the host aggregation; no writer is left to abort) */
     wk->writers_open = 0;
     double dt = now_s() - t_start;
+    int lzw = 0;
+    for (int k = 0; in->gpu_inflate && k < in->nparts; k++)
+        lzw |= in->parts[k].tiles.compression == 5;
+    const char *where = !in->gpu_inflate ? ""
+                        : lzw ? (in->nparts > 1 ? " [land cover: mosaic parts (LZW) decoded on the gpu]"
+                                                : " [land cover: LZW tiles decoded on the gpu]")
+                              : (in->nparts > 1 ? " [land cover: mosaic parts inflated on the gpu]"
+                                                : " [land cover inflated on the gpu]");
     snprintf(msg, sizeof msg,
              "block %d: %d x %d px, 18 rasters in %.3f s (%.1f Mpx/s; read %.3f s [overlapped], gpu+copies+write %.3f s; %s deflate)%s",
-             block_id, w, h, dt, (double)w * h / dt / 1e6, t_read, t_gpu, host_deflate ? "host" : "gpu",
-             in->gpu_inflate ? (in->nparts > 1 ? " [land cover: mosaic parts inflated on the gpu]"
-                                               : " [land cover inflated on the gpu]") : "");
+             block_id, w, h, dt, (double)w * h / dt / 1e6, t_read, t_gpu, host_deflate ? "host" : "gpu", where);
     gh_log_message(wk->log, "INFO", msg, 0);
     return ok ? 0 : -1;
 }

@@ -664,7 +664,7 @@ int gh_tiff_read_window(gh_tiff *t, int xoff, int yoff, int xcount, int ycount, 
 
 int gh_tiff_window_tiles_plan(const gh_tiff *t, int xoff, int yoff, int xcount, int ycount, gh_tile_plan *plan)
 {
-    if (!t->tiled || (t->compression != 8 && t->compression != 32946) || t->predictor != 1)
+    if (!t->tiled || (t->compression != 8 && t->compression != 32946 && t->compression != 5) || t->predictor != 1)
         return 1;
     if (xoff < 0 || yoff < 0 || xcount <= 0 || ycount <= 0 || xoff + xcount > t->w || yoff + ycount > t->h)
         return 1;
@@ -687,6 +687,7 @@ int gh_tiff_window_tiles_plan(const gh_tiff *t, int xoff, int yoff, int xcount, 
             total += (size_t)n;
         }
     plan->blob_bytes = total;
+    plan->compression = t->compression;
     return 0;
 }
 

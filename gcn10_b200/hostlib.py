@@ -252,8 +252,8 @@ class Tiff:
 
     def window_tiles(self, xoff=0, yoff=0, xcount=None, ycount=None, threads=4):
         """The compressed tiles of a window as they lie in the file (gh_tiff_window_tiles_plan / _read), or None when
-        the dataset cannot be handed to the GPU inflater (not tiled, not DEFLATE, predictor 2).
-        Returns dict(tile_w, tile_h, tiles_x, tiles_y, x_in, y_in, blob, offsets, sizes)."""
+        the dataset cannot be handed to the GPU decoder (not tiled, neither DEFLATE nor LZW, predictor 2).
+        Returns dict(tile_w, tile_h, tiles_x, tiles_y, x_in, y_in, blob, offsets, sizes, compression)."""
         xcount = self.width - xoff if xcount is None else xcount
         ycount = self.height - yoff if ycount is None else ycount
         plan = TilePlan()
@@ -269,7 +269,8 @@ class Tiff:
         if rc:
             raise HostError(rc, e.value.decode(errors="replace"))
         return dict(tile_w=plan.tile_w, tile_h=plan.tile_h, tiles_x=plan.tiles_x, tiles_y=plan.tiles_y, x_in=plan.x_in,
-                    y_in=plan.y_in, blob=blob[:plan.blob_bytes], offsets=offsets, sizes=sizes)
+                    y_in=plan.y_in, blob=blob[:plan.blob_bytes], offsets=offsets, sizes=sizes,
+                    compression=plan.compression)
 
     def close(self):
         if self.h:
@@ -280,7 +281,8 @@ class Tiff:
 class TilePlan(C.Structure):
     """gh_tile_plan of gcn10_host.h."""
     _fields_ = [("tile_w", C.c_int), ("tile_h", C.c_int), ("tx0", C.c_int), ("ty0", C.c_int), ("tiles_x", C.c_int),
-                ("tiles_y", C.c_int), ("x_in", C.c_int), ("y_in", C.c_int), ("blob_bytes", C.c_size_t)]
+                ("tiles_y", C.c_int), ("x_in", C.c_int), ("y_in", C.c_int), ("blob_bytes", C.c_size_t),
+                ("compression", C.c_int)]
 
 
 class RasterPart(C.Structure):
@@ -321,7 +323,7 @@ class Raster:
 
     def window_parts(self, xoff, yoff, xcount, ycount, max_parts=9, threads=4):
         """(rc, parts): rc 0 -> parts = [dict(dst_x, dst_y, w, h, tile_w, tile_h, tiles_x, tiles_y, x_in, y_in, blob,
-        offsets, sizes)] ready for capi.TileSource; rc 1 -> decode on the host; raises when a source is missing."""
+        offsets, sizes, compression)] ready for capi.TileSource; rc 1 -> decode on the host; raises when a source is missing."""
         arr = (RasterPart * max_parts)()
         n = C.c_int()
         e = _err()
@@ -341,7 +343,8 @@ class Raster:
                 raise HostError(r2, e.value.decode(errors="replace"))
             parts.append(dict(dst_x=arr[k].dst_x, dst_y=arr[k].dst_y, w=arr[k].w, h=arr[k].h, tile_w=plan.tile_w,
                               tile_h=plan.tile_h, tiles_x=plan.tiles_x, tiles_y=plan.tiles_y, x_in=plan.x_in,
-                              y_in=plan.y_in, blob=blob[:plan.blob_bytes], offsets=offsets, sizes=sizes))
+                              y_in=plan.y_in, blob=blob[:plan.blob_bytes], offsets=offsets, sizes=sizes,
+                              compression=plan.compression))
         return rc, parts
 
     def close(self):

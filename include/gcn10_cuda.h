@@ -313,6 +313,14 @@ int gcn10_cuda_block_deflate_rows(gcn10_ctx *ctx,
  *   blob, blob_bytes   the tiles' bytes (host memory; page-locked memory makes the copy asynchronous)
  *   offsets, sizes     per tile: start of its zlib stream in blob and its length; size 0 = a sparse tile,
  *                      read as zeros (what GDAL returns for a tile that was never written)
+ *   compression        the file's TIFF Compression tag: 0, 8 or 32946 = zlib streams; 5 = LZW (new style, no
+ *                      predictor: what gdal_translate -co COMPRESS=LZW writes), decoded on the GPU as well, with
+ *                      libtiff's rules.  Any other value is refused with GCN10_EINVAL.  Every _tiles_ and _parts_ call
+ *                      takes it per part, so the parts of one mosaic may differ.
+ *
+ * The compression field was appended to the struct; 0 selects zlib, so a caller that zero-initialises the struct
+ * keeps working unchanged.  The change is source-compatible but not binary-compatible (gcn10_tile_part embeds the
+ * struct): callers must be recompiled.
  */
 typedef struct {
     int tile_w, tile_h;
@@ -322,13 +330,17 @@ typedef struct {
     size_t blob_bytes;
     const uint64_t *offsets;
     const uint32_t *sizes;
+    int compression;
 } gcn10_tile_source;
 
 /* Inflate the tiles of `src` on the GPU and return the w x h window as a raster in HOST memory
  * (the load_raster() half alone).  tile_status, if not NULL, receives tiles_x * tiles_y codes: 0 = ok,
  * 1..10 = the reason a tile could not be decoded (see inflate_core.h; 10 = the stream's Adler-32 trailer does not
- * match the decoded bytes, which zlib reports to GDAL as a data error).  Returns GCN10_EDATA if any tile failed (the
- * window is then incomplete). */
+ * match the decoded bytes, which zlib reports to GDAL as a data error).  LZW tiles (compression 5) report 8 when the
+ * input ends and 9 when EOI comes before the tile is full (libtiff's "Not enough data"), 11 for an old-style
+ * (pre-TIFF 5.0, LSB-first) stream, which is not supported, and 12 for a code libtiff refuses: above the next free
+ * entry, a first code after Clear above 257, a code before the first Clear, or a table that overflows without a Clear
+ * (lzw_core.h).  Returns GCN10_EDATA if any tile failed (the window is then incomplete). */
 int gcn10_cuda_inflate_tiles(gcn10_ctx *ctx, const gcn10_tile_source *src, int w, int h,
                              uint8_t *out, size_t out_pitch, int *tile_status);
 
