@@ -105,18 +105,9 @@ int main(int argc, char **argv)
         fprintf(stderr, "[rank 0] missing -c/--config <file>; see 'gcn10 -h' for usage.\n");    /* main.c:103-107 */
         return 1;
     }
-    if (opt.cog) {
-        /* a COG's levels come before its full resolution: the GPU makes them from the whole block first.  The
-         * host-deflate path encodes band by band on the host and cannot. */
-        const char *hd = getenv("GCN10_HOST_DEFLATE");
-        if (hd && *hd && *hd != '0') {
-            fprintf(stderr, "[rank 0] --cog cannot be combined with GCN10_HOST_DEFLATE=1: that diagnostic path encodes "
-                            "the outputs band by band on the host, and a COG's overview levels must precede its full "
-                            "resolution\n");
-            return 1;
-        }
+    /* a COG's levels come before its full resolution: the GPU makes them from the whole block first */
+    if (opt.cog)
         opt.overviews = GCN10_MAX_OVERVIEWS;
-    }
     char err[GH_ERRLEN] = "";
     if (gh_config_parse(conf, &opt.cfg, err, sizeof err)) {
         fprintf(stderr, "%s\n", err);                           /* config.c:52,108-111 */

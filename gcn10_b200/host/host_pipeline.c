@@ -18,8 +18,8 @@
  *                   (files are created when the first strip arrives, i.e. after the land cover decoded cleanly,
  *                   under a temporary name that is renamed on success).
  *
- * Land cover that is not tiled DEFLATE is decoded on the host band by band (gcn10_cuda_block_deflate_rows);
- * with GCN10_HOST_DEFLATE=1 the raw planes come back instead and a zlib thread pool encodes them.
+ * Land cover that is not tiled DEFLATE or LZW (or any, with GCN10_HOST_INFLATE=1) is decoded on the host: band by
+ * band (gcn10_cuda_block_deflate_rows), or whole with --cog (gcn10_cuda_block_deflate).  Every path encodes on the GPU.
  *
  * gh_run_blocks() replaces the MPI round-robin of main.c:171: one worker and one gcn10_ctx per GPU, block ids
  * popped from a shared atomic counter; the join of the workers is the barrier (main.c:187).  No data moves
@@ -48,7 +48,6 @@ static const char *const k_arcs[3] = { "i", "ii", "iii" };             /* cn.c:1
 
 typedef struct {
     uint8_t *esa;                   /* pinned: BAND_ROWS x pitch */
-    uint8_t *planes[NPLANES];       /* pinned: BAND_ROWS x pitch each */
     int y0, rows;
     int state;                      /* 0 free, 1 filled (waiting for its consumer), -1 read failed */
 } band_buf;
@@ -96,25 +95,21 @@ typedef struct worker {
     pthread_mutex_t lmu;
     pthread_cond_t lcv;
     size_t pitch_cap;
-    int have_planes;
     band_buf bands[2];
     uint8_t *whole;                 /* --cog, land cover decoded on the host: the whole window, pinned */
     size_t whole_cap;
-    /* encoder hand-off */
+    /* band reader hand-off */
     pthread_mutex_t mu;
     pthread_cond_t cv;
     gh_tiffw *writers[NPLANES];
     int writers_open;
     char paths[NPLANES][PATH_MAX];
-    /* --aggregate: the mean rasters' files, opened and closed with the 18 outputs, and (host-deflate path) the host
-     * aggregation of each plane */
+    /* --aggregate: the mean rasters' files, opened and closed with the 18 outputs */
     gh_tiffw *agg_writers[NPLANES];
-    gh_aggregate *aggs[NPLANES];
     char agg_paths[NPLANES][PATH_MAX];
     int out_w, out_h;
     double out_gt[6];
     int cur_block;
-    size_t pitch;
     atomic_int encode_failed;       /* set by I/O pool threads, read by the worker */
     int encoder_quit;
 } worker;
@@ -133,25 +128,18 @@ static void fatal(worker *wk, const char *msg)
     exit(1);
 }
 
-static int ensure_bands(worker *wk, size_t pitch, int need_planes)
+static int ensure_bands(worker *wk, size_t pitch)
 {
-    if (wk->pitch_cap >= pitch && (!need_planes || wk->have_planes))
+    if (wk->pitch_cap >= pitch)
         return 0;
     for (int b = 0; b < 2; b++) {
         gcn10_cuda_host_free(wk->bands[b].esa);
         wk->bands[b].esa = gcn10_cuda_host_alloc(pitch * BAND_ROWS);
-        for (int k = 0; k < NPLANES; k++) {
-            gcn10_cuda_host_free(wk->bands[b].planes[k]);
-            wk->bands[b].planes[k] = need_planes ? gcn10_cuda_host_alloc(pitch * BAND_ROWS) : NULL;
-            if (need_planes && !wk->bands[b].planes[k])
-                return -1;
-        }
         if (!wk->bands[b].esa)
             return -1;
         wk->bands[b].state = 0;
     }
     wk->pitch_cap = pitch;
-    wk->have_planes = need_planes;
     return 0;
 }
 
@@ -181,8 +169,6 @@ static void abort_agg_writers(worker *wk)
         if (wk->agg_writers[k])
             gh_tiffw_abort(wk->agg_writers[k]);
         wk->agg_writers[k] = NULL;
-        gh_aggregate_free(wk->aggs[k]);
-        wk->aggs[k] = NULL;
     }
 }
 
@@ -207,9 +193,7 @@ static int open_agg_writers(worker *wk)
         if (wk->esa_r && gh_raster_geokeys(wk->esa_r, &gk) == 0)
             gh_tiffw_set_geokeys(wk->agg_writers[k], &gk);
         pthread_mutex_unlock(&wk->rmu);
-        wk->aggs[k] = gh_aggregate_new(wk->out_w, wk->out_h, f);
-        if (gh_tiffw_set_nodata(wk->agg_writers[k], 1) || (wk->opt->cog && gh_tiffw_set_cog(wk->agg_writers[k], 1)) ||
-            !wk->aggs[k]) {
+        if (gh_tiffw_set_nodata(wk->agg_writers[k], 1) || (wk->opt->cog && gh_tiffw_set_cog(wk->agg_writers[k], 1))) {
             snprintf(err, sizeof err, "write error 3 on %s (aggregate)", wk->agg_paths[k]);
             gh_log_message(wk->log, "ERROR", err, 1);
             abort_agg_writers(wk);
@@ -260,37 +244,7 @@ static int open_writers(worker *wk)
     return 0;
 }
 
-/* encoder thread: compresses and appends filled bands in order */
-static void *encoder_main(void *arg)
-{
-    worker *wk = arg;
-    int turn = 0;
-    for (;;) {
-        pthread_mutex_lock(&wk->mu);
-        while (wk->bands[turn].state != 1 && !wk->encoder_quit)
-            pthread_cond_wait(&wk->cv, &wk->mu);
-        if (wk->bands[turn].state != 1 && wk->encoder_quit) {
-            pthread_mutex_unlock(&wk->mu);
-            return NULL;
-        }
-        pthread_mutex_unlock(&wk->mu);
-        band_buf *bb = &wk->bands[turn];
-        if (open_writers(wk))
-            atomic_store(&wk->encode_failed, 1);
-        for (int k = 0; k < NPLANES && !atomic_load(&wk->encode_failed); k++)
-            if (gh_tiffw_write_rows(wk->writers[k], bb->planes[k], wk->pitch, bb->y0, bb->rows, wk->io_threads) ||
-                (wk->opt->aggregate && gh_aggregate_write_rows(wk->aggs[k], wk->agg_writers[k], bb->planes[k], wk->pitch,
-                                                               bb->y0, bb->rows, wk->io_threads)))
-                atomic_store(&wk->encode_failed, 1);
-        pthread_mutex_lock(&wk->mu);
-        bb->state = 0;
-        pthread_cond_broadcast(&wk->cv);
-        pthread_mutex_unlock(&wk->mu);
-        turn ^= 1;
-    }
-}
-
-/* ---- GPU-deflate path: reader thread -> gcn10_cuda_block_deflate_rows -> append compressed tiles ---- */
+/* ---- host-decoded bands: reader thread -> gcn10_cuda_block_deflate_rows -> append compressed tiles ---- */
 
 typedef struct {
     worker *wk;
@@ -376,10 +330,9 @@ static int tile_sink(void *user, const gcn10_tile_strip *st)
     return atomic_load(&wk->encode_failed) ? 1 : 0;
 }
 
-/* option "stats" on the GPU-deflate paths: the histograms the GPU counted while it encoded the block go to the writers,
- * which turn them into the files' statistics on close (after the block's last band, or its one call).  Runs on the
- * thread that called the library, which is also the one whose tile sink opened the writers.  (The host-deflate path
- * needs none: gh_tiffw_write_rows counts the rows it compresses.) */
+/* option "stats": the histograms the GPU counted while it encoded the block go to the writers, which turn them into the
+ * files' statistics on close (after the block's last band, or its one call).  Runs on the thread that called the
+ * library, which is also the one whose tile sink opened the writers. */
 static void put_gpu_histograms(worker *wk)
 {
     if (!wk->opt->stats || !wk->writers_open || atomic_load(&wk->encode_failed))
@@ -508,58 +461,6 @@ static int block_gpu_whole(worker *wk, int block_id, const gh_window *we, const 
     return 0;
 }
 
-/* ---- host-deflate path: raw planes back, zlib thread pool encodes band i while band i+1 is computed ---- */
-
-static int bands_host_deflate(worker *wk, int block_id, const gh_window *we, const uint8_t *hsg, const gh_window *wh,
-                              size_t pitch, double *t_read, double *t_gpu)
-{
-    char msg[1024], err[GH_ERRLEN] = "";
-    const int w = we->xcount, h = we->ycount;
-    wk->encoder_quit = 0;
-    wk->bands[0].state = wk->bands[1].state = 0;
-    pthread_t enc;
-    if (pthread_create(&enc, NULL, encoder_main, wk) != 0)
-        fatal(wk, "cannot start the encoder thread");
-    gcn10_cuda_set_option(wk->ctx, "strip_rows", BAND_STRIP_ROWS);
-    int turn = 0, failed = 0;
-    for (int y0 = 0; y0 < h && !failed; y0 += BAND_ROWS, turn ^= 1) {
-        band_buf *bb = &wk->bands[turn];
-        int rows = h - y0 < BAND_ROWS ? h - y0 : BAND_ROWS;
-        pthread_mutex_lock(&wk->mu);
-        while (bb->state != 0)
-            pthread_cond_wait(&wk->cv, &wk->mu);
-        pthread_mutex_unlock(&wk->mu);
-        double t0 = now_s();
-        if (read_band(wk, we, y0, rows, bb->esa, pitch, err, sizeof err)) {
-            gh_log_message(wk->log, "ERROR", err, 1);                               /* raster.c:182-186 */
-            failed = 1;
-            break;
-        }
-        double t1 = now_s();
-        int rc = gcn10_cuda_block_rows(wk->ctx, bb->esa, w, h, y0, rows, pitch, we->gt, hsg, wh->xcount, wh->ycount,
-                                       (size_t)wh->xcount, wh->gt, GCN10_MASK_ALL, bb->planes, pitch);
-        if (rc) {
-            snprintf(msg, sizeof msg, "cuda failure on block %d: %s", block_id, gcn10_cuda_last_error());
-            fatal(wk, msg);
-        }
-        *t_read += t1 - t0;
-        *t_gpu += now_s() - t1;
-        bb->y0 = y0;
-        bb->rows = rows;
-        pthread_mutex_lock(&wk->mu);
-        bb->state = 1;
-        pthread_cond_broadcast(&wk->cv);
-        pthread_mutex_unlock(&wk->mu);
-    }
-    gcn10_cuda_set_option(wk->ctx, "strip_rows", 2048);
-    pthread_mutex_lock(&wk->mu);
-    wk->encoder_quit = 1;
-    pthread_cond_broadcast(&wk->cv);
-    pthread_mutex_unlock(&wk->mu);
-    pthread_join(enc, NULL);
-    return failed;
-}
-
 /* ---- the loader: everything of process_block() that happens before the first pixel is computed ---------- */
 
 static gh_raster *open_once(worker *wk, gh_raster **slot, const char *path)
@@ -642,12 +543,12 @@ static void load_block(worker *wk, block_input *in, int block_id)
 
     /* a tiled DEFLATE or LZW land-cover file without predictor (what GDAL writes for COMPRESS=DEFLATE / LZW TILED=YES;
      * the ESA WorldCover files are DEFLATE) is handed to the GPU compressed; anything else is decoded later, band by band */
-    const char *hd = getenv("GCN10_HOST_DEFLATE"), *hi = getenv("GCN10_HOST_INFLATE");
-    const int host_side = (hd && *hd && *hd != '0') || (hi && *hi && *hi != '0');
+    const char *hi = getenv("GCN10_HOST_INFLATE");
+    const int host_inflate = hi && *hi && *hi != '0';
     gh_raster_part rp[MAX_PARTS];
     int np = 0;
-    int prc = host_side ? 1 : gh_raster_window_parts(wk->esa_r, in->we.xoff, in->we.yoff, in->we.xcount, in->we.ycount, rp,
-                                                     MAX_PARTS, &np, err, sizeof err);
+    int prc = host_inflate ? 1 : gh_raster_window_parts(wk->esa_r, in->we.xoff, in->we.yoff, in->we.xcount, in->we.ycount,
+                                                        rp, MAX_PARTS, &np, err, sizeof err);
     if (prc < 0) {
         gh_log_message(wk->log, "ERROR", err, 1);
         in->failed = 1;
@@ -755,13 +656,10 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
     const gh_window *we = &in->we, *wh = &in->wh;
     const int w = we->xcount, h = we->ycount;
     const size_t pitch = ((size_t)w + 255) / 256 * 256;
-    const char *hd = getenv("GCN10_HOST_DEFLATE");
-    const int host_deflate = hd && *hd && *hd != '0';
-    if (!in->gpu_inflate && !wk->opt->cog && ensure_bands(wk, pitch, host_deflate)) {
+    if (!in->gpu_inflate && !wk->opt->cog && ensure_bands(wk, pitch)) {
         snprintf(msg, sizeof msg, "pinned allocation failed for block %d: %s", block_id, gcn10_cuda_last_error());
         fatal(wk, msg);
     }
-    wk->pitch = pitch;
 
     /* output directories and file names (cn.c:236-256, 293-360); the files themselves appear with the first rows */
     const char *root = (wk->opt->out_root && *wk->opt->out_root) ? wk->opt->out_root : ".";
@@ -797,7 +695,6 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
     atomic_store(&wk->encode_failed, 0);
     double t_read = in->t_read, t_gpu = 0;
     int failed = in->gpu_inflate ? block_gpu_tiles(wk, in, &t_gpu)
-                 : host_deflate ? bands_host_deflate(wk, block_id, we, in->hsg, wh, pitch, &t_read, &t_gpu)
                  : wk->opt->cog ? block_gpu_whole(wk, block_id, we, in->hsg, wh, pitch, &t_read, &t_gpu)
                                 : bands_gpu_deflate(wk, block_id, we, in->hsg, wh, pitch, &t_read, &t_gpu);
 
@@ -842,7 +739,6 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
         }
         wk->agg_writers[k] = NULL;
     }
-    abort_agg_writers(wk);                      /* (frees the host aggregation; no writer is left to abort) */
     wk->writers_open = 0;
     double dt = now_s() - t_start;
     int lzw = 0;
@@ -854,8 +750,8 @@ static int gh_process_block(worker *wk, block_input *in, int total_blocks, doubl
                               : (in->nparts > 1 ? " [land cover: mosaic parts inflated on the gpu]"
                                                 : " [land cover inflated on the gpu]");
     snprintf(msg, sizeof msg,
-             "block %d: %d x %d px, 18 rasters in %.3f s (%.1f Mpx/s; read %.3f s [overlapped], gpu+copies+write %.3f s; %s deflate)%s",
-             block_id, w, h, dt, (double)w * h / dt / 1e6, t_read, t_gpu, host_deflate ? "host" : "gpu", where);
+             "block %d: %d x %d px, 18 rasters in %.3f s (%.1f Mpx/s; read %.3f s [overlapped], gpu+copies+write %.3f s; gpu deflate)%s",
+             block_id, w, h, dt, (double)w * h / dt / 1e6, t_read, t_gpu, where);
     gh_log_message(wk->log, "INFO", msg, 0);
     return ok ? 0 : -1;
 }
@@ -864,7 +760,7 @@ static void *worker_main(void *arg)
 {
     worker *wk = arg;
     char msg[256];
-    /* keep this worker (and the loader / reader / encoder threads it spawns, which inherit the mask) on the
+    /* keep this worker (and the loader / reader threads it spawns, which inherit the mask) on the
      * NUMA node of its GPU so that the pinned buffers are node-local */
     int node = gcn10_cuda_bind_host_thread(wk->device);
     snprintf(msg, sizeof msg, "worker %d on gpu %d, numa node %d", wk->index, wk->device, node);
@@ -911,11 +807,8 @@ static void *worker_main(void *arg)
         pthread_mutex_unlock(&wk->lmu);
     }
     pthread_join(loader, NULL);
-    for (int b = 0; b < 2; b++) {
+    for (int b = 0; b < 2; b++)
         gcn10_cuda_host_free(wk->bands[b].esa);
-        for (int k = 0; k < NPLANES; k++)
-            gcn10_cuda_host_free(wk->bands[b].planes[k]);
-    }
     gcn10_cuda_host_free(wk->whole);
     for (int i = 0; i < LOAD_SLOTS; i++) {
         gcn10_cuda_host_free(wk->in[i].blob);

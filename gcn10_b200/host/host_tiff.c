@@ -1569,110 +1569,3 @@ int gh_tiff_write_cog(const char *path, const uint8_t *data, int w, int h, size_
     }
     return 0;
 }
-
-/* ---- mean rasters on the host (gh_aggregate_*) ---- */
-
-struct gh_aggregate {
-    int w, h, f, cw, ch;
-    uint32_t *sum, *cnt;        /* the cell row in progress */
-    int next_y, next_cell;      /* the next plane row and cell row */
-    uint8_t *buf;               /* completed cell rows not yet written: rows buf_row0 .. + buf_rows */
-    int buf_rows, buf_cap, buf_row0;
-};
-
-gh_aggregate *gh_aggregate_new(int w, int h, int f)
-{
-    if (w <= 0 || h <= 0 || f < 2 || f > GCN10_MAX_AGGREGATE)
-        return NULL;
-    gh_aggregate *a = calloc(1, sizeof *a);
-    if (!a)
-        return NULL;
-    a->w = w;
-    a->h = h;
-    a->f = f;
-    a->cw = gcn10_aggregate_dim(w, f);
-    a->ch = gcn10_aggregate_dim(h, f);
-    a->sum = calloc((size_t)a->cw, sizeof *a->sum);
-    a->cnt = calloc((size_t)a->cw, sizeof *a->cnt);
-    if (!a->sum || !a->cnt) {
-        gh_aggregate_free(a);
-        return NULL;
-    }
-    return a;
-}
-
-void gh_aggregate_free(gh_aggregate *a)
-{
-    if (!a)
-        return;
-    free(a->sum);
-    free(a->cnt);
-    free(a->buf);
-    free(a);
-}
-
-int gh_aggregate_rows(gh_aggregate *a, const uint8_t *data, size_t pitch, int y0, int nrows, uint8_t *out, size_t out_pitch,
-                      int *row0)
-{
-    if (!a || !data || !out || nrows < 0 || y0 != a->next_y || nrows > a->h - y0 || out_pitch < (size_t)a->cw)
-        return -1;
-    if (row0)
-        *row0 = a->next_cell;
-    int n = 0;
-    for (int y = y0; y < y0 + nrows; y++) {
-        const uint8_t *row = data + (size_t)(y - y0) * pitch;
-        for (int cx = 0, x = 0; cx < a->cw; cx++) {
-            const int xe = x + a->f < a->w ? x + a->f : a->w;
-            uint32_t s = 0, c = 0;
-            for (; x < xe; x++)
-                if (row[x] != GCN10_NODATA) {
-                    s += row[x];
-                    c++;
-                }
-            a->sum[cx] += s;
-            a->cnt[cx] += c;
-        }
-        if ((y + 1) % a->f == 0 || y + 1 == a->h) {
-            uint8_t *o = out + (size_t)n * out_pitch;
-            for (int cx = 0; cx < a->cw; cx++)
-                o[cx] = gcn10_aggregate_value(a->sum[cx], a->cnt[cx]);
-            memset(a->sum, 0, (size_t)a->cw * sizeof *a->sum);
-            memset(a->cnt, 0, (size_t)a->cw * sizeof *a->cnt);
-            n++;
-        }
-    }
-    a->next_y = y0 + nrows;
-    a->next_cell += n;
-    return n;
-}
-
-int gh_aggregate_write_rows(gh_aggregate *a, gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0, int nrows, int threads)
-{
-    if (!a || !tw)
-        return -1;
-    const int most = nrows / a->f + 2;                  /* cell rows this band can complete (the last one short) */
-    if (a->buf_rows + most > a->buf_cap) {
-        const int cap = a->buf_rows + most + TILE;
-        uint8_t *b = realloc(a->buf, (size_t)cap * (size_t)a->cw);
-        if (!b)
-            return -1;
-        a->buf = b;
-        a->buf_cap = cap;
-    }
-    if (a->buf_rows == 0)
-        a->buf_row0 = a->next_cell;
-    const int n = gh_aggregate_rows(a, data, pitch, y0, nrows, a->buf + (size_t)a->buf_rows * a->cw, (size_t)a->cw, NULL);
-    if (n < 0)
-        return -1;
-    a->buf_rows += n;
-    const int done = a->buf_row0 + a->buf_rows == a->ch;
-    const int put = done ? a->buf_rows : a->buf_rows / TILE * TILE;
-    if (put > 0) {
-        if (gh_tiffw_write_rows(tw, a->buf, (size_t)a->cw, a->buf_row0, put, threads))
-            return -1;
-        memmove(a->buf, a->buf + (size_t)put * a->cw, (size_t)(a->buf_rows - put) * a->cw);
-        a->buf_rows -= put;
-        a->buf_row0 += put;
-    }
-    return 0;
-}

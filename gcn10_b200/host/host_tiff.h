@@ -70,20 +70,6 @@ int gh_tiffw_put_level_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nro
  * tile whose framing is wrong fails the file. */
 int gh_tiffw_put_framed_tile_rows(gh_tiffw *tw, int level, int tile_row0, int nrows, const uint8_t *blob,
                                   const uint64_t *offsets, const uint32_t *sizes);
-/* Mean rasters on the host (option "aggregate" where the raw planes come back): the rule of gcn10_aggregate_dim /
- * _value (include/gcn10_cuda.h) applied band by band.  A gh_aggregate belongs to one plane of a w x h block and keeps the
- * partial cell row between bands.
- *   gh_aggregate_rows        adds rows [y0, y0 + nrows) (y0 continues the previous call) and writes the cell rows they
- *                            complete to out (cw bytes each, out_pitch apart), the first of them cell row *row0; returns
- *                            how many (at most nrows / f + 2), -1 on a bad argument or a band out of order
- *   gh_aggregate_write_rows  the same, appended to the w / f x h / f GeoTIFF tw with gh_tiffw_write_rows (cell rows wait
- *                            until a whole 256-row tile row of the mean raster or the raster's end is there) */
-typedef struct gh_aggregate gh_aggregate;
-gh_aggregate *gh_aggregate_new(int w, int h, int f);
-int gh_aggregate_rows(gh_aggregate *a, const uint8_t *data, size_t pitch, int y0, int nrows, uint8_t *out, size_t out_pitch,
-                      int *row0);
-int gh_aggregate_write_rows(gh_aggregate *a, gh_tiffw *tw, const uint8_t *data, size_t pitch, int y0, int nrows, int threads);
-void gh_aggregate_free(gh_aggregate *a);
 /* Runs fn(arg, 0..n-1) on up to `threads` threads (the calling thread included). */
 void gh_parallel_for(int n, int threads, void (*fn)(void *arg, int index), void *arg);
 /* Writes the tile tables, georeferencing and IFD; 0 ok. */

@@ -83,12 +83,6 @@ def load(path: str | None = None) -> C.CDLL:
     L.gh_tiffw_set_cog.argtypes = [_vp, C.c_int]
     L.gh_tiffw_put_framed_tile_rows.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, C.POINTER(C.c_uint64),
                                                 C.POINTER(C.c_uint32)]
-    L.gh_aggregate_new.argtypes = [C.c_int, C.c_int, C.c_int]
-    L.gh_aggregate_new.restype = _vp
-    L.gh_aggregate_rows.argtypes = [_vp, _vp, C.c_size_t, C.c_int, C.c_int, _vp, C.c_size_t, _ip]
-    L.gh_aggregate_write_rows.argtypes = [_vp, _vp, _vp, C.c_size_t, C.c_int, C.c_int, C.c_int]
-    L.gh_aggregate_free.argtypes = [_vp]
-    L.gh_aggregate_free.restype = None
     L.gh_tiffw_put_level_tile_rows.argtypes = [_vp, C.c_int, C.c_int, C.c_int, _vp, C.POINTER(C.c_uint64),
                                                C.POINTER(C.c_uint32)]
     L.gh_tiffw_close.argtypes = [_vp]
@@ -357,17 +351,10 @@ class TiffWriter:
     """Incremental tiled-DEFLATE GeoTIFF writer (gh_tiffw_*): raw row bands or pre-compressed tile rows.
     ``overviews=n`` adds up to n overview levels (gh_tiffw_set_overviews); ``levels`` is how many the file gets.
     ``stats=True`` adds the NoData tag and the band statistics (gh_tiffw_set_stats): write_rows counts the pixels itself,
-    tiles put already compressed need ``put_histogram``.  ``nodata=True`` adds the NoData tag alone (gh_tiffw_set_nodata).
-    ``aggregate=f`` makes the file the f x f mean raster of a w x h plane: the file is ceil(w / f) x ceil(h / f) with the
-    geotransform scaled by f, NoData 255, and ``write_plane_rows`` feeds it the plane's rows (gh_aggregate_write_rows)."""
+    tiles put already compressed need ``put_histogram``.  ``nodata=True`` adds the NoData tag alone (gh_tiffw_set_nodata)."""
 
     def __init__(self, path: str, w: int, h: int, gt, overviews: int = 0, stats: bool = False, nodata: bool = False,
-                 aggregate: int = 0, geokeys=None, cog: bool = False):
-        self.agg = Aggregate(w, h, aggregate) if aggregate else None
-        if aggregate:
-            f = aggregate
-            w, h, gt = -(-w // f), -(-h // f), (gt[0], gt[1] * f, gt[2] * f, gt[3], gt[4] * f, gt[5] * f)
-            nodata = True
+                 geokeys=None, cog: bool = False):
         self.L = load()
         h_ = _vp()
         e = _err()
@@ -443,46 +430,10 @@ class TiffWriter:
         data = np.ascontiguousarray(data, dtype=np.uint8)
         return self.L.gh_tiffw_write_rows(self.h, data.ctypes.data, data.shape[1], y0, data.shape[0], threads)
 
-    def write_plane_rows(self, data: np.ndarray, y0: int, threads: int = 2):
-        """Mean-raster files (``aggregate=f``): rows [y0, y0 + len) of the full-resolution plane."""
-        data = np.ascontiguousarray(data, dtype=np.uint8)
-        return self.L.gh_aggregate_write_rows(self.agg.h, self.h, data.ctypes.data, data.shape[1], y0, data.shape[0],
-                                              threads)
-
     def close(self):
         rc = self.L.gh_tiffw_close(self.h)
         self.h = None
-        if self.agg is not None:
-            self.agg.free()
         return rc
-
-
-class Aggregate:
-    """The host's mean-raster rule over one w x h plane fed band by band (gh_aggregate_*)."""
-
-    def __init__(self, w: int, h: int, f: int):
-        self.L = load()
-        self.h = self.L.gh_aggregate_new(w, h, f)
-        if not self.h:
-            raise HostError(-1, f"gh_aggregate_new({w}, {h}, {f}) failed")
-        self.cw = -(-w // f)
-        self.f = f
-
-    def rows(self, data: np.ndarray, y0: int):
-        """Adds rows [y0, y0 + len) of the plane; returns (first cell row, uint8 [n, cw]) of the cell rows completed."""
-        data = np.ascontiguousarray(data, dtype=np.uint8)
-        out = np.zeros((data.shape[0] // self.f + 2, self.cw), np.uint8)     # (+ the block's last, short cell row)
-        row0 = C.c_int()
-        n = self.L.gh_aggregate_rows(self.h, data.ctypes.data, data.shape[1], y0, data.shape[0], out.ctypes.data,
-                                     self.cw, C.byref(row0))
-        if n < 0:
-            raise HostError(n, f"gh_aggregate_rows(y0={y0}, rows={data.shape[0]}) refused")
-        return row0.value, out[:n]
-
-    def free(self):
-        if self.h:
-            self.L.gh_aggregate_free(self.h)
-            self.h = None
 
 
 def write_tiled_deflate_tiff(path: str, w: int, h: int, tile_w: int, tile_h: int, blob, offsets, sizes, gt):

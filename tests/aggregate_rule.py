@@ -35,8 +35,3 @@ def value(s, n):
 def mean(plane, f):
     """uint8 [ceil(h / f), ceil(w / f)]: the mean raster of a plane."""
     return value(*sums(plane, f))
-
-
-def gt(t, f):
-    """The mean raster's geotransform."""
-    return (t[0], t[1] * f, t[2] * f, t[3], t[4] * f, t[5] * f)

@@ -1,9 +1,23 @@
 """Fixture writers for the host-program tests: a block shapefile (.shp/.shx/.dbf, PolygonZ records with
-an integer ID attribute, like /root/reference/blocks/esa_extent_blocks.*) and GeoTIFF rasters."""
+an integer ID attribute, like /root/reference/blocks/esa_extent_blocks.*) and GeoTIFF rasters; and the runner of the
+gcn10 executable on such a world."""
 import os
 import struct
+import subprocess
 
 import numpy as np
+
+from gcn10_b200 import hostlib
+
+
+def run_program(root, config="config.txt", *extra, host_inflate=False):
+    """gcn10 on one GPU with the config <root>/<config> and the block list <root>/blocks.txt, run from root; the land
+    cover is decoded on the host with host_inflate (GCN10_HOST_INFLATE=1).  Returns the CompletedProcess."""
+    assert os.path.exists(hostlib.EXE_PATH), "gcn10 executable not built (make host)"
+    env = dict(os.environ, GCN10_HOST_INFLATE="1" if host_inflate else "0")
+    return subprocess.run([hostlib.EXE_PATH, "-c", os.path.join(root, config), "-l", os.path.join(root, "blocks.txt"),
+                           "--gpus", "1", "--io-threads", "4", *extra], cwd=str(root), capture_output=True, text=True,
+                          timeout=300, env=env)
 
 
 def write_block_shapefile(path_shp, blocks):

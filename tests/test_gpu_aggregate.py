@@ -3,14 +3,13 @@ behind the block's full-resolution strips and overview levels.  Every mean tile 
 must equal the rule of include/gcn10_cuda.h (tests/aggregate_rule.py) applied to the oracle's planes, byte for byte;
 the full-resolution strips must be byte-identical to the same call without the option."""
 import os
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 
-from gcn10_b200 import capi, hostlib, synth
+from gcn10_b200 import capi, synth
 from tests import aggregate_rule as A
+from tests import fixtures
 from tests import overview_rule as R
 from tests.cases import SMALL_CASES, make_block
 from tests.test_gpu_overviews import T, _assemble, _parts, world  # noqa: F401  (world: the program's input fixture)
@@ -338,18 +337,6 @@ def test_full_size_block(shape, ctx, port, tables):
 
 # ---- the program, file to file ---------------------------------------------------------------------------------
 
-def _program(world, config, outdir, host_deflate=False, host_inflate=False, extra=("--aggregate", "25")):
-    env = dict(os.environ, GCN10_HOST_DEFLATE="1" if host_deflate else "0",
-               GCN10_HOST_INFLATE="1" if host_inflate else "0")
-    root = world["root"]
-    shutil.rmtree(outdir, ignore_errors=True)
-    os.makedirs(outdir)
-    r = subprocess.run([hostlib.EXE_PATH, "-c", str(root / config), "-l", str(root / "blocks.txt"), "--gpus", "1",
-                        "--io-threads", "4", "-o", "--outdir", str(outdir)] + list(extra), cwd=str(root),
-                       capture_output=True, text=True, timeout=300, env=env)
-    assert r.returncode == 0, r.stderr
-
-
 def _read(path):
     from PIL import Image
     with Image.open(path) as im:
@@ -360,9 +347,11 @@ def _read(path):
 @pytest.mark.parametrize("config", ["config.txt", "config_vrt.txt"], ids=["geotiff", "vrt_mosaic"])
 def test_program_aggregate(world, reference, config, tmp_path):
     root = world["root"]
-    modes = dict(gpu=(False, False), host_inflate=(False, True), host_deflate=(True, True))
-    for mode, (hd, hi) in modes.items():
-        _program(world, config, tmp_path / mode, hd, hi)
+    modes = dict(gpu=False, host_inflate=True)
+    for mode, hi in modes.items():
+        r = fixtures.run_program(root, config, "-o", "--outdir", str(tmp_path / mode), "--aggregate", "25",
+                                 host_inflate=hi)
+        assert r.returncode == 0, r.stderr
     for bid, x0, y0, x1, y1 in world["blocks"]:
         want = reference.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
                                    str(root / "lookups"), block_id=bid)
@@ -379,5 +368,5 @@ def test_program_aggregate(world, reference, config, tmp_path):
             assert keys == full[4], agg_rel                 # the land cover's GeoKeys
             assert tuple(scale)[:2] == pytest.approx((full[3][0] * 25, full[3][1] * 25), rel=1e-15)
             assert tuple(tie) == tuple(full[2])
-            for m in modes:                                 # the three paths write the same file contents
+            for m in modes:                                 # both paths write the same file contents
                 assert np.array_equal(got[m][0], img) and got[m][1:] == got["gpu"][1:], (agg_rel, m)

@@ -3,15 +3,12 @@ then the full resolution, then the mean rasters, and with "ordered" every tile l
 Optimized GeoTIFF.  The tile streams must be byte-identical to the same call without the option; the framing is
 checked on every tile; the program's outputs must pass tests/cog_rule.py and equal the reference."""
 import ctypes as C
-import os
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 
-from gcn10_b200 import capi, hostlib, synth
-from tests import cog_rule
+from gcn10_b200 import capi, synth
+from tests import cog_rule, fixtures
 from tests import overview_rule as R
 from tests.cases import SMALL_CASES, make_block
 from tests.test_gpu_overviews import _assemble, _frames, _parts, world  # noqa: F401  (world: module fixture)
@@ -238,22 +235,12 @@ def test_full_size_block(shape, ctx, port, tables):
 
 # ---- the program, file to file ---------------------------------------------------------------------------------
 
-def _program(world, config, outdir, host_inflate=False, host_deflate=False, extra=()):
-    env = dict(os.environ, GCN10_HOST_DEFLATE="1" if host_deflate else "0",
-               GCN10_HOST_INFLATE="1" if host_inflate else "0")
-    root = world["root"]
-    shutil.rmtree(outdir, ignore_errors=True)
-    os.makedirs(outdir)
-    return subprocess.run([hostlib.EXE_PATH, "-c", str(root / config), "-l", str(root / "blocks.txt"), "--gpus", "1",
-                           "--io-threads", "4", "-o", "--outdir", str(outdir), *extra], cwd=str(root),
-                          capture_output=True, text=True, timeout=300, env=env)
-
-
 @pytest.mark.parametrize("config,host_inflate", [("config.txt", False), ("config_vrt.txt", False), ("config.txt", True)],
                          ids=["geotiff", "vrt_mosaic", "host_inflate"])
 def test_program_cog(world, reference, config, host_inflate, tmp_path):  # noqa: F811
     root = world["root"]
-    r = _program(world, config, tmp_path, host_inflate, extra=("--cog", "--stats", "--aggregate", str(AGG)))
+    r = fixtures.run_program(root, config, "-o", "--outdir", str(tmp_path), "--cog", "--stats", "--aggregate", str(AGG),
+                             host_inflate=host_inflate)
     assert r.returncode == 0, r.stderr
     for bid, x0, y0, x1, y1 in world["blocks"]:
         want = reference.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
@@ -270,9 +257,3 @@ def test_program_cog(world, reference, config, host_inflate, tmp_path):  # noqa:
             agg = str(tmp_path / f"{cond}_agg{AGG}" / name)
             assert len(cog_rule.check(agg)) == 1, agg               # the mean raster: a COG without levels
             assert len(_frames(agg)) == 1
-
-
-def test_program_cog_refuses_host_deflate(world, tmp_path):  # noqa: F811
-    r = _program(world, "config.txt", tmp_path, host_deflate=True, extra=("--cog",))
-    assert r.returncode != 0
-    assert "--cog cannot be combined with GCN10_HOST_DEFLATE=1" in r.stderr

@@ -194,8 +194,6 @@ def test_full_size_block_equals_deflate_input(shape, gpu_ctx):
 def test_program_on_lzw_land_cover(mosaic, reference, tmp_path):
     """gcn10 on an LZW GeoTIFF, and on a VRT whose sources are LZW and DEFLATE files: the land cover is decoded on the
     GPU, the 18 rasters equal the reference's process_block() and the GCN10_HOST_INFLATE=1 run."""
-    import os
-    import subprocess
     from gcn10_b200 import hostlib
     from tests import fixtures, lookups
     from tests.lzw_files import recode_to_lzw
@@ -229,9 +227,7 @@ def test_program_on_lzw_land_cover(mosaic, reference, tmp_path):
         fixtures.write_config(str(run / "config.txt"), land, str(tmp_path / "hsg.tif"), str(tmp_path / "blocks.shp"),
                               str(tmp_path / "lookups"), str(run / "logs"))
         (run / "blocks.txt").write_text("21\n")
-        env = dict(os.environ, GCN10_HOST_INFLATE="1" if host_inflate else "0", GCN10_HOST_DEFLATE="0")
-        r = subprocess.run([hostlib.EXE_PATH, "-c", str(run / "config.txt"), "-l", str(run / "blocks.txt"), "--gpus",
-                            "1", "-o"], cwd=str(run), capture_output=True, text=True, timeout=300, env=env)
+        r = fixtures.run_program(run, "config.txt", "-o", host_inflate=host_inflate)
         assert r.returncode == 0, r.stderr
         log = (run / "logs" / "rank_0.log").read_text()
         assert (tag in log) == (not host_inflate), log[-2000:]

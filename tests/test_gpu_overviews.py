@@ -2,9 +2,6 @@
 selected plane behind the block's full-resolution strips.  Every level tile is inflated with CPython's zlib and must
 equal the rule of include/gcn10_cuda.h (tests/overview_rule.py) applied to the oracle's planes; the full-resolution
 strips must be byte-identical to the same call without the option."""
-import os
-import shutil
-import subprocess
 import zlib
 
 import numpy as np
@@ -301,18 +298,6 @@ def world(tmp_path_factory):
     return dict(root=root, esa=esa, esa_t=esa_t, hsg=hsg, hsg_t=hsg_t, blocks=blocks)
 
 
-def _program(world, config, outdir, host_deflate=False, host_inflate=False):
-    env = dict(os.environ, GCN10_HOST_DEFLATE="1" if host_deflate else "0",
-               GCN10_HOST_INFLATE="1" if host_inflate else "0")
-    root = world["root"]
-    shutil.rmtree(outdir, ignore_errors=True)
-    os.makedirs(outdir)
-    r = subprocess.run([hostlib.EXE_PATH, "-c", str(root / config), "-l", str(root / "blocks.txt"), "--gpus", "1",
-                        "--io-threads", "4", "-o", "--overviews", "--outdir", str(outdir)], cwd=str(root),
-                       capture_output=True, text=True, timeout=300, env=env)
-    assert r.returncode == 0, r.stderr
-
-
 def _frames(path):
     from PIL import Image
     out = []
@@ -326,9 +311,10 @@ def _frames(path):
 @pytest.mark.parametrize("config", ["config.txt", "config_vrt.txt"], ids=["geotiff", "vrt_mosaic"])
 def test_program_overviews(world, reference, config, tmp_path):
     root = world["root"]
-    modes = dict(gpu=(False, False), host_inflate=(False, True), host_deflate=(True, True))
-    for mode, (hd, hi) in modes.items():
-        _program(world, config, tmp_path / mode, hd, hi)
+    modes = dict(gpu=False, host_inflate=True)
+    for mode, hi in modes.items():
+        r = fixtures.run_program(root, config, "-o", "--overviews", "--outdir", str(tmp_path / mode), host_inflate=hi)
+        assert r.returncode == 0, r.stderr
     for bid, x0, y0, x1, y1 in world["blocks"]:
         want = reference.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
                                    str(root / "lookups"), block_id=bid)

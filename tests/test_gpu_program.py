@@ -44,27 +44,15 @@ def world(tmp_path_factory):
     return dict(root=root, esa=esa, esa_t=esa_t, hsg=hsg, hsg_t=hsg_t, blocks=blocks)
 
 
-def _run(world, *extra, host_deflate=False, host_inflate=False):
-    exe = hostlib.EXE_PATH
-    assert os.path.exists(exe), "gcn10 executable not built (make host)"
-    root = world["root"]
-    env = dict(os.environ, GCN10_HOST_DEFLATE="1" if host_deflate else "0",
-               GCN10_HOST_INFLATE="1" if host_inflate else "0")
-    return subprocess.run([exe, "-c", str(root / "config.txt"), "-l", str(root / "blocks.txt"), "--gpus", "1",
-                           "--io-threads", "4", *extra], cwd=str(root), capture_output=True, text=True, timeout=300,
-                          env=env)
-
-
-@pytest.mark.parametrize("host_deflate,host_inflate", [(False, False), (False, True), (True, True)],
-                         ids=["gpu_inflate_gpu_deflate", "host_inflate_gpu_deflate", "host_inflate_host_deflate"])
-def test_program_matches_reference_process_block(world, reference, host_deflate, host_inflate):
+@pytest.mark.parametrize("host_inflate", [False, True], ids=["gpu_inflate_gpu_deflate", "host_inflate_gpu_deflate"])
+def test_program_matches_reference_process_block(world, reference, host_inflate):
     from PIL import Image
     import shutil
     shutil.rmtree(world["root"] / "logs", ignore_errors=True)      # log files are opened for append (log.c:79)
-    r = _run(world, "-o", host_deflate=host_deflate, host_inflate=host_inflate)
+    r = fixtures.run_program(world["root"], "config.txt", "-o", host_inflate=host_inflate)
     assert r.returncode == 0, r.stderr
     log_all = (world["root"] / "logs" / "rank_0.log").read_text()
-    assert ("land cover inflated on the gpu" in log_all) == (not host_deflate and not host_inflate)
+    assert ("land cover inflated on the gpu" in log_all) == (not host_inflate)
     root = world["root"]
     for bid, x0, y0, x1, y1 in world["blocks"][:2]:
         want = reference.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
@@ -108,22 +96,22 @@ def test_damaged_land_cover_tile_skips_the_block(world, tmp_path):
     shutil.copy(str(root / "esa.tif"), str(tmp_path / "esa_good.tif"))
     try:
         (root / "esa.tif").write_bytes(bytes(data))
-        r = _run(world, "-o")
+        r = fixtures.run_program(root, "config.txt", "-o")
     finally:
         shutil.copy(str(tmp_path / "esa_good.tif"), str(root / "esa.tif"))
     assert r.returncode == 0, r.stderr
     assert "gdalrasterio error 3" in r.stderr and "esa load failed for block 11" in r.stderr
     assert "esa load failed for block 12" not in r.stderr
-    _run(world, "-o")                               # leave intact outputs behind for the following tests
+    fixtures.run_program(root, "config.txt", "-o")            # leave intact outputs behind for the following tests
 
 
 def test_no_overwrite_appends_underscore(world):
     root = world["root"]
     first = root / "cn_rasters_undrained" / "cn_g_iii_11.tif"
     if not first.exists():
-        assert _run(world, "-o").returncode == 0
+        assert fixtures.run_program(root, "config.txt", "-o").returncode == 0
     before = first.read_bytes()
-    r = _run(world)                                             # no -o: existing outputs are kept (cn.c:320-360)
+    r = fixtures.run_program(root)                              # no -o: existing outputs are kept (cn.c:320-360)
     assert r.returncode == 0, r.stderr
     second = root / "cn_rasters_undrained" / "cn_g_iii_11_.tif"
     assert second.exists() and first.read_bytes() == before
@@ -163,17 +151,15 @@ def test_program_reads_a_vrt_mosaic(world, reference, tmp_path):
     write_vrt(str(vroot / "mosaic.vrt"), W, H, esa_t, srcs)
     fixtures.write_config(str(vroot / "config.txt"), str(vroot / "mosaic.vrt"), str(root / "hsg.tif"),
                           str(root / "blocks.shp"), str(root / "lookups"), str(vroot / "logs"))
-    exe = hostlib.EXE_PATH
-    for host_inflate in ("0", "1"):
-        out = vroot / f"out{host_inflate}"
+    shutil.copy(str(root / "blocks.txt"), str(vroot / "blocks.txt"))
+    for host_inflate in (False, True):
+        out = vroot / f"out{int(host_inflate)}"
         out.mkdir()
         shutil.rmtree(vroot / "logs", ignore_errors=True)
-        r = subprocess.run([exe, "-c", str(vroot / "config.txt"), "-l", str(root / "blocks.txt"), "--gpus", "1", "-o",
-                            "--io-threads", "4", "--outdir", str(out)], cwd=str(vroot), capture_output=True, text=True,
-                           timeout=300, env=dict(os.environ, GCN10_HOST_INFLATE=host_inflate, GCN10_HOST_DEFLATE="0"))
+        r = fixtures.run_program(vroot, "config.txt", "-o", "--outdir", str(out), host_inflate=host_inflate)
         assert r.returncode == 0, r.stderr
         log = (vroot / "logs" / "rank_0.log").read_text()
-        assert ("mosaic parts inflated on the gpu" in log) == (host_inflate == "0")
+        assert ("mosaic parts inflated on the gpu" in log) == (not host_inflate)
         for bid, x0, y0, x1, y1 in world["blocks"][:2]:
             want = reference.run_block(esa, esa_t, world["hsg"], world["hsg_t"], (x0, y0, x1, y1), str(root / "lookups"),
                                  block_id=bid)
@@ -185,8 +171,7 @@ def test_program_reads_a_vrt_mosaic(world, reference, tmp_path):
     os.remove(vroot / "lc_11.tif")
     out = vroot / "out_missing"
     out.mkdir()
-    r = subprocess.run([exe, "-c", str(vroot / "config.txt"), "-l", str(root / "blocks.txt"), "--gpus", "1", "-o",
-                        "--outdir", str(out)], cwd=str(vroot), capture_output=True, text=True, timeout=300)
+    r = fixtures.run_program(vroot, "config.txt", "-o", "--outdir", str(out))
     assert r.returncode == 0
     assert "gdal open failed" in r.stderr and "esa load failed for block 12" in r.stderr
     assert not list(out.glob("cn_rasters_*/cn_*_12*"))

@@ -2,14 +2,11 @@
 (gcn10_cuda_last_histograms).  Every histogram must equal np.bincount of the oracle's planes, and the tiles must be
 byte-identical to the same call without the option.  The program's --stats outputs must carry the tags of
 tests/stats_rule.py applied to their decoded planes."""
-import os
-import shutil
-import subprocess
-
 import numpy as np
 import pytest
 
 from gcn10_b200 import capi, hostlib, synth
+from tests import fixtures
 from tests import overview_rule as R
 from tests import stats_rule as S
 from tests.cases import SMALL_CASES, make_block
@@ -243,18 +240,6 @@ def test_full_size_block(shape, ctx, port, tables):
 
 # ---- the program, file to file ---------------------------------------------------------------------------------
 
-def _program(world, config, outdir, stats, host_deflate=False, host_inflate=False):
-    env = dict(os.environ, GCN10_HOST_DEFLATE="1" if host_deflate else "0",
-               GCN10_HOST_INFLATE="1" if host_inflate else "0")
-    root = world["root"]
-    shutil.rmtree(outdir, ignore_errors=True)
-    os.makedirs(outdir)
-    r = subprocess.run([hostlib.EXE_PATH, "-c", str(root / config), "-l", str(root / "blocks.txt"), "--gpus", "1",
-                        "--io-threads", "4", "-o", "--outdir", str(outdir)] + (["--stats"] if stats else []),
-                       cwd=str(root), capture_output=True, text=True, timeout=300, env=env)
-    assert r.returncode == 0, r.stderr
-
-
 def _tags(path):
     from PIL import Image
     with Image.open(path) as im:
@@ -264,10 +249,12 @@ def _tags(path):
 @pytest.mark.parametrize("config", ["config.txt", "config_vrt.txt"], ids=["geotiff", "vrt_mosaic"])
 def test_program_stats(world, reference, config, tmp_path):
     root = world["root"]
-    modes = dict(gpu=(False, False), host_inflate=(False, True), host_deflate=(True, True))
-    for mode, (hd, hi) in modes.items():
-        _program(world, config, tmp_path / mode, True, hd, hi)
-    _program(world, config, tmp_path / "plain", False)
+    modes = dict(gpu=False, host_inflate=True)
+    for mode, hi in modes.items():
+        r = fixtures.run_program(root, config, "-o", "--outdir", str(tmp_path / mode), "--stats", host_inflate=hi)
+        assert r.returncode == 0, r.stderr
+    r = fixtures.run_program(root, config, "-o", "--outdir", str(tmp_path / "plain"))
+    assert r.returncode == 0, r.stderr
     for bid, x0, y0, x1, y1 in world["blocks"]:
         want = reference.run_block(world["esa"], world["esa_t"], world["hsg"], world["hsg_t"], (x0, y0, x1, y1),
                                    str(root / "lookups"), block_id=bid)
@@ -277,7 +264,7 @@ def test_program_stats(world, reference, config, tmp_path):
             assert np.array_equal(img, want["planes"][k]), rel
             assert nodata == "255", rel
             assert S.close(S.parse(meta), S.of_plane(img)), rel
-            for m in modes:                             # the three paths write the same tags
+            for m in modes:                             # both paths write the same tags
                 assert tags[m][1:] == tags["gpu"][1:], (rel, m)
                 assert np.array_equal(tags[m][0], img), (rel, m)
             img, nodata, meta = _tags(str(tmp_path / "plain" / rel))
@@ -287,8 +274,8 @@ def test_program_stats(world, reference, config, tmp_path):
 
 @pytest.fixture(scope="module")
 def tall_world(tmp_path_factory):
-    """A block of 4500 rows: three 2048-row bands on the host-decode and host-deflate paths of the program."""
-    from tests import fixtures, lookups
+    """A block of 4500 rows: three 2048-row bands on the host-decode path of the program."""
+    from tests import lookups
     root = tmp_path_factory.mktemp("gcn10_stats_tall")
     px, hpx = 1.0 / 12000.0, 1.0 / 480.0
     esa_t = (-114.0, px, 0.0, 42.0, 0.0, -px)
@@ -308,12 +295,13 @@ def tall_world(tmp_path_factory):
 
 
 def test_program_stats_multi_band_block(tall_world, reference, tmp_path):
-    """A block taller than two 2048-row bands: the host-decode path hands the GPU's histograms over after its last band,
-    the host-deflate path counts in the writer; every path writes the tags of the decoded planes."""
+    """A block taller than two 2048-row bands: the host-decode path hands the GPU's histograms over after its last band;
+    both paths write the tags of the decoded planes."""
     root = tall_world["root"]
-    modes = dict(gpu=(False, False), host_inflate=(False, True), host_deflate=(True, True))
-    for mode, (hd, hi) in modes.items():
-        _program(tall_world, "config.txt", tmp_path / mode, True, hd, hi)
+    modes = dict(gpu=False, host_inflate=True)
+    for mode, hi in modes.items():
+        r = fixtures.run_program(root, "config.txt", "-o", "--outdir", str(tmp_path / mode), "--stats", host_inflate=hi)
+        assert r.returncode == 0, r.stderr
     bid, x0, y0, x1, y1 = tall_world["blocks"][0]
     want = reference.run_block(tall_world["esa"], tall_world["esa_t"], tall_world["hsg"], tall_world["hsg_t"],
                                (x0, y0, x1, y1), str(root / "lookups"), block_id=bid)

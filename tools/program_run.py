@@ -27,7 +27,6 @@ def main():
     ap.add_argument("--io-threads", type=int, default=0)
     ap.add_argument("--workers-per-gpu", type=int, default=1)
     ap.add_argument("--keep", action="store_true")
-    ap.add_argument("--host-deflate", action="store_true", help="raw planes over PCIe + zlib on the host")
     ap.add_argument("--host-inflate", action="store_true", help="decode the land cover on the host (zlib threads)")
     a = ap.parse_args()
     px = 1.0 / 12000.0
@@ -61,8 +60,7 @@ def main():
     if a.workers_per_gpu > 1:
         cmd += ["--workers-per-gpu", str(a.workers_per_gpu)]
     t0 = time.time()
-    env = dict(os.environ, GCN10_HOST_DEFLATE="1" if a.host_deflate else "0",
-               GCN10_HOST_INFLATE="1" if a.host_inflate else "0")
+    env = dict(os.environ, GCN10_HOST_INFLATE="1" if a.host_inflate else "0")
     r = subprocess.run(cmd, cwd=root, capture_output=True, text=True, env=env)
     dt = time.time() - t0
     print(f"gcn10 rc={r.returncode} wall {dt:.2f} s -> {n * s * s / dt / 1e6:.1f} Mpx/s end to end "
