@@ -47,29 +47,6 @@ class TileStrip(C.Structure):
                 ("framed", C.c_int)]
 
 
-def _tile_collector(tiles, overviews, total, on_strip=None, aggregate=None):
-    """A sink that files every tile of a strip: level 0 into tiles = {plane: {(tile_row, tile_x): bytes}}, overview
-    level k into overviews = {k: {plane: {...}}}, the mean rasters (option "aggregate") into aggregate = {plane: {...}};
-    with ``on_strip(strip_struct)`` the tiles are not copied."""
-
-    def _sink(_user, sp):
-        st = sp.contents
-        total[0] += st.blob_bytes
-        if on_strip is not None:
-            return int(on_strip(st) or 0)
-        blob = C.string_at(st.blob, st.blob_bytes)
-        dest = aggregate if st.aggregate else tiles if st.level == 0 else overviews.setdefault(st.level, {})
-        for k in range(st.n_planes):
-            d = dest.setdefault(st.plane_ids[k], {})
-            for tr in range(st.n_tile_rows):
-                for tx in range(st.tiles_x):
-                    i = (k * st.n_tile_rows + tr) * st.tiles_x + tx
-                    d[(st.tile_row0 + tr, tx)] = blob[st.offsets[i]: st.offsets[i] + st.sizes[i]]
-        return 0
-
-    return _sink
-
-
 TILE_SINK = C.CFUNCTYPE(C.c_int, C.c_void_p, C.POINTER(TileStrip))
 
 
@@ -377,6 +354,31 @@ class Context:
             hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask, ptrs, out.strides[1]))
         return out
 
+    def _deflate_call(self, fn, on_strip, *args):
+        """Runs the compressed-tile library call ``fn(ctx, *args, sink, NULL)`` with a sink that files every tile of a
+        strip (level 0 under tiles, overview level k under overviews[k], the mean rasters under aggregate) unless
+        ``on_strip(strip_struct)`` takes the strips instead; returns block_deflate's result dict."""
+        tiles, overviews, aggregate, total = {}, {}, {}, [0]
+
+        def sink(_user, sp):
+            st = sp.contents
+            total[0] += st.blob_bytes
+            if on_strip is not None:
+                return int(on_strip(st) or 0)
+            blob = C.string_at(st.blob, st.blob_bytes)
+            dest = aggregate if st.aggregate else tiles if st.level == 0 else overviews.setdefault(st.level, {})
+            for k in range(st.n_planes):
+                d = dest.setdefault(st.plane_ids[k], {})
+                for tr in range(st.n_tile_rows):
+                    for tx in range(st.tiles_x):
+                        i = (k * st.n_tile_rows + tr) * st.tiles_x + tx
+                        d[(st.tile_row0 + tr, tx)] = blob[st.offsets[i]: st.offsets[i] + st.sizes[i]]
+            return 0
+
+        cb = TILE_SINK(sink)
+        self._check(fn(self.h, *args, cb, None))
+        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
+
     def block_deflate(self, esa, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
         """Compressed-tile call.  Returns dict(tiles={plane: {(tile_row, tile_x): bytes}},
         overviews={level: {plane: {(tile_row, tile_x): bytes}}} (option "overviews"), bytes=total,
@@ -387,12 +389,8 @@ class Context:
         hsg, hsg_pitch = _rows(hsg)
         h, w = esa.shape
         hsy, hsx = hsg.shape
-        tiles, overviews, aggregate, total = {}, {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
-        self._check(self.lib.gcn10_cuda_block_deflate(
-            self.h, esa.ctypes.data, w, h, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
-            _d6(soil_gt), plane_mask, cb, None))
-        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
+        return self._deflate_call(self.lib.gcn10_cuda_block_deflate, on_strip, esa.ctypes.data, w, h, esa_pitch,
+                                  _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask)
 
     def block_deflate_rows(self, esa_rows, h, row0, gt, hsg, soil_gt, plane_mask=MASK_ALL, on_strip=None):
         """Band form of block_deflate: esa_rows holds rows [row0, row0+len) of a block that is h rows tall; the
@@ -401,12 +399,9 @@ class Context:
         hsg, hsg_pitch = _rows(hsg)
         nrows, w = esa_rows.shape
         hsy, hsx = hsg.shape
-        tiles, overviews, aggregate, total = {}, {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
-        self._check(self.lib.gcn10_cuda_block_deflate_rows(
-            self.h, esa_rows.ctypes.data, w, h, row0, nrows, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch,
-            _d6(soil_gt), plane_mask, cb, None))
-        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
+        return self._deflate_call(self.lib.gcn10_cuda_block_deflate_rows, on_strip, esa_rows.ctypes.data, w, h, row0,
+                                  nrows, esa_pitch, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt),
+                                  plane_mask)
 
     def inflate_tiles(self, src: "TileSource", w, h, out=None, want_status=False):
         """GPU inflate of a tile source into a host raster uint8 [h, w]."""
@@ -426,13 +421,9 @@ class Context:
         block_deflate)."""
         hsg, hsg_pitch = _rows(hsg)
         hsy, hsx = hsg.shape
-        tiles, overviews, aggregate, total = {}, {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
         st = src.struct()
-        self._check(self.lib.gcn10_cuda_block_tiles_deflate(
-            self.h, C.byref(st), w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
-            cb, None))
-        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
+        return self._deflate_call(self.lib.gcn10_cuda_block_tiles_deflate, on_strip, C.byref(st), w, h, _d6(gt),
+                                  hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask)
 
     def inflate_parts(self, parts, fill, w, h, want_status=False):
         """GPU inflate of a mosaic ([(TileSource, dst_x, dst_y, w, h), ...]) into a host raster uint8 [h, w]."""
@@ -451,13 +442,8 @@ class Context:
         """Mosaic form of block_tiles_deflate; same result layout."""
         hsg, hsg_pitch = _rows(hsg)
         hsy, hsx = hsg.shape
-        tiles, overviews, aggregate, total = {}, {}, {}, [0]
-        cb = TILE_SINK(_tile_collector(tiles, overviews, total, on_strip, aggregate))
-        arr = parts_array(parts)
-        self._check(self.lib.gcn10_cuda_block_parts_deflate(
-            self.h, arr, len(parts), fill, w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask,
-            cb, None))
-        return dict(tiles=tiles, overviews=overviews, aggregate=aggregate, bytes=total[0], histograms=self._histograms())
+        return self._deflate_call(self.lib.gcn10_cuda_block_parts_deflate, on_strip, parts_array(parts), len(parts), fill,
+                                  w, h, _d6(gt), hsg.ctypes.data, hsx, hsy, hsg_pitch, _d6(soil_gt), plane_mask)
 
     def tiles_prefetch(self, src: "TileSource", w, h):
         """Start upload + GPU inflate of a block's tiles; the next block_tiles_deflate / inflate_tiles call with the

@@ -7,82 +7,40 @@ import os
 import numpy as np
 import pytest
 
-from gcn10_b200 import capi, synth
+from gcn10_b200 import capi
 from tests import aggregate_rule as A
 from tests import fixtures
 from tests import overview_rule as R
+from tests.block_options import (CALLS, FULL_SIZE, T, assemble, config_for, ctx, full_size_block,  # noqa: F401
+                                 full_size_parts, options, run_call, world)
 from tests.cases import SMALL_CASES, make_block
-from tests.test_gpu_overviews import T, _assemble, _parts, world  # noqa: F401  (world: the program's input fixture)
 
 pytestmark = pytest.mark.gpu
 
-MASKS = [capi.MASK_ALL, capi.MASK_DRAINED, 1 << 13]
-# (mask, fused, ordered, ship): all 24 combinations, dealt out over the cases x calls below
-CONFIGS = [(m, f, o, s) for m in MASKS for f in (1, 0) for o in (0, 1) for s in (0, 1)]
-CALLS = ["deflate", "rows", "tiles", "parts"]
 FACTORS = [25, 2, 7, 100, 256, 1024]
-
-
-@pytest.fixture(scope="module")
-def ctx(tables):
-    with capi.Context(0) as c:
-        c.set_luts(tables)
-        yield c
-
-
-def _set(ctx, aggregate=0, overviews=0, stats=0, fused=1, ordered=0, ship=0, strip_rows=2048):
-    for k, v in dict(aggregate=aggregate, overviews=overviews, stats=stats, fused=fused, ordered=ordered, ship=ship,
-                     strip_rows=strip_rows).items():
-        ctx.set_option(k, v)
-
-
-def _run(ctx, call, b, mask=capi.MASK_ALL, band=768):
-    esa = b["esa"]
-    h, w = esa.shape
-    if call == "deflate":
-        return ctx.block_deflate(esa, b["gt"], b["hsg"], b["soil_gt"], mask)
-    if call == "rows":
-        res = dict(tiles={}, overviews={}, aggregate={}, histograms=None)
-        for y0 in range(0, h, band):
-            r = ctx.block_deflate_rows(esa[y0:y0 + band], h, y0, b["gt"], b["hsg"], b["soil_gt"], mask)
-            for k, d in r["tiles"].items():
-                res["tiles"].setdefault(k, {}).update(d)
-            assert not r["aggregate"] or y0 + band >= h, "mean rasters before the band that ends the block"
-            res["overviews"].update(r["overviews"])
-            res["aggregate"].update(r["aggregate"])
-            res["histograms"] = r["histograms"]
-        return res
-    if call == "tiles":
-        src = capi.TileSource.from_raster(esa, 256, 256)
-        return ctx.block_tiles_deflate(src, w, h, b["gt"], b["hsg"], b["soil_gt"], mask)
-    return ctx.block_parts_deflate(_parts(esa), 0, w, h, b["gt"], b["hsg"], b["soil_gt"], mask)
 
 
 def _check_means(res, want, mask, f, w, h):
     planes = [p for p in range(18) if mask >> p & 1]
     assert sorted(res["aggregate"]) == planes
     for p in planes:
-        got = _assemble(res["aggregate"][p], A.dim(w, f), A.dim(h, f))
+        got = assemble(res["aggregate"][p], A.dim(w, f), A.dim(h, f))
         assert np.array_equal(got, A.mean(want[p], f)), f"plane {p} f={f}"
 
 
 @pytest.mark.parametrize("call", CALLS)
 @pytest.mark.parametrize("name,kw", SMALL_CASES, ids=[c[0] for c in SMALL_CASES])
 def test_means_equal_oracle(name, kw, call, ctx, port, tables):
-    i = [c[0] for c in SMALL_CASES].index(name) * len(CALLS) + CALLS.index(call)
-    mask, fused, ordered, ship = CONFIGS[i % len(CONFIGS)]
-    f = FACTORS[i % len(FACTORS)]
+    mask, fused, ordered, ship = config_for(name, call)
+    f = config_for(name, call, FACTORS)
     b = make_block(**kw)
     h, w = b["esa"].shape
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
-    _set(ctx, 0, fused=fused, ordered=ordered, ship=ship)
-    base = _run(ctx, call, b, mask)
+    with options(ctx, fused=fused, ordered=ordered, ship=ship):
+        base = run_call(ctx, call, b, mask)
     assert base["aggregate"] == {}
-    _set(ctx, f, fused=fused, ordered=ordered, ship=ship)
-    try:
-        res = _run(ctx, call, b, mask)
-    finally:
-        _set(ctx)
+    with options(ctx, aggregate=f, fused=fused, ordered=ordered, ship=ship):
+        res = run_call(ctx, call, b, mask)
     assert res["tiles"] == base["tiles"]            # the same bytes as without the option
     _check_means(res, want, mask, f, w, h)
 
@@ -91,13 +49,10 @@ def test_strip_fields_and_order(ctx):
     b = make_block(w=3001, h=2600, seed=21)
     h, w = b["esa"].shape
     seen = []
-    _set(ctx, 2, overviews=16, strip_rows=512)
-    try:
+    with options(ctx, aggregate=2, overviews=16, strip_rows=512):
         ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], capi.MASK_DRAINED,
                           on_strip=lambda st: seen.append((st.aggregate, st.level, st.tile_row0, st.n_tile_rows,
                                                            st.tiles_x, st.level_w, st.level_h)))
-    finally:
-        _set(ctx)
     expect = []
     for k in range(R.levels(w, h) + 1):             # full resolution, then the overview levels
         lw, lh = R.dim(w, k), R.dim(h, k)
@@ -115,19 +70,13 @@ def test_factors_and_strip_sizes(f, ctx, port, tables):
     b = make_block(w=1777, h=1290, seed=31 + f)
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
     for fused in (1, 0):
-        _set(ctx, f, fused=fused, strip_rows=256)
-        try:
+        with options(ctx, aggregate=f, fused=fused, strip_rows=256):
             res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])
-        finally:
-            _set(ctx)
         _check_means(res, want, capi.MASK_ALL, f, 1777, 1290)
     b = make_block(w=300, h=200, seed=5)
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
-    _set(ctx, 1024)
-    try:
+    with options(ctx, aggregate=1024):
         res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])       # one cell holds the whole block
-    finally:
-        _set(ctx)
     _check_means(res, want, capi.MASK_ALL, 1024, 300, 200)
 
 
@@ -149,22 +98,19 @@ def test_launch_counts(ctx, tables):
         base = fresh.launch_count() - n0
 
     def count(agg, fused):
-        _set(ctx, agg, fused=fused, strip_rows=512)
-        n0 = ctx.launch_count()
-        ctx.block_deflate(*args)
-        return ctx.launch_count() - n0
+        with options(ctx, aggregate=agg, fused=fused, strip_rows=512):
+            n0 = ctx.launch_count()
+            ctx.block_deflate(*args)
+            return ctx.launch_count() - n0
 
-    try:
-        _set(ctx, 25)
-        _set(ctx, 0)                                    # set, then back off: exactly the launches of a fresh context
+    with options(ctx, aggregate=25):
+        ctx.set_option("aggregate", 0)                  # set, then back off: exactly the launches of a fresh context
         n0 = ctx.launch_count()
         ctx.block_deflate(*args)
         assert ctx.launch_count() - n0 == base
-        # three accumulate kernels (1100 rows in 512-row strips), the finish kernel, one encoder for the 52 x 44 mean
-        for fused in (1, 0):
-            assert count(25, fused) == count(0, fused) + 3 + 1 + 1
-    finally:
-        _set(ctx)
+    # three accumulate kernels (1100 rows in 512-row strips), the finish kernel, one encoder for the 52 x 44 mean
+    for fused in (1, 0):
+        assert count(25, fused) == count(0, fused) + 3 + 1 + 1
 
 
 def test_with_overviews_and_stats(ctx, port, tables):
@@ -172,13 +118,10 @@ def test_with_overviews_and_stats(ctx, port, tables):
     b = make_block(w=2100, h=1900, seed=41)
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
     for fused in (1, 0):
-        _set(ctx, 0, 16, 1, fused)
-        try:
+        with options(ctx, overviews=16, stats=1, fused=fused):
             base = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])
-            _set(ctx, 25, 16, 1, fused)
+        with options(ctx, aggregate=25, overviews=16, stats=1, fused=fused):
             res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])
-        finally:
-            _set(ctx)
         assert res["tiles"] == base["tiles"] and res["overviews"] == base["overviews"]
         assert np.array_equal(res["histograms"], base["histograms"])
         assert all(int(res["histograms"][p].sum()) == 2100 * 1900 for p in range(18))
@@ -189,8 +132,7 @@ def test_bands_order_restart_and_mask(ctx, port, tables):
     b = make_block(w=700, h=1100, seed=23)
     esa, h = b["esa"], 1100
     want = port.block_rows(esa, b["gt"], b["hsg"], b["soil_gt"], tables)
-    _set(ctx, 25)
-    try:
+    with options(ctx, aggregate=25):
         with pytest.raises(capi.Gcn10Error) as e:       # no block open
             ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])
         assert e.value.code == -1
@@ -210,8 +152,6 @@ def test_bands_order_restart_and_mask(ctx, port, tables):
         # the whole block again in one call: the same means, not sums of two blocks
         r3 = ctx.block_deflate(esa, b["gt"], b["hsg"], b["soil_gt"])
         assert r3["aggregate"] == r2["aggregate"]
-    finally:
-        _set(ctx)
     ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])     # free again without the option
 
 
@@ -219,28 +159,24 @@ def test_prefetch_and_ship_paths(ctx, port, tables):
     blocks = [make_block(w=2100, h=1900, seed=24 + i) for i in range(3)]
     srcs = [capi.TileSource.from_raster(b["esa"], 256, 256) for b in blocks]
     for ordered, ship in ((0, 0), (1, 1)):
-        _set(ctx, 25, ordered=ordered, ship=ship)
-        try:
+        with options(ctx, aggregate=25, ordered=ordered, ship=ship):
             ctx.tiles_prefetch(srcs[0], 2100, 1900)
             results = []
             for i, b in enumerate(blocks):
                 if i + 1 < len(blocks):
                     ctx.tiles_prefetch(srcs[i + 1], 2100, 1900)
                 results.append(ctx.block_tiles_deflate(srcs[i], 2100, 1900, b["gt"], b["hsg"], b["soil_gt"]))
-        finally:
-            _set(ctx)
         for b, res in zip(blocks, results):
             want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
             for p in (0, 17):
-                assert np.array_equal(_assemble(res["tiles"][p], 2100, 1900), want[p])
+                assert np.array_equal(assemble(res["tiles"][p], 2100, 1900), want[p])
             _check_means(res, want, capi.MASK_ALL, 25, 2100, 1900)
 
 
 def test_sink_failure_and_damaged_tile(ctx, port, tables):
     b = make_block(w=1500, h=1300, seed=30)
     h, w = b["esa"].shape
-    _set(ctx, 7, strip_rows=256)
-    try:
+    with options(ctx, aggregate=7, strip_rows=256):
         seen = []
 
         def fail_in_mean(st):
@@ -261,8 +197,6 @@ def test_sink_failure_and_damaged_tile(ctx, port, tables):
         assert e.value.code == -6 and seen == []
         # the context is usable afterwards: the aborted blocks left nothing in the accumulators
         res = ctx.block_tiles_deflate(src, w, h, b["gt"], b["hsg"], b["soil_gt"])
-    finally:
-        _set(ctx)
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
     _check_means(res, want, capi.MASK_ALL, 7, w, h)
 
@@ -279,11 +213,10 @@ def test_random_tables_two_kernel_path(fused, ctx, port, tables):
     try:
         ctx.set_luts(t)
         for mask in (capi.MASK_ALL, capi.MASK_UNDRAINED, 0x3 | 1 << 10):
-            _set(ctx, 25, fused=fused, strip_rows=256)
-            res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
+            with options(ctx, aggregate=25, fused=fused, strip_rows=256):
+                res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
             _check_means(res, want, mask, 25, 1040, 700)
     finally:
-        _set(ctx)
         ctx.set_luts(tables)
 
 
@@ -307,32 +240,21 @@ def _oracle_means(port, tables, esa, gt, hsg, sgt, n, f):
     return A.value(s.cpu().numpy().astype(np.uint64), cnt.cpu().numpy().astype(np.uint64))
 
 
-@pytest.mark.parametrize("shape", ["worldcover_36000", "vrt_36001_four_parts"])
+@pytest.mark.parametrize("shape", FULL_SIZE)
 def test_full_size_block(shape, ctx, port, tables):
-    if shape == "worldcover_36000":
-        n, px, lon0, lat0 = 36000, 1.0 / 12000.0, -114.0, 42.0
-    else:
-        n, px, lon0, lat0 = 36001, 8.3333333333330430e-05, 33.0, -3.0
-    gt, sgt, hsx, hsy = synth.block_geometry(lon0, lat0, n, n, px, 1.0 / 480.0, (0.0011, 0.0004), 2)
-    esa = synth.esa_tile(n, n, 77, patch=64)
+    n, gt, sgt, esa, hsg = full_size_block(shape)
     esa[::41, ::13] = 0                                 # land cover without a Curve Number: nodata pixels in every cell
-    hsg = synth.hsg_tile(hsx, hsy, 78, patch=3)
-    _set(ctx, 25)
-    try:
-        if shape == "worldcover_36000":
-            res = ctx.block_tiles_deflate(capi.TileSource.from_raster(esa, 1024, 1024), n, n, gt, hsg, sgt)
-        else:                                           # the real VRT's four files around a block corner
-            c = 35000
-            parts = [(capi.TileSource.from_raster(np.ascontiguousarray(esa[y:y + hh, x:x + ww]), 1024, 1024), x, y,
-                      ww, hh) for (y, hh) in ((0, c), (c, n - c)) for (x, ww) in ((0, c), (c, n - c))]
+    parts = full_size_parts(shape, esa)
+    with options(ctx, aggregate=25):
+        if len(parts) == 1:
+            res = ctx.block_tiles_deflate(parts[0][0], n, n, gt, hsg, sgt)
+        else:
             res = ctx.block_parts_deflate(parts, 0, n, n, gt, hsg, sgt)
-    finally:
-        _set(ctx)
     cw = A.dim(n, 25)
     assert cw == (1440 if n == 36000 else 1441)
     want = _oracle_means(port, tables, esa, gt, hsg, sgt, n, 25)
     for p in range(18):
-        assert np.array_equal(_assemble(res["aggregate"][p], cw, cw), want[p]), p
+        assert np.array_equal(assemble(res["aggregate"][p], cw, cw), want[p]), p
 
 
 # ---- the program, file to file ---------------------------------------------------------------------------------

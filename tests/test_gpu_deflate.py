@@ -9,11 +9,11 @@ import pytest
 
 from gcn10_b200 import capi
 from tests import stream_ref as S
+from tests.block_options import assemble
 from tests.cases import make_block
 
 pytestmark = pytest.mark.gpu
 
-T = 256
 _PATH = [None]          # the encoder path of the running test (fixture encoder_path)
 
 
@@ -36,21 +36,6 @@ def _reference(want, tables, mask=capi.MASK_ALL):
     p = _PATH[0]
     reg = S.regime(tables, mask, fused=int(p != "two_kernel"), tuned_code=int(p == "fused_tuned_code"))
     return S.expected_tiles({k: want[k] for k in reg.planes}, reg)
-
-
-def _assemble(tiles, w, h, exact=None):
-    """The plane the tiles decode to; with ``exact`` (the reference's tiles of the plane) every stream must equal the
-    reference's, byte for byte."""
-    tx_n, ty_n = (w + T - 1) // T, (h + T - 1) // T
-    full = np.zeros((ty_n * T, tx_n * T), dtype=np.uint8)
-    assert sorted(tiles) == [(r, c) for r in range(ty_n) for c in range(tx_n)], "tile grid incomplete"
-    for (r, c), z in tiles.items():
-        if exact is not None:
-            assert z == exact[(r, c)], f"{_PATH[0]}: tile {(r, c)}: {len(z)} bytes, reference {len(exact[(r, c)])}"
-        raw = zlib.decompress(z)
-        assert len(raw) == T * T
-        full[r * T:(r + 1) * T, c * T:(c + 1) * T] = np.frombuffer(raw, dtype=np.uint8).reshape(T, T)
-    return full
 
 
 CASES = [
@@ -81,9 +66,7 @@ def test_deflate_tiles_decode_to_oracle_planes(name, kw, gpu_ctx, port, tables):
     assert sorted(res["tiles"]) == list(range(18))
     ref = _reference(want, tables)
     for k in range(18):
-        full = _assemble(res["tiles"][k], w, h, ref[k])
-        assert np.array_equal(full[:h, :w], want[k]), f"{name}: plane {k}"
-        assert not full[h:, :].any() and not full[:, w:].any(), "edge padding must be zero"
+        assert np.array_equal(assemble(res["tiles"][k], w, h, ref[k]), want[k]), f"{name}: plane {k}"
 
 
 def test_deflate_stored_fallback_and_masks(gpu_ctx, port, tables):
@@ -106,7 +89,7 @@ def test_deflate_stored_fallback_and_masks(gpu_ctx, port, tables):
     assert max(sizes) == 2 + 10 + 65536 + 4, "expected at least one stored tile"
     ref = _reference(want, t, mask)
     for k in range(9):
-        assert np.array_equal(_assemble(res["tiles"][k], 520, 300, ref[k])[:300, :520], want[k])
+        assert np.array_equal(assemble(res["tiles"][k], 520, 300, ref[k]), want[k])
 
 
 @pytest.mark.parametrize("holes", [1, 2, 5], ids=["2_literal_classes", "3_literal_classes", "too_many_classes"])
@@ -131,7 +114,7 @@ def test_tables_with_missing_rows_per_variant(holes, gpu_ctx, port, tables):
         gpu_ctx.set_luts(tables)
     ref = _reference(want, t)
     for k in range(18):
-        assert np.array_equal(_assemble(res["tiles"][k], 700, 540, ref[k])[:540, :700], want[k]), f"plane {k}"
+        assert np.array_equal(assemble(res["tiles"][k], 700, 540, ref[k]), want[k]), f"plane {k}"
 
 
 @pytest.mark.parametrize("mask", [1 << 7, (1 << 0) | (1 << 4) | (1 << 9) | (1 << 17), 0x3FFFF & ~(1 << 8), 0x2AAAA])
@@ -145,7 +128,7 @@ def test_arbitrary_plane_masks(mask, gpu_ctx, port, tables):
     assert sorted(res["tiles"]) == sel
     ref = _reference(want, tables, mask)
     for k in sel:
-        assert np.array_equal(_assemble(res["tiles"][k], 777, 515, ref[k])[:515, :777], want[k]), f"plane {k}"
+        assert np.array_equal(assemble(res["tiles"][k], 777, 515, ref[k]), want[k]), f"plane {k}"
 
 
 def test_deflate_compresses_cn_rasters(gpu_ctx):
@@ -207,8 +190,7 @@ def test_deflate_rows_bands_equal_whole_block(gpu_ctx, port, tables):
     ref = _reference(want, tables, capi.MASK_UNDRAINED)
     for k in range(9, 18):
         tiles = {(r, c): z for (p, r, c), z in got.items() if p == k}
-        full = _assemble(tiles, w, h, ref[k])
-        assert np.array_equal(full[:h, :w], want[k]), k
+        assert np.array_equal(assemble(tiles, w, h, ref[k]), want[k]), k
 
 
 @pytest.mark.parametrize("break_row", [None, 129, 2, 255, 130, 3])
@@ -227,7 +209,7 @@ def test_long_row_runs(break_row, gpu_ctx, port, tables, encoder_path):
     res = gpu_ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])
     ref = _reference(want, tables)
     for k in range(18):
-        assert np.array_equal(_assemble(res["tiles"][k], w, h, ref[k])[:h, :w], want[k]), f"plane {k}"
+        assert np.array_equal(assemble(res["tiles"][k], w, h, ref[k]), want[k]), f"plane {k}"
     # a tile of 256 repeated rows: 254 tokens of 10 bits (tuned code), 19 bits (fixed code), or one 24-bit token per
     # row (two-kernel path), plus a few tokens where the raster changes
     per_tile = {"fused_tuned_code": 450, "fused_fixed_code": 750, "two_kernel": 900}[encoder_path]
@@ -264,8 +246,7 @@ def test_strip_hand_over_paths_agree(gpu_ctx, port, tables, encoder_path):
     ref = _reference(want, tables)
     for k in range(18):
         assert got[0]["tiles"][k] == got[1]["tiles"][k] == again["tiles"][k]
-        full = _assemble(got[1]["tiles"][k], w, h, ref[k])
-        assert np.array_equal(full[:h, :w], want[k])
+        assert np.array_equal(assemble(got[1]["tiles"][k], w, h, ref[k]), want[k])
 
 
 def test_ordered_strips(gpu_ctx, port, tables, encoder_path):
@@ -299,5 +280,4 @@ def test_ordered_strips(gpu_ctx, port, tables, encoder_path):
     ref = _reference(want, tables)
     for k in range(18):
         assert res["tiles"][k] == plain["tiles"][k]
-        full = _assemble(res["tiles"][k], w, h, ref[k])
-        assert np.array_equal(full[:h, :w], want[k])
+        assert np.array_equal(assemble(res["tiles"][k], w, h, ref[k]), want[k])

@@ -13,7 +13,6 @@ DESIGN.md section 4.5: the same parse, tie-break, code, stored fallbacks and enc
 """
 import os
 import time
-import zlib
 from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
@@ -22,6 +21,7 @@ import pytest
 from gcn10_b200 import capi
 from tests import aggregate_rule, overview_rule
 from tests import stream_ref as S
+from tests.block_options import assemble
 from tests.cases import make_block
 from tests.encoder_cases import (SHAPES, noisy_tile, random_block, tables_with_classes, tables_with_records,
                                   tables_with_values)
@@ -30,14 +30,6 @@ pytestmark = pytest.mark.gpu
 
 T = 256
 ONE, NINE, ALL = 1 << 7, capi.MASK_DRAINED, capi.MASK_ALL
-
-
-def _decode_check(tiles, want, w, h):
-    for k, d in tiles.items():
-        full = np.zeros(((h + T - 1) // T * T, (w + T - 1) // T * T), np.uint8)
-        for (r, c), z in d.items():
-            full[r * T:(r + 1) * T, c * T:(c + 1) * T] = np.frombuffer(zlib.decompress(z), np.uint8).reshape(T, T)
-        assert np.array_equal(full[:h, :w], want[k]), k
 
 
 def _launches(ctx, fn):
@@ -117,7 +109,8 @@ def test_code_regimes(name, kind, n, mask, call, gpu_ctx, port, tables):
         assert n_fused == n_plain, (n_fused, n_plain)
     _regime_table.append((f"{name} {reg.shape or reg.path}", len(sel), call, f"{reg.path} ({n_fused} / {n_plain})"))
     planes = {k: want[k] for k in sel}
-    _decode_check(res["tiles"], planes, w, h)
+    for k, tiles in res["tiles"].items():
+        assert np.array_equal(assemble(tiles, w, h), planes[k]), k
     S.check_tiles(res["tiles"], planes, reg, name)
     S.check_tiles(res0["tiles"], planes, S.regime(t, mask, fused=0), name + " fused=0")
 
@@ -241,7 +234,8 @@ def test_kernel_modes(gpu_ctx, port, tables):
         finally:
             gpu_ctx.set_option("tuned_code", 1)
             gpu_ctx.set_luts(tables)
-        _decode_check(res["tiles"], planes, b["esa"].shape[1], T)
+        for k, tiles in res["tiles"].items():
+            assert np.array_equal(assemble(tiles, b["esa"].shape[1], T), planes[k]), k
         S.check_tiles(res["tiles"], planes, reg, name)
     count = mode_counts(blocks)
     print("\nmode coverage:", count)

@@ -3,7 +3,6 @@ import numpy as np
 import pytest
 
 from tests import golden_io
-from tests.test_oracle_pinned import _window_inputs
 
 pytestmark = pytest.mark.gpu
 
@@ -13,7 +12,7 @@ BLOCKS = golden_io.block_cases()
 @pytest.mark.parametrize("name", sorted(BLOCKS))
 def test_gpu_matches_golden_blocks(name, gpu_ctx, port):
     c = BLOCKS[name]
-    esa, gt, hsg, sgt = _window_inputs(port, c)
+    esa, gt, hsg, sgt = golden_io.window_inputs(port, c)
     got = gpu_ctx.block(np.ascontiguousarray(esa), gt, np.ascontiguousarray(hsg), sgt)
     assert np.array_equal(got, c["planes"])
 

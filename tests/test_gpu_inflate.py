@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 
 from gcn10_b200 import capi, synth
+from tests.block_options import assemble
 from tests.cases import make_block
 
 pytestmark = pytest.mark.gpu
@@ -194,14 +195,6 @@ def test_bad_arguments(gpu_ctx):
     assert rc == -1
 
 
-def _assemble(tiles, w, h, T=256):
-    tx_n, ty_n = (w + T - 1) // T, (h + T - 1) // T
-    full = np.zeros((ty_n * T, tx_n * T), dtype=np.uint8)
-    for (r, c), z in tiles.items():
-        full[r * T:(r + 1) * T, c * T:(c + 1) * T] = np.frombuffer(zlib.decompress(z), dtype=np.uint8).reshape(T, T)
-    return full[:h, :w]
-
-
 @pytest.mark.parametrize("kw,tile,off", [
     (dict(w=1300, h=777, seed=4), 256, (0, 0)),
     (dict(w=2300, h=2600, seed=6), 1024, (100, 900)),
@@ -218,7 +211,7 @@ def test_compressed_in_compressed_out_matches_oracle(kw, tile, off, gpu_ctx, por
     res = gpu_ctx.block_tiles_deflate(src, w, h, b["gt"], b["hsg"], b["soil_gt"])
     assert sorted(res["tiles"]) == list(range(18))
     for k in range(18):
-        assert np.array_equal(_assemble(res["tiles"][k], w, h), want[k]), f"plane {k}"
+        assert np.array_equal(assemble(res["tiles"][k], w, h), want[k]), f"plane {k}"
     # identical to the raw-raster entry point, tile for tile
     ref = gpu_ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])
     assert ref["tiles"] == res["tiles"]
@@ -246,7 +239,7 @@ def test_prefetch_overlaps_the_next_block_and_results_do_not_change(gpu_ctx, por
 
     def check(res, want):
         for k in range(18):
-            assert np.array_equal(_assemble(res["tiles"][k], 900, 700), want[k])
+            assert np.array_equal(assemble(res["tiles"][k], 900, 700), want[k])
 
     gpu_ctx.tiles_prefetch(srcs[0], 900, 700)
     for i in range(4):
@@ -291,8 +284,7 @@ def test_mosaic_parts(gpu_ctx, port, tables):
     want = port.block_rows(esa, b["gt"], b["hsg"], b["soil_gt"], tables)
     res = gpu_ctx.block_parts_deflate(parts, 0, w, h, b["gt"], b["hsg"], b["soil_gt"])
     for k in range(18):
-        full = _assemble(res["tiles"][k], w, h)
-        assert np.array_equal(full[:h, :w], want[k]), k
+        assert np.array_equal(assemble(res["tiles"][k], w, h), want[k]), k
     # a missing source: its rectangle reads as the fill value (VRT NoDataValue)
     holed = esa.copy()
     x, y, pw, ph = rects[2]

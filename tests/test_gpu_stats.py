@@ -9,28 +9,11 @@ from gcn10_b200 import capi, hostlib, synth
 from tests import fixtures
 from tests import overview_rule as R
 from tests import stats_rule as S
+from tests.block_options import (CALLS, FULL_SIZE, config_for, ctx, full_size_block, full_size_parts,  # noqa: F401
+                                 options, run_call, world)
 from tests.cases import SMALL_CASES, make_block
-from tests.test_gpu_overviews import _parts, world  # noqa: F401  (world: the program's input fixture)
 
 pytestmark = pytest.mark.gpu
-
-MASKS = [capi.MASK_ALL, capi.MASK_DRAINED, 1 << 13]
-# (mask, fused, ordered, ship): all 24 combinations, dealt out over the cases x calls below
-CONFIGS = [(m, f, o, s) for m in MASKS for f in (1, 0) for o in (0, 1) for s in (0, 1)]
-CALLS = ["deflate", "rows", "tiles", "parts"]
-
-
-@pytest.fixture(scope="module")
-def ctx(tables):
-    with capi.Context(0) as c:
-        c.set_luts(tables)
-        yield c
-
-
-def _set(ctx, stats=0, overviews=0, fused=1, ordered=0, ship=0, strip_rows=2048):
-    for k, v in dict(stats=stats, overviews=overviews, fused=fused, ordered=ordered, ship=ship,
-                     strip_rows=strip_rows).items():
-        ctx.set_option(k, v)
 
 
 def _want(planes, mask):
@@ -42,42 +25,18 @@ def _want(planes, mask):
     return out
 
 
-def _run(ctx, call, b, mask, band=768):
-    esa = b["esa"]
-    h, w = esa.shape
-    if call == "deflate":
-        return ctx.block_deflate(esa, b["gt"], b["hsg"], b["soil_gt"], mask)
-    if call == "rows":
-        res = dict(tiles={}, histograms=None)
-        for y0 in range(0, h, band):
-            r = ctx.block_deflate_rows(esa[y0:y0 + band], h, y0, b["gt"], b["hsg"], b["soil_gt"], mask)
-            for k, d in r["tiles"].items():
-                res["tiles"].setdefault(k, {}).update(d)
-            assert r["histograms"] is None or y0 + band >= h, "histograms before the band that ends the block"
-            res["histograms"] = r["histograms"]
-        return res
-    if call == "tiles":
-        src = capi.TileSource.from_raster(esa, 256, 256)
-        return ctx.block_tiles_deflate(src, w, h, b["gt"], b["hsg"], b["soil_gt"], mask)
-    return ctx.block_parts_deflate(_parts(esa), 0, w, h, b["gt"], b["hsg"], b["soil_gt"], mask)
-
-
 @pytest.mark.parametrize("call", CALLS)
 @pytest.mark.parametrize("name,kw", SMALL_CASES, ids=[c[0] for c in SMALL_CASES])
 def test_histograms_equal_oracle(name, kw, call, ctx, port, tables):
-    i = [c[0] for c in SMALL_CASES].index(name) * len(CALLS) + CALLS.index(call)
-    mask, fused, ordered, ship = CONFIGS[i % len(CONFIGS)]
+    mask, fused, ordered, ship = config_for(name, call)
     b = make_block(**kw)
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
-    _set(ctx, 0, 0, fused, ordered, ship)
-    base = _run(ctx, call, b, mask)
+    with options(ctx, fused=fused, ordered=ordered, ship=ship):
+        base = run_call(ctx, call, b, mask)
     assert base["histograms"] is None
-    _set(ctx, 1, 0, fused, ordered, ship)
-    try:
-        res = _run(ctx, call, b, mask)
+    with options(ctx, stats=1, fused=fused, ordered=ordered, ship=ship):
+        res = run_call(ctx, call, b, mask)
         assert np.array_equal(ctx.last_histograms(), res["histograms"])
-    finally:
-        _set(ctx)
     assert res["tiles"] == base["tiles"]            # the same bytes as without the option
     assert np.array_equal(res["histograms"], _want(want, mask))
 
@@ -93,18 +52,18 @@ def test_random_tables_two_kernel_path(fused, ctx, port, tables):
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], t)
     try:
         ctx.set_luts(t)
-        for mask in (capi.MASK_ALL, capi.MASK_UNDRAINED):
-            _set(ctx, 1, fused=fused, strip_rows=256)
-            n0 = ctx.launch_count()
-            res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
-            n_on = ctx.launch_count() - n0
-            _set(ctx, 0, fused=fused, strip_rows=256)
-            n0 = ctx.launch_count()
-            ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
-            assert n_on - (ctx.launch_count() - n0) == 3        # one histogram kernel per strip (3 of 256 rows)
-            assert np.array_equal(res["histograms"], _want(want, mask)), mask
+        with options(ctx, fused=fused, strip_rows=256):
+            for mask in (capi.MASK_ALL, capi.MASK_UNDRAINED):
+                ctx.set_option("stats", 1)
+                n0 = ctx.launch_count()
+                res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
+                n_on = ctx.launch_count() - n0
+                ctx.set_option("stats", 0)
+                n0 = ctx.launch_count()
+                ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"], mask)
+                assert n_on - (ctx.launch_count() - n0) == 3        # one histogram kernel per strip (3 of 256 rows)
+                assert np.array_equal(res["histograms"], _want(want, mask)), mask
     finally:
-        _set(ctx)
         ctx.set_luts(tables)
 
 
@@ -112,11 +71,8 @@ def test_with_overviews_level_zero_only(ctx, port, tables):
     b = make_block(w=2100, h=1900, seed=41)
     want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
     for fused in (1, 0):
-        _set(ctx, 1, 16, fused)
-        try:
+        with options(ctx, stats=1, overviews=16, fused=fused):
             res = ctx.block_deflate(b["esa"], b["gt"], b["hsg"], b["soil_gt"])
-        finally:
-            _set(ctx)
         assert sorted(res["overviews"]) == list(range(1, R.levels(2100, 1900) + 1))
         assert np.array_equal(res["histograms"], _want(want, capi.MASK_ALL)), fused
         assert all(int(res["histograms"][p].sum()) == 2100 * 1900 for p in range(18))
@@ -126,8 +82,7 @@ def test_bands_order_and_restart(ctx, port, tables):
     b = make_block(w=700, h=1100, seed=23)
     esa, h = b["esa"], 1100
     want = port.block_rows(esa, b["gt"], b["hsg"], b["soil_gt"], tables)
-    _set(ctx, 1)
-    try:
+    with options(ctx, stats=1):
         with pytest.raises(capi.Gcn10Error) as e:       # no block open
             ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])
         assert e.value.code == -1
@@ -148,8 +103,6 @@ def test_bands_order_and_restart(ctx, port, tables):
         # the whole block again in one call: the same counts, not twice them
         r3 = ctx.block_deflate(esa, b["gt"], b["hsg"], b["soil_gt"])
         assert np.array_equal(r3["histograms"], r2["histograms"])
-    finally:
-        _set(ctx)
     ctx.block_deflate_rows(esa[512:], h, 512, b["gt"], b["hsg"], b["soil_gt"])     # free again without the option
 
 
@@ -163,37 +116,31 @@ def test_launch_counts(ctx, tables):
         base = fresh.launch_count() - n0
 
     def count(stats, fused):
-        _set(ctx, stats, fused=fused, strip_rows=512)
-        n0 = ctx.launch_count()
-        ctx.block_deflate(*args)
-        return ctx.launch_count() - n0
+        with options(ctx, stats=stats, fused=fused, strip_rows=512):
+            n0 = ctx.launch_count()
+            ctx.block_deflate(*args)
+            return ctx.launch_count() - n0
 
-    try:
-        _set(ctx, 1)
-        _set(ctx, 0)                                    # set, then back off: exactly the launches of a fresh context
+    with options(ctx, stats=1):
+        ctx.set_option("stats", 0)                      # set, then back off: exactly the launches of a fresh context
         n0 = ctx.launch_count()
         ctx.block_deflate(*args)
         assert ctx.launch_count() - n0 == base
-        assert count(1, 1) == count(0, 1)               # fused: no launch of its own
-        assert count(1, 0) == count(0, 0) + 3           # two-kernel path: one per strip (1100 rows in 512-row strips)
-    finally:
-        _set(ctx)
+    assert count(1, 1) == count(0, 1)                   # fused: no launch of its own
+    assert count(1, 0) == count(0, 0) + 3               # two-kernel path: one per strip (1100 rows in 512-row strips)
 
 
 def test_prefetch_and_ship_paths(ctx, port, tables):
     blocks = [make_block(w=2100, h=1900, seed=24 + i) for i in range(3)]
     srcs = [capi.TileSource.from_raster(b["esa"], 256, 256) for b in blocks]
     for ordered, ship in ((0, 0), (1, 1)):
-        _set(ctx, 1, ordered=ordered, ship=ship)
-        try:
+        with options(ctx, stats=1, ordered=ordered, ship=ship):
             ctx.tiles_prefetch(srcs[0], 2100, 1900)
             results = []
             for i, b in enumerate(blocks):
                 if i + 1 < len(blocks):
                     ctx.tiles_prefetch(srcs[i + 1], 2100, 1900)
                 results.append(ctx.block_tiles_deflate(srcs[i], 2100, 1900, b["gt"], b["hsg"], b["soil_gt"]))
-        finally:
-            _set(ctx)
         for b, res in zip(blocks, results):
             want = port.block_rows(b["esa"], b["gt"], b["hsg"], b["soil_gt"], tables)
             assert np.array_equal(res["histograms"], _want(want, capi.MASK_ALL))
@@ -212,27 +159,15 @@ def _oracle_histograms(port, tables, esa, gt, hsg, sgt, n):
     return hist.cpu().numpy().astype(np.uint64)
 
 
-@pytest.mark.parametrize("shape", ["worldcover_36000", "vrt_36001_four_parts"])
+@pytest.mark.parametrize("shape", FULL_SIZE)
 def test_full_size_block(shape, ctx, port, tables):
-    if shape == "worldcover_36000":
-        n, px, lon0, lat0 = 36000, 1.0 / 12000.0, -114.0, 42.0
-    else:
-        n, px, lon0, lat0 = 36001, 8.3333333333330430e-05, 33.0, -3.0
-    gt, sgt, hsx, hsy = synth.block_geometry(lon0, lat0, n, n, px, 1.0 / 480.0, (0.0011, 0.0004), 2)
-    esa = synth.esa_tile(n, n, 77, patch=64)
-    hsg = synth.hsg_tile(hsx, hsy, 78, patch=3)
-    _set(ctx, 1)
-    try:
-        if shape == "worldcover_36000":
-            res = ctx.block_tiles_deflate(capi.TileSource.from_raster(esa, 1024, 1024), n, n, gt, hsg, sgt,
-                                          on_strip=lambda st: 0)
-        else:                                           # the real VRT's four files around a block corner
-            c = 35000
-            parts = [(capi.TileSource.from_raster(np.ascontiguousarray(esa[y:y + hh, x:x + ww]), 1024, 1024), x, y,
-                      ww, hh) for (y, hh) in ((0, c), (c, n - c)) for (x, ww) in ((0, c), (c, n - c))]
+    n, gt, sgt, esa, hsg = full_size_block(shape)
+    parts = full_size_parts(shape, esa)
+    with options(ctx, stats=1):
+        if len(parts) == 1:
+            res = ctx.block_tiles_deflate(parts[0][0], n, n, gt, hsg, sgt, on_strip=lambda st: 0)
+        else:
             res = ctx.block_parts_deflate(parts, 0, n, n, gt, hsg, sgt, on_strip=lambda st: 0)
-    finally:
-        _set(ctx)
     got = res["histograms"]
     assert all(int(got[p].sum()) == n * n for p in range(18))
     assert np.array_equal(got, _oracle_histograms(port, tables, esa, gt, hsg, sgt, n))

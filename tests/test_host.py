@@ -12,7 +12,6 @@ import pytest
 from gcn10_b200 import hostlib
 from tests import lookups
 from tests import fixtures, golden_io
-from tests.test_oracle_pinned import _effective_lut
 
 PX = 1.0 / 12000.0
 
@@ -23,7 +22,7 @@ def test_lookup_reader_matches_oracle_and_golden(port, lookup_dir, tmp_path):
     for label, d in (("default", lookup_dir), ("hostile", write_hostile(str(tmp_path / "hostile")))):
         t = hostlib.load_lookup_tables(d)
         assert np.array_equal(t, port.load_tables(d)), label
-        assert np.array_equal(_effective_lut(t), g[label]), label
+        assert np.array_equal(golden_io.effective_lut(t), g[label]), label
 
 
 def test_lookup_reader_errors(tmp_path):

@@ -11,7 +11,7 @@ from PIL import Image
 from gcn10_b200 import hostlib
 from tests import cog_rule, stats_rule
 from tests import overview_rule as R
-from tests.test_host_overviews import GT, SIZES, _raster, _tile_rows
+from tests.tiff_cases import GT, SIZES, raster, tile_rows
 
 # the land cover's GeoKeys as the writer copies them (a projected CRS with double and ascii params)
 GEOKEYS = ([1, 1, 0, 4, 1024, 0, 1, 1, 1025, 0, 1, 1, 3072, 0, 1, 32611, 3076, 34736, 1, 0],
@@ -61,7 +61,7 @@ def _framed(rows):
 
 
 def _put_level(tw, k, img, framed, rows_per_call=3):
-    rows = _tile_rows(img)
+    rows = tile_rows(img)
     for r0 in range(0, len(rows), rows_per_call):
         part = rows[r0:r0 + rows_per_call]
         blob, offs, sizes = (_framed if framed else _plain)(part)
@@ -71,7 +71,7 @@ def _put_level(tw, k, img, framed, rows_per_call=3):
 @pytest.mark.parametrize("w,h", SIZES)
 def test_whole_raster_cog(tmp_path, w, h):
     """gh_tiff_write_cog, the CPU reference: rules 1-4 hold and every IFD decodes to the raster and its levels."""
-    a = _raster(w, h, seed=w * 3 + h)
+    a = raster(w, h, seed=w * 3 + h)
     path = str(tmp_path / "c.tif")
     hostlib.tiff_write_cog(path, a, GT, 16)
     ifds = cog_rule.check(path)
@@ -87,7 +87,7 @@ def test_whole_raster_cog(tmp_path, w, h):
 @pytest.mark.parametrize("overviews", [0, 16])
 @pytest.mark.parametrize("framed", [False, True])
 def test_writer_cog(tmp_path, w, h, tags, overviews, framed):
-    a = _raster(w, h, seed=w + 5 * h)
+    a = raster(w, h, seed=w + 5 * h)
     nlev = R.levels(w, h) if overviews else 0
     path = str(tmp_path / "c.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, overviews=overviews, stats="stats" in tags, nodata=tags == "nodata",
@@ -118,7 +118,7 @@ def test_writer_cog(tmp_path, w, h, tags, overviews, framed):
 def test_same_streams_as_plain_layout(tmp_path):
     """Same tile streams, different order and framing: the tiles of a COG are byte for byte those of the plain file."""
     w, h = 3001, 517
-    a = _raster(w, h, seed=11)
+    a = raster(w, h, seed=11)
     plain, cog = str(tmp_path / "p.tif"), str(tmp_path / "c.tif")
     tw = hostlib.TiffWriter(plain, w, h, GT, overviews=16)
     for y0 in range(0, h, 512):
@@ -143,7 +143,7 @@ def test_same_streams_as_plain_layout(tmp_path):
 def test_rule_rejects_plain_overviews(tmp_path):
     """A file in the plain layout (level data behind the full resolution, IFDs at the end) is not a COG."""
     w, h = 4111, 260
-    a = _raster(w, h, seed=3)
+    a = raster(w, h, seed=3)
     path = str(tmp_path / "p.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, overviews=16)
     assert tw.write_rows(a, 0) == 0
@@ -154,7 +154,7 @@ def test_rule_rejects_plain_overviews(tmp_path):
 
 def test_rule_rejects_altered_trailer(tmp_path):
     w, h = 4111, 260
-    a = _raster(w, h, seed=4)
+    a = raster(w, h, seed=4)
     path = str(tmp_path / "c.tif")
     hostlib.tiff_write_cog(path, a, GT, 16)
     ifds = cog_rule.check(path)
@@ -175,13 +175,13 @@ def _left_behind(tmp_path):
 @pytest.mark.parametrize("order", ["full_first", "largest_first", "skip_level"])
 def test_out_of_order_levels_refused(tmp_path, order):
     w, h = 3001, 517
-    a = _raster(w, h, seed=5)
+    a = raster(w, h, seed=5)
     nlev = R.levels(w, h)
     assert nlev >= 2
     path = str(tmp_path / "c.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, overviews=16, cog=True)
     first = {"full_first": 0, "largest_first": 1, "skip_level": nlev - 1}[order]
-    rows = _tile_rows(R.decimate(a, first) if first else a)
+    rows = tile_rows(R.decimate(a, first) if first else a)
     blob, offs, sizes = _plain(rows[:1])
     assert tw.put_tile_rows(first, 0, 1, blob, offs, sizes) != 0
     assert tw.close() != 0
@@ -190,10 +190,10 @@ def test_out_of_order_levels_refused(tmp_path, order):
 
 def test_bad_framing_refused(tmp_path):
     w, h = 600, 300
-    a = _raster(w, h, seed=6)
+    a = raster(w, h, seed=6)
     path = str(tmp_path / "c.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, cog=True)
-    blob, offs, sizes = _framed(_tile_rows(a))
+    blob, offs, sizes = _framed(tile_rows(a))
     bad = bytearray(blob)
     bad[int(offs[1]) - 4] ^= 1                  # tile 1's leader
     assert tw.put_tile_rows(0, 0, 2, bytes(bad), offs, sizes, framed=True) != 0
@@ -203,13 +203,13 @@ def test_bad_framing_refused(tmp_path):
 
 def test_cog_refuses_bands_and_late_settings(tmp_path):
     w, h = 600, 300
-    a = _raster(w, h, seed=7)
+    a = raster(w, h, seed=7)
     path = str(tmp_path / "c.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, stats=True, cog=True)
     assert tw.write_rows(a, 0) != 0                                     # bands: the levels would trail
     assert tw.L.gh_tiffw_set_nodata(tw.h, 1) != 0                       # the header region is sized already
     assert tw.L.gh_tiffw_set_cog(tw.h, 1) != 0
-    rows = _tile_rows(a)
+    rows = tile_rows(a)
     blob, offs, sizes = _plain(rows)
     assert tw.put_tile_rows(0, 0, len(rows), blob, offs, sizes) == 0
     assert tw.put_histogram(np.bincount(a.ravel(), minlength=256)) == 0
@@ -221,13 +221,13 @@ def test_cog_refuses_bands_and_late_settings(tmp_path):
 def test_streams_decode(tmp_path):
     """Each framed tile is still a complete zlib stream of its 256 x 256 tile."""
     w, h = 700, 513
-    a = _raster(w, h, seed=8)
+    a = raster(w, h, seed=8)
     path = str(tmp_path / "c.tif")
     hostlib.tiff_write_cog(path, a, GT, 16)
     ifds = cog_rule.check(path)
     with open(path, "rb") as f:
         data = f.read()
-    tiles = _tile_rows(a)
+    tiles = tile_rows(a)
     flat = [z for row in tiles for z in row]
     for o, n, z in zip(ifds[0]["offsets"], ifds[0]["counts"], flat):
         assert zlib.decompress(data[o:o + n]) == zlib.decompress(z)

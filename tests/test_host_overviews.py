@@ -3,7 +3,6 @@ gh_tiffw_put_level_tile_rows, gh_tiffw_close) and of the three overview rules of
 libtiff reader is the independent reader of the files."""
 import os
 import subprocess
-import zlib
 
 import numpy as np
 import pytest
@@ -11,20 +10,9 @@ from PIL import Image
 
 from gcn10_b200 import hostlib
 from tests import overview_rule as R
+from tests.tiff_cases import GT, SIZES, raster, tile_rows
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GT = (-114.0, 1.0 / 12000.0, 0.0, 42.0, 0.0, -1.0 / 12000.0)
-SIZES = [(1, 1), (15, 7), (257, 257), (4111, 260), (48, 3000), (3001, 517)]
-
-
-def _raster(w, h, seed):
-    rng = np.random.default_rng(seed)
-    # patches, so that the tiles compress like land cover and the levels differ from plain subsampling by rows
-    a = rng.integers(0, 12, size=((h + 6) // 7, (w + 4) // 5), dtype=np.uint8) * 10
-    a = np.repeat(np.repeat(a, 7, axis=0), 5, axis=1)[:h, :w]
-    return np.ascontiguousarray(a + rng.integers(0, 2, size=(h, w), dtype=np.uint8))
-
-
 def _frames(path):
     out = []
     with Image.open(path) as im:
@@ -48,7 +36,7 @@ def _check_file(path, a, nlev):
 
 @pytest.mark.parametrize("w,h", SIZES)
 def test_write_rows_levels(tmp_path, w, h):
-    a = _raster(w, h, seed=w * 7 + h)
+    a = raster(w, h, seed=w * 7 + h)
     path = str(tmp_path / "o.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, overviews=16)
     assert tw.levels == R.levels(w, h)
@@ -63,39 +51,24 @@ def test_write_rows_levels(tmp_path, w, h):
     t.close()
 
 
-def _tile_rows(img):
-    """[tile_row] -> the zlib streams of that row of 256 x 256 tiles, zero padded."""
-    h, w = img.shape
-    out = []
-    for ty in range(0, h, 256):
-        row = []
-        for tx in range(0, w, 256):
-            t = np.zeros((256, 256), np.uint8)
-            part = img[ty:ty + 256, tx:tx + 256]
-            t[:part.shape[0], :part.shape[1]] = part
-            row.append(zlib.compress(t.tobytes(), 6))
-        out.append(row)
-    return out
-
-
 @pytest.mark.parametrize("w,h", SIZES)
 def test_put_level_tile_rows(tmp_path, w, h):
-    a = _raster(w, h, seed=w + 3 * h)
+    a = raster(w, h, seed=w + 3 * h)
     nlev = R.levels(w, h)
     path = str(tmp_path / "p.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, overviews=16)
     for level in range(nlev + 1):
-        for r, streams in enumerate(_tile_rows(R.decimate(a, level) if level else a)):
+        for r, streams in enumerate(tile_rows(R.decimate(a, level) if level else a)):
             assert tw.put_tile_row(r, streams, level=level) == 0, (level, r)
     assert tw.close() == 0
     _check_file(path, a, nlev)
 
 
 def test_level_cap_and_order(tmp_path):
-    a = _raster(3001, 517, seed=5)
+    a = raster(3001, 517, seed=5)
     tw = hostlib.TiffWriter(str(tmp_path / "c.tif"), 3001, 517, GT, overviews=2)
     assert tw.levels == 2
-    rows = _tile_rows(R.decimate(a, 1))
+    rows = tile_rows(R.decimate(a, 1))
     assert tw.put_tile_row(1, rows[1], level=1) != 0         # tile rows of a level come in order
     assert tw.put_tile_row(0, rows[0], level=3) != 0         # no such level
     tw.L.gh_tiffw_abort(tw.h)
@@ -103,20 +76,20 @@ def test_level_cap_and_order(tmp_path):
 
 def test_incomplete_level_fails_and_leaves_no_file(tmp_path):
     w, h = 3001, 517
-    a = _raster(w, h, seed=9)
+    a = raster(w, h, seed=9)
     path = str(tmp_path / "i.tif")
     tw = hostlib.TiffWriter(path, w, h, GT, overviews=16)
-    for r, streams in enumerate(_tile_rows(a)):
+    for r, streams in enumerate(tile_rows(a)):
         assert tw.put_tile_row(r, streams) == 0
     for level in range(1, R.levels(w, h)):                  # the last level is missing
-        for r, streams in enumerate(_tile_rows(R.decimate(a, level))):
+        for r, streams in enumerate(tile_rows(R.decimate(a, level))):
             assert tw.put_tile_row(r, streams, level=level) == 0
     assert tw.close() != 0
     assert not os.path.exists(path) and not os.path.exists(path + ".part")
 
 
 def test_without_overviews_one_ifd(tmp_path):
-    a = _raster(600, 300, seed=1)
+    a = raster(600, 300, seed=1)
     path = str(tmp_path / "n.tif")
     tw = hostlib.TiffWriter(path, 600, 300, GT)
     assert tw.levels == 0

@@ -21,22 +21,10 @@ from tests.cases import SMALL_CASES, make_block, PX, PX_VRT, HSG_PX
 BLOCKS = golden_io.block_cases()
 
 
-def _window_inputs(port, c):
-    """Cut the ESA / HSG windows of a golden block case with the restated window arithmetic."""
-    eh, ew = c["esa"].shape
-    hh, hw = c["hsg"].shape
-    we = port.window(ew, eh, c["esa_t"], c["bbox"])
-    wh = port.window(hw, hh, c["hsg_t"], c["bbox"])
-    assert we is not None and wh is not None
-    xo, yo, xc, yc, gt = we
-    hxo, hyo, hxc, hyc, sgt = wh
-    return c["esa"][yo:yo + yc, xo:xo + xc], gt, c["hsg"][hyo:hyo + hyc, hxo:hxo + hxc], sgt
-
-
 @pytest.mark.parametrize("name", sorted(BLOCKS))
 def test_restatement_matches_golden_blocks(name, port, tables, lookup_dir):
     c = BLOCKS[name]
-    esa, gt, hsg, sgt = _window_inputs(port, c)
+    esa, gt, hsg, sgt = golden_io.window_inputs(port, c)
     assert np.array_equal(np.array(gt), c["gt"]), "clipped geotransform differs from the reference's"
     got = port.block_rows(esa, gt, hsg, sgt, tables)
     assert got.shape == c["planes"].shape
@@ -52,7 +40,7 @@ def test_restatement_matches_golden_blocks(name, port, tables, lookup_dir):
 @pytest.mark.parametrize("name", sorted(BLOCKS))
 def test_numpy_restatement_matches_golden_blocks(name, port, tables):
     c = BLOCKS[name]
-    esa, gt, hsg, sgt = _window_inputs(port, c)
+    esa, gt, hsg, sgt = golden_io.window_inputs(port, c)
     assert np.array_equal(O.numpy_block(esa, gt, hsg, sgt, tables), c["planes"])
 
 
@@ -76,27 +64,9 @@ def test_real_vrt_blocks_are_36001(port):
     assert (w[2], w[3]) == (36000, 36000)
 
 
-def _effective_lut(tabs):
-    """uint8 [18, codes, 256] behaviour of int tables for the probe raster of luts.npz."""
-    g = golden_io.luts()
-    codes = g["hsg_codes"]
-    out = np.full((18, len(codes), 256), 255, dtype=np.uint8)
-    for c in range(2):
-        for i, hv in enumerate(codes):
-            s = hv
-            if 11 <= hv <= 14:
-                s = 4 if c == 0 else hv - 10
-            if s >= 5:
-                continue
-            for t in range(9):
-                v = tabs[t][:, s]
-                out[c * 9 + t, i] = np.where(v < 255, v & 0xFF, 255).astype(np.uint8)
-    return out
-
-
 def test_default_lookup_tables_match_golden(port, lookup_dir):
     tabs = port.load_tables(lookup_dir)
-    assert np.array_equal(_effective_lut(tabs), golden_io.luts()["default"])
+    assert np.array_equal(golden_io.effective_lut(tabs), golden_io.luts()["default"])
     # known answers straight from the shipped CSVs (SURVEY 8c)
     g_ii = tabs[7]
     assert (g_ii[10, 1], g_ii[10, 4], g_ii[50, 2], g_ii[100, 4]) == (15, 59, 81, 62)
@@ -109,7 +79,7 @@ def test_hostile_lookup_tables_match_golden(port, tmp_path):
     from tests.golden.make_golden import write_hostile
     d = write_hostile(str(tmp_path / "hostile"))
     tabs = port.load_tables(d)
-    assert np.array_equal(_effective_lut(tabs), golden_io.luts()["hostile"])
+    assert np.array_equal(golden_io.effective_lut(tabs), golden_io.luts()["hostile"])
     assert tabs[0][20, 4] == 11 and tabs[0][7, 4] == 51 and tabs[0][0, 1] == 61 and tabs[0][200, 2] == 1
 
 

@@ -24,7 +24,7 @@ sys.path.insert(0, ROOT)
 
 from gcn10_b200 import capi, hostlib, synth, tiff_lzw  # noqa: E402
 from tests import lookups  # noqa: E402
-from tools.overview_bench import N, T_IN, gpu_info, tile_source  # noqa: E402
+from tools.option_bench import N, T_IN, gpu_info, tile_source  # noqa: E402
 
 
 def lzw_source(ctx, esa):
